@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- region-scored triplets/s for CORE's region pooling / scoring / loss path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one forward + backward of the region path over one batch of synthetic triplets
@@ -178,7 +178,8 @@ def cpu_port_step(sample, tau, kind=None):
 
 def cpu_what(kind):
     return ("reference functions utils/loss_func.py (oracle/_ref, unmodified copy) + Class-N InfoNCE restatement" if kind == "reference"
-            else "oracle/aten_port.py = reference ATen op sequence (oracle/_ref absent)")
+            else "oracle/aten_port.py = reference ATen op sequence (oracle/_ref absent: build() copies the reference's modules there "
+                 "only when COR_REFERENCE names a reference checkout)")
 
 
 def cpu_baseline(inputs_cpu, cfg, triplets, iters, warm=1):
@@ -509,6 +510,26 @@ def emit_result(line):
         os.write(_RESULT_FD, data)
 
 
+DUMP_SAMPLE = 1 << 20      # elements kept of an output larger than this: a fixed, seeded sample (bounds the dump to a few 4 MB files)
+
+
+def dump_outputs(out_dir, loss, grads):
+    """What one timed step hands its caller -- the loss and the gradients of pred, comb and emb -- as float32
+    DIR/<name>.npy, so that two builds can be compared output for output on the same seeded inputs.  An output with
+    more than DUMP_SAMPLE elements is stored as the flat sample at sorted indices drawn once from a generator seeded
+    with 0: the same positions in every run of the same configuration."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss.detach().float().reshape(1)}
+    arrays.update({f"grad_{k}": g.detach().float() for k, g in sorted(grads.items()) if g is not None})
+    for name, t in arrays.items():
+        a = t.cpu().numpy()
+        if a.size > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
+        print(f"[bench] {name}: {tuple(t.shape)} -> {out_dir}/{name}.npy {a.shape}", file=sys.stderr)
+
+
 def main():
     quiet_stdout()
     ap_ = argparse.ArgumentParser()
@@ -528,7 +549,15 @@ def main():
     ap_.add_argument("--no-secondary", action="store_true", help="skip the extra tensor-core / top-k kernel lines (N=1 only)")
     ap_.add_argument("--pool-engine", default="auto")
     ap_.add_argument("--sim-engine", default="auto")
+    ap_.add_argument("--dump-outputs", metavar="DIR", help="write the loss and gradients of the last timed step as DIR/<name>.npy "
+                                                           "(rank 0; outputs above 2^20 elements as a fixed, seeded sample).  --impl ours "
+                                                           "only: the reference arm draws its inputs on the host, from another generator and "
+                                                           "in fp32, so its outputs would not line up element for element with these")
     args = ap_.parse_args()
+    if args.steps < 1:
+        ap_.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap_.error("--dump-outputs writes what --impl ours computed (the reference arm's inputs differ; see --help)")
     cfg = dict(CFG, B=args.batch, M=args.masks)
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
@@ -583,7 +612,12 @@ def main():
             print(f"[bench] CUDA-graph capture failed ({type(e).__name__}: {e}); timing eager launches", file=sys.stderr)
             bufs.graph = None
             torch.cuda.synchronize()
-    step = bufs.replay if graphed else (lambda: bufs._step(True, True, kw)[0])
+
+    def eager_step():
+        bufs.loss, bufs.grads = bufs._step(True, True, kw)
+        return bufs.loss
+
+    step = bufs.replay if graphed else eager_step
     for _ in range(2):
         step()
     barrier()
@@ -607,6 +641,8 @@ def main():
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     ms_step = float(ms) / args.steps
     value = cfg["B"] * world / (ms_step * 1e-3)
+    if args.dump_outputs and rank == 0:     # before any later leg replays the step into the same buffers
+        dump_outputs(args.dump_outputs, loss, bufs.grads)
 
     trace("events pass")
     # ---- per-kernel durations: the same K steps once more, eager, with CUDA events around every C-ABI call

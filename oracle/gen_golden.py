@@ -1,8 +1,8 @@
 """Generate tests/golden/*.npz by running the UNMODIFIED reference (wangtong627/COR) here.
 
-Run in the build container only (needs /root/reference, which does not exist on the GPU box):
+Needs a checkout of the reference, named by COR_REFERENCE (the same variable oracle/build_ref.py reads):
 
-    python oracle/gen_golden.py
+    COR_REFERENCE=/path/to/COR python oracle/gen_golden.py
 
 Every fixture stores the inputs (compressed) and the reference's outputs and autograd
 gradients, all float32, computed on CPU in fp32 by importing the reference's own modules
@@ -20,13 +20,14 @@ import numpy as np
 import torch
 import torch.nn.functional as F
 
-REF = os.environ.get("COR_REFERENCE", "/root/reference")
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 OUT = os.path.join(ROOT, "tests", "golden")
 sys.path.insert(0, ROOT)
-sys.path.insert(0, REF)
 
 from cor_b200 import synth  # noqa: E402
+from oracle.build_ref import REFERENCE as REF  # noqa: E402
+
+sys.path.insert(0, REF)
 
 
 def _stub(name, **attrs):
@@ -62,6 +63,8 @@ def save(name, **arrays):
 
 
 def main():
+    if not os.path.isdir(REF):
+        raise SystemExit("set COR_REFERENCE to a checkout of the reference (wangtong627/COR)")
     torch.manual_seed(0)
     torch.set_num_threads(4)
     lf, ma, trainer = load_reference()

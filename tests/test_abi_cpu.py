@@ -8,6 +8,7 @@ import pytest
 import torch
 
 from cor_b200 import _lib, build
+from oracle.build_ref import REFERENCE
 
 
 @pytest.fixture(scope="module")
@@ -97,10 +98,9 @@ def test_mask_adapter_parameter_names_match_reference_checkpoints():
               "get_mask_map.mask_downscaling.3.weight", "get_mask_map.mask_downscaling.4.bias",
               "get_mask_map.mask_downscaling.6.weight"}
     assert expect <= keys
-    ref_dir = "/root/reference"
-    if os.path.isdir(ref_dir):   # build container only: compare against the real module
+    if os.path.isdir(REFERENCE):   # with a reference checkout: compare against the real module
         import sys
-        sys.path.insert(0, ref_dir)
+        sys.path.insert(0, REFERENCE)
         from lib.support_model.mask_adapter import MaskAdapterPooling as Ref
         r = Ref(x_in_channel=64, mask_adatpet_network_in_channel=32, mask_downscaling_mid_channel=16,
                 mask_adatpet_network_mid_channel=32, num_output_maps=8)
@@ -108,13 +108,13 @@ def test_mask_adapter_parameter_names_match_reference_checkpoints():
         m.load_state_dict(r.state_dict(), strict=True)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference checkout only exists in the build container")
+@pytest.mark.skipif(not os.path.isdir(REFERENCE), reason="needs a checkout of the reference named by COR_REFERENCE")
 def test_hooks_install_into_the_real_reference():
     """hooks.install() rebinds the reference's own names; SupportBranch (support_branch.py:29-40) then
     builds with the patched pooling classes, parameters and error behaviour untouched."""
     import sys
     import types
-    sys.path.insert(0, "/root/reference")
+    sys.path.insert(0, REFERENCE)
     for name in ("open_clip", "accelerate"):
         if name not in sys.modules:
             m = types.ModuleType(name)

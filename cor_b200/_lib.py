@@ -76,6 +76,10 @@ def load(path: str = LIB_PATH):
         _sig(lib, "cor_fgbg_loss_fwd", i, p, ll, p, ll, p, ll, p, ll, i, i, i, p, p, p)
         _sig(lib, "cor_fgbg_loss_bwd", i, p, ll, p, ll, p, ll, i, i, i, p, p, p, ll, f, f, p, ll, i, p, ll, p, ll, i, p)
         _sig(lib, "cor_step_combine", i, p, p, p, f, f, f, p, p)
+        _sig(lib, "cor_step_tail_counter_words", i)
+        _sig(lib, "cor_step_tail_work_bytes", sz, i, i, i)
+        _sig(lib, "cor_step_tail_fwd", i, p, i, ll, i, i, i, i, f, p, p, p, p, f, p, f, f, f, p, p, p, p, p, p, p, p, p, p, p, p, p, p)
+        _sig(lib, "cor_step_tail_bwd", i, p, p, p, p, i, i, i, f, p, f, p, p, p, p, p, p, f, f, p, i, p, p, p, p)
         _sig(lib, "cor_seg_loss_work_bytes", sz, i, i, i)
         _sig(lib, "cor_seg_loss_npartials", i)
         fp = C.POINTER(C.c_float)

@@ -32,7 +32,7 @@ _KERNELS_PER_CALL = {
     "cor_fgbg_loss_bwd": 1, "cor_step_combine": 1, "cor_seg_loss_fwd": 2, "cor_seg_loss_bwd": 1, "cor_sim_stream_fwd": 2,
     "cor_sim_umma_fwd": 2, "cor_infonce_coef": 1, "cor_sim_umma_coef": 1, "cor_infonce_bwd_umma": 3, "cor_gemm_bf16": 1, "cor_cast_cat_bf16": 1, "cor_act_bwd": 2, "cor_ln_rows_fwd": 1, "cor_ln_rows_bwd": 2, "cor_dwconv7_cl": 1, "cor_dwconv7_cl_wgrad": 2,
     "cor_hyper_logits_fwd": 1, "cor_hyper_logits_bwd": 2, "cor_sim_lse_parts": 1, "cor_infonce_tail": 1, "cor_infonce_fwd": 1, "cor_infonce_bwd": 2, "cor_topk": 1, "cor_l2_normalize": 1,
-    "cor_val_post": 3, "cor_soft_metrics": 2,
+    "cor_val_post": 3, "cor_soft_metrics": 2, "cor_step_tail_fwd": 1, "cor_step_tail_bwd": 1,
 }
 
 

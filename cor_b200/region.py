@@ -99,6 +99,33 @@ def _overlap_enabled():
     return os.environ.get("COR_STEP_OVERLAP", "1") != "0"
 
 
+def _pool_bwd_gemm_enabled():
+    return os.environ.get("COR_POOL_BWD_GEMM", "1") != "0"
+
+
+def _step_tail_ok(B: int, M: int, C: int, multi_rank: bool, bg_mode: int, sim_engine: str) -> bool:
+    """Whether the fused step runs its region tail as one forward and one backward launch (csrc/step_tail.cu): one rank's
+    rows only, bg_mode 0, a streaming-similarity shape (<= 16 queries, C % 8 == 0, C <= 256) and the pooling backward on the
+    batched GEMM.  ``COR_STEP_TAIL=0`` keeps the kernel chain it replaces (A/B)."""
+    return (os.environ.get("COR_STEP_TAIL", "1") != "0" and not multi_rank and bg_mode == 0 and B <= 16 and C % 8 == 0 and C <= 256
+            and ops._sim_engine(B, B * M, C, sim_engine) == "stream" and _pool_bwd_gemm_enabled())
+
+
+_tail_counters = {}
+
+
+def _tail_counter(dev, B, M, C):
+    """Zero-initialised arrival counters of the step-tail kernels, cached per shape: every launch leaves them zero again."""
+    key = (dev.index, B, M, C)
+    t = _tail_counters.get(key)
+    if t is None:
+        # never evicted (128 bytes each): captured graphs hold the raw pointer
+        from . import _lib as L
+        t = torch.zeros(L.load().cor_step_tail_counter_words(), dtype=torch.int32, device=dev)
+        _tail_counters[key] = t
+    return t
+
+
 def _peer_fused_ok(n_queries: int, C: int, n_regions: int = 0, sim_engine: str = "auto") -> bool:
     """Shapes the fused gather + similarity kernel serves (a rank's <= 16 queries, one 16-byte vector per lane) and for which
     it wins: whenever the separate path would score on the streaming kernel.  Once the gathered gallery is large enough for
@@ -186,84 +213,111 @@ class _FusedStepFn(torch.autograd.Function):
         ks = lib.cor_pool_umma_ksplit(B, Cc, P)
         part = torch.empty((ks, B, Rp, Cc), **f32)
         call("cor_pool_umma_fwd", dev, ptr(emb_c), ptr(w16), B, Cc, P, Rp, ptr(part))
-        fg = torch.empty((B * M, Cc), **f32)
-        fg16 = px.pub if px is not None else torch.empty((B * M, Cc), dtype=torch.bfloat16, device=dev)
-        if ev_px is not None:
-            cur.wait_event(ev_px)
-        inv_fg = torch.empty((B * M,), **f32)
-        split = B * Rp * Cc
-        call("cor_rows_finalize", dev, ptr(part), M, _ll(Rp * Cc), ks, _ll(split), ptr(stats[:, 3:]), 4, _f(1e-8), B * M, Cc, 1, 1,
-             None, _f(0.0), ptr(fg), ptr(fg16), ptr(inv_fg))
-        if px is not None:
-            px.signal(0)                     # the bg rows, fg/bg loss and segmentation loss below hide the rank skew
-        # 4. background rows + fg / bg cosine losses on the GT rows (row b*M of fg, row b of bg): a second branch off the
-        #    fg rows, on the side stream, parallel to the similarity / InfoNCE chain below
-        bg = torch.empty((B, Cc), **f32)
-        inv_bg = torch.empty((B,), **f32)
-        out4 = torch.empty(4, **f32)
-        aux = torch.empty(lib.cor_fgbg_aux_floats(B, Cc), **f32)
-        if side is not None:
-            side.wait_stream(cur)
-        with torch.cuda.stream(side if side is not None else cur):
-            call("cor_rows_finalize", dev, ptr(part), 1, _ll(Rp * Cc), ks, _ll(split), ptr(stats[:, 3:]), 4 * M, _f(1e-8), B, Cc, 1, 1,
-                 ptr(part[0, :, M, :]), _f(float(P)), ptr(bg), None, ptr(inv_bg))
-            call("cor_fgbg_loss_fwd", dev, ptr(fg), _ll(M * Cc), ptr(bg), _ll(Cc), ptr(comb_c), _ll(Cc), ptr(stats), _ll(4 * M), B, Cc,
-                 int(bg_mode), ptr(out4), ptr(aux))
-        # 6. InfoNCE of every composed query against all (gathered) regions
-        if ev_q is not None:
-            cur.wait_event(ev_q)
-        n_local = B * M
-        inv_tau = 1.0 / float(tau)
-        # A/B on one 8xB200 box (profiles/README.md): reduce-scatter of the region gradient 0.951 ms/step, collective-free
-        # variant 0.965 ms/step -> the reduce-scatter stays the default; COR_STEP_BWD=local selects the other.
-        local_bwd = os.environ.get("COR_STEP_BWD", "reduce_scatter") == "local"
-        fused_parts = None
-        if gather and ws > 1:
-            r16 = torch.empty((ws * n_local, Cc), dtype=torch.bfloat16, device=dev)
-            if px is not None and not local_bwd and _peer_fused_ok(B, Cc, ws * n_local, sim_engine):
-                # ONE kernel: pull the peers' rows over NVLink, keep a local copy for the backward, and score every row
-                # against this rank's queries while it is in registers (all-gather fused with its consumer)
-                fused_parts = px.gather_sim(r16, q16, inv_tau)
-            elif px is not None:
-                px.gather(r16)               # our own pull-over-NVLink kernel: no NCCL on the data path
+        tail = _step_tail_ok(B, M, Cc, gather and ws > 1, int(bg_mode), sim_engine)
+        ctx.tail = _tail_counter(dev, B, M, Cc) if tail else None
+        if tail:
+            # 3.-6. in ONE launch: unit rows (+ bf16 copy), their scores against the queries, the bg rows and fg / bg cosine
+            # statistics of the GT masks, and in its last CTA the log-sum-exp merge, the InfoNCE, fg / bg losses and the total
+            fg = torch.empty((B * M, Cc), **f32)
+            fg16 = torch.empty((B * M, Cc), dtype=torch.bfloat16, device=dev)
+            inv_fg = torch.empty((B * M,), **f32)
+            bg = torch.empty((B, Cc), **f32)
+            inv_bg = torch.empty((B,), **f32)
+            out4 = torch.empty(4, **f32)
+            aux = torch.empty(lib.cor_fgbg_aux_floats(B, Cc), **f32)
+            r16, offset, ws, n_local = fg16, 0, 1, B * M
+            q_all = lse_all = tgt_all = None
+            targets = _target_rows(dev, B, M, 0)
+            lse = torch.empty((B,), **f32)
+            nce = torch.empty(1, **f32)
+            tgt = torch.empty((B,), **f32)
+            loss = torch.empty(1, **f32)
+            inv_tau = 1.0 / float(tau)
+            work = ops._work(lib.cor_step_tail_work_bytes(B, M, Cc), dev)
+            if side is not None:
+                cur.wait_stream(side)        # join: the total needs the segmentation loss, the scores the bf16 queries
+            call("cor_step_tail_fwd", dev, ptr(part), ks, _ll(B * Rp * Cc), Rp, B, M, Cc, _f(float(P)), ptr(stats), ptr(q16), ptr(comb_c),
+                 ptr(targets), _f(inv_tau), ptr(out8), _f(w_fg), _f(w_bg), _f(nce_weight), ptr(fg), ptr(fg16), ptr(inv_fg), ptr(bg),
+                 ptr(inv_bg), ptr(out4), ptr(aux), ptr(lse), ptr(nce), ptr(tgt), ptr(loss), ptr(work), ptr(ctx.tail))
+        else:
+            fg = torch.empty((B * M, Cc), **f32)
+            fg16 = px.pub if px is not None else torch.empty((B * M, Cc), dtype=torch.bfloat16, device=dev)
+            if ev_px is not None:
+                cur.wait_event(ev_px)
+            inv_fg = torch.empty((B * M,), **f32)
+            split = B * Rp * Cc
+            call("cor_rows_finalize", dev, ptr(part), M, _ll(Rp * Cc), ks, _ll(split), ptr(stats[:, 3:]), 4, _f(1e-8), B * M, Cc, 1, 1,
+                 None, _f(0.0), ptr(fg), ptr(fg16), ptr(inv_fg))
+            if px is not None:
+                px.signal(0)                     # the bg rows, fg/bg loss and segmentation loss below hide the rank skew
+            # 4. background rows + fg / bg cosine losses on the GT rows (row b*M of fg, row b of bg): a second branch off the
+            #    fg rows, on the side stream, parallel to the similarity / InfoNCE chain below
+            bg = torch.empty((B, Cc), **f32)
+            inv_bg = torch.empty((B,), **f32)
+            out4 = torch.empty(4, **f32)
+            aux = torch.empty(lib.cor_fgbg_aux_floats(B, Cc), **f32)
+            if side is not None:
+                side.wait_stream(cur)
+            with torch.cuda.stream(side if side is not None else cur):
+                call("cor_rows_finalize", dev, ptr(part), 1, _ll(Rp * Cc), ks, _ll(split), ptr(stats[:, 3:]), 4 * M, _f(1e-8), B, Cc, 1, 1,
+                     ptr(part[0, :, M, :]), _f(float(P)), ptr(bg), None, ptr(inv_bg))
+                call("cor_fgbg_loss_fwd", dev, ptr(fg), _ll(M * Cc), ptr(bg), _ll(Cc), ptr(comb_c), _ll(Cc), ptr(stats), _ll(4 * M), B, Cc,
+                     int(bg_mode), ptr(out4), ptr(aux))
+            # 6. InfoNCE of every composed query against all (gathered) regions
+            if ev_q is not None:
+                cur.wait_event(ev_q)
+            n_local = B * M
+            inv_tau = 1.0 / float(tau)
+            # A/B on one 8xB200 box (profiles/README.md): reduce-scatter of the region gradient 0.951 ms/step, collective-free
+            # variant 0.965 ms/step -> the reduce-scatter stays the default; COR_STEP_BWD=local selects the other.
+            local_bwd = os.environ.get("COR_STEP_BWD", "reduce_scatter") == "local"
+            fused_parts = None
+            if gather and ws > 1:
+                r16 = torch.empty((ws * n_local, Cc), dtype=torch.bfloat16, device=dev)
+                if px is not None and not local_bwd and _peer_fused_ok(B, Cc, ws * n_local, sim_engine):
+                    # ONE kernel: pull the peers' rows over NVLink, keep a local copy for the backward, and score every row
+                    # against this rank's queries while it is in registers (all-gather fused with its consumer)
+                    fused_parts = px.gather_sim(r16, q16, inv_tau)
+                elif px is not None:
+                    px.gather(r16)               # our own pull-over-NVLink kernel: no NCCL on the data path
+                else:
+                    torch.distributed.all_gather_into_tensor(r16, fg16)
+                offset = rank * n_local
+                if local_bwd:
+                    # A second small all-gather (the queries) replaces the backward's reduce-scatter: every rank scores
+                    # ALL queries against ALL regions (same HBM-bound cost as scoring its own), which gives it the
+                    # log-sum-exp of the remote queries too, so the backward needs no collective at all.
+                    q_all = torch.empty((ws * B, Cc), dtype=torch.bfloat16, device=dev)
+                    torch.distributed.all_gather_into_tensor(q_all, q16)
+                    _, lse_all = ops._sim_forward(r16, q_all, inv_tau, False, True, sim_engine)
+                    lse = lse_all[rank * B:(rank + 1) * B]
+                    ar = torch.arange(ws * B, device=dev, dtype=torch.int64)
+                    tgt_all = (ar // B) * n_local + (ar % B) * M - offset       # target rows local to THIS rank
+                else:
+                    q_all = lse_all = tgt_all = None
+                    lse = None
             else:
-                torch.distributed.all_gather_into_tensor(r16, fg16)
-            offset = rank * n_local
-            if local_bwd:
-                # A second small all-gather (the queries) replaces the backward's reduce-scatter: every rank scores
-                # ALL queries against ALL regions (same HBM-bound cost as scoring its own), which gives it the
-                # log-sum-exp of the remote queries too, so the backward needs no collective at all.
-                q_all = torch.empty((ws * B, Cc), dtype=torch.bfloat16, device=dev)
-                torch.distributed.all_gather_into_tensor(q_all, q16)
-                _, lse_all = ops._sim_forward(r16, q_all, inv_tau, False, True, sim_engine)
-                lse = lse_all[rank * B:(rank + 1) * B]
-                ar = torch.arange(ws * B, device=dev, dtype=torch.int64)
-                tgt_all = (ar // B) * n_local + (ar % B) * M - offset       # target rows local to THIS rank
-            else:
+                r16, offset, ws = fg16, 0, 1
                 q_all = lse_all = tgt_all = None
                 lse = None
-        else:
-            r16, offset, ws = fg16, 0, 1
-            q_all = lse_all = tgt_all = None
-            lse = None
-        targets = _target_rows(dev, B, M, offset)
-        nce = torch.empty(1, **f32)
-        tgt = torch.empty((B,), **f32)
-        loss = torch.empty(1, **f32)
-        if lse is None:
-            # similarity with its log-sum-exp partials left in the work buffer, then ONE tail kernel: partial merge ->
-            # lse, target logits, InfoNCE mean and the step's total loss
-            sim_work, nparts, qt = fused_parts if fused_parts is not None else ops._sim_lse_parts(r16, q16, inv_tau, sim_engine)
-            lse = torch.empty((B,), **f32)
-            if side is not None:
-                cur.wait_stream(side)        # join: the total needs the segmentation and fg/bg losses
-            call("cor_infonce_tail", dev, ptr(sim_work), nparts, qt, ptr(r16), ptr(q16), ptr(targets), r16.shape[0], B, Cc, _f(inv_tau),
-                 ptr(lse), ptr(nce), ptr(tgt), ptr(out8), ptr(out4), _f(w_fg), _f(w_bg), _f(nce_weight), ptr(loss))
-        else:
-            call("cor_infonce_fwd", dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), r16.shape[0], B, Cc, _f(inv_tau), ptr(nce), ptr(tgt))
-            if side is not None:
-                cur.wait_stream(side)        # join: the combine needs the segmentation loss
-            call("cor_step_combine", dev, ptr(out8), ptr(out4), ptr(nce), _f(w_fg), _f(w_bg), _f(nce_weight), ptr(loss))
+            targets = _target_rows(dev, B, M, offset)
+            nce = torch.empty(1, **f32)
+            tgt = torch.empty((B,), **f32)
+            loss = torch.empty(1, **f32)
+            if lse is None:
+                # similarity with its log-sum-exp partials left in the work buffer, then ONE tail kernel: partial merge ->
+                # lse, target logits, InfoNCE mean and the step's total loss
+                sim_work, nparts, qt = fused_parts if fused_parts is not None else ops._sim_lse_parts(r16, q16, inv_tau, sim_engine)
+                lse = torch.empty((B,), **f32)
+                if side is not None:
+                    cur.wait_stream(side)        # join: the total needs the segmentation and fg/bg losses
+                call("cor_infonce_tail", dev, ptr(sim_work), nparts, qt, ptr(r16), ptr(q16), ptr(targets), r16.shape[0], B, Cc, _f(inv_tau),
+                     ptr(lse), ptr(nce), ptr(tgt), ptr(out8), ptr(out4), _f(w_fg), _f(w_bg), _f(nce_weight), ptr(loss))
+            else:
+                call("cor_infonce_fwd", dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), r16.shape[0], B, Cc, _f(inv_tau), ptr(nce), ptr(tgt))
+                if side is not None:
+                    cur.wait_stream(side)        # join: the combine needs the segmentation loss
+                call("cor_step_combine", dev, ptr(out8), ptr(out4), ptr(nce), _f(w_fg), _f(w_bg), _f(nce_weight), ptr(loss))
         ctx.save_for_backward(pred_c, t_save, w_save, per, fg, bg, inv_fg, inv_bg, comb_c, stats, out4, aux, r16, q16, targets, lse, w32,
                               fg16, q_all, lse_all, tgt_all)
         ctx.cfg = (B, M, Cc, h, w, float(inv_tau), float(nce_weight), int(bg_mode), float(w_fg), float(w_bg), ws, offset, n_local,
@@ -319,71 +373,91 @@ class _FusedStepFn(torch.autograd.Function):
                 px.before_produce(1)
         if px is None or side is not None:
             g_pred = seg_bwd()               # side stream: runs underneath the InfoNCE / pooling backward
-        # InfoNCE backward first: it WRITES g_regions (this rank's rows) and g_queries ...
-        Nr = r16.shape[0]
-        g_regions = torch.empty((n_local, Cc), **f32)
-        g_q = torch.empty((B, Cc), **f32)
-        work = ops._work(lib.cor_sim_work_bytes(B, Nr, Cc), dev)
-        if ws > 1 and q_all is not None:
-            # (all regions, my queries) -> g_queries ; (my regions, ALL queries) -> g_regions.  Every rank's loss is the
-            # mean over its own B queries, so the sum over ranks of d loss_j / d my_regions carries the factor ws.
-            call("cor_infonce_bwd", dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), Nr, B, Cc, _f(inv_tau), ptr(g), _f(nce_weight), None,
-                 ptr(g_q), ptr(work))
-            call("cor_infonce_bwd", dev, ptr(fg16), ptr(q_all), ptr(tgt_all), ptr(lse_all), n_local, ws * B, Cc, _f(inv_tau), ptr(g),
-                 _f(float(ws) * nce_weight), ptr(g_regions), None, None)
-        elif ws > 1:
-            if ev_px is not None:
-                cur.wait_event(ev_px)
-            g_all = px.gall if px is not None else torch.empty((Nr, Cc), **f32)
-            call("cor_infonce_bwd", dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), Nr, B, Cc, _f(inv_tau), ptr(g), _f(nce_weight),
-                 ptr(g_all), ptr(g_q), ptr(work))
-            if px is not None:
-                px.signal(1)
-                if side is None:
-                    g_pred = seg_bwd()       # independent work between the signal and the pull hides the rank skew
-                px.reduce(g_regions)         # fixed rank order: bit-identical from run to run
-            else:
-                torch.distributed.reduce_scatter_tensor(g_regions, g_all, op=torch.distributed.ReduceOp.SUM)
-        else:
-            call("cor_infonce_bwd", dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), Nr, B, Cc, _f(inv_tau), ptr(g), _f(nce_weight),
-                 ptr(g_regions), ptr(g_q), ptr(work))
-        # ... then the fg/bg backward ADDS its GT-row gradients into g_regions (row b*M) and g_queries
-        g_bg = torch.empty((B, Cc), **f32) if bg_mode == 1 else None
-        call("cor_fgbg_loss_bwd", dev, ptr(fg), _ll(M * Cc), ptr(bg), _ll(Cc), ptr(comb_c), _ll(Cc), B, Cc, bg_mode, ptr(out4), ptr(aux),
-             ptr(g), _ll(0), _f(w_fg), _f(w_bg), ptr(g_regions), _ll(M * Cc), 1, ptr(g_bg), _ll(Cc), ptr(g_q), _ll(Cc), 1)
-        if need_comb:
-            g_comb = g_q.view(comb_shape).to(comb_dt)
-        if need_emb:
-            gs_fg = torch.empty((B * M, Cc), **f32)
-            call("cor_rows_finalize_bwd", dev, ptr(g_regions), ptr(fg), ptr(inv_fg), ptr(stats[:, 3:]), 4, _f(1e-8), B * M, Cc, 1, 1, 0,
-                 _f(0.0), ptr(gs_fg))
-            gs_bg_full = None
-            if g_bg is not None:          # paired bg mode: background gradient lives on the GT rows only
-                gs_bg = torch.empty((B, Cc), **f32)
-                call("cor_rows_finalize_bwd", dev, ptr(g_bg), ptr(bg), ptr(inv_bg), ptr(stats[:, 3:]), 4 * M, _f(1e-8), B, Cc, 1, 1, 1,
-                     _f(float(P)), ptr(gs_bg))
-                gs_bg_full = torch.zeros((B, M, Cc), **f32)
-                gs_bg_full[:, 0, :] = gs_bg
-            g_emb_c = torch.empty((B, Cc, h, w), dtype=emb_dt if emb_dt in (torch.float32, torch.bfloat16) else torch.float32, device=dev)
-            w16, w16_epoch = ctx.w16
-            if (gs_bg_full is None and w16 is not None and getattr(w16, "_cor_epoch", -1) == w16_epoch and Cc % 8 == 0 and P % 8 == 0
-                    and os.environ.get("COR_POOL_BWD_GEMM", "1") != "0"):
-                # d emb[b] (C x P) = gs[b]^T (C x M) w[b] (M x P): one batched tcgen05 GEMM on the bf16 weights the forward's
-                # pooling GEMM used (still in their buffer: no later forward of this shape has rewritten them), both operands
-                # MN-major as they lie; the gradient rows are cast to bf16 and zero-padded to a whole 64-row K block, which makes
-                # the other operand's rows beyond M (the ones row, the next image) irrelevant.  Persistent tiles with coalesced
-                # stores: 2-3x faster than the one-shot pool_bwd_umma kernel, which rebuilds both operands from fp32.
+        w16, w16_epoch = ctx.w16
+        gemm_ok = (bg_mode != 1 and w16 is not None and getattr(w16, "_cor_epoch", -1) == w16_epoch and Cc % 8 == 0 and P % 8 == 0
+                   and _pool_bwd_gemm_enabled())
+        if ctx.tail is not None and (gemm_ok or not need_emb):
+            # ONE launch: InfoNCE + fg-loss gradient of every row, through the row epilogue, cast to bf16 into the K-padded
+            # operand of the pooling-backward GEMM; and the query gradient (+ fg / bg terms) in extra CTAs, one set per query
+            Kp = (M + 63) // 64 * 64
+            a16 = torch.empty((B * Kp, Cc), dtype=torch.bfloat16, device=dev) if need_emb else None
+            g_q = torch.empty((B, Cc), **f32) if need_comb else None
+            work = ops._work(lib.cor_step_tail_work_bytes(B, M, Cc), dev)
+            call("cor_step_tail_bwd", dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), B, M, Cc, _f(inv_tau), ptr(g), _f(nce_weight),
+                 ptr(fg), ptr(inv_fg), ptr(stats), ptr(comb_c), ptr(out4), ptr(aux), _f(w_fg), _f(w_bg), ptr(a16), Kp, ptr(g_q),
+                 ptr(work), ptr(ctx.tail))
+            if need_comb:
+                g_comb = g_q.view(comb_shape).to(comb_dt)
+            if need_emb:
                 from .linear import gemm
-                Kp = (M + 63) // 64 * 64
-                a16 = torch.empty((B * Kp, Cc), dtype=torch.bfloat16, device=dev)
-                call("cor_cast_pad_rows_bf16", dev, ptr(gs_fg), B, M, Kp, Cc, ptr(a16))
                 Rp = w16.shape[1]
-                g_emb_c = gemm(a16, w16.view(B * Rp, P), Cc, P, Kp, a_mn=True, b_mn=True, batch=B, a_batch_rows=Kp, b_batch_rows=Rp,
-                               out_dtype=g_emb_c.dtype).view(B, Cc, h, w)
+                out_dt = emb_dt if emb_dt in (torch.float32, torch.bfloat16) else torch.float32
+                g_emb = gemm(a16, w16.view(B * Rp, P), Cc, P, Kp, a_mn=True, b_mn=True, batch=B, a_batch_rows=Kp, b_batch_rows=Rp,
+                             out_dtype=out_dt).view(B, Cc, h, w).to(emb_dt)
+        else:
+            # InfoNCE backward first: it WRITES g_regions (this rank's rows) and g_queries ...
+            Nr = r16.shape[0]
+            g_regions = torch.empty((n_local, Cc), **f32)
+            g_q = torch.empty((B, Cc), **f32)
+            work = ops._work(lib.cor_sim_work_bytes(B, Nr, Cc), dev)
+            if ws > 1 and q_all is not None:
+                # (all regions, my queries) -> g_queries ; (my regions, ALL queries) -> g_regions.  Every rank's loss is the
+                # mean over its own B queries, so the sum over ranks of d loss_j / d my_regions carries the factor ws.
+                call("cor_infonce_bwd", dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), Nr, B, Cc, _f(inv_tau), ptr(g), _f(nce_weight), None,
+                     ptr(g_q), ptr(work))
+                call("cor_infonce_bwd", dev, ptr(fg16), ptr(q_all), ptr(tgt_all), ptr(lse_all), n_local, ws * B, Cc, _f(inv_tau), ptr(g),
+                     _f(float(ws) * nce_weight), ptr(g_regions), None, None)
+            elif ws > 1:
+                if ev_px is not None:
+                    cur.wait_event(ev_px)
+                g_all = px.gall if px is not None else torch.empty((Nr, Cc), **f32)
+                call("cor_infonce_bwd", dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), Nr, B, Cc, _f(inv_tau), ptr(g), _f(nce_weight),
+                     ptr(g_all), ptr(g_q), ptr(work))
+                if px is not None:
+                    px.signal(1)
+                    if side is None:
+                        g_pred = seg_bwd()       # independent work between the signal and the pull hides the rank skew
+                    px.reduce(g_regions)         # fixed rank order: bit-identical from run to run
+                else:
+                    torch.distributed.reduce_scatter_tensor(g_regions, g_all, op=torch.distributed.ReduceOp.SUM)
             else:
-                name = "cor_pool_bwd_umma" if lib.cor_pool_bwd_umma_ok(B, Cc, P, M, int(gs_bg_full is not None)) else "cor_pool_bwd_feat"
-                call(name, dev, ptr(gs_fg), ptr(gs_bg_full), ptr(w32), _ll(P), B, Cc, P, M, ops.W_CLAMP, ptr(g_emb_c), L._DTYPES[g_emb_c.dtype])
-            g_emb = g_emb_c.to(emb_dt)
+                call("cor_infonce_bwd", dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), Nr, B, Cc, _f(inv_tau), ptr(g), _f(nce_weight),
+                     ptr(g_regions), ptr(g_q), ptr(work))
+            # ... then the fg/bg backward ADDS its GT-row gradients into g_regions (row b*M) and g_queries
+            g_bg = torch.empty((B, Cc), **f32) if bg_mode == 1 else None
+            call("cor_fgbg_loss_bwd", dev, ptr(fg), _ll(M * Cc), ptr(bg), _ll(Cc), ptr(comb_c), _ll(Cc), B, Cc, bg_mode, ptr(out4), ptr(aux),
+                 ptr(g), _ll(0), _f(w_fg), _f(w_bg), ptr(g_regions), _ll(M * Cc), 1, ptr(g_bg), _ll(Cc), ptr(g_q), _ll(Cc), 1)
+            if need_comb:
+                g_comb = g_q.view(comb_shape).to(comb_dt)
+            if need_emb:
+                gs_fg = torch.empty((B * M, Cc), **f32)
+                call("cor_rows_finalize_bwd", dev, ptr(g_regions), ptr(fg), ptr(inv_fg), ptr(stats[:, 3:]), 4, _f(1e-8), B * M, Cc, 1, 1, 0,
+                     _f(0.0), ptr(gs_fg))
+                gs_bg_full = None
+                if g_bg is not None:          # paired bg mode: background gradient lives on the GT rows only
+                    gs_bg = torch.empty((B, Cc), **f32)
+                    call("cor_rows_finalize_bwd", dev, ptr(g_bg), ptr(bg), ptr(inv_bg), ptr(stats[:, 3:]), 4 * M, _f(1e-8), B, Cc, 1, 1, 1,
+                         _f(float(P)), ptr(gs_bg))
+                    gs_bg_full = torch.zeros((B, M, Cc), **f32)
+                    gs_bg_full[:, 0, :] = gs_bg
+                g_emb_c = torch.empty((B, Cc, h, w), dtype=emb_dt if emb_dt in (torch.float32, torch.bfloat16) else torch.float32, device=dev)
+                if gs_bg_full is None and gemm_ok:
+                    # d emb[b] (C x P) = gs[b]^T (C x M) w[b] (M x P): one batched tcgen05 GEMM on the bf16 weights the forward's
+                    # pooling GEMM used (still in their buffer: no later forward of this shape has rewritten them), both operands
+                    # MN-major as they lie; the gradient rows are cast to bf16 and zero-padded to a whole 64-row K block, which makes
+                    # the other operand's rows beyond M (the ones row, the next image) irrelevant.  Persistent tiles with coalesced
+                    # stores: 2-3x faster than the one-shot pool_bwd_umma kernel, which rebuilds both operands from fp32.
+                    from .linear import gemm
+                    Kp = (M + 63) // 64 * 64
+                    a16 = torch.empty((B * Kp, Cc), dtype=torch.bfloat16, device=dev)
+                    call("cor_cast_pad_rows_bf16", dev, ptr(gs_fg), B, M, Kp, Cc, ptr(a16))
+                    Rp = w16.shape[1]
+                    g_emb_c = gemm(a16, w16.view(B * Rp, P), Cc, P, Kp, a_mn=True, b_mn=True, batch=B, a_batch_rows=Kp, b_batch_rows=Rp,
+                                   out_dtype=g_emb_c.dtype).view(B, Cc, h, w)
+                else:
+                    name = "cor_pool_bwd_umma" if lib.cor_pool_bwd_umma_ok(B, Cc, P, M, int(gs_bg_full is not None)) else "cor_pool_bwd_feat"
+                    call(name, dev, ptr(gs_fg), ptr(gs_bg_full), ptr(w32), _ll(P), B, Cc, P, M, ops.W_CLAMP, ptr(g_emb_c), L._DTYPES[g_emb_c.dtype])
+                g_emb = g_emb_c.to(emb_dt)
         if side is not None:
             cur.wait_stream(side)
         if g_pred is not None:

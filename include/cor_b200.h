@@ -147,6 +147,33 @@ int cor_step_combine(const float* seg, const float* fgbg, const float* nce, floa
                      float* loss, cor_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
+ * The fused step's region tail in one launch each way (csrc/step_tail.cu; cor_b200/region.py, one rank, bg_mode 0):
+ * B <= 16 triplets with M candidate masks each, C % 8 == 0, C <= 256; query b's target is region row b*M.
+ *   cor_step_tail_fwd: the pooling GEMM's split-K partials part [nsplit][B][Rp][C] (row M of each image = the all-ones
+ *     weight row) -> unit rows fg [B*M, C] f32 + bf16 + inv_fg [B*M] (= cor_rows_finalize), background rows of the
+ *     ground-truth masks bg [B, C] + inv_bg [B], the InfoNCE of every query against all B*M rows (lse [B], nce [1],
+ *     tgt_logit [B]), the fg / bg losses out4 [4] + aux (= cor_fgbg_loss_fwd, bg_mode 0) and
+ *     total = seg[0] + w_fg * out4[0] + w_bg * out4[1] + w_nce * nce (= cor_infonce_tail).  stats [B*M, 4] from
+ *     cor_mask_prep; queries [B, C] bf16, comb [B, C] f32 (the same queries).
+ *   cor_step_tail_bwd: for upstream scalar *g_loss, the InfoNCE + fg-loss gradient of every region row taken back
+ *     through the row epilogue, cast to bf16 into a16 [B][Kp][C] (rows M..Kp-1 zeroed: the K-padded operand of the
+ *     pooling-backward GEMM; NULL = not wanted) and the gradient of the queries g_queries [B, C] f32 (NULL = not wanted).
+ *   work: cor_step_tail_work_bytes() bytes; counter: cor_step_tail_counter_words() u32 words, zero before the first
+ *   launch and left zero by every launch (graph-replayable).  Deterministic.
+ * ---------------------------------------------------------------------------------------- */
+int cor_step_tail_counter_words(void);
+size_t cor_step_tail_work_bytes(int B, int M, int C);
+int cor_step_tail_fwd(const float* part, int nsplit, long long split_stride, int Rp, int B, int M, int C, float p_total,
+                      const float* stats, const void* queries_bf16, const float* comb, const long long* targets, float inv_tau,
+                      const float* seg, float w_fg, float w_bg, float w_nce, float* fg, void* fg_bf16, float* inv_fg, float* bg,
+                      float* inv_bg, float* fgbg_out4, float* aux, float* lse, float* nce, float* tgt_logit, float* total,
+                      void* work, unsigned* counter, cor_stream_t stream);
+int cor_step_tail_bwd(const void* regions_bf16, const void* queries_bf16, const long long* targets, const float* lse, int B, int M,
+                      int C, float inv_tau, const float* g_loss, float w_nce, const float* fg, const float* inv_fg,
+                      const float* stats, const float* comb, const float* fgbg_out4, const float* aux, float w_fg, float w_bg,
+                      void* a16, int Kp, float* g_queries, void* work, unsigned* counter, cor_stream_t stream);
+
+/* ------------------------------------------------------------------------------------------
  * Segmentation loss (loss_func.py:5-32) with the target resample of trainer_v3_g.py:67 fused in.
  *   pred [N, H, W] f32/bf16 logits; mask [N, Hm, Wm] f32/bf16/u8 (resampled to HxW if sizes differ)
  *   Per sample, from ONE pass over (pred, mask), seven terms (t = target, p = sigmoid(pred),

@@ -80,6 +80,8 @@ def load(path: str = LIB_PATH):
         _sig(lib, "cor_step_tail_work_bytes", sz, i, i, i)
         _sig(lib, "cor_step_tail_fwd", i, p, i, ll, i, i, i, i, f, p, p, p, p, f, p, f, f, f, p, p, p, p, p, p, p, p, p, p, p, p, p, p)
         _sig(lib, "cor_step_tail_bwd", i, p, p, p, p, i, i, i, f, p, f, p, p, p, p, p, p, f, f, p, i, p, p, p, p)
+        _sig(lib, "cor_step_tail_fwd_ls", i, p, i, ll, i, i, i, i, f, p, p, p, p, p, p, f, f, f, p, p, p, p, p, p, p, p, p, p, p, p, p, p)
+        _sig(lib, "cor_step_tail_bwd_ls", i, p, p, p, p, i, i, i, p, p, f, p, p, p, p, p, p, f, f, p, i, p, p, p, p, p)
         _sig(lib, "cor_seg_loss_work_bytes", sz, i, i, i)
         _sig(lib, "cor_seg_loss_npartials", i)
         fp = C.POINTER(C.c_float)
@@ -96,6 +98,14 @@ def load(path: str = LIB_PATH):
         _sig(lib, "cor_infonce_bwd", i, p, p, p, p, i, i, i, f, p, f, p, p, p, p)
         _sig(lib, "cor_infonce_bwd_umma_work_bytes", sz, i, i, i)
         _sig(lib, "cor_infonce_bwd_umma", i, p, p, i, i, i, f, p, p, p, f, p, p, p, p)
+        # the same entries with the logit scale read from device memory (and its gradient written there)
+        _sig(lib, "cor_sim_stream_fwd_ls", i, p, p, i, i, i, p, p, p, p, p)
+        _sig(lib, "cor_sim_umma_fwd_ls", i, p, p, i, i, i, p, p, p, p, p)
+        _sig(lib, "cor_sim_lse_parts_ls", i, i, p, p, i, i, i, p, p, C.POINTER(i), C.POINTER(i), p)
+        _sig(lib, "cor_infonce_tail_ls", i, p, i, i, p, p, p, i, i, i, p, p, p, p, p, p, f, f, f, p, p)
+        _sig(lib, "cor_infonce_fwd_ls", i, p, p, p, p, i, i, i, p, p, p, p)
+        _sig(lib, "cor_infonce_bwd_ls", i, p, p, p, p, i, i, i, p, p, f, p, p, p, p, p)
+        _sig(lib, "cor_infonce_bwd_umma_ls", i, p, p, i, i, i, p, p, p, p, f, p, p, p, p, p)
         _sig(lib, "cor_topk", i, p, p, p, i, i, i, i, p, p, p)
         _sig(lib, "cor_l2_normalize", i, p, i, i, i, p, p, p, p)
         _sig(lib, "cor_gemm_bf16_work_bytes", sz, i, i, i, i, i)
@@ -137,6 +147,7 @@ def load(path: str = LIB_PATH):
         _sig(lib, "cor_peer_reduce_rows", i, p, p, ll, p, p, i, i, i, p)
         _sig(lib, "cor_peer_gather_sim_work_bytes", sz)
         _sig(lib, "cor_peer_gather_sim", i, p, p, ll, i, p, i, f, p, p, p, p, i, i, i, p)
+        _sig(lib, "cor_peer_gather_sim_ls", i, p, p, ll, i, p, i, p, p, p, p, p, i, i, i, p)
         if lib.cor_abi_version() != ABI_VERSION:
             raise CorError(f"ABI version mismatch: library {lib.cor_abi_version()}, binding {ABI_VERSION}; rebuild with `python -m cor_b200.build`")
         _lib = lib

@@ -23,6 +23,8 @@
 // 128-byte row of one P k-block per thread), 8 = TMA producer, 9 = TMEM owner + MMA issuer (highest warp ids: the
 // issue arbiter favours them, see sim_umma.cu).  The producer prefetches Y tiles into L2 ahead of the stage loads.
 // Split over Y (gridDim.x) leaves fp32 partials [split][Nx][D] that a fixed-order fold sums (deterministic).
+// Logit-scale gradient (mode 0 only): the epilogue thread of query row x also keeps sum_y (P/gscale)[x][y] S[x][y] in a
+// register across its Y tiles and leaves one partial per (split, column half, query); nce_scale_fold_kernel sums them.
 #include <stdlib.h>
 
 #include "umma.cuh"
@@ -52,10 +54,13 @@ struct NceArgs {
   int Nx, Ny, Nq, nkb, nslots, mode;       // mode 0: X = queries (G = dQ), 1: X = regions (G = dR)
   float c2;                                // log2(e) / tau
   float gmul;                              // g_mul / (tau * Nq); multiplied by g_loss[0] on the device
+  float g_mul;
+  const float* scale;                      // device logit scale replacing 1/tau in c2 and gmul, or NULL
+  float* lspart;                           // mode 0: [gridDim.x][2][Nq] logit-scale gradient partials, or NULL
   const float* lse;                        // [Nq]
   const long long* targets;                // [Nq] region index of each query's positive
   const float* g_loss;                     // [1]
-  float* out;                              // [gridDim.x][Nx][D] partials (or the result itself when gridDim.x == 1)
+  float* out;                              // [gridDim.x][Nx][D] partials (or the result itself when gridDim.x == 1); NULL = not written
   const bf16* X;                           // [Nx][D] the CTA's rows, read by the epilogue threads when the X tile lives in TMEM
 };
 
@@ -224,7 +229,14 @@ __global__ void __launch_bounds__(320, 1) nce_bwd_umma_kernel(const __grid_const
     }
 #endif
     const float log2e = 1.4426950408889634f;
-    const float gscale = a.g_loss[0] * a.gmul;
+    float c2 = a.c2, gmul = a.gmul;
+    if (a.scale) {
+      const float s = __ldg(a.scale);
+      c2 = s * log2e;
+      gmul = a.g_mul * s / (float)a.Nq;
+    }
+    const float gscale = a.g_loss[0] * gmul;
+    float ls = 0.f;                                 // mode 0 with lspart: sum over this thread's S columns of coef * S
     float my_nl = 0.f;                              // mode 0: -lse[q] log2e of this thread's query
     int my_tg = -1;
     if (a.mode == 0 && xok) {
@@ -267,10 +279,14 @@ __global__ void __launch_bounds__(320, 1) nce_bwd_umma_kernel(const __grid_const
           hit0 = (__shfl_sync(0xffffffffu, tg_a, 2 * j) == xg);
           hit1 = (__shfl_sync(0xffffffffu, tg_a, 2 * j + 1) == xg);
         }
-        float c0 = ex2_approx(fmaf(__uint_as_float(va[2 * j]), a.c2, n0));
-        float c1 = ex2_approx(fmaf(__uint_as_float(va[2 * j + 1]), a.c2, n1));
+        float c0 = ex2_approx(fmaf(__uint_as_float(va[2 * j]), c2, n0));
+        float c1 = ex2_approx(fmaf(__uint_as_float(va[2 * j + 1]), c2, n1));
         if (hit0) c0 -= 1.f;
         if (hit1) c1 -= 1.f;
+        if (a.lspart) {                             // columns past Ny hold S = 0 (TMA zero fill): they add nothing
+          ls = fmaf(c0, __uint_as_float(va[2 * j]), ls);
+          ls = fmaf(c1, __uint_as_float(va[2 * j + 1]), ls);
+        }
         w[j] = pack_bf16x2_rn(c0 * gscale, c1 * gscale);
       }
       // P row -> shared memory, K-major SW128: 16-byte chunk c of row r at c ^ (r & 7); this thread owns chunks half*4 .. +3
@@ -284,6 +300,7 @@ __global__ void __launch_bounds__(320, 1) nce_bwd_umma_kernel(const __grid_const
       __syncwarp();
       if (lane == 0) mbar_arrive(&tail->p_full[pb]);
     }
+    if (a.lspart && a.mode == 0 && xok) a.lspart[((long long)blockIdx.x * 2 + half) * a.Nq + xg] = ls;
     // ---- drain G: this thread's X row, columns [half * D/2, +D/2) ----
     if (n_my > 0) {
       mbar_wait(&tail->g_full, 0);
@@ -294,7 +311,7 @@ __global__ void __launch_bounds__(320, 1) nce_bwd_umma_kernel(const __grid_const
         uint32_t v[32];
         tmem_ld_32(tmem_g + ((uint32_t)(qd * 32) << 16) + (uint32_t)(half * ncol + c), v);
         tmem_ld_wait();
-        if (xok) {
+        if (xok && a.out) {
 #pragma unroll
           for (int j = 0; j < 8; ++j)
             reinterpret_cast<float4*>(dst + c)[j] = make_float4(__uint_as_float(v[4 * j]), __uint_as_float(v[4 * j + 1]),
@@ -320,6 +337,25 @@ __global__ void __launch_bounds__(256) nce_fold_kernel(const float4* __restrict_
   }
 }
 
+// *g_scale = g_loss[0] * g_mul / Nq * sum_q sum_p lspart[p][q]: one CTA, partials in order per query, queries in a fixed tree
+__global__ void __launch_bounds__(256) nce_scale_fold_kernel(const float* __restrict__ lspart, int nparts, int Nq, const float* __restrict__ g_loss,
+                                                             float g_mul, float* __restrict__ g_scale) {
+  __shared__ float red[256];
+  float v = 0.f;
+  for (int q = threadIdx.x; q < Nq; q += 256) {
+    float s = 0.f;
+    for (int p = 0; p < nparts; ++p) s += lspart[(long long)p * Nq + q];
+    v += s;
+  }
+  red[threadIdx.x] = v;
+  __syncthreads();
+  for (int o = 128; o > 0; o >>= 1) {
+    if (threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) g_scale[0] = red[0] * (g_loss[0] * g_mul / (float)Nq);
+}
+
 static int nce_splits(int xtiles, int ytiles) {
   int s = sm_count() / xtiles;
   if (s < 1) s = 1;
@@ -327,8 +363,10 @@ static int nce_splits(int xtiles, int ytiles) {
   return s;
 }
 
-static int nce_launch(const void* X, const void* Y, int Nx, int Ny, int Nq, int D, int mode, float inv_tau, const float* lse,
-                      const long long* targets, const float* g_loss, float g_mul, float* out, float* part, cudaStream_t st) {
+// out == NULL (mode 0): only the logit-scale partials are wanted -- the dQ GEMM still runs, its result is not stored
+static int nce_launch(const void* X, const void* Y, int Nx, int Ny, int Nq, int D, int mode, float inv_tau, const float* scale,
+                      const float* lse, const long long* targets, const float* g_loss, float g_mul, float* out, float* part,
+                      float* lspart, cudaStream_t st) {
   const int nkb = D / kNbBK;
   const int xtiles = ceil_div(Nx, kNbM), ytiles = ceil_div(Ny, kNbN);
   const int nsplit = nce_splits(xtiles, ytiles);
@@ -348,12 +386,13 @@ static int nce_launch(const void* X, const void* Y, int Nx, int Ny, int Nq, int 
   a.Nx = Nx; a.Ny = Ny; a.Nq = Nq; a.nkb = nkb; a.nslots = nslots; a.mode = mode;
   a.c2 = inv_tau * 1.4426950408889634f;
   a.gmul = g_mul * inv_tau / (float)Nq;
+  a.g_mul = g_mul; a.scale = scale; a.lspart = lspart;
   a.lse = lse; a.targets = targets; a.g_loss = g_loss;
   a.X = reinterpret_cast<const bf16*>(X);
-  a.out = nsplit == 1 ? out : part;
+  a.out = !out ? nullptr : (nsplit == 1 ? out : part);
   nce_bwd_umma_kernel<<<dim3(nsplit, xtiles), 320, smem, st>>>(tmX, tmY, a);
   rc = check_launch("nce_bwd_umma_kernel");
-  if (rc || nsplit == 1) return rc;
+  if (rc || nsplit == 1 || !out) return rc;
   const long long vecs = (long long)Nx * D / 4;
   const int blocks = (int)((vecs + 255) / 256 < (long long)sm_count() * 4 ? (vecs + 255) / 256 : (long long)sm_count() * 4);
   nce_fold_kernel<<<blocks, 256, 0, st>>>(reinterpret_cast<const float4*>(part), reinterpret_cast<float4*>(out), vecs, nsplit);
@@ -364,24 +403,54 @@ static int nce_launch(const void* X, const void* Y, int Nx, int Ny, int Nq, int 
 
 using namespace cor;
 
-extern "C" size_t cor_infonce_bwd_umma_work_bytes(int Nq, int Nr, int D) {
-  // the two launches' partials (nce_launch: X tiles of kNbM rows, Y tiles of kNbN rows), one after the other in the same buffer
+// the two launches' partials (nce_launch: X tiles of kNbM rows, Y tiles of kNbN rows), one after the other in the same buffer,
+// then the logit-scale partials of the dQ launch [splits][2][Nq]
+static size_t nce_part_bytes(int Nq, int Nr, int D) {
   const size_t sq = (size_t)nce_splits(ceil_div(Nq, kNbM), ceil_div(Nr, kNbN)) * Nq * D * sizeof(float);      // mode 0: X = queries
   const size_t sr = (size_t)nce_splits(ceil_div(Nr, kNbM), ceil_div(Nq, kNbN)) * Nr * D * sizeof(float);      // mode 1: X = regions
-  return (sq > sr ? sq : sr) + 256;
+  return ((sq > sr ? sq : sr) + 255) / 256 * 256;
+}
+
+extern "C" size_t cor_infonce_bwd_umma_work_bytes(int Nq, int Nr, int D) {
+  const size_t ls = (size_t)nce_splits(ceil_div(Nq, kNbM), ceil_div(Nr, kNbN)) * 2 * Nq * sizeof(float);
+  return nce_part_bytes(Nq, Nr, D) + ls + 256;
+}
+
+static int infonce_bwd_umma(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, const float* scale,
+                            const float* lse, const long long* targets, const float* g_loss, float g_mul, float* g_regions,
+                            float* g_queries, float* g_scale, void* work, cor_stream_t stream) {
+  COR_REQUIRE(regions && queries && lse && targets && g_loss && work, "cor_infonce_bwd_umma: null pointer");
+  COR_REQUIRE(Nr > 0 && Nq > 0 && D % kNbBK == 0 && D >= kNbBK && D <= 256, "cor_infonce_bwd_umma: need D in {64,128,192,256} (D=%d)", D);
+  COR_REQUIRE(g_regions || g_queries || g_scale, "cor_infonce_bwd_umma: nothing to compute");
+  cudaStream_t st = as_stream(stream);
+  float* part = reinterpret_cast<float*>(work);
+  float* lspart = g_scale ? reinterpret_cast<float*>(reinterpret_cast<char*>(work) + nce_part_bytes(Nq, Nr, D)) : nullptr;
+  int rc = COR_OK;
+  if (g_queries || g_scale)
+    rc = nce_launch(queries, regions, Nq, Nr, Nq, D, 0, inv_tau, scale, lse, targets, g_loss, g_mul, g_queries, part, lspart, st);
+  if (rc) return rc;
+  if (g_scale) {
+    const int nparts = 2 * nce_splits(ceil_div(Nq, kNbM), ceil_div(Nr, kNbN));
+    nce_scale_fold_kernel<<<1, 256, 0, st>>>(lspart, nparts, Nq, g_loss, g_mul, g_scale);
+    rc = check_launch("nce_scale_fold_kernel");
+    if (rc) return rc;
+  }
+  if (g_regions)
+    rc = nce_launch(regions, queries, Nr, Nq, Nq, D, 1, inv_tau, scale, lse, targets, g_loss, g_mul, g_regions, part, nullptr, st);
+  return rc;
 }
 
 extern "C" int cor_infonce_bwd_umma(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, const float* lse,
                                     const long long* targets, const float* g_loss, float g_mul, float* g_regions, float* g_queries,
                                     void* work, cor_stream_t stream) {
-  COR_REQUIRE(regions && queries && lse && targets && g_loss && work, "cor_infonce_bwd_umma: null pointer");
-  COR_REQUIRE(Nr > 0 && Nq > 0 && D % kNbBK == 0 && D >= kNbBK && D <= 256, "cor_infonce_bwd_umma: need D in {64,128,192,256} (D=%d)", D);
-  COR_REQUIRE(g_regions || g_queries, "cor_infonce_bwd_umma: nothing to compute");
-  cudaStream_t st = as_stream(stream);
-  float* part = reinterpret_cast<float*>(work);
-  int rc = COR_OK;
-  if (g_queries) rc = nce_launch(queries, regions, Nq, Nr, Nq, D, 0, inv_tau, lse, targets, g_loss, g_mul, g_queries, part, st);
-  if (rc) return rc;
-  if (g_regions) rc = nce_launch(regions, queries, Nr, Nq, Nq, D, 1, inv_tau, lse, targets, g_loss, g_mul, g_regions, part, st);
-  return rc;
+  return infonce_bwd_umma(regions, queries, Nr, Nq, D, inv_tau, nullptr, lse, targets, g_loss, g_mul, g_regions, g_queries, nullptr, work,
+                          stream);
+}
+
+extern "C" int cor_infonce_bwd_umma_ls(const void* regions, const void* queries, int Nr, int Nq, int D, const float* logit_scale,
+                                       const float* lse, const long long* targets, const float* g_loss, float g_mul, float* g_regions,
+                                       float* g_queries, float* g_logit_scale, void* work, cor_stream_t stream) {
+  COR_REQUIRE(logit_scale, "cor_infonce_bwd_umma_ls: null logit_scale");
+  return infonce_bwd_umma(regions, queries, Nr, Nq, D, 0.f, logit_scale, lse, targets, g_loss, g_mul, g_regions, g_queries, g_logit_scale,
+                          work, stream);
 }

@@ -162,7 +162,8 @@ __global__ void __launch_bounds__(kPeerThreads) peer_gather_kernel(const uint4* 
 constexpr int kPgsThreads = 256;
 __global__ void __launch_bounds__(kPgsThreads) peer_gather_sim_kernel(const uint4* const* __restrict__ src, uint4* __restrict__ all,
                                                                       long long n_local, int D, const bf16* __restrict__ queries, int Nq,
-                                                                      float inv_tau, float* __restrict__ part, PeerCtl c) {
+                                                                      float inv_tau, const float* __restrict__ scale, float* __restrict__ part,
+                                                                      PeerCtl c) {
   extern __shared__ float qs[];   // [kQT][D]
   __shared__ float cm[kPgsThreads / 32][kQT], cs[kPgsThreads / 32][kQT];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -171,6 +172,7 @@ __global__ void __launch_bounds__(kPgsThreads) peer_gather_sim_kernel(const uint
     qs[i] = q < Nq ? __bfloat162float(queries[(long long)q * D + d]) : 0.f;
   }
   const unsigned epoch = peer_enter(c);          // includes a __syncthreads: qs is complete, every peer's rows are published
+  if (scale) inv_tau = __ldg(scale);
   const int nvec = D / 8;
   const bool has = lane < nvec;
   const long long total = n_local * c.world, step = (long long)gridDim.x * (kPgsThreads / 32);
@@ -385,9 +387,9 @@ int cor_peer_gather_rows(const void* const* peer_src, void* all, long long bytes
 
 size_t cor_peer_gather_sim_work_bytes(void) { return (size_t)sm_count() * kQT * 2 * sizeof(float) + 16; }
 
-int cor_peer_gather_sim(const void* const* peer_src, void* all, long long n_local, int D, const void* queries, int Nq, float inv_tau,
-                        float* part, int* nparts, void* const* peer_flags, void* state, int rank, int world, int channel,
-                        cor_stream_t stream) {
+static int peer_gather_sim_launch(const void* const* peer_src, void* all, long long n_local, int D, const void* queries, int Nq,
+                                 float inv_tau, const float* scale, float* part, int* nparts, void* const* peer_flags, void* state, int rank,
+                                 int world, int channel, cor_stream_t stream) {
   COR_REQUIRE(peer_src && all && queries && part && nparts && peer_flags && state, "cor_peer_gather_sim: null pointer");
   COR_REQUIRE(world >= 1 && world <= kPeerMaxWorld && rank >= 0 && rank < world, "cor_peer_gather_sim: rank %d / world %d (max %d)", rank,
               world, kPeerMaxWorld);
@@ -400,9 +402,24 @@ int cor_peer_gather_sim(const void* const* peer_src, void* all, long long n_loca
   const size_t smem = (size_t)kQT * D * sizeof(float);
   peer_gather_sim_kernel<<<grid, kPgsThreads, smem, as_stream(stream)>>>(reinterpret_cast<const uint4* const*>(peer_src),
                                                                         reinterpret_cast<uint4*>(all), n_local, D,
-                                                                        reinterpret_cast<const bf16*>(queries), Nq, inv_tau, part, c);
+                                                                        reinterpret_cast<const bf16*>(queries), Nq, inv_tau, scale, part, c);
   *nparts = grid;
   return check_launch("peer_gather_sim_kernel");
+}
+
+int cor_peer_gather_sim(const void* const* peer_src, void* all, long long n_local, int D, const void* queries, int Nq, float inv_tau,
+                        float* part, int* nparts, void* const* peer_flags, void* state, int rank, int world, int channel,
+                        cor_stream_t stream) {
+  return peer_gather_sim_launch(peer_src, all, n_local, D, queries, Nq, inv_tau, nullptr, part, nparts, peer_flags, state, rank, world,
+                                channel, stream);
+}
+
+int cor_peer_gather_sim_ls(const void* const* peer_src, void* all, long long n_local, int D, const void* queries, int Nq,
+                           const float* logit_scale, float* part, int* nparts, void* const* peer_flags, void* state, int rank, int world,
+                           int channel, cor_stream_t stream) {
+  COR_REQUIRE(logit_scale, "cor_peer_gather_sim_ls: null logit_scale");
+  return peer_gather_sim_launch(peer_src, all, n_local, D, queries, Nq, 0.f, logit_scale, part, nparts, peer_flags, state, rank, world,
+                                channel, stream);
 }
 
 int cor_peer_reduce_rows(const void* const* peer_src, float* out, long long floats_per_rank, void* const* peer_flags, void* state,

@@ -34,10 +34,11 @@ __global__ void __launch_bounds__(128) l2_normalize_kernel(const T* __restrict__
 // grid = (region CTAs, query tiles); block = 256.  dynamic smem = kQT * D floats.
 // work layout: part [qtiles][gridDim.x][kQT][2] (running max, sum) -> lse by sim_lse_combine_kernel.
 __global__ void __launch_bounds__(256) sim_stream_kernel(const bf16* __restrict__ regions, const bf16* __restrict__ queries, int Nr,
-                                                         int Nq, int D, float inv_tau, float* __restrict__ S,
-                                                         float* __restrict__ part) {
+                                                         int Nq, int D, float inv_tau, const float* __restrict__ scale,
+                                                         float* __restrict__ S, float* __restrict__ part) {
   extern __shared__ float qs[];   // [kQT][D]
   __shared__ float cm[8][kQT], cs[8][kQT];
+  if (scale) inv_tau = __ldg(scale);
   const int q0 = blockIdx.y * kQT;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   for (int i = threadIdx.x; i < kQT * D; i += blockDim.x) {
@@ -110,9 +111,10 @@ __global__ void __launch_bounds__(256) sim_lse_combine_kernel(const float* __res
 // ---- InfoNCE forward: target logits and the mean loss ------------------------------------------------
 __global__ void __launch_bounds__(1024) infonce_fwd_kernel(const bf16* __restrict__ regions, const bf16* __restrict__ queries,
                                                            const long long* __restrict__ targets, const float* __restrict__ lse, int Nr,
-                                                           int Nq, int D, float inv_tau, float* __restrict__ loss,
-                                                           float* __restrict__ tgt_logit) {
+                                                           int Nq, int D, float inv_tau, const float* __restrict__ scale,
+                                                           float* __restrict__ loss, float* __restrict__ tgt_logit) {
   __shared__ double scratch[32];
+  if (scale) inv_tau = __ldg(scale);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarp = blockDim.x >> 5;
   double acc[1] = {0.0};
   for (int q = warp; q < Nq; q += nwarp) {
@@ -135,10 +137,12 @@ __global__ void __launch_bounds__(1024) infonce_fwd_kernel(const bf16* __restric
 __global__ void __launch_bounds__(1024) infonce_tail_kernel(const float* __restrict__ part, int nparts, int qt,
                                                             const bf16* __restrict__ regions, const bf16* __restrict__ queries,
                                                             const long long* __restrict__ targets, int Nr, int Nq, int D, float inv_tau,
-                                                            float* __restrict__ lse, float* __restrict__ nce, float* __restrict__ tgt_logit,
-                                                            const float* __restrict__ seg, const float* __restrict__ fgbg, float w_fg,
-                                                            float w_bg, float w_nce, float* __restrict__ total) {
+                                                            const float* __restrict__ scale, float* __restrict__ lse, float* __restrict__ nce,
+                                                            float* __restrict__ tgt_logit, const float* __restrict__ seg,
+                                                            const float* __restrict__ fgbg, float w_fg, float w_bg, float w_nce,
+                                                            float* __restrict__ total) {
   __shared__ double scratch[32];
+  if (scale) inv_tau = __ldg(scale);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarp = blockDim.x >> 5;
   double acc[1] = {0.0};
   for (int q = warp; q < Nq; q += nwarp) {
@@ -215,17 +219,22 @@ __global__ void __launch_bounds__(256) infonce_coef_kernel(const float* __restri
 //   g_regions[r,:] = sum_q coef[q,r] Q[q,:]      g_queries[q,:] = sum_r coef[q,r] R[r,:]
 // grid = region CTAs (persistent), block = 256; loops over query tiles of 16 so that every region row
 // is owned by exactly one warp (deterministic, no atomics).  qpart [gridDim.x][Nq][D] per-CTA partials
-// of g_queries are reduced in fixed order by infonce_bwd_q_kernel.
+// of g_queries are reduced in fixed order by infonce_bwd_q_kernel.  With lspart (the logit-scale gradient wanted) every
+// CTA also leaves sum_r (exp(s S - lse) - [r == t(q)]) S[q,r] over its rows per query, lspart [gridDim.x][Nq], for the same
+// fold kernel.
 template <bool WANT_R>
 __global__ void __launch_bounds__(256, 1) infonce_bwd_kernel(const bf16* __restrict__ regions, const bf16* __restrict__ queries,
                                                              const long long* __restrict__ targets, const float* __restrict__ lse,
-                                                             int Nr, int Nq, int D, float inv_tau, const float* __restrict__ g_loss,
-                                                             float g_mul, float* __restrict__ g_regions, float* __restrict__ qpart) {
+                                                             int Nr, int Nq, int D, float inv_tau, const float* __restrict__ scale,
+                                                             const float* __restrict__ g_loss, float g_mul, float* __restrict__ g_regions,
+                                                             float* __restrict__ qpart, float* __restrict__ lspart) {
   extern __shared__ float smem[];
   float* qs = smem;                    // [kQT][D]
   float* red = smem + kQT * D;         // [8 warps][kQT][D] reduction scratch (reuses after the row loop)
   __shared__ float lse_s[kQT];
   __shared__ long long tgt_s[kQT];
+  __shared__ float ls_s[8][kQT];
+  if (scale) inv_tau = __ldg(scale);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int nvec = D / 8;              // <= 32: one 16-byte vector per lane
   const bool has = lane < nvec;
@@ -252,6 +261,7 @@ __global__ void __launch_bounds__(256, 1) infonce_bwd_kernel(const bf16* __restr
     long long r = (long long)blockIdx.x * 8 + warp;
     uint4 raw_next = make_uint4(0u, 0u, 0u, 0u);
     if (has && r < Nr) raw_next = ld_stream16(reinterpret_cast<const uint4*>(regions + r * D) + lane);
+    float ls = 0.f;                    // lane q: this warp's share of the logit-scale gradient sum of query q0 + q
     for (; r < Nr; r += rstep) {
       float f[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
       const uint4 raw = raw_next;
@@ -276,6 +286,7 @@ __global__ void __launch_bounds__(256, 1) infonce_bwd_kernel(const bf16* __restr
       if (lane < kQT && q0 + lane < Nq) {
         coef = __expf(sv * inv_tau - lse_s[lane]);
         if (tgt_s[lane] == r) coef -= 1.f;
+        if (lspart) ls = fmaf(coef, sv, ls);
         coef *= gscale;
       }
       float gr[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
@@ -312,6 +323,7 @@ __global__ void __launch_bounds__(256, 1) infonce_bwd_kernel(const bf16* __restr
 #pragma unroll
         for (int e = 0; e < 8; ++e) red[(warp * kQT + q) * D + lane * 8 + e] = dq[q][e];
     }
+    if (lspart && lane < kQT) ls_s[warp][lane] = ls;
     __syncthreads();
     for (int i = threadIdx.x; i < kQT * D; i += blockDim.x) {
       const int q = i / D;
@@ -319,6 +331,11 @@ __global__ void __launch_bounds__(256, 1) infonce_bwd_kernel(const bf16* __restr
       float t = 0.f;
       for (int w = 0; w < 8; ++w) t += red[w * kQT * D + i];
       qpart[((long long)blockIdx.x * Nq + q0 + q) * D + (i % D)] = t;
+    }
+    if (lspart && threadIdx.x < kQT && q0 + threadIdx.x < Nq) {
+      float t = 0.f;
+      for (int w = 0; w < 8; ++w) t += ls_s[w][threadIdx.x];
+      lspart[(long long)blockIdx.x * Nq + q0 + threadIdx.x] = t;
     }
   }
 }
@@ -329,11 +346,13 @@ __global__ void __launch_bounds__(256, 1) infonce_bwd_kernel(const bf16* __restr
 constexpr int kRQ = 128;
 __global__ void __launch_bounds__(256, 1) infonce_bwd_regions_kernel(const bf16* __restrict__ regions, const bf16* __restrict__ queries,
                                                                      const long long* __restrict__ targets, const float* __restrict__ lse,
-                                                                     int Nr, int Nq, int D, float inv_tau, const float* __restrict__ g_loss,
-                                                                     float g_mul, float* __restrict__ g_regions) {
+                                                                     int Nr, int Nq, int D, float inv_tau, const float* __restrict__ scale,
+                                                                     const float* __restrict__ g_loss, float g_mul,
+                                                                     float* __restrict__ g_regions) {
   extern __shared__ float qs[];        // [kRQ][D]
   __shared__ float lse_s[kRQ];
   __shared__ long long tgt_s[kRQ];
+  if (scale) inv_tau = __ldg(scale);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int nvec = D / 8;
   const bool has = lane < nvec;
@@ -412,20 +431,43 @@ __global__ void __launch_bounds__(256, 1) infonce_bwd_regions_kernel(const bf16*
   }
 }
 
-// g_queries[i] = sum_p qpart[p][i]: block (32, 8) -- 8 thread rows split the partials, fixed-order smem fold
-__global__ void __launch_bounds__(256) infonce_bwd_q_kernel(const float* __restrict__ qpart, int nparts, long long n, float* __restrict__ g_queries) {
+// g_queries[i] = sum_p qpart[p][i]: block (32, 8) -- 8 thread rows split the partials, fixed-order smem fold.
+// With g_scale, block 0 also folds lspart [nparts][Nq] (partials in CTA order per query, then the queries in a fixed
+// tree) into the logit-scale gradient *g_scale = g_loss[0] * g_mul / Nq * sum.
+__global__ void __launch_bounds__(256) infonce_bwd_q_kernel(const float* __restrict__ qpart, int nparts, long long n, float* __restrict__ g_queries,
+                                                            const float* __restrict__ lspart, int Nq, const float* __restrict__ g_loss,
+                                                            float g_mul, float* __restrict__ g_scale) {
   __shared__ float red[8][33];
   const long long i = (long long)blockIdx.x * 32 + threadIdx.x;
   float t = 0.f;
-  if (i < n)
-    for (int p = threadIdx.y; p < nparts; p += 8) t += qpart[(long long)p * n + i];
-  red[threadIdx.y][threadIdx.x] = t;
-  __syncthreads();
-  if (threadIdx.y == 0 && i < n) {
-    float a = 0.f;
+  if (g_queries) {
+    if (i < n)
+      for (int p = threadIdx.y; p < nparts; p += 8) t += qpart[(long long)p * n + i];
+    red[threadIdx.y][threadIdx.x] = t;
+    __syncthreads();
+    if (threadIdx.y == 0 && i < n) {
+      float a = 0.f;
 #pragma unroll
-    for (int y = 0; y < 8; ++y) a += red[y][threadIdx.x];
-    g_queries[i] = a;
+      for (int y = 0; y < 8; ++y) a += red[y][threadIdx.x];
+      g_queries[i] = a;
+    }
+  }
+  if (g_scale && blockIdx.x == 0) {
+    __shared__ float ls_red[256];
+    const int tid = threadIdx.y * 32 + threadIdx.x;
+    float v = 0.f;
+    for (int q = tid; q < Nq; q += 256) {
+      float s = 0.f;
+      for (int p = 0; p < nparts; ++p) s += lspart[(long long)p * Nq + q];
+      v += s;
+    }
+    ls_red[tid] = v;
+    __syncthreads();
+    for (int o = 128; o > 0; o >>= 1) {
+      if (tid < o) ls_red[tid] += ls_red[tid + o];
+      __syncthreads();
+    }
+    if (tid == 0) g_scale[0] = ls_red[0] * (g_loss[0] * g_mul / (float)Nq);
   }
 }
 
@@ -594,7 +636,7 @@ extern "C" size_t cor_sim_work_bytes(int Nq, int Nr, int D) {
   // LSE partials (either producer) and the g_queries partials of the streaming backward
   const size_t ctas = (size_t)sm_count() * 2 + 1024;
   const size_t lse_part = (size_t)ceil_div(Nq, kQT) * ctas * 256 * 2 * sizeof(float);
-  const size_t qpart = ctas * (size_t)Nq * D * sizeof(float);
+  const size_t qpart = ctas * (size_t)Nq * (D + 1) * sizeof(float);     // + the logit-scale partials [ctas][Nq]
   (void)Nr;
   return (lse_part > qpart ? lse_part : qpart) + 256;
 }
@@ -608,8 +650,8 @@ extern "C" int cor_l2_normalize(const void* x, int x_dtype, int n, int D, float*
   return check_launch("l2_normalize_kernel");
 }
 
-static int sim_stream_launch(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, float* S, float* lse,
-                             void* work, int* nparts, int* qt, cudaStream_t st) {
+static int sim_stream_launch(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, const float* scale, float* S,
+                             float* lse, void* work, int* nparts, int* qt, cudaStream_t st) {
   const bool want_lse = lse || nparts;
   COR_REQUIRE(regions && queries && (S || want_lse), "cor_sim_stream: null pointer");
   COR_REQUIRE(Nr > 0 && Nq > 0 && D > 0 && D % 8 == 0, "cor_sim_stream: need D %% 8 == 0 (D=%d)", D);
@@ -620,7 +662,7 @@ static int sim_stream_launch(const void* regions, const void* queries, int Nr, i
   COR_CUDA(cudaFuncSetAttribute(sim_stream_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int ctas = stream_region_ctas(Nr), qtiles = ceil_div(Nq, kQT);
   float* part = want_lse ? (float*)work : nullptr;
-  sim_stream_kernel<<<dim3(ctas, qtiles), 256, smem, st>>>((const bf16*)regions, (const bf16*)queries, Nr, Nq, D, inv_tau, S, part);
+  sim_stream_kernel<<<dim3(ctas, qtiles), 256, smem, st>>>((const bf16*)regions, (const bf16*)queries, Nr, Nq, D, inv_tau, scale, S, part);
   int rc = check_launch("sim_stream_kernel");
   if (rc || !want_lse) return rc;
   if (nparts) {                       // deferred: the caller merges the partials (cor_infonce_tail)
@@ -633,70 +675,131 @@ static int sim_stream_launch(const void* regions, const void* queries, int Nr, i
 
 extern "C" int cor_sim_stream_fwd(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, float* S,
                                   float* lse, void* work, cor_stream_t stream) {
-  return sim_stream_launch(regions, queries, Nr, Nq, D, inv_tau, S, lse, work, nullptr, nullptr, as_stream(stream));
+  return sim_stream_launch(regions, queries, Nr, Nq, D, inv_tau, nullptr, S, lse, work, nullptr, nullptr, as_stream(stream));
+}
+
+extern "C" int cor_sim_stream_fwd_ls(const void* regions, const void* queries, int Nr, int Nq, int D, const float* logit_scale, float* S,
+                                     float* lse, void* work, cor_stream_t stream) {
+  COR_REQUIRE(logit_scale, "cor_sim_stream_fwd_ls: null logit_scale");
+  return sim_stream_launch(regions, queries, Nr, Nq, D, 0.f, logit_scale, S, lse, work, nullptr, nullptr, as_stream(stream));
+}
+
+static int sim_lse_parts(int engine, const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, const float* scale,
+                         void* work, int* nparts, int* qt, cor_stream_t stream) {
+  COR_REQUIRE(nparts && qt, "cor_sim_lse_parts: null pointer");
+  if (engine == 1)
+    return cor::sim_umma_launch(regions, queries, Nr, Nq, D, inv_tau, scale, nullptr, nullptr, work, nparts, qt, as_stream(stream));
+  COR_REQUIRE(engine == 0, "cor_sim_lse_parts: engine %d (0 = stream, 1 = umma)", engine);
+  return sim_stream_launch(regions, queries, Nr, Nq, D, inv_tau, scale, nullptr, nullptr, work, nparts, qt, as_stream(stream));
 }
 
 extern "C" int cor_sim_lse_parts(int engine, const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, void* work,
                                  int* nparts, int* qt, cor_stream_t stream) {
-  COR_REQUIRE(nparts && qt, "cor_sim_lse_parts: null pointer");
-  if (engine == 1) return cor::sim_umma_launch(regions, queries, Nr, Nq, D, inv_tau, nullptr, nullptr, work, nparts, qt, as_stream(stream));
-  COR_REQUIRE(engine == 0, "cor_sim_lse_parts: engine %d (0 = stream, 1 = umma)", engine);
-  return sim_stream_launch(regions, queries, Nr, Nq, D, inv_tau, nullptr, nullptr, work, nparts, qt, as_stream(stream));
+  return sim_lse_parts(engine, regions, queries, Nr, Nq, D, inv_tau, nullptr, work, nparts, qt, stream);
+}
+
+extern "C" int cor_sim_lse_parts_ls(int engine, const void* regions, const void* queries, int Nr, int Nq, int D, const float* logit_scale,
+                                    void* work, int* nparts, int* qt, cor_stream_t stream) {
+  COR_REQUIRE(logit_scale, "cor_sim_lse_parts_ls: null logit_scale");
+  return sim_lse_parts(engine, regions, queries, Nr, Nq, D, 0.f, logit_scale, work, nparts, qt, stream);
+}
+
+static int infonce_tail(const float* lse_part, int nparts, int qt, const void* regions, const void* queries, const long long* targets, int Nr,
+                        int Nq, int D, float inv_tau, const float* scale, float* lse, float* nce, float* tgt_logit, const float* seg,
+                        const float* fgbg, float w_fg, float w_bg, float w_nce, float* total, cor_stream_t stream) {
+  COR_REQUIRE(lse_part && regions && queries && targets && lse && nce && tgt_logit, "cor_infonce_tail: null pointer");
+  COR_REQUIRE(nparts > 0 && qt > 0 && Nr > 0 && Nq > 0 && D > 0, "cor_infonce_tail: bad sizes");
+  COR_REQUIRE(!total || (seg && fgbg), "cor_infonce_tail: total needs seg and fgbg");
+  infonce_tail_kernel<<<1, 1024, 0, as_stream(stream)>>>(lse_part, nparts, qt, (const bf16*)regions, (const bf16*)queries, targets, Nr, Nq, D,
+                                                        inv_tau, scale, lse, nce, tgt_logit, seg, fgbg, w_fg, w_bg, w_nce, total);
+  return check_launch("infonce_tail_kernel");
 }
 
 extern "C" int cor_infonce_tail(const float* lse_part, int nparts, int qt, const void* regions, const void* queries,
                                 const long long* targets, int Nr, int Nq, int D, float inv_tau, float* lse, float* nce, float* tgt_logit,
                                 const float* seg, const float* fgbg, float w_fg, float w_bg, float w_nce, float* total,
                                 cor_stream_t stream) {
-  COR_REQUIRE(lse_part && regions && queries && targets && lse && nce && tgt_logit, "cor_infonce_tail: null pointer");
-  COR_REQUIRE(nparts > 0 && qt > 0 && Nr > 0 && Nq > 0 && D > 0, "cor_infonce_tail: bad sizes");
-  COR_REQUIRE(!total || (seg && fgbg), "cor_infonce_tail: total needs seg and fgbg");
-  infonce_tail_kernel<<<1, 1024, 0, as_stream(stream)>>>(lse_part, nparts, qt, (const bf16*)regions, (const bf16*)queries, targets, Nr, Nq, D,
-                                                        inv_tau, lse, nce, tgt_logit, seg, fgbg, w_fg, w_bg, w_nce, total);
-  return check_launch("infonce_tail_kernel");
+  return infonce_tail(lse_part, nparts, qt, regions, queries, targets, Nr, Nq, D, inv_tau, nullptr, lse, nce, tgt_logit, seg, fgbg, w_fg,
+                      w_bg, w_nce, total, stream);
+}
+
+extern "C" int cor_infonce_tail_ls(const float* lse_part, int nparts, int qt, const void* regions, const void* queries,
+                                   const long long* targets, int Nr, int Nq, int D, const float* logit_scale, float* lse, float* nce,
+                                   float* tgt_logit, const float* seg, const float* fgbg, float w_fg, float w_bg, float w_nce, float* total,
+                                   cor_stream_t stream) {
+  COR_REQUIRE(logit_scale, "cor_infonce_tail_ls: null logit_scale");
+  return infonce_tail(lse_part, nparts, qt, regions, queries, targets, Nr, Nq, D, 0.f, logit_scale, lse, nce, tgt_logit, seg, fgbg, w_fg,
+                      w_bg, w_nce, total, stream);
+}
+
+static int infonce_fwd(const void* regions, const void* queries, const long long* targets, const float* lse, int Nr, int Nq, int D,
+                       float inv_tau, const float* scale, float* loss, float* tgt_logit, cor_stream_t stream) {
+  COR_REQUIRE(regions && queries && targets && lse && loss && tgt_logit, "cor_infonce_fwd: null pointer");
+  infonce_fwd_kernel<<<1, 1024, 0, as_stream(stream)>>>((const bf16*)regions, (const bf16*)queries, targets, lse, Nr, Nq, D, inv_tau,
+                                                       scale, loss, tgt_logit);
+  return check_launch("infonce_fwd_kernel");
 }
 
 extern "C" int cor_infonce_fwd(const void* regions, const void* queries, const long long* targets, const float* lse, int Nr,
                                int Nq, int D, float inv_tau, float* loss, float* tgt_logit, cor_stream_t stream) {
-  COR_REQUIRE(regions && queries && targets && lse && loss && tgt_logit, "cor_infonce_fwd: null pointer");
-  infonce_fwd_kernel<<<1, 1024, 0, as_stream(stream)>>>((const bf16*)regions, (const bf16*)queries, targets, lse, Nr, Nq, D, inv_tau,
-                                                       loss, tgt_logit);
-  return check_launch("infonce_fwd_kernel");
+  return infonce_fwd(regions, queries, targets, lse, Nr, Nq, D, inv_tau, nullptr, loss, tgt_logit, stream);
 }
 
-extern "C" int cor_infonce_bwd(const void* regions, const void* queries, const long long* targets, const float* lse, int Nr,
-                               int Nq, int D, float inv_tau, const float* g_loss, float g_mul, float* g_regions, float* g_queries,
-                               void* work, cor_stream_t stream) {
-  COR_REQUIRE(regions && queries && targets && lse && g_loss && (g_regions || g_queries), "cor_infonce_bwd: null pointer");
-  COR_REQUIRE(!g_queries || work, "cor_infonce_bwd: g_queries needs a work buffer");
+extern "C" int cor_infonce_fwd_ls(const void* regions, const void* queries, const long long* targets, const float* lse, int Nr,
+                                  int Nq, int D, const float* logit_scale, float* loss, float* tgt_logit, cor_stream_t stream) {
+  COR_REQUIRE(logit_scale, "cor_infonce_fwd_ls: null logit_scale");
+  return infonce_fwd(regions, queries, targets, lse, Nr, Nq, D, 0.f, logit_scale, loss, tgt_logit, stream);
+}
+
+static int infonce_bwd(const void* regions, const void* queries, const long long* targets, const float* lse, int Nr, int Nq, int D,
+                       float inv_tau, const float* scale, const float* g_loss, float g_mul, float* g_regions, float* g_queries,
+                       float* g_scale, void* work, cor_stream_t stream) {
+  COR_REQUIRE(regions && queries && targets && lse && g_loss && (g_regions || g_queries || g_scale), "cor_infonce_bwd: null pointer");
+  COR_REQUIRE(!(g_queries || g_scale) || work, "cor_infonce_bwd: g_queries / g_logit_scale need a work buffer");
   COR_REQUIRE(D % 8 == 0 && D <= 256, "cor_infonce_bwd: streaming backward supports D %% 8 == 0 and D <= 256 (D=%d)", D);
   COR_REQUIRE((((uintptr_t)regions) & 15) == 0 && (((uintptr_t)g_regions) & 15) == 0, "cor_infonce_bwd: 16-byte alignment required");
   cudaStream_t st = as_stream(stream);
   int ctas = sm_count();
   const int need = ceil_div(Nr, 8);
   if (ctas > need) ctas = need;
-  if (!g_queries) {
+  if (!g_queries && !g_scale) {
     const size_t smem_r = (size_t)kRQ * D * sizeof(float);
     COR_CUDA(cudaFuncSetAttribute(infonce_bwd_regions_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_r));
     infonce_bwd_regions_kernel<<<ctas, 256, smem_r, st>>>((const bf16*)regions, (const bf16*)queries, targets, lse, Nr, Nq, D, inv_tau,
-                                                         g_loss, g_mul, g_regions);
+                                                         scale, g_loss, g_mul, g_regions);
     return check_launch("infonce_bwd_regions_kernel");
   }
   const size_t smem = (size_t)(kQT * D + 8 * kQT * D) * sizeof(float);
+  // work: qpart [ctas][Nq][D], then (logit-scale gradient wanted) lspart [ctas][Nq]
+  float* lspart = g_scale ? (float*)work + (size_t)ctas * Nq * D : nullptr;
   if (g_regions) {
     COR_CUDA(cudaFuncSetAttribute(infonce_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    infonce_bwd_kernel<true><<<ctas, 256, smem, st>>>((const bf16*)regions, (const bf16*)queries, targets, lse, Nr, Nq, D, inv_tau, g_loss,
-                                                     g_mul, g_regions, (float*)work);
+    infonce_bwd_kernel<true><<<ctas, 256, smem, st>>>((const bf16*)regions, (const bf16*)queries, targets, lse, Nr, Nq, D, inv_tau, scale,
+                                                     g_loss, g_mul, g_regions, (float*)work, lspart);
   } else {
     COR_CUDA(cudaFuncSetAttribute(infonce_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    infonce_bwd_kernel<false><<<ctas, 256, smem, st>>>((const bf16*)regions, (const bf16*)queries, targets, lse, Nr, Nq, D, inv_tau, g_loss,
-                                                      g_mul, nullptr, (float*)work);
+    infonce_bwd_kernel<false><<<ctas, 256, smem, st>>>((const bf16*)regions, (const bf16*)queries, targets, lse, Nr, Nq, D, inv_tau, scale,
+                                                      g_loss, g_mul, nullptr, (float*)work, lspart);
   }
   int rc = check_launch("infonce_bwd_kernel");
   if (rc) return rc;
   const long long n = (long long)Nq * D;
-  infonce_bwd_q_kernel<<<ceil_div(n, 32), dim3(32, 8), 0, st>>>((const float*)work, ctas, n, g_queries);
+  infonce_bwd_q_kernel<<<ceil_div(n, 32), dim3(32, 8), 0, st>>>((const float*)work, ctas, n, g_queries, lspart, Nq, g_loss, g_mul, g_scale);
   return check_launch("infonce_bwd_q_kernel");
+}
+
+extern "C" int cor_infonce_bwd(const void* regions, const void* queries, const long long* targets, const float* lse, int Nr,
+                               int Nq, int D, float inv_tau, const float* g_loss, float g_mul, float* g_regions, float* g_queries,
+                               void* work, cor_stream_t stream) {
+  return infonce_bwd(regions, queries, targets, lse, Nr, Nq, D, inv_tau, nullptr, g_loss, g_mul, g_regions, g_queries, nullptr, work, stream);
+}
+
+extern "C" int cor_infonce_bwd_ls(const void* regions, const void* queries, const long long* targets, const float* lse, int Nr,
+                                  int Nq, int D, const float* logit_scale, const float* g_loss, float g_mul, float* g_regions,
+                                  float* g_queries, float* g_logit_scale, void* work, cor_stream_t stream) {
+  COR_REQUIRE(logit_scale, "cor_infonce_bwd_ls: null logit_scale");
+  return infonce_bwd(regions, queries, targets, lse, Nr, Nq, D, 0.f, logit_scale, g_loss, g_mul, g_regions, g_queries, g_logit_scale, work,
+                     stream);
 }
 
 extern "C" int cor_infonce_coef(const float* S, const float* lse, const long long* targets, int Nq, int Nr, float inv_tau,

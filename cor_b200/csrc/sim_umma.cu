@@ -78,7 +78,7 @@ struct SimCoef {
 // part layout (shared with the streaming producer's combine kernel): [qtile][gridDim.x][kSimBM][2]
 __global__ void __launch_bounds__(320, 1) sim_umma_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmR,
                                                           int Nr, int Nq, int nkb, int nstages, int q_slots, int cl, float inv_tau,
-                                                          float* __restrict__ S, float* __restrict__ part, SimCoef coef) {
+                                                          const float* __restrict__ scale, float* __restrict__ S, float* __restrict__ part, SimCoef coef) {
   extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t* base = reinterpret_cast<uint8_t*>(((uintptr_t)smem + 1023) & ~(uintptr_t)1023);
   uint8_t* q_smem = base;                                                   // [half][kb] x 16 KB
@@ -188,6 +188,7 @@ __global__ void __launch_bounds__(320, 1) sim_umma_kernel(const __grid_constant_
     const int q = q0 + hf * kSimHalf + qd * 32 + lane;
     const bool active = hf < nhalf;
     const bool qok = active && q < Nq;
+    if (scale) inv_tau = __ldg(scale);
     const float c2 = inv_tau * 1.4426950408889634f;   // exp(x/tau) = exp2(x * c2)
     float m = -INFINITY, ssum = 0.f;               // running max of raw S and sum exp2((S - m) c2)
     const bool vec_ok = (Nr % 4 == 0) && ((((uintptr_t)S) & 15) == 0);
@@ -341,7 +342,7 @@ __global__ void __launch_bounds__(320, 1) sim_umma_kernel(const __grid_constant_
 using namespace cor;
 
 namespace cor {
-static int sim_umma_launch_impl(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, float* S, float* lse,
+static int sim_umma_launch_impl(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, const float* scale, float* S, float* lse,
                                 void* work, int* nparts, int* qt, SimCoef coef, cudaStream_t st) {
   const bool want_lse = lse || nparts;
   COR_REQUIRE(regions && queries && (S || want_lse || coef.P), "cor_sim_umma_fwd: null pointer");
@@ -360,7 +361,7 @@ static int sim_umma_launch_impl(const void* regions, const void* queries, int Nr
     const char* e = getenv("COR_SIM_TS");
     if (want_lse && !S && !coef.P && cl == 1 && !(e && atoi(e) == 0)) {
       int gx_ts = 0;
-      int rc_ts = sim_umma_ts_launch(regions, queries, Nr, Nq, D, inv_tau, work, &gx_ts, st);
+      int rc_ts = sim_umma_ts_launch(regions, queries, Nr, Nq, D, inv_tau, scale, work, &gx_ts, st);
       if (rc_ts) return rc_ts;
       if (nparts) {
         *nparts = gx_ts;
@@ -410,7 +411,7 @@ static int sim_umma_launch_impl(const void* regions, const void* queries, int Nr
       cfg.gridDim = dim3(gx, qtiles);
     }
   }
-  COR_CUDA(cudaLaunchKernelEx(&cfg, sim_umma_kernel, tmQ, tmR, Nr, Nq, nkb_arg, nstages, q_slots, cl, inv_tau, S, part, coef));
+  COR_CUDA(cudaLaunchKernelEx(&cfg, sim_umma_kernel, tmQ, tmR, Nr, Nq, nkb_arg, nstages, q_slots, cl, inv_tau, scale, S, part, coef));
   rc = check_launch("sim_umma_kernel");
   if (rc || !want_lse) return rc;
   if (nparts) {                       // deferred: the caller merges the partials (cor_infonce_tail)
@@ -422,22 +423,29 @@ static int sim_umma_launch_impl(const void* regions, const void* queries, int Nr
   return launch_lse_combine(part, Nq, gx, kSimBM, lse, st);
 }
 
-int sim_umma_launch(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, float* S, float* lse, void* work,
-                    int* nparts, int* qt, cudaStream_t st) {
-  return sim_umma_launch_impl(regions, queries, Nr, Nq, D, inv_tau, S, lse, work, nparts, qt, SimCoef{nullptr, nullptr, nullptr, 0.f, nullptr}, st);
+int sim_umma_launch(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, const float* scale, float* S, float* lse,
+                    void* work, int* nparts, int* qt, cudaStream_t st) {
+  return sim_umma_launch_impl(regions, queries, Nr, Nq, D, inv_tau, scale, S, lse, work, nparts, qt, SimCoef{nullptr, nullptr, nullptr, 0.f, nullptr}, st);
 }
 }  // namespace cor
 
 extern "C" int cor_sim_umma_coef(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, const float* lse,
                                  const long long* targets, const float* g_loss, float g_mul, void* P_bf16, cor_stream_t stream) {
   COR_REQUIRE(lse && targets && g_loss && P_bf16, "cor_sim_umma_coef: null pointer");
-  return cor::sim_umma_launch_impl(regions, queries, Nr, Nq, D, inv_tau, nullptr, nullptr, nullptr, nullptr, nullptr,
+  return cor::sim_umma_launch_impl(regions, queries, Nr, Nq, D, inv_tau, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr,
                                    cor::SimCoef{lse, targets, g_loss, g_mul, (cor::bf16*)P_bf16}, cor::as_stream(stream));
 }
 
 extern "C" int cor_sim_umma_fwd(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, float* S, float* lse,
                                 void* work, cor_stream_t stream) {
-  return cor::sim_umma_launch(regions, queries, Nr, Nq, D, inv_tau, S, lse, work, nullptr, nullptr, as_stream(stream));
+  return cor::sim_umma_launch(regions, queries, Nr, Nq, D, inv_tau, nullptr, S, lse, work, nullptr, nullptr, as_stream(stream));
+}
+
+// cor_sim_umma_fwd with the logit scale read from device memory
+extern "C" int cor_sim_umma_fwd_ls(const void* regions, const void* queries, int Nr, int Nq, int D, const float* logit_scale, float* S,
+                                   float* lse, void* work, cor_stream_t stream) {
+  COR_REQUIRE(logit_scale, "cor_sim_umma_fwd_ls: null logit_scale");
+  return cor::sim_umma_launch(regions, queries, Nr, Nq, D, 0.f, logit_scale, S, lse, work, nullptr, nullptr, as_stream(stream));
 }
 
 #ifdef COR_SIM_TRACE

@@ -36,7 +36,8 @@ struct TsSmemTail {
 };
 
 __global__ void __launch_bounds__(320, 1) sim_umma_ts_kernel(const __grid_constant__ CUtensorMap tmR, const bf16* __restrict__ queries, int Nr,
-                                                             int Nq, int nkb, int nstages, float inv_tau, float* __restrict__ part) {
+                                                             int Nq, int nkb, int nstages, float inv_tau, const float* __restrict__ scale,
+                                                             float* __restrict__ part) {
   extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t* base = reinterpret_cast<uint8_t*>(((uintptr_t)smem + 1023) & ~(uintptr_t)1023);
   uint8_t* r_smem = base;
@@ -138,6 +139,7 @@ __global__ void __launch_bounds__(320, 1) sim_umma_ts_kernel(const __grid_consta
     __syncwarp();
     if (lane == 0) mbar_arrive(&tail->afull);
 
+    if (scale) inv_tau = __ldg(scale);
     const float c2 = inv_tau * 1.4426950408889634f;
     float m = -INFINITY, ssum = 0.f;
     auto proc = [&](uint32_t (&v)[32], int r0, int col) {
@@ -220,8 +222,8 @@ __global__ void __launch_bounds__(320, 1) sim_umma_ts_kernel(const __grid_consta
 
 // LSE-only launcher (sim_umma.cu falls back to the SS kernel for the S / coefficient modes).  Returns the number of
 // partial records per query tile in *nparts.
-int sim_umma_ts_launch(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, void* work, int* nparts,
-                       cudaStream_t st) {
+int sim_umma_ts_launch(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, const float* scale, void* work,
+                       int* nparts, cudaStream_t st) {
   const int qtiles = ceil_div(Nq, kTsBM), ntiles = ceil_div(Nr, kTsBN);
   CUtensorMap tmR;
   int rc = umma::encode_tmap_bf16_2d(&tmR, regions, (uint64_t)Nr, (uint64_t)D, kTsBN, kTsBK);
@@ -235,7 +237,7 @@ int sim_umma_ts_launch(const void* regions, const void* queries, int Nr, int Nq,
   const size_t smem = (size_t)nstages * kTsBBytes + sizeof(TsSmemTail) + 1024;
   COR_CUDA(cudaFuncSetAttribute(sim_umma_ts_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   sim_umma_ts_kernel<<<dim3(gx, qtiles), 320, smem, st>>>(tmR, reinterpret_cast<const bf16*>(queries), Nr, Nq, nkb, nstages, inv_tau,
-                                                         reinterpret_cast<float*>(work));
+                                                         scale, reinterpret_cast<float*>(work));
   *nparts = gx;
   return check_launch("sim_umma_ts_kernel");
 }

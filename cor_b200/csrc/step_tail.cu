@@ -18,7 +18,7 @@ namespace {
 constexpr float kDenEps = 1e-8f;    // eps added to the pooling denominator (cor_rows_finalize's eps in region.py)
 constexpr float kCosEps = 1e-8f;    // F.cosine_similarity default eps (fgbg_loss.cu)
 constexpr int kTailRowsQ = 64;      // region rows per dQ CTA of the backward: 8 per warp, held in registers
-constexpr int kCounterWords = 32;   // [0]: forward; [1 + q]: backward query q
+constexpr int kCounterWords = 32;   // [0]: forward; [1 + q]: backward query q; [1 + kQT]: backward, all queries (logit scale)
 
 __device__ __forceinline__ void load8(const float* p, float (&v)[8]) {
   const float4 a = *reinterpret_cast<const float4*>(p), b = *reinterpret_cast<const float4*>(p + 4);
@@ -83,7 +83,7 @@ __device__ __forceinline__ bool arrive_last(unsigned* counter, unsigned n, bool*
 
 struct StepTailFwd {
   const float* part; int nsplit; long long split_stride; long long img_stride; int B, M, C; float p_total;
-  const float* stats; const bf16* q16; const float* comb; const long long* targets; float inv_tau;
+  const float* stats; const bf16* q16; const float* comb; const long long* targets; float inv_tau; const float* scale;
   const float* seg; float w_fg, w_bg, w_nce;
   float* fg; bf16* fg16; float* inv_fg; float* bg; float* inv_bg; float* out4; float* aux;
   float* lse; float* nce; float* tgt; float* total; float* lse_part; unsigned* counter;
@@ -98,6 +98,7 @@ __global__ void __launch_bounds__(256, 1) step_tail_fwd_kernel(const StepTailFwd
   __shared__ bool last;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int C = a.C, M = a.M, Nq = a.B, Nr = a.B * a.M;
+  const float inv_tau = a.scale ? __ldg(a.scale) : a.inv_tau;
   fill_queries(qs, a.q16, Nq, C);
   const bool has = lane * 8 < C;
   const int c0 = lane * 8;
@@ -136,7 +137,7 @@ __global__ void __launch_bounds__(256, 1) step_tail_fwd_kernel(const StepTailFwd
     }
     const float sv = transpose_reduce16(s, lane);
     if (lane < Nq) {           // lane < kQT: lane l holds query l
-      m_run = sv * a.inv_tau;
+      m_run = sv * inv_tau;
       s_run = 1.f;
       if (a.targets[lane] == r) a.tgt[lane] = sv;
     }
@@ -267,7 +268,7 @@ __global__ void __launch_bounds__(256, 1) step_tail_fwd_kernel(const StepTailFwd
   block_sum<1>(quirk, dscratch);
   if (threadIdx.x == 0) {
     double acc = 0.0;
-    for (int q = 0; q < Nq; ++q) acc += (double)lse_s[q] - (double)tgt_s[q] * (double)a.inv_tau;
+    for (int q = 0; q < Nq; ++q) acc += (double)lse_s[q] - (double)tgt_s[q] * (double)inv_tau;
     const float nce = (float)(acc / (double)Nq);
     const float fl = nfg > 0 ? (float)(1.0 - v0 / nfg) : 0.f;
     const float bl = nbg > 0 ? (float)(1.0 + quirk[0] / (nbg * (double)C)) : 0.f;
@@ -278,14 +279,16 @@ __global__ void __launch_bounds__(256, 1) step_tail_fwd_kernel(const StepTailFwd
 }
 
 struct StepTailBwd {
-  const bf16* r16; const bf16* q16; const long long* targets; const float* lse; int B, M, C; float inv_tau;
+  const bf16* r16; const bf16* q16; const long long* targets; const float* lse; int B, M, C; float inv_tau; const float* scale;
   const float* g_loss; float w_nce; const float* fg; const float* inv_fg; const float* stats; const float* comb;
   const float* out4; const float* aux; float w_fg, w_bg;
-  bf16* a16; int Kp; float* g_q; float* qpart; unsigned* counter; int nreg, nsplit_q;
+  bf16* a16; int Kp; float* g_q; float* g_scale; float* qpart; float* lspart; float* lsq; unsigned* counter; int nreg, nsplit_q;
 };
 
 // grid = nreg region CTAs (warp per row: InfoNCE + fg-loss gradient of the row, epilogue backward, bf16 GEMM operand) +
 // B * nsplit_q dQ CTAs (query q, kTailRowsQ rows each; the last of a query's CTAs folds the partials in split order).
+// The logit-scale gradient sum_r (p_qr - [r == t(q)]) S_qr rides on the dQ CTAs: one partial per (query, split), folded in
+// split order by the query's last CTA, and the last of those folds the queries in order into *g_scale.
 // block = 256; dynamic smem = kQT * C floats.
 __global__ void __launch_bounds__(256, 1) step_tail_bwd_kernel(const StepTailBwd a) {
   extern __shared__ float sm[];
@@ -295,7 +298,8 @@ __global__ void __launch_bounds__(256, 1) step_tail_bwd_kernel(const StepTailBwd
   const bool has = lane * 8 < C;
   const int c0 = lane * 8;
   const float g = a.g_loss[0];
-  const float gscale = g * a.w_nce * a.inv_tau / (float)Nq;
+  const float inv_tau = a.scale ? __ldg(a.scale) : a.inv_tau;
+  const float gscale = g * a.w_nce * inv_tau / (float)Nq;
   const float nfg = a.out4[2], nbg = a.out4[3];
   if ((int)blockIdx.x < a.nreg) {
     float* qs = sm;   // [kQT][C]
@@ -322,7 +326,7 @@ __global__ void __launch_bounds__(256, 1) step_tail_bwd_kernel(const StepTailBwd
       const float sv = transpose_reduce16(s, lane);
       float coef = 0.f;
       if (lane < Nq) {
-        coef = __expf(sv * a.inv_tau - a.lse[lane]);
+        coef = __expf(sv * inv_tau - a.lse[lane]);
         if (a.targets[lane] == r) coef -= 1.f;
         coef *= gscale;
       }
@@ -393,11 +397,14 @@ __global__ void __launch_bounds__(256, 1) step_tail_bwd_kernel(const StepTailBwd
     for (int u = 0; u < 8; ++u) t[u] += __shfl_xor_sync(0xffffffffu, t[u], o);
   // 2. sum_r coef[r] R[r] over the warp's rows in row order, then the 8 warp sums in warp order
   float acc[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+  float ls = 0.f;                   // sum_r coef[r] S[r] / gscale over the warp's rows (the same in every lane)
+  __shared__ float ls_w[8];
 #pragma unroll
   for (int u = 0; u < 8; ++u) {
     if (rw + u < Nr) {
-      float c = __expf(t[u] * a.inv_tau - lq);
+      float c = __expf(t[u] * inv_tau - lq);
       if (tq == rw + u) c -= 1.f;
+      if (a.g_scale) ls = fmaf(c, t[u], ls);
       c *= gscale;
       float f[8];
       unpack8(raw[u], f);
@@ -406,11 +413,19 @@ __global__ void __launch_bounds__(256, 1) step_tail_bwd_kernel(const StepTailBwd
     }
   }
   if (has) store8(red + warp * C + c0, acc);
+  if (lane == 0) ls_w[warp] = ls;
   __syncthreads();
-  for (int c = threadIdx.x; c < C; c += blockDim.x) {
+  if (a.g_q) {
+    for (int c = threadIdx.x; c < C; c += blockDim.x) {
+      float v = 0.f;
+      for (int w = 0; w < 8; ++w) v += red[w * C + c];
+      a.qpart[((long long)q * a.nsplit_q + split) * C + c] = v;
+    }
+  }
+  if (a.g_scale && threadIdx.x == 0) {
     float v = 0.f;
-    for (int w = 0; w < 8; ++w) v += red[w * C + c];
-    a.qpart[((long long)q * a.nsplit_q + split) * C + c] = v;
+    for (int w = 0; w < 8; ++w) v += ls_w[w];
+    a.lspart[q * a.nsplit_q + split] = v;
   }
   if (!arrive_last(a.counter + q, a.nsplit_q, &last)) return;
   // last dQ CTA of query q: fold the splits in order, add the fg-loss and bg-quirk gradients (fgbg_bwd_kernel, bg_mode 0)
@@ -419,7 +434,7 @@ __global__ void __launch_bounds__(256, 1) step_tail_bwd_kernel(const StepTailBwd
   const float quirk = (rs[6] > 0.f && nbg > 0.f) ? (g * a.w_bg) / (nbg * (float)C) : 0.f;
   const float cf = rs[0], nf = rs[2], nq = rs[4];
   const float* colstat = a.aux + (long long)Nq * 8;
-  for (int c = threadIdx.x; c < C; c += blockDim.x) {
+  for (int c = threadIdx.x; a.g_q && c < C; c += blockDim.x) {
     float t = 0.f;
     for (int k0 = 0; k0 < a.nsplit_q; k0 += 8) {      // eight partials in flight, added in split order
       float pk[8];
@@ -437,6 +452,19 @@ __global__ void __launch_bounds__(256, 1) step_tail_bwd_kernel(const StepTailBwd
     }
     a.g_q[(long long)q * C + c] = t + gq;
   }
+  if (!a.g_scale) return;
+  if (threadIdx.x == 0) {
+    float v = 0.f;
+    for (int k = 0; k < a.nsplit_q; ++k) v += __ldcg(a.lspart + q * a.nsplit_q + k);
+    a.lsq[q] = v;
+  }
+  if (!arrive_last(a.counter + 1 + kQT, Nq, &last)) return;
+  // last query to finish: the queries in order, scaled like the InfoNCE term of the total loss
+  if (threadIdx.x == 0) {
+    float v = 0.f;
+    for (int i = 0; i < Nq; ++i) v += __ldcg(a.lsq + i);
+    a.g_scale[0] = v * (g * a.w_nce / (float)Nq);
+  }
 }
 
 }  // namespace cor
@@ -450,7 +478,7 @@ extern "C" int cor_step_tail_counter_words(void) { return kCounterWords; }
 extern "C" size_t cor_step_tail_work_bytes(int B, int M, int C) {
   if (B <= 0 || M <= 0 || C <= 0) return 0;
   const size_t fwd = (size_t)ceil_div((long long)B * M, 8) * kQT * 2 * sizeof(float);
-  const size_t bwd = (size_t)B * tail_nsplit_q(B, M) * C * sizeof(float);
+  const size_t bwd = (size_t)B * tail_nsplit_q(B, M) * (C + 1) * sizeof(float) + kQT * sizeof(float);   // + logit-scale partials
   return fwd > bwd ? fwd : bwd;
 }
 
@@ -460,11 +488,11 @@ static int tail_shape_ok(int B, int M, int C, const char* who) {
   return COR_OK;
 }
 
-extern "C" int cor_step_tail_fwd(const float* part, int nsplit, long long split_stride, int Rp, int B, int M, int C, float p_total,
-                                 const float* stats, const void* queries_bf16, const float* comb, const long long* targets, float inv_tau,
-                                 const float* seg, float w_fg, float w_bg, float w_nce, float* fg, void* fg_bf16, float* inv_fg, float* bg,
-                                 float* inv_bg, float* fgbg_out4, float* aux, float* lse, float* nce, float* tgt_logit, float* total,
-                                 void* work, unsigned* counter, cor_stream_t stream) {
+static int step_tail_fwd(const float* part, int nsplit, long long split_stride, int Rp, int B, int M, int C, float p_total,
+                         const float* stats, const void* queries_bf16, const float* comb, const long long* targets, float inv_tau,
+                         const float* scale, const float* seg, float w_fg, float w_bg, float w_nce, float* fg, void* fg_bf16, float* inv_fg,
+                         float* bg, float* inv_bg, float* fgbg_out4, float* aux, float* lse, float* nce, float* tgt_logit, float* total,
+                         void* work, unsigned* counter, cor_stream_t stream) {
   int rc = tail_shape_ok(B, M, C, "cor_step_tail_fwd");
   if (rc) return rc;
   COR_REQUIRE(part && stats && queries_bf16 && comb && targets && seg && fg && fg_bf16 && inv_fg && bg && inv_bg && fgbg_out4 && aux &&
@@ -474,31 +502,72 @@ extern "C" int cor_step_tail_fwd(const float* part, int nsplit, long long split_
                                                                      (uintptr_t)comb) & 15) == 0,
               "cor_step_tail_fwd: bad partial layout or alignment (nsplit=%d Rp=%d M=%d)", nsplit, Rp, M);
   StepTailFwd a{part, nsplit, split_stride, (long long)Rp * C, B, M, C, p_total, stats, (const bf16*)queries_bf16, comb, targets, inv_tau,
-                seg, w_fg, w_bg, w_nce, fg, (bf16*)fg_bf16, inv_fg, bg, inv_bg, fgbg_out4, aux, lse, nce, tgt_logit, total,
+                scale, seg, w_fg, w_bg, w_nce, fg, (bf16*)fg_bf16, inv_fg, bg, inv_bg, fgbg_out4, aux, lse, nce, tgt_logit, total,
                 (float*)work, counter};
   const int grid = ceil_div((long long)B * M, 8);
   step_tail_fwd_kernel<<<grid, 256, (size_t)kQT * C * sizeof(float), as_stream(stream)>>>(a);
   return check_launch("step_tail_fwd_kernel");
 }
 
-extern "C" int cor_step_tail_bwd(const void* regions_bf16, const void* queries_bf16, const long long* targets, const float* lse, int B, int M,
-                                 int C, float inv_tau, const float* g_loss, float w_nce, const float* fg, const float* inv_fg,
-                                 const float* stats, const float* comb, const float* fgbg_out4, const float* aux, float w_fg, float w_bg,
-                                 void* a16, int Kp, float* g_queries, void* work, unsigned* counter, cor_stream_t stream) {
+extern "C" int cor_step_tail_fwd(const float* part, int nsplit, long long split_stride, int Rp, int B, int M, int C, float p_total,
+                                 const float* stats, const void* queries_bf16, const float* comb, const long long* targets, float inv_tau,
+                                 const float* seg, float w_fg, float w_bg, float w_nce, float* fg, void* fg_bf16, float* inv_fg, float* bg,
+                                 float* inv_bg, float* fgbg_out4, float* aux, float* lse, float* nce, float* tgt_logit, float* total,
+                                 void* work, unsigned* counter, cor_stream_t stream) {
+  return step_tail_fwd(part, nsplit, split_stride, Rp, B, M, C, p_total, stats, queries_bf16, comb, targets, inv_tau, nullptr, seg, w_fg, w_bg,
+                       w_nce, fg, fg_bf16, inv_fg, bg, inv_bg, fgbg_out4, aux, lse, nce, tgt_logit, total, work, counter, stream);
+}
+
+extern "C" int cor_step_tail_fwd_ls(const float* part, int nsplit, long long split_stride, int Rp, int B, int M, int C, float p_total,
+                                    const float* stats, const void* queries_bf16, const float* comb, const long long* targets,
+                                    const float* logit_scale, const float* seg, float w_fg, float w_bg, float w_nce, float* fg, void* fg_bf16,
+                                    float* inv_fg, float* bg, float* inv_bg, float* fgbg_out4, float* aux, float* lse, float* nce,
+                                    float* tgt_logit, float* total, void* work, unsigned* counter, cor_stream_t stream) {
+  COR_REQUIRE(logit_scale, "cor_step_tail_fwd_ls: null logit_scale");
+  return step_tail_fwd(part, nsplit, split_stride, Rp, B, M, C, p_total, stats, queries_bf16, comb, targets, 0.f, logit_scale, seg, w_fg,
+                       w_bg, w_nce, fg, fg_bf16, inv_fg, bg, inv_bg, fgbg_out4, aux, lse, nce, tgt_logit, total, work, counter, stream);
+}
+
+static int step_tail_bwd(const void* regions_bf16, const void* queries_bf16, const long long* targets, const float* lse, int B, int M,
+                         int C, float inv_tau, const float* scale, const float* g_loss, float w_nce, const float* fg, const float* inv_fg,
+                         const float* stats, const float* comb, const float* fgbg_out4, const float* aux, float w_fg, float w_bg,
+                         void* a16, int Kp, float* g_queries, float* g_scale, void* work, unsigned* counter, cor_stream_t stream) {
   int rc = tail_shape_ok(B, M, C, "cor_step_tail_bwd");
   if (rc) return rc;
   COR_REQUIRE(regions_bf16 && queries_bf16 && targets && lse && g_loss && fg && inv_fg && stats && comb && fgbg_out4 && aux,
               "cor_step_tail_bwd: null pointer");
-  COR_REQUIRE(!g_queries || (work && counter), "cor_step_tail_bwd: g_queries needs a work buffer and the counters");
+  COR_REQUIRE(!(g_queries || g_scale) || (work && counter), "cor_step_tail_bwd: g_queries / g_logit_scale need a work buffer and the counters");
   COR_REQUIRE(!a16 || Kp >= M, "cor_step_tail_bwd: Kp=%d < M=%d", Kp, M);
   COR_REQUIRE((((uintptr_t)regions_bf16 | (uintptr_t)queries_bf16 | (uintptr_t)fg | (uintptr_t)comb | (uintptr_t)a16) & 15) == 0,
               "cor_step_tail_bwd: 16-byte alignment required");
-  if (!a16 && !g_queries) return COR_OK;
+  if (!a16 && !g_queries && !g_scale) return COR_OK;
   const int nreg = a16 ? ceil_div((long long)B * M, 8) : 0;
   const int nsq = tail_nsplit_q(B, M);
-  const int grid = nreg + (g_queries ? B * nsq : 0);
-  StepTailBwd a{(const bf16*)regions_bf16, (const bf16*)queries_bf16, targets, lse, B, M, C, inv_tau, g_loss, w_nce, fg, inv_fg, stats,
-                comb, fgbg_out4, aux, w_fg, w_bg, (bf16*)a16, Kp, g_queries, (float*)work, counter, nreg, nsq};
+  const int grid = nreg + (g_queries || g_scale ? B * nsq : 0);
+  // work: qpart [B][nsq][C], then the logit-scale partials lspart [B][nsq] and per-query sums lsq [kQT]
+  float* qpart = (float*)work;
+  float* lspart = qpart ? qpart + (size_t)B * nsq * C : nullptr;
+  float* lsq = lspart ? lspart + (size_t)B * nsq : nullptr;
+  StepTailBwd a{(const bf16*)regions_bf16, (const bf16*)queries_bf16, targets, lse, B, M, C, inv_tau, scale, g_loss, w_nce, fg, inv_fg,
+                stats, comb, fgbg_out4, aux, w_fg, w_bg, (bf16*)a16, Kp, g_queries, g_scale, qpart, lspart, lsq, counter, nreg, nsq};
   step_tail_bwd_kernel<<<grid, 256, (size_t)kQT * C * sizeof(float), as_stream(stream)>>>(a);
   return check_launch("step_tail_bwd_kernel");
+}
+
+extern "C" int cor_step_tail_bwd(const void* regions_bf16, const void* queries_bf16, const long long* targets, const float* lse, int B, int M,
+                                 int C, float inv_tau, const float* g_loss, float w_nce, const float* fg, const float* inv_fg,
+                                 const float* stats, const float* comb, const float* fgbg_out4, const float* aux, float w_fg, float w_bg,
+                                 void* a16, int Kp, float* g_queries, void* work, unsigned* counter, cor_stream_t stream) {
+  return step_tail_bwd(regions_bf16, queries_bf16, targets, lse, B, M, C, inv_tau, nullptr, g_loss, w_nce, fg, inv_fg, stats, comb, fgbg_out4,
+                       aux, w_fg, w_bg, a16, Kp, g_queries, nullptr, work, counter, stream);
+}
+
+extern "C" int cor_step_tail_bwd_ls(const void* regions_bf16, const void* queries_bf16, const long long* targets, const float* lse, int B,
+                                    int M, int C, const float* logit_scale, const float* g_loss, float w_nce, const float* fg,
+                                    const float* inv_fg, const float* stats, const float* comb, const float* fgbg_out4, const float* aux,
+                                    float w_fg, float w_bg, void* a16, int Kp, float* g_queries, float* g_logit_scale, void* work,
+                                    unsigned* counter, cor_stream_t stream) {
+  COR_REQUIRE(logit_scale, "cor_step_tail_bwd_ls: null logit_scale");
+  return step_tail_bwd(regions_bf16, queries_bf16, targets, lse, B, M, C, 0.f, logit_scale, g_loss, w_nce, fg, inv_fg, stats, comb,
+                       fgbg_out4, aux, w_fg, w_bg, a16, Kp, g_queries, g_logit_scale, work, counter, stream);
 }

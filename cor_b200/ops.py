@@ -33,6 +33,11 @@ _KERNELS_PER_CALL = {
     "cor_sim_umma_fwd": 2, "cor_infonce_coef": 1, "cor_sim_umma_coef": 1, "cor_infonce_bwd_umma": 3, "cor_gemm_bf16": 1, "cor_cast_cat_bf16": 1, "cor_act_bwd": 2, "cor_ln_rows_fwd": 1, "cor_ln_rows_bwd": 2, "cor_dwconv7_cl": 1, "cor_dwconv7_cl_wgrad": 2,
     "cor_hyper_logits_fwd": 1, "cor_hyper_logits_bwd": 2, "cor_sim_lse_parts": 1, "cor_infonce_tail": 1, "cor_infonce_fwd": 1, "cor_infonce_bwd": 2, "cor_topk": 1, "cor_l2_normalize": 1,
     "cor_val_post": 3, "cor_soft_metrics": 2, "cor_step_tail_fwd": 1, "cor_step_tail_bwd": 1,
+    # device-resident logit scale: the same kernels; the tensor-core backward adds one fold launch when the scale's
+    # gradient is wanted
+    "cor_sim_stream_fwd_ls": 2, "cor_sim_umma_fwd_ls": 2, "cor_sim_lse_parts_ls": 1, "cor_infonce_tail_ls": 1, "cor_infonce_fwd_ls": 1,
+    "cor_infonce_bwd_ls": 2, "cor_infonce_bwd_umma_ls": 4, "cor_step_tail_fwd_ls": 1, "cor_step_tail_bwd_ls": 1,
+    "cor_peer_gather_sim_ls": 1,
 }
 
 
@@ -470,7 +475,25 @@ def _sim_engine(Nq: int, Nr: int, D: int, engine: str) -> str:
     return "stream"
 
 
-def _sim_forward(r16, q16, inv_tau, want_S, want_lse, engine):
+def check_logit_scale(logit_scale: Optional[torch.Tensor], tau: Optional[float], who: str) -> None:
+    """A logit scale replaces ``tau``: a 0-dim fp32 CUDA tensor, never passed together with ``tau``."""
+    if logit_scale is None:
+        return
+    if tau is not None:
+        raise CorError(f"{who}: pass either tau or logit_scale, not both")
+    if not isinstance(logit_scale, torch.Tensor) or logit_scale.dim() != 0 or logit_scale.dtype != torch.float32:
+        raise CorError(f"{who}: logit_scale must be a 0-dim float32 tensor, got "
+                       + (f"shape {tuple(logit_scale.shape)} {logit_scale.dtype}" if isinstance(logit_scale, torch.Tensor) else repr(logit_scale)))
+    if not logit_scale.is_cuda:
+        raise CorError(f"{who}: logit_scale must be a CUDA tensor (the kernels read it from device memory)")
+
+
+def _tau_arg(name: str, inv_tau: float, scale: Optional[torch.Tensor]):
+    """(entry name, argument) of an InfoNCE entry: the float inv_tau, or the ``_ls`` twin that reads the device scale."""
+    return (name, _f(inv_tau)) if scale is None else (name + "_ls", ptr(scale))
+
+
+def _sim_forward(r16, q16, inv_tau, want_S, want_lse, engine, scale=None):
     dev = r16.device
     Nr, D = r16.shape
     Nq = q16.shape[0]
@@ -478,12 +501,12 @@ def _sim_forward(r16, q16, inv_tau, want_S, want_lse, engine):
     S = torch.empty((Nq, Nr), dtype=torch.float32, device=dev) if want_S else None
     lse = torch.empty((Nq,), dtype=torch.float32, device=dev) if want_lse else None
     work = _work(lib.cor_sim_work_bytes(Nq, Nr, D), dev)
-    name = "cor_sim_umma_fwd" if _sim_engine(Nq, Nr, D, engine) == "umma" else "cor_sim_stream_fwd"
-    _call(name, dev, ptr(r16), ptr(q16), Nr, Nq, D, _f(inv_tau), ptr(S), ptr(lse), ptr(work))
+    name, ta = _tau_arg("cor_sim_umma_fwd" if _sim_engine(Nq, Nr, D, engine) == "umma" else "cor_sim_stream_fwd", inv_tau, scale)
+    _call(name, dev, ptr(r16), ptr(q16), Nr, Nq, D, ta, ptr(S), ptr(lse), ptr(work))
     return S, lse
 
 
-def _sim_lse_parts(r16, q16, inv_tau, engine):
+def _sim_lse_parts(r16, q16, inv_tau, engine, scale=None):
     """Similarity producer that leaves its log-sum-exp partials in a work buffer: (work, nparts, qt) for cor_infonce_tail."""
     import ctypes as C
     dev = r16.device
@@ -493,7 +516,8 @@ def _sim_lse_parts(r16, q16, inv_tau, engine):
     work = _work(lib.cor_sim_work_bytes(Nq, Nr, D), dev)
     nparts, qt = C.c_int(0), C.c_int(0)
     eng = 1 if _sim_engine(Nq, Nr, D, engine) == "umma" else 0
-    _call("cor_sim_lse_parts", dev, eng, ptr(r16), ptr(q16), Nr, Nq, D, _f(inv_tau), ptr(work), C.byref(nparts), C.byref(qt))
+    name, ta = _tau_arg("cor_sim_lse_parts", inv_tau, scale)
+    _call(name, dev, eng, ptr(r16), ptr(q16), Nr, Nq, D, ta, ptr(work), C.byref(nparts), C.byref(qt))
     return work, nparts.value, qt.value
 
 
@@ -525,19 +549,21 @@ def _infonce_bwd_dense(Nq: int, Nr: int, D: int, engine: str) -> bool:
 
 class _InfoNCEFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, regions, queries, targets, tau, engine, regions_bf16):
-        dev = require_cuda(regions, queries, targets)
+    def forward(ctx, regions, queries, targets, tau, engine, regions_bf16, logit_scale):
+        dev = require_cuda(regions, queries, targets, logit_scale)
         r16 = regions_bf16.reshape(-1, regions_bf16.shape[-1]).contiguous() if regions_bf16 is not None else _to_bf16_rows(regions)
         q16 = _to_bf16_rows(queries)
         Nr, D = r16.shape
         Nq = q16.shape[0]
         tg = targets.to(torch.int64).contiguous()
-        inv_tau = 1.0 / float(tau)
-        _, lse = _sim_forward(r16, q16, inv_tau, False, True, engine)
+        inv_tau = 1.0 / float(tau) if logit_scale is None else 0.0
+        _, lse = _sim_forward(r16, q16, inv_tau, False, True, engine, logit_scale)
         loss = torch.empty(1, dtype=torch.float32, device=dev)
         tgt = torch.empty((Nq,), dtype=torch.float32, device=dev)
-        _call("cor_infonce_fwd", dev, ptr(r16), ptr(q16), ptr(tg), ptr(lse), Nr, Nq, D, _f(inv_tau), ptr(loss), ptr(tgt))
-        ctx.save_for_backward(r16, q16, tg, lse)
+        name, ta = _tau_arg("cor_infonce_fwd", inv_tau, logit_scale)
+        _call(name, dev, ptr(r16), ptr(q16), ptr(tg), ptr(lse), Nr, Nq, D, ta, ptr(loss), ptr(tgt))
+        # the scale is saved as an input: an in-place write to it before backward trips autograd's version check
+        ctx.save_for_backward(r16, q16, tg, lse, logit_scale)
         ctx.engine = engine
         ctx.cfg = (inv_tau, regions.dtype, queries.dtype, tuple(regions.shape), tuple(queries.shape),
                    regions.requires_grad, queries.requires_grad)
@@ -545,35 +571,44 @@ class _InfoNCEFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, g):
-        r16, q16, tg, lse = ctx.saved_tensors
+        r16, q16, tg, lse, sc = ctx.saved_tensors
         inv_tau, rdt, qdt, rshape, qshape, r_need, q_need = ctx.cfg
+        s_need = sc is not None and ctx.needs_input_grad[6]
         dev = r16.device
         Nr, D = r16.shape
         Nq = q16.shape[0]
         lib = L.load()
         gl = g.reshape(1).float().contiguous()
+        gs = torch.empty((), dtype=torch.float32, device=dev) if s_need else None
+        gs_arg = () if sc is None else (ptr(gs),)
         if _infonce_bwd_dense(Nq, Nr, D, ctx.engine):
             # hundreds of queries: both products on our tensor-core kernel (csrc/nce_bwd_umma.cu) -- the S tile is
             # recomputed, turned into bf16 coefficients in registers and fed straight back as an MMA operand; no S, no P,
-            # no library GEMM
+            # no library GEMM.  The scale's gradient comes out of the dQ launch, which therefore runs whenever it is wanted.
             gq = torch.empty((Nq, D), dtype=torch.float32, device=dev) if q_need else None
             gr = torch.empty((Nr, D), dtype=torch.float32, device=dev) if r_need else None
             work = _work(lib.cor_infonce_bwd_umma_work_bytes(Nq, Nr, D), dev)
-            _call("cor_infonce_bwd_umma", dev, ptr(r16), ptr(q16), Nr, Nq, D, _f(inv_tau), ptr(lse), ptr(tg), ptr(gl), _f(1.0), ptr(gr),
-                  ptr(gq), ptr(work))
+            name, ta = _tau_arg("cor_infonce_bwd_umma", inv_tau, sc)
+            _call(name, dev, ptr(r16), ptr(q16), Nr, Nq, D, ta, ptr(lse), ptr(tg), ptr(gl), _f(1.0), ptr(gr), ptr(gq), *gs_arg, ptr(work))
         else:
             gr = torch.empty((Nr, D), dtype=torch.float32, device=dev)
             gq = torch.empty((Nq, D), dtype=torch.float32, device=dev)
             work = _work(lib.cor_sim_work_bytes(Nq, Nr, D), dev)
-            _call("cor_infonce_bwd", dev, ptr(r16), ptr(q16), ptr(tg), ptr(lse), Nr, Nq, D, _f(inv_tau), ptr(gl), _f(1.0), ptr(gr), ptr(gq), ptr(work))
-        return (gr.view(rshape).to(rdt) if r_need else None), (gq.view(qshape).to(qdt) if q_need else None), None, None, None, None
+            name, ta = _tau_arg("cor_infonce_bwd", inv_tau, sc)
+            _call(name, dev, ptr(r16), ptr(q16), ptr(tg), ptr(lse), Nr, Nq, D, ta, ptr(gl), _f(1.0), ptr(gr), ptr(gq), *gs_arg, ptr(work))
+        return ((gr.view(rshape).to(rdt) if r_need else None), (gq.view(qshape).to(qdt) if q_need else None), None, None, None, None, gs)
 
 
-def infonce_loss(regions: torch.Tensor, queries: torch.Tensor, targets: torch.Tensor, tau: float = 0.07, engine: str = "auto",
-                 regions_bf16: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """mean_q CE(S[q,:]/tau, targets[q]) with S = queries @ regions^T (bf16 operands, fp32 accumulate).
-    Gradients flow straight through the bf16 rounding to ``regions`` and ``queries``."""
-    return _InfoNCEFn.apply(regions, queries, targets, float(tau), engine, regions_bf16)
+def infonce_loss(regions: torch.Tensor, queries: torch.Tensor, targets: torch.Tensor, tau: Optional[float] = None, engine: str = "auto",
+                 regions_bf16: Optional[torch.Tensor] = None, logit_scale: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """mean_q CE(s * S[q,:], targets[q]) with S = queries @ regions^T (bf16 operands, fp32 accumulate) and s = 1/tau
+    (tau defaults to 0.07).  Gradients flow straight through the bf16 rounding to ``regions`` and ``queries``.
+
+    ``logit_scale``: a learnable temperature -- a 0-dim float32 CUDA tensor s > 0 used in place of 1/tau (pass one or
+    the other).  The kernels read it from device memory, and when it requires grad d loss / d s reaches it through
+    autograd, e.g. ``logit_scale = log_s.exp()`` with a parameter ``log_s`` as in CLIP."""
+    check_logit_scale(logit_scale, tau, "infonce_loss")
+    return _InfoNCEFn.apply(regions, queries, targets, 0.07 if tau is None else float(tau), engine, regions_bf16, logit_scale)
 
 
 def topk_retrieve(regions: torch.Tensor, queries: torch.Tensor, k: int, engine: str = "auto"):

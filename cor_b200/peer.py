@@ -145,16 +145,18 @@ class PeerExchange:
         self._last = 0
         return out
 
-    def gather_sim(self, out: torch.Tensor, q16: torch.Tensor, inv_tau: float):
+    def gather_sim(self, out: torch.Tensor, q16: torch.Tensor, inv_tau: float, logit_scale: Optional[torch.Tensor] = None):
         """Fused all-gather + similarity (csrc/peer.cu, peer_gather_sim_kernel): fills ``out`` [world*n_local, C] bf16 like
         :meth:`gather` AND scores every row against this rank's queries ``q16`` [Nq <= 16, C] bf16 while it is in registers.
+        ``logit_scale`` (0-dim f32 on the device) replaces ``inv_tau`` when given.
         Returns ``(work, nparts, qt)`` -- the log-sum-exp partials for ``cor_infonce_tail``."""
         import ctypes as C_
         from . import ops
         work = ops._work(self.lib.cor_peer_gather_sim_work_bytes(), self.device)
         nparts = C_.c_int(0)
-        ops._call("cor_peer_gather_sim", self.device, ops.ptr(self.pub_ptrs), ops.ptr(out), ops._ll(self.n_local), self.C, ops.ptr(q16),
-                  int(q16.shape[0]), ops._f(inv_tau), ops.ptr(work), C_.byref(nparts), ops.ptr(self.flag_ptrs), ops.ptr(self.state),
+        name, ta = ops._tau_arg("cor_peer_gather_sim", inv_tau, logit_scale)
+        ops._call(name, self.device, ops.ptr(self.pub_ptrs), ops.ptr(out), ops._ll(self.n_local), self.C, ops.ptr(q16),
+                  int(q16.shape[0]), ta, ops.ptr(work), C_.byref(nparts), ops.ptr(self.flag_ptrs), ops.ptr(self.state),
                   self.rank, self.world, 0)
         self._last = 0
         return work, nparts.value, 16

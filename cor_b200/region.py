@@ -34,11 +34,15 @@ def region_query_similarity(regions: torch.Tensor, queries: torch.Tensor, engine
     return ops.similarity(regions, queries, engine)
 
 
-def region_infonce_loss(regions: torch.Tensor, queries: torch.Tensor, targets: torch.Tensor, tau: float = 0.07,
-                        gather: bool = True, engine: str = "auto", regions_bf16: Optional[torch.Tensor] = None) -> torch.Tensor:
+def region_infonce_loss(regions: torch.Tensor, queries: torch.Tensor, targets: torch.Tensor, tau: Optional[float] = None,
+                        gather: bool = True, engine: str = "auto", regions_bf16: Optional[torch.Tensor] = None,
+                        logit_scale: Optional[torch.Tensor] = None) -> torch.Tensor:
     """InfoNCE of each local query against ALL regions.  With ``gather`` (and an initialised process
     group) the region rows are all-gathered across ranks first and ``targets`` -- indices into the
-    LOCAL region rows -- are offset by rank * n_local.  tau is a build choice (the reference defines none)."""
+    LOCAL region rows -- are offset by rank * n_local.  tau (default 0.07) is a build choice (the reference defines
+    none); ``logit_scale`` replaces 1/tau with a device tensor that can be learned (see ``ops.infonce_loss``).  Each
+    rank's loss is the mean over its own queries, so the scale's gradient is rank-local, like the queries'."""
+    ops.check_logit_scale(logit_scale, tau, "region_infonce_loss")
     regions = regions.reshape(-1, regions.shape[-1])
     rank, ws = cdist.world()
     if gather and ws > 1:
@@ -46,12 +50,13 @@ def region_infonce_loss(regions: torch.Tensor, queries: torch.Tensor, targets: t
         regions = cdist.all_gather_rows(regions)
         targets = targets + rank * n_local
         regions_bf16 = None
-    return ops.infonce_loss(regions, queries.reshape(-1, queries.shape[-1]), targets, tau, engine, regions_bf16)
+    return ops.infonce_loss(regions, queries.reshape(-1, queries.shape[-1]), targets, tau, engine, regions_bf16, logit_scale)
 
 
 def topk_regions(regions: torch.Tensor, queries: torch.Tensor, k: int, sharded: bool = False, engine: str = "auto"):
     """Top-k regions per query, total order (score desc, index asc).  With ``sharded`` each rank holds
-    a contiguous, equal shard of the gallery: local top-k, all-gather of k*(score,idx), k-way merge."""
+    a contiguous, equal shard of the gallery: local top-k, all-gather of k*(score,idx), k-way merge.
+    Takes no temperature or logit scale: a positive scale does not change the ranking."""
     idx, score = ops.topk_retrieve(regions, queries, min(k, regions.shape[0]), engine)
     rank, ws = cdist.world()
     if sharded and ws > 1:
@@ -147,10 +152,12 @@ class _FusedStepFn(torch.autograd.Function):
     pooling engine applies; the modular ops remain the general path."""
 
     @staticmethod
-    def forward(ctx, pred, emb, comb, masks, tau, nce_weight, gather, sim_engine, bg_mode, w_fg, w_bg):
+    def forward(ctx, pred, emb, comb, masks, tau, nce_weight, gather, sim_engine, bg_mode, w_fg, w_bg, logit_scale):
         from . import _lib as L
         ptr, _f, _ll, call = ops.ptr, ops._f, ops._ll, ops._call
-        dev = L.require_cuda(pred, emb, comb, masks)
+        dev = L.require_cuda(pred, emb, comb, masks, logit_scale)
+        sc = logit_scale                       # device logit scale (replaces 1/tau in every InfoNCE launch) or None
+        tau_arg = lambda name, inv_tau: ops._tau_arg(name, inv_tau, sc)
         lib = L.load()
         B, M = masks.shape[:2]
         Cc, h, w = emb.shape[1:]
@@ -236,8 +243,9 @@ class _FusedStepFn(torch.autograd.Function):
             work = ops._work(lib.cor_step_tail_work_bytes(B, M, Cc), dev)
             if side is not None:
                 cur.wait_stream(side)        # join: the total needs the segmentation loss, the scores the bf16 queries
-            call("cor_step_tail_fwd", dev, ptr(part), ks, _ll(B * Rp * Cc), Rp, B, M, Cc, _f(float(P)), ptr(stats), ptr(q16), ptr(comb_c),
-                 ptr(targets), _f(inv_tau), ptr(out8), _f(w_fg), _f(w_bg), _f(nce_weight), ptr(fg), ptr(fg16), ptr(inv_fg), ptr(bg),
+            name, ta = tau_arg("cor_step_tail_fwd", inv_tau)
+            call(name, dev, ptr(part), ks, _ll(B * Rp * Cc), Rp, B, M, Cc, _f(float(P)), ptr(stats), ptr(q16), ptr(comb_c),
+                 ptr(targets), ta, ptr(out8), _f(w_fg), _f(w_bg), _f(nce_weight), ptr(fg), ptr(fg16), ptr(inv_fg), ptr(bg),
                  ptr(inv_bg), ptr(out4), ptr(aux), ptr(lse), ptr(nce), ptr(tgt), ptr(loss), ptr(work), ptr(ctx.tail))
         else:
             fg = torch.empty((B * M, Cc), **f32)
@@ -277,7 +285,7 @@ class _FusedStepFn(torch.autograd.Function):
                 if px is not None and not local_bwd and _peer_fused_ok(B, Cc, ws * n_local, sim_engine):
                     # ONE kernel: pull the peers' rows over NVLink, keep a local copy for the backward, and score every row
                     # against this rank's queries while it is in registers (all-gather fused with its consumer)
-                    fused_parts = px.gather_sim(r16, q16, inv_tau)
+                    fused_parts = px.gather_sim(r16, q16, inv_tau, sc)
                 elif px is not None:
                     px.gather(r16)               # our own pull-over-NVLink kernel: no NCCL on the data path
                 else:
@@ -289,7 +297,7 @@ class _FusedStepFn(torch.autograd.Function):
                     # log-sum-exp of the remote queries too, so the backward needs no collective at all.
                     q_all = torch.empty((ws * B, Cc), dtype=torch.bfloat16, device=dev)
                     torch.distributed.all_gather_into_tensor(q_all, q16)
-                    _, lse_all = ops._sim_forward(r16, q_all, inv_tau, False, True, sim_engine)
+                    _, lse_all = ops._sim_forward(r16, q_all, inv_tau, False, True, sim_engine, sc)
                     lse = lse_all[rank * B:(rank + 1) * B]
                     ar = torch.arange(ws * B, device=dev, dtype=torch.int64)
                     tgt_all = (ar // B) * n_local + (ar % B) * M - offset       # target rows local to THIS rank
@@ -307,19 +315,22 @@ class _FusedStepFn(torch.autograd.Function):
             if lse is None:
                 # similarity with its log-sum-exp partials left in the work buffer, then ONE tail kernel: partial merge ->
                 # lse, target logits, InfoNCE mean and the step's total loss
-                sim_work, nparts, qt = fused_parts if fused_parts is not None else ops._sim_lse_parts(r16, q16, inv_tau, sim_engine)
+                sim_work, nparts, qt = fused_parts if fused_parts is not None else ops._sim_lse_parts(r16, q16, inv_tau, sim_engine, sc)
                 lse = torch.empty((B,), **f32)
                 if side is not None:
                     cur.wait_stream(side)        # join: the total needs the segmentation and fg/bg losses
-                call("cor_infonce_tail", dev, ptr(sim_work), nparts, qt, ptr(r16), ptr(q16), ptr(targets), r16.shape[0], B, Cc, _f(inv_tau),
+                name, ta = tau_arg("cor_infonce_tail", inv_tau)
+                call(name, dev, ptr(sim_work), nparts, qt, ptr(r16), ptr(q16), ptr(targets), r16.shape[0], B, Cc, ta,
                      ptr(lse), ptr(nce), ptr(tgt), ptr(out8), ptr(out4), _f(w_fg), _f(w_bg), _f(nce_weight), ptr(loss))
             else:
-                call("cor_infonce_fwd", dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), r16.shape[0], B, Cc, _f(inv_tau), ptr(nce), ptr(tgt))
+                name, ta = tau_arg("cor_infonce_fwd", inv_tau)
+                call(name, dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), r16.shape[0], B, Cc, ta, ptr(nce), ptr(tgt))
                 if side is not None:
                     cur.wait_stream(side)        # join: the combine needs the segmentation loss
                 call("cor_step_combine", dev, ptr(out8), ptr(out4), ptr(nce), _f(w_fg), _f(w_bg), _f(nce_weight), ptr(loss))
+        # the scale is saved as an input: an in-place write to it before backward trips autograd's version check
         ctx.save_for_backward(pred_c, t_save, w_save, per, fg, bg, inv_fg, inv_bg, comb_c, stats, out4, aux, r16, q16, targets, lse, w32,
-                              fg16, q_all, lse_all, tgt_all)
+                              fg16, q_all, lse_all, tgt_all, sc)
         ctx.cfg = (B, M, Cc, h, w, float(inv_tau), float(nce_weight), int(bg_mode), float(w_fg), float(w_bg), ws, offset, n_local,
                    pred.dtype, emb.dtype, comb.dtype, tuple(comb.shape), need_pred, need_emb, comb.requires_grad)
         ctx.px = px
@@ -333,7 +344,7 @@ class _FusedStepFn(torch.autograd.Function):
         from . import _lib as L
         ptr, _f, _ll, call = ops.ptr, ops._f, ops._ll, ops._call
         (pred_c, t_save, w_save, per, fg, bg, inv_fg, inv_bg, comb_c, stats, out4, aux, r16, q16, targets, lse, w32,
-         fg16, q_all, lse_all, tgt_all) = ctx.saved_tensors
+         fg16, q_all, lse_all, tgt_all, sc) = ctx.saved_tensors
         (B, M, Cc, h, w, inv_tau, nce_weight, bg_mode, w_fg, w_bg, ws, offset, n_local, pred_dt, emb_dt, comb_dt, comb_shape,
          need_pred, need_emb, need_comb) = ctx.cfg
         dev = fg.device
@@ -341,9 +352,15 @@ class _FusedStepFn(torch.autograd.Function):
         P = h * w
         f32 = dict(dtype=torch.float32, device=dev)
         if g_loss is None:
-            return (None,) * 11
+            return (None,) * 12
         g = g_loss.reshape(1).float().contiguous()
         g_pred = g_emb = g_comb = None
+        need_scale = sc is not None and ctx.needs_input_grad[11]
+        # d loss / d scale: written by the InfoNCE backward over THIS rank's queries (the launch that writes g_queries)
+        g_scale = torch.empty((), **f32) if need_scale else None
+        tau_arg = lambda name: ops._tau_arg(name, inv_tau, sc)
+        gs_arg = () if sc is None else (ptr(g_scale),)          # the _ls backward entries take the gradient pointer
+        gs_none = () if sc is None else (None,)
         cur = torch.cuda.current_stream(dev)
         side = _side_stream(dev) if (_overlap_enabled() and need_pred) else None
 
@@ -383,9 +400,10 @@ class _FusedStepFn(torch.autograd.Function):
             a16 = torch.empty((B * Kp, Cc), dtype=torch.bfloat16, device=dev) if need_emb else None
             g_q = torch.empty((B, Cc), **f32) if need_comb else None
             work = ops._work(lib.cor_step_tail_work_bytes(B, M, Cc), dev)
-            call("cor_step_tail_bwd", dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), B, M, Cc, _f(inv_tau), ptr(g), _f(nce_weight),
+            name, ta = tau_arg("cor_step_tail_bwd")
+            call(name, dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), B, M, Cc, ta, ptr(g), _f(nce_weight),
                  ptr(fg), ptr(inv_fg), ptr(stats), ptr(comb_c), ptr(out4), ptr(aux), _f(w_fg), _f(w_bg), ptr(a16), Kp, ptr(g_q),
-                 ptr(work), ptr(ctx.tail))
+                 *gs_arg, ptr(work), ptr(ctx.tail))
             if need_comb:
                 g_comb = g_q.view(comb_shape).to(comb_dt)
             if need_emb:
@@ -403,16 +421,18 @@ class _FusedStepFn(torch.autograd.Function):
             if ws > 1 and q_all is not None:
                 # (all regions, my queries) -> g_queries ; (my regions, ALL queries) -> g_regions.  Every rank's loss is the
                 # mean over its own B queries, so the sum over ranks of d loss_j / d my_regions carries the factor ws.
-                call("cor_infonce_bwd", dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), Nr, B, Cc, _f(inv_tau), ptr(g), _f(nce_weight), None,
-                     ptr(g_q), ptr(work))
-                call("cor_infonce_bwd", dev, ptr(fg16), ptr(q_all), ptr(tgt_all), ptr(lse_all), n_local, ws * B, Cc, _f(inv_tau), ptr(g),
-                     _f(float(ws) * nce_weight), ptr(g_regions), None, None)
+                name, ta = tau_arg("cor_infonce_bwd")
+                call(name, dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), Nr, B, Cc, ta, ptr(g), _f(nce_weight), None,
+                     ptr(g_q), *gs_arg, ptr(work))
+                call(name, dev, ptr(fg16), ptr(q_all), ptr(tgt_all), ptr(lse_all), n_local, ws * B, Cc, ta, ptr(g),
+                     _f(float(ws) * nce_weight), ptr(g_regions), None, *gs_none, None)
             elif ws > 1:
                 if ev_px is not None:
                     cur.wait_event(ev_px)
                 g_all = px.gall if px is not None else torch.empty((Nr, Cc), **f32)
-                call("cor_infonce_bwd", dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), Nr, B, Cc, _f(inv_tau), ptr(g), _f(nce_weight),
-                     ptr(g_all), ptr(g_q), ptr(work))
+                name, ta = tau_arg("cor_infonce_bwd")
+                call(name, dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), Nr, B, Cc, ta, ptr(g), _f(nce_weight),
+                     ptr(g_all), ptr(g_q), *gs_arg, ptr(work))
                 if px is not None:
                     px.signal(1)
                     if side is None:
@@ -421,8 +441,9 @@ class _FusedStepFn(torch.autograd.Function):
                 else:
                     torch.distributed.reduce_scatter_tensor(g_regions, g_all, op=torch.distributed.ReduceOp.SUM)
             else:
-                call("cor_infonce_bwd", dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), Nr, B, Cc, _f(inv_tau), ptr(g), _f(nce_weight),
-                     ptr(g_regions), ptr(g_q), ptr(work))
+                name, ta = tau_arg("cor_infonce_bwd")
+                call(name, dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), Nr, B, Cc, ta, ptr(g), _f(nce_weight),
+                     ptr(g_regions), ptr(g_q), *gs_arg, ptr(work))
             # ... then the fg/bg backward ADDS its GT-row gradients into g_regions (row b*M) and g_queries
             g_bg = torch.empty((B, Cc), **f32) if bg_mode == 1 else None
             call("cor_fgbg_loss_bwd", dev, ptr(fg), _ll(M * Cc), ptr(bg), _ll(Cc), ptr(comb_c), _ll(Cc), B, Cc, bg_mode, ptr(out4), ptr(aux),
@@ -462,7 +483,7 @@ class _FusedStepFn(torch.autograd.Function):
             cur.wait_stream(side)
         if g_pred is not None:
             g_pred = g_pred.to(pred_dt)
-        return g_pred, g_emb, g_comb, None, None, None, None, None, None, None, None
+        return g_pred, g_emb, g_comb, None, None, None, None, None, None, None, None, g_scale
 
 
 def _fused_ok(emb, masks, pool_engine):
@@ -471,9 +492,9 @@ def _fused_ok(emb, masks, pool_engine):
     return pool_engine in ("auto", "umma") and ops.umma_pool_eligible(emb, M, P, ops.W_CLAMP, 1, True) and emb.shape[1] % 8 == 0
 
 
-def region_step(pred: torch.Tensor, emb: torch.Tensor, comb: torch.Tensor, masks: torch.Tensor, *, tau: float = 0.07,
+def region_step(pred: torch.Tensor, emb: torch.Tensor, comb: torch.Tensor, masks: torch.Tensor, *, tau: Optional[float] = None,
                 nce_weight: float = 1.0, gather: bool = True, pool_engine: str = "auto", sim_engine: str = "auto",
-                bg_mode: int = 0, fused: bool = True) -> RegionStepOut:
+                bg_mode: int = 0, fused: bool = True, logit_scale: Optional[torch.Tensor] = None) -> RegionStepOut:
     """One forward of the whole region path for a batch of triplets with M candidate masks each
     (mask 0 of every image is the ground-truth ``query_mask``):
 
@@ -482,10 +503,17 @@ def region_step(pred: torch.Tensor, emb: torch.Tensor, comb: torch.Tensor, masks
         nce  = InfoNCE(comb_b vs all B*M (x world) pooled regions, target = region (b,0))   [Class N]
         loss = seg + 5 fg + 5 bg + nce_weight * nce
 
+    The InfoNCE logits are S / tau (tau defaults to 0.07), or ``logit_scale * S`` for a learnable temperature:
+    ``logit_scale`` is a 0-dim float32 tensor s > 0 on the step's device, passed instead of ``tau``.  The kernels read
+    it from device memory, and d loss / d s reaches it through autograd when it requires grad.
+
     ONE pass over the masks and ONE pass over the feature map serve fg, bg and all M regions.  With bf16
     features and >= 16 masks the step runs as a single fused autograd node (tensor-core pooling, hand
     written backward); other shapes compose the modular ops.
     """
+    ops.check_logit_scale(logit_scale, tau, "region_step")
+    if logit_scale is not None and logit_scale.device != emb.device:
+        raise CorError(f"region_step: logit_scale is on {logit_scale.device}, the step on {emb.device}")
     B, M = masks.shape[:2]
     if comb.shape[0] != B or emb.shape[0] != B or pred.shape[0] != B:
         raise CorError("region_step: batch sizes differ")
@@ -493,8 +521,8 @@ def region_step(pred: torch.Tensor, emb: torch.Tensor, comb: torch.Tensor, masks
         raise CorError(f"region_step: comb {tuple(comb.shape)} must hold one row of C={emb.shape[1]} channels per triplet "
                        "(the kernels read the queries with the feature map's row width)")
     if fused and _fused_ok(emb, masks, pool_engine) and pred.dim() == 4 and pred.shape[1] == 1:
-        loss, out8, out4, nce, fg = _FusedStepFn.apply(pred, emb, comb, masks, float(tau), float(nce_weight), bool(gather), sim_engine,
-                                                       int(bg_mode), 5.0, 5.0)
+        loss, out8, out4, nce, fg = _FusedStepFn.apply(pred, emb, comb, masks, 0.07 if tau is None else float(tau), float(nce_weight),
+                                                       bool(gather), sim_engine, int(bg_mode), 5.0, 5.0, logit_scale)
         return RegionStepOut(loss=loss, seg=out8[0], fg=out4[0], bg=out4[1], nce=nce[0], regions=fg.view(B, M, -1))
     pool = ops.region_pool(emb, masks, transform=ops.W_CLAMP, normalize=True, pair=True, engine=pool_engine, want_bf16=True)
     Cc = pool.fg.shape[-1]
@@ -503,7 +531,7 @@ def region_step(pred: torch.Tensor, emb: torch.Tensor, comb: torch.Tensor, masks
     losses, _ = ops.fgbg_losses(pool.fg[:, 0, :], pool.bg[:, 0, :], q, pool.stats.view(B, M, 4)[:, 0, :], bg_mode)
     seg = ops.seg_loss(pred, masks[:, 0:1])
     nce = region_infonce_loss(pool.fg.reshape(B * M, Cc), q, gt_rows, tau, gather, sim_engine,
-                              regions_bf16=pool.fg_bf16)
+                              regions_bf16=pool.fg_bf16, logit_scale=logit_scale)
     loss = seg + 5 * losses[0] + 5 * losses[1] + nce_weight * nce
     return RegionStepOut(loss=loss, seg=seg, fg=losses[0], bg=losses[1], nce=nce, regions=pool.fg.detach())
 
@@ -516,7 +544,11 @@ class StepBuffers:
 
     ``capture()`` records forward + backward of the step ONCE into a CUDA graph over these static
     buffers (launch-bound inner loop: ~30 small kernels); afterwards ``run`` / ``replay`` re-issue
-    the whole step with a single graph launch.  Gradients land in ``self.grads``."""
+    the whole step with a single graph launch.  Gradients land in ``self.grads``.
+
+    ``capture(logit_scale=s)`` (s a 0-dim float32 tensor on the device) learns the temperature: the graph reads ``s``
+    from device memory at every replay, so a value written into it (``s.copy_(log_s.exp())``) takes effect without a
+    recapture, and d loss / d s lands in ``self.grads["logit_scale"]``, overwritten by every replay."""
 
     def __init__(self, B, M, C=256, h=64, w=64, H=1024, W=1024, hp=256, wp=256, D=None, device="cuda",
                  emb_dtype=torch.bfloat16, mask_dtype=torch.float32):
@@ -547,10 +579,16 @@ class StepBuffers:
         pred = self.d["pred"].detach().requires_grad_(backward)
         comb = self.d["comb"].detach().requires_grad_(backward)
         emb = self.d["emb"].detach().requires_grad_(backward and emb_grad)
-        out = region_step(pred, emb, comb, self.d["masks"], **kw)
+        kw = dict(kw)
+        scale = kw.pop("logit_scale", None)
+        if scale is not None:
+            scale = scale.detach().requires_grad_(backward)      # a leaf over the caller's storage: read in place
+        out = region_step(pred, emb, comb, self.d["masks"], logit_scale=scale, **kw)
         if backward:
             out.loss.backward(gradient=self._seed)      # a resident 1.0: no per-step fill kernel from autograd
         grads = {"pred": pred.grad, "comb": comb.grad, "emb": emb.grad}
+        if scale is not None:
+            grads["logit_scale"] = scale.grad
         return out.loss.detach(), grads
 
     def capture(self, backward: bool = True, emb_grad: bool = True, warmup: int = 3, **kw):

@@ -172,6 +172,20 @@ int cor_step_tail_bwd(const void* regions_bf16, const void* queries_bf16, const 
                       int C, float inv_tau, const float* g_loss, float w_nce, const float* fg, const float* inv_fg,
                       const float* stats, const float* comb, const float* fgbg_out4, const float* aux, float w_fg, float w_bg,
                       void* a16, int Kp, float* g_queries, void* work, unsigned* counter, cor_stream_t stream);
+/* Extend cor_step_tail_fwd / _bwd: the logit scale s = 1/tau is read from device memory (logit_scale, one f32; a CUDA
+ * graph that captured the call picks up a new value at every replay).  _bwd also writes d total / d s to g_logit_scale
+ * (one f32; NULL = not wanted): w_nce * g_loss[0] * mean_q sum_r (softmax(s S_q)_r - [r == t(q)]) S_qr, folded in a fixed
+ * order by the dQ CTAs (which then run even when g_queries is NULL). */
+int cor_step_tail_fwd_ls(const float* part, int nsplit, long long split_stride, int Rp, int B, int M, int C, float p_total,
+                         const float* stats, const void* queries_bf16, const float* comb, const long long* targets,
+                         const float* logit_scale, const float* seg, float w_fg, float w_bg, float w_nce, float* fg, void* fg_bf16,
+                         float* inv_fg, float* bg, float* inv_bg, float* fgbg_out4, float* aux, float* lse, float* nce,
+                         float* tgt_logit, float* total, void* work, unsigned* counter, cor_stream_t stream);
+int cor_step_tail_bwd_ls(const void* regions_bf16, const void* queries_bf16, const long long* targets, const float* lse, int B,
+                         int M, int C, const float* logit_scale, const float* g_loss, float w_nce, const float* fg,
+                         const float* inv_fg, const float* stats, const float* comb, const float* fgbg_out4, const float* aux,
+                         float w_fg, float w_bg, void* a16, int Kp, float* g_queries, float* g_logit_scale, void* work,
+                         unsigned* counter, cor_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
  * Segmentation loss (loss_func.py:5-32) with the target resample of trainer_v3_g.py:67 fused in.
@@ -256,6 +270,40 @@ size_t cor_infonce_bwd_umma_work_bytes(int Nq, int Nr, int D);
 int cor_infonce_bwd_umma(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, const float* lse,
                          const long long* targets, const float* g_loss, float g_mul, float* g_regions, float* g_queries,
                          void* work, cor_stream_t stream);
+
+/* Learnable temperature: the entries above with the logit scale s (= 1/tau) read from device memory instead of the
+ * float inv_tau.  logit_scale: one f32 on the device, positive; read once per CTA when the kernel runs, so a captured
+ * CUDA graph picks up a new value at every replay.  S, lse and every coefficient are those of the float entries at
+ * inv_tau = *logit_scale (bit-equal for the same f32 value).  Same arguments otherwise, same kernels, same launches.
+ * The backward entries also write g_logit_scale (one f32 on the device; NULL = not wanted):
+ *   d loss / d s = g_loss[0] * g_mul * mean_q sum_r (exp(s S[q,r] - lse[q]) - [r == target(q)]) S[q,r]
+ * from per-query partials folded in a fixed order (no float atomics, no host synchronisation: deterministic and
+ * graph-capturable).  The legacy coefficient entries cor_infonce_coef and cor_sim_umma_coef stay float-only.
+ *   cor_sim_stream_fwd_ls, cor_sim_umma_fwd_ls, cor_sim_lse_parts_ls, cor_infonce_tail_ls, cor_infonce_fwd_ls: as the
+ *     entries without the suffix.
+ *   cor_infonce_bwd_ls: extends cor_infonce_bwd.  The gradient comes from the (regions, queries) pair of the call, so a
+ *     data-parallel rank asks for it on its (all regions, its queries) call; g_logit_scale needs `work`.
+ *   cor_infonce_bwd_umma_ls: extends cor_infonce_bwd_umma.  The dQ launch forms the partials; with g_logit_scale but
+ *     no g_queries it still runs (the whole dQ GEMM, result not stored), plus one single-CTA fold launch.
+ * ---------------------------------------------------------------------------------------- */
+int cor_sim_stream_fwd_ls(const void* regions, const void* queries, int Nr, int Nq, int D, const float* logit_scale,
+                          float* S, float* lse, void* work, cor_stream_t stream);
+int cor_sim_umma_fwd_ls(const void* regions, const void* queries, int Nr, int Nq, int D, const float* logit_scale,
+                        float* S, float* lse, void* work, cor_stream_t stream);
+int cor_sim_lse_parts_ls(int engine, const void* regions, const void* queries, int Nr, int Nq, int D, const float* logit_scale,
+                         void* work, int* nparts, int* qt, cor_stream_t stream);
+int cor_infonce_tail_ls(const float* lse_part, int nparts, int qt, const void* regions, const void* queries,
+                        const long long* targets, int Nr, int Nq, int D, const float* logit_scale, float* lse, float* nce,
+                        float* tgt_logit, const float* seg, const float* fgbg, float w_fg, float w_bg, float w_nce,
+                        float* total, cor_stream_t stream);
+int cor_infonce_fwd_ls(const void* regions, const void* queries, const long long* targets, const float* lse,
+                       int Nr, int Nq, int D, const float* logit_scale, float* loss, float* tgt_logit, cor_stream_t stream);
+int cor_infonce_bwd_ls(const void* regions, const void* queries, const long long* targets, const float* lse,
+                       int Nr, int Nq, int D, const float* logit_scale, const float* g_loss, float g_mul, float* g_regions,
+                       float* g_queries, float* g_logit_scale, void* work, cor_stream_t stream);
+int cor_infonce_bwd_umma_ls(const void* regions, const void* queries, int Nr, int Nq, int D, const float* logit_scale,
+                            const float* lse, const long long* targets, const float* g_loss, float g_mul, float* g_regions,
+                            float* g_queries, float* g_logit_scale, void* work, cor_stream_t stream);
 
 /* Top-k retrieval: per query the k best regions under (score desc, index asc), where score is the
  * canonical value fl32(sum in fp64 of exact bf16 products).  S is the (tensor-core) prefilter
@@ -428,6 +476,10 @@ size_t cor_peer_gather_sim_work_bytes(void);
 int cor_peer_gather_sim(const void* const* peer_src, void* all, long long n_local, int D, const void* queries, int Nq, float inv_tau,
                         float* part, int* nparts, void* const* peer_flags, void* state, int rank, int world, int channel,
                         cor_stream_t stream);
+/* Extends cor_peer_gather_sim: the logit scale is read from device memory (logit_scale, one f32), as the _ls InfoNCE entries. */
+int cor_peer_gather_sim_ls(const void* const* peer_src, void* all, long long n_local, int D, const void* queries, int Nq,
+                           const float* logit_scale, float* part, int* nparts, void* const* peer_flags, void* state, int rank, int world,
+                           int channel, cor_stream_t stream);
 
 #ifdef __cplusplus
 }

@@ -1,6 +1,6 @@
 #!/bin/bash
 # A/B builds of ONE kernel file with other -D knobs, linked against the other (current) objects:
-#   benchmarks/build_variants.sh sim_umma pf0 "-DCOR_SIM_PREFETCH=0"   ->  cor_b200/build/ab/libcor_b200_pf0.so
+#   benchmarks/build_variants.sh sim_umma_ts poly1 "-DCOR_SIM_TS_POLY_OF4=1"   ->  cor_b200/build/ab/libcor_b200_poly1.so
 # Select one at run time with COR_B200_LIB=<path>.  cor_b200/build/ is git-ignored but travels to the GPU box.
 set -e
 ROOT=$(cd "$(dirname "$0")/.." && pwd)

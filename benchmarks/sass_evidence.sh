@@ -1,6 +1,6 @@
 #!/usr/bin/env bash
 # Counts the SASS mnemonics that prove which hardware paths the built objects use (B200_PROFILING.md): tcgen05
-# (UTCHMMA, LDTM, UTCBAR, UTCATOMSWS = tcgen05.alloc), TMA (UTMALDG, .MULTICAST), mbarrier (SYNCS.*), system-scope
+# (UTCHMMA, LDTM, UTCBAR, UTCATOMSWS = tcgen05.alloc), TMA (UTMALDG), mbarrier (SYNCS.*), system-scope
 # peer loads/stores (LDG/STG ...STRONG.SYS), 128-bit streaming loads, dp4a.  Runs on the CPU build host:
 #   python -m cor_b200.build && benchmarks/sass_evidence.sh > profiles/rNN_sass_evidence.txt
 cd "$(dirname "$0")/.." || exit 1

@@ -1,4 +1,4 @@
-"""Hand-off timeline of the similarity kernel's first tiles (debug build with -DCOR_SIM_TRACE, see sim_umma.cu):
+"""Hand-off timeline of the S-store similarity kernel's first tiles (debug build with -DCOR_SIM_TRACE, see sim_umma.cu):
 COR_B200_LIB=cor_b200/build/ab/libcor_b200_trace.so python benchmarks/sim_trace.py [Nq Nr]"""
 import ctypes as C
 import os
@@ -11,7 +11,7 @@ g = torch.Generator(device="cuda").manual_seed(0)
 R = torch.nn.functional.normalize(torch.randn(Nr, 256, device="cuda", generator=g), dim=-1).bfloat16()
 Q = torch.nn.functional.normalize(torch.randn(Nq, 256, device="cuda", generator=g), dim=-1).bfloat16()
 for _ in range(3):
-    ops._sim_lse_parts(R, Q, 1 / 0.07, "umma")
+    ops._sim_forward(R, Q, 1.0, True, False, "umma")
 torch.cuda.synchronize()
 lib = L.load()
 buf = (C.c_longlong * 256)()

@@ -121,7 +121,8 @@ def main():
             t = timeit(lambda: ops.topk_retrieve(R, Q, k), a.iters)
             emit(f"topk_retrieve (sim+select+rerank) Nq256 Nr4096 k{k}", t)
 
-    # ---- InfoNCE forward + backward: dense (tensor-core S + bf16 coefficients + library GEMMs) vs streaming backward
+    # ---- InfoNCE forward + backward: tensor-core backward (nce_bwd_umma: coefficients formed in registers, no S / P written,
+    #      no library GEMM) vs streaming backward
     if want("nce"):
         for (Nq, Nr, D) in [(256, 4096, 256), (1024, 102400, 256)]:
             R = unit(Nr, D, g).requires_grad_(True)

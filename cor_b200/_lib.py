@@ -14,7 +14,7 @@ LIB_PATH = os.path.join(HERE, "libcor_b200.so")
 HEADER = os.path.join(os.path.dirname(HERE), "include", "cor_b200.h")
 
 F32, BF16, U8 = 0, 1, 2
-ABI_VERSION = 2
+ABI_VERSION = 3
 # terms of the segmentation loss (include/cor_b200.h COR_SEG_*)
 ACT_NONE, ACT_RELU, ACT_GELU, ACT_SIGMOID = range(4)
 SEG_WBCE, SEG_WIOU, SEG_DICE, SEG_BCE, SEG_IOU, SEG_WDICE, SEG_FOCAL, SEG_NTERMS = range(8)
@@ -75,7 +75,6 @@ def load(path: str = LIB_PATH):
         _sig(lib, "cor_fgbg_aux_floats", sz, i, i)
         _sig(lib, "cor_fgbg_loss_fwd", i, p, ll, p, ll, p, ll, p, ll, i, i, i, p, p, p)
         _sig(lib, "cor_fgbg_loss_bwd", i, p, ll, p, ll, p, ll, i, i, i, p, p, p, ll, f, f, p, ll, i, p, ll, p, ll, i, p)
-        _sig(lib, "cor_step_combine", i, p, p, p, f, f, f, p, p)
         _sig(lib, "cor_step_tail_counter_words", i)
         _sig(lib, "cor_step_tail_work_bytes", sz, i, i, i)
         _sig(lib, "cor_step_tail_fwd", i, p, i, ll, i, i, i, i, f, p, p, p, p, f, p, f, f, f, p, p, p, p, p, p, p, p, p, p, p, p, p, p)
@@ -91,8 +90,6 @@ def load(path: str = LIB_PATH):
         _sig(lib, "cor_sim_stream_fwd", i, p, p, i, i, i, f, p, p, p, p)
         _sig(lib, "cor_sim_umma_fwd", i, p, p, i, i, i, f, p, p, p, p)
         _sig(lib, "cor_infonce_fwd", i, p, p, p, p, i, i, i, f, p, p, p)
-        _sig(lib, "cor_sim_umma_coef", i, p, p, i, i, i, f, p, p, p, f, p, p)
-        _sig(lib, "cor_infonce_coef", i, p, p, p, i, i, f, p, f, p, p)
         _sig(lib, "cor_sim_lse_parts", i, i, p, p, i, i, i, f, p, C.POINTER(i), C.POINTER(i), p)
         _sig(lib, "cor_infonce_tail", i, p, i, i, p, p, p, i, i, i, f, p, p, p, p, p, f, f, f, p, p)
         _sig(lib, "cor_infonce_bwd", i, p, p, p, p, i, i, i, f, p, f, p, p, p, p)

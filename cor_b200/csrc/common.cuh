@@ -15,8 +15,9 @@ int check_launch(const char* what);   // cudaGetLastError -> COR_ECUDA
 int sm_count();                       // cached multiprocessor count of the current device
 // lse[q] from `nparts` (max,sum) partials laid out [qtile][nparts][qt][2] (sim_stream.cu)
 int launch_lse_combine(const float* part, int Nq, int nparts, int qt, float* lse, cudaStream_t st);
-// tcgen05 similarity producer (sim_umma.cu); nparts/qt non-NULL: leave the LSE partials in `work`, report their layout.
-// Every InfoNCE kernel takes (inv_tau, scale): a non-NULL scale is the device-resident logit scale that replaces inv_tau.
+// tcgen05 similarity producer (sim_umma.cu): S or lse, not both; nparts/qt non-NULL: leave the LSE partials in `work`,
+// report their layout.  Every InfoNCE kernel takes (inv_tau, scale): a non-NULL scale is the device-resident logit scale
+// that replaces inv_tau.
 int sim_umma_launch(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, const float* scale, float* S,
                     float* lse, void* work, int* nparts, int* qt, cudaStream_t st);
 

@@ -139,12 +139,6 @@ __global__ void __launch_bounds__(128) fgbg_bwd_kernel(const float* __restrict__
   }
 }
 
-// loss = seg + w_fg * fg + w_bg * bg + w_nce * nce  (utils/trainer_v3_g.py:67-73 plus the Class-N term)
-__global__ void step_combine_kernel(const float* seg, const float* fgbg, const float* nce, float w_fg, float w_bg, float w_nce,
-                                    float* loss) {
-  loss[0] = seg[0] + w_fg * fgbg[0] + w_bg * fgbg[1] + (nce ? w_nce * nce[0] : 0.f);
-}
-
 }  // namespace cor
 
 using namespace cor;
@@ -173,11 +167,4 @@ extern "C" int cor_fgbg_loss_bwd(const float* fg_rows, long long fg_stride, cons
                                                     aux + (size_t)n * 8, out4, g2, g2_stride, gw_fg, gw_bg, g_fg_rows, gfg_stride, fg_accumulate, g_bg_rows,
                                                     gbg_stride, g_comb, gcomb_stride, comb_accumulate);
   return check_launch("fgbg_bwd_kernel");
-}
-
-extern "C" int cor_step_combine(const float* seg, const float* fgbg, const float* nce, float w_fg, float w_bg, float w_nce, float* loss,
-                                cor_stream_t stream) {
-  COR_REQUIRE(seg && fgbg && loss, "cor_step_combine: null pointer");
-  step_combine_kernel<<<1, 1, 0, as_stream(stream)>>>(seg, fgbg, nce, w_fg, w_bg, w_nce, loss);
-  return check_launch("step_combine_kernel");
 }

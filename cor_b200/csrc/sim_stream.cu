@@ -4,7 +4,7 @@
 // diagonal, F.cosine_similarity at utils/loss_func.py:84,123.  These kernels cover the HBM-bound
 // regime (a handful of queries against many regions, AI ~ Nq flop/B) and the small utility steps
 // (row L2-normalise of lib/support_branch.py:85, target logits, exact top-k re-rank); the
-// tensor-core variant for many queries lives in sim_umma.cu and shares the work-buffer layout.
+// tensor-core variants for many queries live in sim_umma.cu (S) and sim_umma_ts.cu (lse, same work-buffer layout).
 #include "common.cuh"
 
 namespace cor {
@@ -133,7 +133,7 @@ __global__ void __launch_bounds__(1024) infonce_fwd_kernel(const bf16* __restric
 }
 
 // ---- the fused step's tail in ONE launch: merge of the log-sum-exp partials (as sim_lse_combine_kernel), target
-//      logits, mean InfoNCE loss and the step's total loss (as step_combine_kernel).  One CTA, one warp per query.
+//      logits, mean InfoNCE loss and the step's total loss (seg + w_fg fg + w_bg bg + w_nce nce).  One CTA, one warp per query.
 __global__ void __launch_bounds__(1024) infonce_tail_kernel(const float* __restrict__ part, int nparts, int qt,
                                                             const bf16* __restrict__ regions, const bf16* __restrict__ queries,
                                                             const long long* __restrict__ targets, int Nr, int Nq, int D, float inv_tau,
@@ -176,41 +176,6 @@ __global__ void __launch_bounds__(1024) infonce_tail_kernel(const float* __restr
     const float v = (float)(acc[0] / (double)Nq);
     nce[0] = v;
     if (total) total[0] = seg[0] + w_fg * fgbg[0] + w_bg * fgbg[1] + w_nce * v;
-  }
-}
-
-// ---- InfoNCE backward, many-query regime: the coefficient matrix in bf16 for two plain GEMMs ------------------------
-//   P[q,r] = (exp(S[q,r]/tau - lse[q]) - [r == t(q)]) * g * g_mul / (tau * Nq)      (S = raw dot products, f32)
-// dQ = P R and dR = P^T Q are then library GEMMs (cuBLAS through torch.mm, fp32 output): with hundreds of queries the
-// backward is 4*Nq*Nr*D flops of dense GEMM, which the per-row streaming kernel above cannot feed.
-__global__ void __launch_bounds__(256) infonce_coef_kernel(const float* __restrict__ S, const float* __restrict__ lse,
-                                                           const long long* __restrict__ targets, int Nq, long long Nr, float inv_tau,
-                                                           const float* __restrict__ g_loss, float g_mul, bf16* __restrict__ P) {
-  const int q = blockIdx.y;
-  const float l = lse[q];
-  const long long t = targets[q];
-  const float gscale = g_loss[0] * g_mul * inv_tau / (float)Nq;
-  const float* s = S + (long long)q * Nr;
-  bf16* p = P + (long long)q * Nr;
-  const long long nvec = Nr / 4;
-  const bool aligned = (Nr % 4 == 0);
-  if (aligned) {
-    for (long long v = (long long)blockIdx.x * blockDim.x + threadIdx.x; v < nvec; v += (long long)gridDim.x * blockDim.x) {
-      const float4 x = *reinterpret_cast<const float4*>(s + 4 * v);
-      float c[4] = {__expf(x.x * inv_tau - l), __expf(x.y * inv_tau - l), __expf(x.z * inv_tau - l), __expf(x.w * inv_tau - l)};
-      if (t >= 4 * v && t < 4 * v + 4) c[t - 4 * v] -= 1.f;
-      uint2 o;
-      __nv_bfloat162 lo = __floats2bfloat162_rn(c[0] * gscale, c[1] * gscale), hi = __floats2bfloat162_rn(c[2] * gscale, c[3] * gscale);
-      o.x = *reinterpret_cast<uint32_t*>(&lo);
-      o.y = *reinterpret_cast<uint32_t*>(&hi);
-      *reinterpret_cast<uint2*>(p + 4 * v) = o;
-    }
-  } else {
-    for (long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x; r < Nr; r += (long long)gridDim.x * blockDim.x) {
-      float c = __expf(s[r] * inv_tau - l);
-      if (r == t) c -= 1.f;
-      p[r] = __float2bfloat16_rn(c * gscale);
-    }
   }
 }
 
@@ -342,7 +307,7 @@ __global__ void __launch_bounds__(256, 1) infonce_bwd_kernel(const bf16* __restr
 
 // g_regions only (no dQ): all queries (chunks of kRQ) stay in shared memory, every region row is read once
 // and its gradient accumulates in registers across ALL query tiles -- one write per row, no block syncs
-// inside the row loop.  This is the (my regions, all queries) half of the collective-free multi-rank backward.
+// inside the row loop.  cor_infonce_bwd takes it when neither g_queries nor the logit-scale gradient is wanted.
 constexpr int kRQ = 128;
 __global__ void __launch_bounds__(256, 1) infonce_bwd_regions_kernel(const bf16* __restrict__ regions, const bf16* __restrict__ queries,
                                                                      const long long* __restrict__ targets, const float* __restrict__ lse,
@@ -800,18 +765,6 @@ extern "C" int cor_infonce_bwd_ls(const void* regions, const void* queries, cons
   COR_REQUIRE(logit_scale, "cor_infonce_bwd_ls: null logit_scale");
   return infonce_bwd(regions, queries, targets, lse, Nr, Nq, D, 0.f, logit_scale, g_loss, g_mul, g_regions, g_queries, g_logit_scale, work,
                      stream);
-}
-
-extern "C" int cor_infonce_coef(const float* S, const float* lse, const long long* targets, int Nq, int Nr, float inv_tau,
-                                const float* g_loss, float g_mul, void* P_bf16, cor_stream_t stream) {
-  COR_REQUIRE(S && lse && targets && g_loss && P_bf16, "cor_infonce_coef: null pointer");
-  COR_REQUIRE(Nq > 0 && Nq <= 65535 && Nr > 0, "cor_infonce_coef: bad shape Nq=%d Nr=%d", Nq, Nr);
-  COR_REQUIRE(Nr % 4 != 0 || ((((uintptr_t)S) & 15) == 0 && (((uintptr_t)P_bf16) & 7) == 0), "cor_infonce_coef: alignment");
-  int gx = ceil_div(ceil_div(Nr, 4), 256);
-  const int cap = ceil_div((long long)sm_count() * 8, Nq);
-  if (gx > cap) gx = cap < 1 ? 1 : cap;
-  infonce_coef_kernel<<<dim3(gx, Nq), 256, 0, as_stream(stream)>>>(S, lse, targets, Nq, Nr, inv_tau, g_loss, g_mul, (bf16*)P_bf16);
-  return check_launch("infonce_coef_kernel");
 }
 
 extern "C" int cor_topk(const float* S, const void* regions, const void* queries, int Nr, int Nq, int D, int k, long long* idx,

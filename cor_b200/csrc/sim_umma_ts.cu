@@ -13,7 +13,7 @@
 // ping-pong (the epilogue of half 0 runs under the MMAs of half 1 and vice versa) -- and the queries [256, 256 + D).
 // With <= 128 queries there is one half and its accumulator alternates between the two slots tile by tile.
 // Warp roles (320 threads): 0..7 epilogue (lane quarter w % 4, half w / 4), 8 TMA producer, 9 TMEM owner + MMA issuer.
-// LSE partials in the work buffer exactly as sim_umma.cu leaves them ([qtile][gridDim.x][256][2]).
+// LSE partials in the work buffer as [qtile][gridDim.x][256][2], the layout sim_lse_combine_kernel and cor_infonce_tail read.
 #include <stdlib.h>
 
 #include "umma.cuh"
@@ -220,8 +220,8 @@ __global__ void __launch_bounds__(320, 1) sim_umma_ts_kernel(const __grid_consta
   if (warp == kTsMmaWarp) tmem_dealloc(tmem, 512);
 }
 
-// LSE-only launcher (sim_umma.cu falls back to the SS kernel for the S / coefficient modes).  Returns the number of
-// partial records per query tile in *nparts.
+// LSE-only launcher (sim_umma.cu stores S with the kernel that keeps both operands in shared memory).  Returns the
+// number of partial records per query tile in *nparts.
 int sim_umma_ts_launch(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, const float* scale, void* work,
                        int* nparts, cudaStream_t st) {
   const int qtiles = ceil_div(Nq, kTsBM), ntiles = ceil_div(Nr, kTsBN);

@@ -80,27 +80,6 @@ __device__ __forceinline__ void tma_load_4d(void* smem_dst, const CUtensorMap* m
       : "memory");
 }
 
-// One slice of a stage, delivered to the same shared-memory offset of EVERY CTA in `mask` (and signalling the
-// mbarrier at the same offset in each of them): the cluster fetches the tile from L2 once.
-__device__ __forceinline__ void tma_load_2d_mc(void* smem_dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, uint16_t mask,
-                                               uint64_t hint) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster.L2::cache_hint"
-      " [%0], [%1, {%4, %5}], [%2], %3, %6;"
-      ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "h"(mask), "r"(c0), "r"(c1), "l"(hint)
-      : "memory");
-}
-
-// ---- thread-block clusters -----------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync() {
-  asm volatile("barrier.cluster.arrive.aligned;\n\tbarrier.cluster.wait.aligned;" ::: "memory");
-}
-
 // ---- tcgen05 -----------------------------------------------------------------------------------------
 __device__ __forceinline__ void tmem_alloc(uint32_t* smem_slot, uint32_t ncols) {   // one full warp; ncols pow2 >= 32
   asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_slot)), "r"(ncols) : "memory");
@@ -135,12 +114,6 @@ __device__ __forceinline__ void mma_bf16_ss_acc(uint32_t tmem_d, uint64_t desc_a
 // tcgen05.fence::before_thread_sync).
 __device__ __forceinline__ void mma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-
-// Same, arriving on the mbarrier at this offset in every CTA of `mask` (stage release in a multicast ring).
-__device__ __forceinline__ void mma_commit_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(smem_u32(bar)), "h"(mask) : "memory");
 }
 
 // Instruction descriptor, kind::f16: D=f32, A=B=bf16, both K-major, M x N tile (PTX ISA "Instruction

@@ -104,16 +104,12 @@ def _overlap_enabled():
     return os.environ.get("COR_STEP_OVERLAP", "1") != "0"
 
 
-def _pool_bwd_gemm_enabled():
-    return os.environ.get("COR_POOL_BWD_GEMM", "1") != "0"
-
-
 def _step_tail_ok(B: int, M: int, C: int, multi_rank: bool, bg_mode: int, sim_engine: str) -> bool:
     """Whether the fused step runs its region tail as one forward and one backward launch (csrc/step_tail.cu): one rank's
-    rows only, bg_mode 0, a streaming-similarity shape (<= 16 queries, C % 8 == 0, C <= 256) and the pooling backward on the
-    batched GEMM.  ``COR_STEP_TAIL=0`` keeps the kernel chain it replaces (A/B)."""
+    rows only, bg_mode 0 and a streaming-similarity shape (<= 16 queries, C % 8 == 0, C <= 256).  ``COR_STEP_TAIL=0`` keeps
+    the kernel chain it replaces (A/B)."""
     return (os.environ.get("COR_STEP_TAIL", "1") != "0" and not multi_rank and bg_mode == 0 and B <= 16 and C % 8 == 0 and C <= 256
-            and ops._sim_engine(B, B * M, C, sim_engine) == "stream" and _pool_bwd_gemm_enabled())
+            and ops._sim_engine(B, B * M, C, sim_engine) == "stream")
 
 
 _tail_counters = {}
@@ -193,7 +189,7 @@ class _FusedStepFn(torch.autograd.Function):
         # start of the step (one 32-thread CTA polling local flags): by the time the row epilogue needs the answer the
         # 0.7 ms mask resample has gone by, so the wait never sits on the critical path.
         rank, ws = cdist.world()
-        px = peer.get_exchange(B * M, Cc, dev) if (gather and ws > 1 and os.environ.get("COR_STEP_BWD", "reduce_scatter") != "local") else None
+        px = peer.get_exchange(B * M, Cc, dev) if (gather and ws > 1) else None
         ev_px = None
         if px is not None:
             with torch.cuda.stream(side if side is not None else cur):
@@ -233,7 +229,6 @@ class _FusedStepFn(torch.autograd.Function):
             out4 = torch.empty(4, **f32)
             aux = torch.empty(lib.cor_fgbg_aux_floats(B, Cc), **f32)
             r16, offset, ws, n_local = fg16, 0, 1, B * M
-            q_all = lse_all = tgt_all = None
             targets = _target_rows(dev, B, M, 0)
             lse = torch.empty((B,), **f32)
             nce = torch.empty(1, **f32)
@@ -276,13 +271,10 @@ class _FusedStepFn(torch.autograd.Function):
                 cur.wait_event(ev_q)
             n_local = B * M
             inv_tau = 1.0 / float(tau)
-            # A/B on one 8xB200 box (profiles/README.md): reduce-scatter of the region gradient 0.951 ms/step, collective-free
-            # variant 0.965 ms/step -> the reduce-scatter stays the default; COR_STEP_BWD=local selects the other.
-            local_bwd = os.environ.get("COR_STEP_BWD", "reduce_scatter") == "local"
             fused_parts = None
             if gather and ws > 1:
                 r16 = torch.empty((ws * n_local, Cc), dtype=torch.bfloat16, device=dev)
-                if px is not None and not local_bwd and _peer_fused_ok(B, Cc, ws * n_local, sim_engine):
+                if px is not None and _peer_fused_ok(B, Cc, ws * n_local, sim_engine):
                     # ONE kernel: pull the peers' rows over NVLink, keep a local copy for the backward, and score every row
                     # against this rank's queries while it is in registers (all-gather fused with its consumer)
                     fused_parts = px.gather_sim(r16, q16, inv_tau, sc)
@@ -291,46 +283,23 @@ class _FusedStepFn(torch.autograd.Function):
                 else:
                     torch.distributed.all_gather_into_tensor(r16, fg16)
                 offset = rank * n_local
-                if local_bwd:
-                    # A second small all-gather (the queries) replaces the backward's reduce-scatter: every rank scores
-                    # ALL queries against ALL regions (same HBM-bound cost as scoring its own), which gives it the
-                    # log-sum-exp of the remote queries too, so the backward needs no collective at all.
-                    q_all = torch.empty((ws * B, Cc), dtype=torch.bfloat16, device=dev)
-                    torch.distributed.all_gather_into_tensor(q_all, q16)
-                    _, lse_all = ops._sim_forward(r16, q_all, inv_tau, False, True, sim_engine, sc)
-                    lse = lse_all[rank * B:(rank + 1) * B]
-                    ar = torch.arange(ws * B, device=dev, dtype=torch.int64)
-                    tgt_all = (ar // B) * n_local + (ar % B) * M - offset       # target rows local to THIS rank
-                else:
-                    q_all = lse_all = tgt_all = None
-                    lse = None
             else:
                 r16, offset, ws = fg16, 0, 1
-                q_all = lse_all = tgt_all = None
-                lse = None
             targets = _target_rows(dev, B, M, offset)
             nce = torch.empty(1, **f32)
             tgt = torch.empty((B,), **f32)
             loss = torch.empty(1, **f32)
-            if lse is None:
-                # similarity with its log-sum-exp partials left in the work buffer, then ONE tail kernel: partial merge ->
-                # lse, target logits, InfoNCE mean and the step's total loss
-                sim_work, nparts, qt = fused_parts if fused_parts is not None else ops._sim_lse_parts(r16, q16, inv_tau, sim_engine, sc)
-                lse = torch.empty((B,), **f32)
-                if side is not None:
-                    cur.wait_stream(side)        # join: the total needs the segmentation and fg/bg losses
-                name, ta = tau_arg("cor_infonce_tail", inv_tau)
-                call(name, dev, ptr(sim_work), nparts, qt, ptr(r16), ptr(q16), ptr(targets), r16.shape[0], B, Cc, ta,
-                     ptr(lse), ptr(nce), ptr(tgt), ptr(out8), ptr(out4), _f(w_fg), _f(w_bg), _f(nce_weight), ptr(loss))
-            else:
-                name, ta = tau_arg("cor_infonce_fwd", inv_tau)
-                call(name, dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), r16.shape[0], B, Cc, ta, ptr(nce), ptr(tgt))
-                if side is not None:
-                    cur.wait_stream(side)        # join: the combine needs the segmentation loss
-                call("cor_step_combine", dev, ptr(out8), ptr(out4), ptr(nce), _f(w_fg), _f(w_bg), _f(nce_weight), ptr(loss))
+            # similarity with its log-sum-exp partials left in the work buffer, then ONE tail kernel: partial merge -> lse,
+            # target logits, InfoNCE mean and the step's total loss
+            sim_work, nparts, qt = fused_parts if fused_parts is not None else ops._sim_lse_parts(r16, q16, inv_tau, sim_engine, sc)
+            lse = torch.empty((B,), **f32)
+            if side is not None:
+                cur.wait_stream(side)        # join: the total needs the segmentation and fg/bg losses
+            name, ta = tau_arg("cor_infonce_tail", inv_tau)
+            call(name, dev, ptr(sim_work), nparts, qt, ptr(r16), ptr(q16), ptr(targets), r16.shape[0], B, Cc, ta,
+                 ptr(lse), ptr(nce), ptr(tgt), ptr(out8), ptr(out4), _f(w_fg), _f(w_bg), _f(nce_weight), ptr(loss))
         # the scale is saved as an input: an in-place write to it before backward trips autograd's version check
-        ctx.save_for_backward(pred_c, t_save, w_save, per, fg, bg, inv_fg, inv_bg, comb_c, stats, out4, aux, r16, q16, targets, lse, w32,
-                              fg16, q_all, lse_all, tgt_all, sc)
+        ctx.save_for_backward(pred_c, t_save, w_save, per, fg, bg, inv_fg, inv_bg, comb_c, stats, out4, aux, r16, q16, targets, lse, w32, sc)
         ctx.cfg = (B, M, Cc, h, w, float(inv_tau), float(nce_weight), int(bg_mode), float(w_fg), float(w_bg), ws, offset, n_local,
                    pred.dtype, emb.dtype, comb.dtype, tuple(comb.shape), need_pred, need_emb, comb.requires_grad)
         ctx.px = px
@@ -343,8 +312,7 @@ class _FusedStepFn(torch.autograd.Function):
     def backward(ctx, g_loss, *_unused):
         from . import _lib as L
         ptr, _f, _ll, call = ops.ptr, ops._f, ops._ll, ops._call
-        (pred_c, t_save, w_save, per, fg, bg, inv_fg, inv_bg, comb_c, stats, out4, aux, r16, q16, targets, lse, w32,
-         fg16, q_all, lse_all, tgt_all, sc) = ctx.saved_tensors
+        (pred_c, t_save, w_save, per, fg, bg, inv_fg, inv_bg, comb_c, stats, out4, aux, r16, q16, targets, lse, w32, sc) = ctx.saved_tensors
         (B, M, Cc, h, w, inv_tau, nce_weight, bg_mode, w_fg, w_bg, ws, offset, n_local, pred_dt, emb_dt, comb_dt, comb_shape,
          need_pred, need_emb, need_comb) = ctx.cfg
         dev = fg.device
@@ -360,7 +328,6 @@ class _FusedStepFn(torch.autograd.Function):
         g_scale = torch.empty((), **f32) if need_scale else None
         tau_arg = lambda name: ops._tau_arg(name, inv_tau, sc)
         gs_arg = () if sc is None else (ptr(g_scale),)          # the _ls backward entries take the gradient pointer
-        gs_none = () if sc is None else (None,)
         cur = torch.cuda.current_stream(dev)
         side = _side_stream(dev) if (_overlap_enabled() and need_pred) else None
 
@@ -378,7 +345,7 @@ class _FusedStepFn(torch.autograd.Function):
 
         px = ctx.px
         ev_px = None
-        if px is not None and ws > 1 and q_all is None:
+        if px is not None and ws > 1:
             # same idea as in the forward: ask early, on the side stream, whether the peers are done with last step's `gall`
             if side is not None:
                 side.wait_stream(cur)
@@ -391,8 +358,7 @@ class _FusedStepFn(torch.autograd.Function):
         if px is None or side is not None:
             g_pred = seg_bwd()               # side stream: runs underneath the InfoNCE / pooling backward
         w16, w16_epoch = ctx.w16
-        gemm_ok = (bg_mode != 1 and w16 is not None and getattr(w16, "_cor_epoch", -1) == w16_epoch and Cc % 8 == 0 and P % 8 == 0
-                   and _pool_bwd_gemm_enabled())
+        gemm_ok = bg_mode != 1 and w16 is not None and getattr(w16, "_cor_epoch", -1) == w16_epoch and Cc % 8 == 0 and P % 8 == 0
         if ctx.tail is not None and (gemm_ok or not need_emb):
             # ONE launch: InfoNCE + fg-loss gradient of every row, through the row epilogue, cast to bf16 into the K-padded
             # operand of the pooling-backward GEMM; and the query gradient (+ fg / bg terms) in extra CTAs, one set per query
@@ -418,15 +384,9 @@ class _FusedStepFn(torch.autograd.Function):
             g_regions = torch.empty((n_local, Cc), **f32)
             g_q = torch.empty((B, Cc), **f32)
             work = ops._work(lib.cor_sim_work_bytes(B, Nr, Cc), dev)
-            if ws > 1 and q_all is not None:
-                # (all regions, my queries) -> g_queries ; (my regions, ALL queries) -> g_regions.  Every rank's loss is the
-                # mean over its own B queries, so the sum over ranks of d loss_j / d my_regions carries the factor ws.
-                name, ta = tau_arg("cor_infonce_bwd")
-                call(name, dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), Nr, B, Cc, ta, ptr(g), _f(nce_weight), None,
-                     ptr(g_q), *gs_arg, ptr(work))
-                call(name, dev, ptr(fg16), ptr(q_all), ptr(tgt_all), ptr(lse_all), n_local, ws * B, Cc, ta, ptr(g),
-                     _f(float(ws) * nce_weight), ptr(g_regions), None, *gs_none, None)
-            elif ws > 1:
+            if ws > 1:
+                # gradient of every gathered row, then a reduce-scatter back to the owning rank: measured faster than a
+                # collective-free backward that all-gathers the queries instead (profiles/README.md)
                 if ev_px is not None:
                     cur.wait_event(ev_px)
                 g_all = px.gall if px is not None else torch.empty((Nr, Cc), **f32)

@@ -19,7 +19,7 @@
 extern "C" {
 #endif
 
-#define COR_ABI_VERSION 2
+#define COR_ABI_VERSION 3
 
 /* element types */
 #define COR_F32 0
@@ -142,9 +142,6 @@ int cor_fgbg_loss_bwd(const float* fg_rows, long long fg_stride, const float* bg
                       float* g_fg_rows, long long gfg_stride, int fg_accumulate,
                       float* g_bg_rows, long long gbg_stride, float* g_comb, long long gcomb_stride,
                       int comb_accumulate, cor_stream_t stream);
-/* loss = seg[0] + w_fg * fgbg[0] + w_bg * fgbg[1] + w_nce * nce[0]   (utils/trainer_v3_g.py:67-73; nce may be NULL) */
-int cor_step_combine(const float* seg, const float* fgbg, const float* nce, float w_fg, float w_bg, float w_nce,
-                     float* loss, cor_stream_t stream);
 
 /* ------------------------------------------------------------------------------------------
  * The fused step's region tail in one launch each way (csrc/step_tail.cu; cor_b200/region.py, one rank, bg_mode 0):
@@ -226,7 +223,9 @@ int cor_seg_loss_bwd(const void* pred, int pred_dtype, const float* t_save, cons
  *   regions [Nr, D] bf16 unit rows, queries [Nq, D] bf16 unit rows, D % 8 == 0.
  *   S [Nq, Nr] f32 or NULL; lse [Nq] (log-sum-exp of S/tau over regions) or NULL.
  * cor_sim_stream_*: CUDA-core streaming kernels, HBM-bound regime (few queries).
- * cor_sim_umma_fwd: tcgen05/TMEM GEMM with the LSE folded into its epilogue (many queries).
+ * cor_sim_umma_fwd: tcgen05/TMEM GEMM (many queries).  It takes S or lse, not both (COR_EINVAL): S comes from a kernel
+ *   with both operands in shared memory, lse from one that holds the queries in tensor memory and folds the
+ *   log-sum-exp into its epilogue.  cor_sim_stream_fwd serves both in one pass.
  * ---------------------------------------------------------------------------------------- */
 size_t cor_sim_work_bytes(int Nq, int Nr, int D);
 int cor_sim_stream_fwd(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau,
@@ -238,26 +237,18 @@ int cor_sim_umma_fwd(const void* regions, const void* queries, int Nr, int Nq, i
 int cor_sim_lse_parts(int engine, const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau,
                       void* work, int* nparts, int* qt, cor_stream_t stream);
 /* The tail of the fused step in ONE launch: merge of those partials -> lse [Nq]; tgt_logit and nce as cor_infonce_fwd;
- * and, when total != NULL, total = seg[0] + w_fg * fgbg[0] + w_bg * fgbg[1] + w_nce * nce (= cor_step_combine,
- * utils/trainer_v3_g.py:67-73 plus the Class-N term). */
+ * and, when total != NULL, total = seg[0] + w_fg * fgbg[0] + w_bg * fgbg[1] + w_nce * nce (utils/trainer_v3_g.py:67-73
+ * plus the Class-N term). */
 int cor_infonce_tail(const float* lse_part, int nparts, int qt, const void* regions, const void* queries,
                      const long long* targets, int Nr, int Nq, int D, float inv_tau, float* lse, float* nce,
                      float* tgt_logit, const float* seg, const float* fgbg, float w_fg, float w_bg, float w_nce,
                      float* total, cor_stream_t stream);
-/* The same coefficient matrix straight out of the tensor-core similarity kernel's epilogue (S is never written):
- * regions / queries as cor_sim_umma_fwd, lse [Nq] from the forward. */
-int cor_sim_umma_coef(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, const float* lse,
-                      const long long* targets, const float* g_loss, float g_mul, void* P_bf16, cor_stream_t stream);
-/* Many-query backward: P [Nq, Nr] bf16 = (exp(S/tau - lse) - onehot(target)) * g_loss[0] * g_mul / (tau * Nq) from the
- * raw similarity matrix S [Nq, Nr] f32; the caller finishes with two plain GEMMs, dQ = P R and dR = P^T Q. */
-int cor_infonce_coef(const float* S, const float* lse, const long long* targets, int Nq, int Nr, float inv_tau,
-                     const float* g_loss, float g_mul, void* P_bf16, cor_stream_t stream);
 /* loss = mean_q (lse[q] - S[q, target[q]] / tau); tgt_logit [Nq] is S[q,target[q]] (f32). */
 int cor_infonce_fwd(const void* regions, const void* queries, const long long* targets, const float* lse,
                     int Nr, int Nq, int D, float inv_tau, float* loss, float* tgt_logit, cor_stream_t stream);
 /* g_regions [Nr, D] f32 and/or g_queries [Nq, D] f32 (either may be NULL) for upstream scalar *g_loss * g_mul.
- * A rank of a data-parallel job calls it twice -- (all regions, its queries) -> g_queries and
- * (its regions, all queries; g_mul = world size) -> g_regions -- so the backward needs no collective. */
+ * A rank of a data-parallel job can call it twice -- (all regions, its queries) -> g_queries and
+ * (its regions, all queries; g_mul = world size) -> g_regions -- so that the backward needs no collective. */
 int cor_infonce_bwd(const void* regions, const void* queries, const long long* targets, const float* lse,
                     int Nr, int Nq, int D, float inv_tau, const float* g_loss, float g_mul, float* g_regions,
                     float* g_queries, void* work, cor_stream_t stream);
@@ -278,7 +269,7 @@ int cor_infonce_bwd_umma(const void* regions, const void* queries, int Nr, int N
  * The backward entries also write g_logit_scale (one f32 on the device; NULL = not wanted):
  *   d loss / d s = g_loss[0] * g_mul * mean_q sum_r (exp(s S[q,r] - lse[q]) - [r == target(q)]) S[q,r]
  * from per-query partials folded in a fixed order (no float atomics, no host synchronisation: deterministic and
- * graph-capturable).  The legacy coefficient entries cor_infonce_coef and cor_sim_umma_coef stay float-only.
+ * graph-capturable).
  *   cor_sim_stream_fwd_ls, cor_sim_umma_fwd_ls, cor_sim_lse_parts_ls, cor_infonce_tail_ls, cor_infonce_fwd_ls: as the
  *     entries without the suffix.
  *   cor_infonce_bwd_ls: extends cor_infonce_bwd.  The gradient comes from the (regions, queries) pair of the call, so a

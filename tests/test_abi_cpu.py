@@ -24,7 +24,7 @@ def test_library_exports_every_declared_symbol(lib):
     raw = ctypes.CDLL(_lib.LIB_PATH)
     missing = [n for n in names if not hasattr(raw, n)]
     assert not missing, f"declared in include/cor_b200.h but not exported: {missing}"
-    assert lib.cor_abi_version() == _lib.ABI_VERSION == 2
+    assert lib.cor_abi_version() == _lib.ABI_VERSION == 3
 
 
 def test_no_torch_types_in_the_header():
@@ -169,7 +169,7 @@ def test_argument_validation_fails_before_any_launch(lib):
         ("cor_peer_signal", (one, one, 0, 2, 5, null)),                                  # channel out of range
         ("cor_infonce_tail", (null, 4, 16, one, one, one, 8, 4, 64, 1.0, one, one, one, null, null, 0.0, 0.0, 0.0, null, null)),
         ("cor_infonce_tail", (one, 4, 16, one, one, one, 8, 4, 64, 1.0, one, one, one, null, null, 0.0, 0.0, 0.0, one, null)),  # total without seg/fgbg
-        ("cor_infonce_coef", (one, one, one, 0, 8, 1.0, one, 1.0, one, null)),           # no queries
+        ("cor_sim_umma_fwd", (one, one, 8, 4, 64, 1.0, one, one, one, null)),             # S and lse in one call
         ("cor_sim_lse_parts", (0, one, one, 8, 4, 64, 1.0, one, None, None, null)),      # nowhere to report the layout
         ("cor_topk", (one, one, one, 8, 4, 64, 9, one, one, null)),                      # k > Nr
         ("cor_gemm_bf16", (one, 0, 8, 0, one, 0, 8, 0, 8, 8, 0, 1, 1.0, null, 0, null, null, null, 0, 8, one, 0, 8, null, 0, null, null)),  # K = 0
@@ -205,4 +205,4 @@ def test_header_is_plain_c_and_a_c_host_can_bind_it(lib, tmp_path):
     assert r.returncode == 0, r.stderr
     r = subprocess.run([exe], capture_output=True, text=True)
     assert r.returncode == 0, (r.returncode, r.stdout, r.stderr)
-    assert "ABI v2" in r.stdout and "-> -1" in r.stdout
+    assert "ABI v3" in r.stdout and "-> -1" in r.stdout

@@ -115,10 +115,9 @@ def test_paired_bg_mode_keeps_the_kernel_chain(monkeypatch):
 
 def test_tail_eligibility(monkeypatch):
     """Host-side choice only: multi-rank gathering, bg_mode 1, more than 16 queries, wide rows, a forced tensor-core
-    similarity, the pooling backward off the batched GEMM and the knob keep today's kernels."""
+    similarity and the knob keep today's kernels."""
     from cor_b200 import region
     monkeypatch.delenv("COR_STEP_TAIL", raising=False)
-    monkeypatch.delenv("COR_POOL_BWD_GEMM", raising=False)
     assert region._step_tail_ok(16, 64, 256, False, 0, "auto")
     assert region._step_tail_ok(1, 17, 128, False, 0, "stream")
     assert not region._step_tail_ok(16, 64, 256, True, 0, "auto")
@@ -127,8 +126,5 @@ def test_tail_eligibility(monkeypatch):
     assert not region._step_tail_ok(16, 64, 384, False, 0, "auto")
     assert not region._step_tail_ok(16, 64, 256, False, 0, "umma")
     assert not region._step_tail_ok(16, 1024, 256, False, 0, "auto")      # 16 384 rows: the tensor-core similarity's regime
-    monkeypatch.setenv("COR_POOL_BWD_GEMM", "0")
-    assert not region._step_tail_ok(16, 64, 256, False, 0, "auto")
-    monkeypatch.delenv("COR_POOL_BWD_GEMM")
     monkeypatch.setenv("COR_STEP_TAIL", "0")
     assert not region._step_tail_ok(16, 64, 256, False, 0, "auto")

@@ -41,4 +41,4 @@ def test_pooling_tail_and_mask_branch_eligibility():
 def test_seg_coefficients_and_act_codes_are_stable():
     from cor_b200 import _lib as L
     assert (L.ACT_NONE, L.ACT_RELU, L.ACT_GELU, L.ACT_SIGMOID) == (0, 1, 2, 3)
-    assert L.ABI_VERSION == 2
+    assert L.ABI_VERSION == 3

@@ -12,3 +12,11 @@ or PyTorch fallback.  ``cor_b200.synth`` (numpy only) generates the benchmark in
 __version__ = "0.1.0"
 
 from ._lib import CorError  # noqa: E402,F401
+
+
+def __getattr__(name):
+    # cor_b200.RegionMemory without importing the region layer (and torch.distributed) at package import
+    if name == "RegionMemory":
+        from .region import RegionMemory
+        return RegionMemory
+    raise AttributeError(f"module {__name__!r} has no attribute {name!r}")

@@ -103,6 +103,17 @@ def load(path: str = LIB_PATH):
         _sig(lib, "cor_infonce_fwd_ls", i, p, p, p, p, i, i, i, p, p, p, p)
         _sig(lib, "cor_infonce_bwd_ls", i, p, p, p, p, i, i, i, p, p, f, p, p, p, p, p)
         _sig(lib, "cor_infonce_bwd_umma_ls", i, p, p, i, i, i, p, p, p, p, f, p, p, p, p, p)
+        # cross-batch region memory
+        _sig(lib, "cor_memory_state_words", i)
+        _sig(lib, "cor_memory_reset", i, p, p)
+        _sig(lib, "cor_memory_enqueue", i, p, i, i, i, p, i, p, p)
+        _sig(lib, "cor_memory_scan_work_bytes", sz, i, i, i)
+        _sig(lib, "cor_memory_scan", i, p, i, p, p, i, i, f, p, p, C.POINTER(i), p)
+        _sig(lib, "cor_infonce_tail_mem", i, p, i, i, p, p, p, i, i, i, f, p, p, i, p, p, p, p, p, p, f, f, f, p, p)
+        _sig(lib, "cor_step_tail_fwd_mem", i, p, i, ll, i, i, i, i, f, p, p, p, p, f, p, p, i, p, p, f, f, f, p, p, p, p, p, p, p, p, p,
+             p, p, p, p, p)
+        _sig(lib, "cor_memory_dq_work_bytes", sz, i, i, i)
+        _sig(lib, "cor_memory_dq", i, p, i, p, p, i, i, f, p, p, p, f, p, p, p, p)
         _sig(lib, "cor_topk", i, p, p, p, i, i, i, i, p, p, p)
         _sig(lib, "cor_l2_normalize", i, p, i, i, i, p, p, p, p)
         _sig(lib, "cor_gemm_bf16_work_bytes", sz, i, i, i, i, i)

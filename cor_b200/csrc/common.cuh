@@ -21,9 +21,14 @@ int launch_lse_combine(const float* part, int Nq, int nparts, int qt, float* lse
 int sim_umma_launch(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, const float* scale, float* S,
                     float* lse, void* work, int* nparts, int* qt, cudaStream_t st);
 
-// same, queries held in tensor memory (sim_umma_ts.cu); log-sum-exp partials only: [qtile][*nparts][256][2] in `work`
+// same, queries held in tensor memory (sim_umma_ts.cu); log-sum-exp partials only: [qtile][*nparts][256][2] in `work`.
+// count non-NULL: the rows actually scored are the first min(Nr, *count), read on the device (a region memory's fill);
+// the grid is sized for Nr and CTAs past the count leave empty partials (-inf, 0).
 int sim_umma_ts_launch(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, const float* scale, void* work,
-                       int* nparts, cudaStream_t st);
+                       int* nparts, cudaStream_t st, const int* count = nullptr);
+
+// queries per tile of the log-sum-exp partials sim_umma_ts_launch leaves: the layout of a region memory's scan
+constexpr int kMemQT = 256;
 
 #define COR_REQUIRE(cond, ...)          \
   do {                                  \
@@ -164,6 +169,43 @@ __device__ __forceinline__ float fold_parts(const float* __restrict__ part, int 
     for (int j = 0; j < kFoldTy; ++j) t += sm[j][threadIdx.x];
   }
   return t;
+}
+
+// "Am I the last CTA?": every thread's global writes are fenced before thread 0 counts; the counter wraps to 0 on the
+// last arrival (atomicInc with limit n - 1), so it is zero again after every launch and every graph replay.
+__device__ __forceinline__ bool arrive_last(unsigned* counter, unsigned n, bool* flag) {
+  __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0) *flag = atomicInc(counter, n - 1) == n - 1;
+  __syncthreads();
+  if (*flag) __threadfence();
+  return *flag;
+}
+
+// Log-sum-exp of query q over a region memory's scan partials [q / kMemQT][nparts][kMemQT][2] (running max, sum), by a
+// group of W consecutive lanes (j = lane within the group, every lane of the warp calls): lane j takes parts j, j + W, ...,
+// max and fp64 sum folded by butterflies (fixed order).  Parts past the memory's fill are (-inf, 0) and add nothing.
+template <int W>
+__device__ __forceinline__ float mem_lse(const float* part, int nparts, int q, int j) {
+  const float2* base = reinterpret_cast<const float2*>(part) + (long long)(q / kMemQT) * nparts * kMemQT + q % kMemQT;
+  float Mx = -INFINITY;
+  for (int p = j; p < nparts; p += W) Mx = fmaxf(Mx, __ldcg(base + (long long)p * kMemQT).x);
+#pragma unroll
+  for (int o = W / 2; o > 0; o >>= 1) Mx = fmaxf(Mx, __shfl_xor_sync(0xffffffffu, Mx, o));
+  double acc = 0.0;
+  for (int p = j; p < nparts; p += W) {
+    const float2 v = __ldcg(base + (long long)p * kMemQT);
+    if (v.x != -INFINITY) acc += (double)(v.y * expf(v.x - Mx));
+  }
+#pragma unroll
+  for (int o = W / 2; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+  return Mx + logf((float)acc);
+}
+
+// log(exp(a) + exp(b)) for finite a, b
+__device__ __forceinline__ float logaddexpf_(float a, float b) {
+  const float hi = fmaxf(a, b), lo = fminf(a, b);
+  return hi + log1pf(expf(lo - hi));
 }
 
 // Block-wide sum of NV values per thread; result valid in every thread.  `scratch` needs

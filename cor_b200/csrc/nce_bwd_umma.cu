@@ -25,6 +25,8 @@
 // Split over Y (gridDim.x) leaves fp32 partials [split][Nx][D] that a fixed-order fold sums (deterministic).
 // Logit-scale gradient (mode 0 only): the epilogue thread of query row x also keeps sum_y (P/gscale)[x][y] S[x][y] in a
 // register across its Y tiles and leaves one partial per (split, column half, query); nce_scale_fold_kernel sums them.
+// Region memory (mode 0, cor_memory_dq): Y = the memory's bank, its row count read on the device (count), no targets (a
+// memory row is never a positive); both folds ADD into the gradients the current rows' backward already wrote.
 #include <stdlib.h>
 
 #include "umma.cuh"
@@ -58,7 +60,8 @@ struct NceArgs {
   const float* scale;                      // device logit scale replacing 1/tau in c2 and gmul, or NULL
   float* lspart;                           // mode 0: [gridDim.x][2][Nq] logit-scale gradient partials, or NULL
   const float* lse;                        // [Nq]
-  const long long* targets;                // [Nq] region index of each query's positive
+  const long long* targets;                // [Nq] region index of each query's positive, or NULL (no positives)
+  const int* count;                        // device row count: Y rows past min(Ny, *count) are not scored; or NULL
   const float* g_loss;                     // [1]
   float* out;                              // [gridDim.x][Nx][D] partials (or the result itself when gridDim.x == 1); NULL = not written
   const bf16* X;                           // [Nx][D] the CTA's rows, read by the epilogue threads when the X tile lives in TMEM
@@ -97,7 +100,8 @@ __global__ void __launch_bounds__(320, 1) nce_bwd_umma_kernel(const __grid_const
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int x0 = blockIdx.y * kNbM;
-  const int ntiles = (a.Ny + kNbN - 1) / kNbN;
+  const int Ny = a.count ? min(a.Ny, max(*a.count, 0)) : a.Ny;
+  const int ntiles = (Ny + kNbN - 1) / kNbN;
   const int D = a.nkb * kNbBK;
   const int n_my = (ntiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;      // tiles blockIdx.x, +gridDim.x, ...
 
@@ -241,7 +245,7 @@ __global__ void __launch_bounds__(320, 1) nce_bwd_umma_kernel(const __grid_const
     int my_tg = -1;
     if (a.mode == 0 && xok) {
       my_nl = -a.lse[xg] * log2e;
-      my_tg = (int)a.targets[xg];
+      my_tg = a.targets ? (int)a.targets[xg] : -1;
     }
     for (int i = 0; i < n_my; ++i) {
       const int t = blockIdx.x + i * gridDim.x;
@@ -270,7 +274,9 @@ __global__ void __launch_bounds__(320, 1) nce_bwd_umma_kernel(const __grid_const
         float n0, n1;
         int hit0, hit1;
         if (a.mode == 0) {
-          n0 = n1 = my_nl;
+          // columns past Ny get no coefficient (exp2(-inf) = 0): a memory's stale rows in its last tile add nothing
+          n0 = y0 + 2 * j < Ny ? my_nl : -INFINITY;
+          n1 = y0 + 2 * j + 1 < Ny ? my_nl : -INFINITY;
           hit0 = (y0 + 2 * j == my_tg);
           hit1 = (y0 + 2 * j + 1 == my_tg);
         } else {
@@ -283,7 +289,7 @@ __global__ void __launch_bounds__(320, 1) nce_bwd_umma_kernel(const __grid_const
         float c1 = ex2_approx(fmaf(__uint_as_float(va[2 * j + 1]), c2, n1));
         if (hit0) c0 -= 1.f;
         if (hit1) c1 -= 1.f;
-        if (a.lspart) {                             // columns past Ny hold S = 0 (TMA zero fill): they add nothing
+        if (a.lspart) {                             // columns past Ny have a zero coefficient: they add nothing
           ls = fmaf(c0, __uint_as_float(va[2 * j]), ls);
           ls = fmaf(c1, __uint_as_float(va[2 * j + 1]), ls);
         }
@@ -318,6 +324,9 @@ __global__ void __launch_bounds__(320, 1) nce_bwd_umma_kernel(const __grid_const
                                                                 __uint_as_float(v[4 * j + 2]), __uint_as_float(v[4 * j + 3]));
         }
       }
+    } else if (xok && a.out) {                    // a split with no Y tile (a memory filled below the grid): zero partials
+      float* dst = a.out + ((long long)blockIdx.x * a.Nx + xg) * D + half * (D / 2);
+      for (int c = 0; c < D / 2; c += 4) *reinterpret_cast<float4*>(dst + c) = make_float4(0.f, 0.f, 0.f, 0.f);
     }
   }
   tc_fence_before();
@@ -325,21 +334,27 @@ __global__ void __launch_bounds__(320, 1) nce_bwd_umma_kernel(const __grid_const
   if (warp == kNbMmaWarp) tmem_dealloc(tmem, 512);
 }
 
-// out[x][d] = sum over splits (ascending) of part[s][x][d]
-__global__ void __launch_bounds__(256) nce_fold_kernel(const float4* __restrict__ part, float4* __restrict__ out, long long vecs, int nsplit) {
+// out[x][d] = sum over splits (ascending) of part[s][x][d]; accumulate: out[x][d] += that sum
+__global__ void __launch_bounds__(256) nce_fold_kernel(const float4* __restrict__ part, float4* __restrict__ out, long long vecs, int nsplit,
+                                                       int accumulate) {
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < vecs; i += (long long)gridDim.x * blockDim.x) {
     float4 acc = part[i];
     for (int s = 1; s < nsplit; ++s) {
       const float4 v = part[(long long)s * vecs + i];
       acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
     }
+    if (accumulate) {
+      const float4 o = out[i];
+      acc.x = o.x + acc.x; acc.y = o.y + acc.y; acc.z = o.z + acc.z; acc.w = o.w + acc.w;
+    }
     out[i] = acc;
   }
 }
 
-// *g_scale = g_loss[0] * g_mul / Nq * sum_q sum_p lspart[p][q]: one CTA, partials in order per query, queries in a fixed tree
+// *g_scale = g_loss[0] * g_mul / Nq * sum_q sum_p lspart[p][q]: one CTA, partials in order per query, queries in a fixed tree.
+// accumulate: *g_scale += that value
 __global__ void __launch_bounds__(256) nce_scale_fold_kernel(const float* __restrict__ lspart, int nparts, int Nq, const float* __restrict__ g_loss,
-                                                             float g_mul, float* __restrict__ g_scale) {
+                                                             float g_mul, float* __restrict__ g_scale, int accumulate) {
   __shared__ float red[256];
   float v = 0.f;
   for (int q = threadIdx.x; q < Nq; q += 256) {
@@ -353,7 +368,10 @@ __global__ void __launch_bounds__(256) nce_scale_fold_kernel(const float* __rest
     if (threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o];
     __syncthreads();
   }
-  if (threadIdx.x == 0) g_scale[0] = red[0] * (g_loss[0] * g_mul / (float)Nq);
+  if (threadIdx.x == 0) {
+    const float v = red[0] * (g_loss[0] * g_mul / (float)Nq);
+    g_scale[0] = accumulate ? g_scale[0] + v : v;
+  }
 }
 
 static int nce_splits(int xtiles, int ytiles) {
@@ -363,10 +381,11 @@ static int nce_splits(int xtiles, int ytiles) {
   return s;
 }
 
-// out == NULL (mode 0): only the logit-scale partials are wanted -- the dQ GEMM still runs, its result is not stored
+// out == NULL (mode 0): only the logit-scale partials are wanted -- the dQ GEMM still runs, its result is not stored.
+// count: device row count of Y (see NceArgs); accumulate: the fold adds into `out` (then the partials always go to `part`)
 static int nce_launch(const void* X, const void* Y, int Nx, int Ny, int Nq, int D, int mode, float inv_tau, const float* scale,
                       const float* lse, const long long* targets, const float* g_loss, float g_mul, float* out, float* part,
-                      float* lspart, cudaStream_t st) {
+                      float* lspart, cudaStream_t st, const int* count = nullptr, int accumulate = 0) {
   const int nkb = D / kNbBK;
   const int xtiles = ceil_div(Nx, kNbM), ytiles = ceil_div(Ny, kNbN);
   const int nsplit = nce_splits(xtiles, ytiles);
@@ -387,15 +406,16 @@ static int nce_launch(const void* X, const void* Y, int Nx, int Ny, int Nq, int 
   a.c2 = inv_tau * 1.4426950408889634f;
   a.gmul = g_mul * inv_tau / (float)Nq;
   a.g_mul = g_mul; a.scale = scale; a.lspart = lspart;
-  a.lse = lse; a.targets = targets; a.g_loss = g_loss;
+  a.lse = lse; a.targets = targets; a.count = count; a.g_loss = g_loss;
   a.X = reinterpret_cast<const bf16*>(X);
-  a.out = !out ? nullptr : (nsplit == 1 ? out : part);
+  const bool direct = nsplit == 1 && !accumulate;
+  a.out = !out ? nullptr : (direct ? out : part);
   nce_bwd_umma_kernel<<<dim3(nsplit, xtiles), 320, smem, st>>>(tmX, tmY, a);
   rc = check_launch("nce_bwd_umma_kernel");
-  if (rc || nsplit == 1 || !out) return rc;
+  if (rc || direct || !out) return rc;
   const long long vecs = (long long)Nx * D / 4;
   const int blocks = (int)((vecs + 255) / 256 < (long long)sm_count() * 4 ? (vecs + 255) / 256 : (long long)sm_count() * 4);
-  nce_fold_kernel<<<blocks, 256, 0, st>>>(reinterpret_cast<const float4*>(part), reinterpret_cast<float4*>(out), vecs, nsplit);
+  nce_fold_kernel<<<blocks, 256, 0, st>>>(reinterpret_cast<const float4*>(part), reinterpret_cast<float4*>(out), vecs, nsplit, accumulate);
   return check_launch("nce_fold_kernel");
 }
 
@@ -431,7 +451,7 @@ static int infonce_bwd_umma(const void* regions, const void* queries, int Nr, in
   if (rc) return rc;
   if (g_scale) {
     const int nparts = 2 * nce_splits(ceil_div(Nq, kNbM), ceil_div(Nr, kNbN));
-    nce_scale_fold_kernel<<<1, 256, 0, st>>>(lspart, nparts, Nq, g_loss, g_mul, g_scale);
+    nce_scale_fold_kernel<<<1, 256, 0, st>>>(lspart, nparts, Nq, g_loss, g_mul, g_scale, 0);
     rc = check_launch("nce_scale_fold_kernel");
     if (rc) return rc;
   }
@@ -453,4 +473,34 @@ extern "C" int cor_infonce_bwd_umma_ls(const void* regions, const void* queries,
   COR_REQUIRE(logit_scale, "cor_infonce_bwd_umma_ls: null logit_scale");
   return infonce_bwd_umma(regions, queries, Nr, Nq, D, 0.f, logit_scale, lse, targets, g_loss, g_mul, g_regions, g_queries, g_logit_scale,
                           work, stream);
+}
+
+// ---- region memory: the queries' gradient through the memory rows (Y = the bank, no positives), added in ----
+static int mem_dq_splits(int Nq, int K) { return nce_splits(ceil_div(Nq, kNbM), ceil_div(K, kNbN)); }
+
+static size_t mem_dq_part_bytes(int Nq, int K, int D) {
+  return ((size_t)mem_dq_splits(Nq, K) * Nq * D * sizeof(float) + 255) / 256 * 256;
+}
+
+extern "C" size_t cor_memory_dq_work_bytes(int Nq, int K, int D) {
+  if (Nq <= 0 || K <= 0 || D <= 0) return 0;
+  return mem_dq_part_bytes(Nq, K, D) + (size_t)mem_dq_splits(Nq, K) * 2 * Nq * sizeof(float) + 256;
+}
+
+extern "C" int cor_memory_dq(const void* bank, int K, const int* state, const void* queries, int Nq, int D, float inv_tau,
+                             const float* logit_scale, const float* lse, const float* g_loss, float g_mul, float* g_queries,
+                             float* g_logit_scale, void* work, cor_stream_t stream) {
+  COR_REQUIRE(bank && state && queries && lse && g_loss && work, "cor_memory_dq: null pointer");
+  COR_REQUIRE(K >= 1 && Nq >= 1, "cor_memory_dq: need K >= 1 and Nq >= 1 (K=%d Nq=%d)", K, Nq);
+  COR_REQUIRE(D % kNbBK == 0 && D >= kNbBK && D <= 256, "cor_memory_dq: need D in {64,128,192,256} (D=%d)", D);
+  COR_REQUIRE(g_queries || g_logit_scale, "cor_memory_dq: nothing to compute");
+  COR_REQUIRE(!g_logit_scale || logit_scale, "cor_memory_dq: g_logit_scale needs logit_scale");
+  cudaStream_t st = as_stream(stream);
+  float* part = reinterpret_cast<float*>(work);
+  float* lspart = g_logit_scale ? reinterpret_cast<float*>(reinterpret_cast<char*>(work) + mem_dq_part_bytes(Nq, K, D)) : nullptr;
+  int rc = nce_launch(queries, bank, Nq, K, Nq, D, 0, inv_tau, logit_scale, lse, nullptr, g_loss, g_mul, g_queries, part, lspart, st,
+                      state + 1, 1);
+  if (rc || !g_logit_scale) return rc;
+  nce_scale_fold_kernel<<<1, 256, 0, st>>>(lspart, 2 * mem_dq_splits(Nq, K), Nq, g_loss, g_mul, g_logit_scale, 1);
+  return check_launch("nce_scale_fold_kernel");
 }

@@ -134,38 +134,51 @@ __global__ void __launch_bounds__(1024) infonce_fwd_kernel(const bf16* __restric
 
 // ---- the fused step's tail in ONE launch: merge of the log-sum-exp partials (as sim_lse_combine_kernel), target
 //      logits, mean InfoNCE loss and the step's total loss (seg + w_fg fg + w_bg bg + w_nce nce).  One CTA, one warp per query.
+//      mem_part non-NULL: a region memory's scan partials (cor_memory_scan), merged in after the current rows' whenever the
+//      memory holds rows (mem_state[1] > 0); an empty memory leaves every output bit-equal to mem_part == NULL.
+//      part == NULL: the current rows' lse is already in lse[] (cor_sim_*_fwd); it is read, merged and written back, and nce
+//      is formed exactly as infonce_fwd_kernel forms the loss.
 __global__ void __launch_bounds__(1024) infonce_tail_kernel(const float* __restrict__ part, int nparts, int qt,
                                                             const bf16* __restrict__ regions, const bf16* __restrict__ queries,
                                                             const long long* __restrict__ targets, int Nr, int Nq, int D, float inv_tau,
                                                             const float* __restrict__ scale, float* __restrict__ lse, float* __restrict__ nce,
                                                             float* __restrict__ tgt_logit, const float* __restrict__ seg,
                                                             const float* __restrict__ fgbg, float w_fg, float w_bg, float w_nce,
-                                                            float* __restrict__ total) {
+                                                            float* __restrict__ total, const float* __restrict__ mem_part, int mem_nparts,
+                                                            const int* __restrict__ mem_state) {
   __shared__ double scratch[32];
   if (scale) inv_tau = __ldg(scale);
+  const int mem_rows = mem_part ? __ldcg(mem_state + 1) : 0;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarp = blockDim.x >> 5;
   double acc[1] = {0.0};
   for (int q = warp; q < Nq; q += nwarp) {
-    const int tile = q / qt, ql = q % qt;
-    const float* base = part + ((long long)tile * nparts * qt + ql) * 2;
-    float M = -INFINITY;
-    for (int p = lane; p < nparts; p += 32) M = fmaxf(M, base[(long long)p * qt * 2]);
-    M = warp_max(M);
-    // fp32 rescale (expf of a non-positive argument, relative error ~1e-7) and fp64 only for the sum: the fp64 exp
-    // of sim_lse_combine_kernel costs microseconds on this single-CTA critical path
-    double a = 0.0;
-    for (int p = lane; p < nparts; p += 32) {
-      const float pm = base[(long long)p * qt * 2], ps = base[(long long)p * qt * 2 + 1];
-      if (pm != -INFINITY) a += (double)(ps * expf(pm - M));
+    float l;
+    if (part) {
+      const int tile = q / qt, ql = q % qt;
+      const float* base = part + ((long long)tile * nparts * qt + ql) * 2;
+      float M = -INFINITY;
+      for (int p = lane; p < nparts; p += 32) M = fmaxf(M, base[(long long)p * qt * 2]);
+      M = warp_max(M);
+      // fp32 rescale (expf of a non-positive argument, relative error ~1e-7) and fp64 only for the sum: the fp64 exp
+      // of sim_lse_combine_kernel costs microseconds on this single-CTA critical path
+      double a = 0.0;
+      for (int p = lane; p < nparts; p += 32) {
+        const float pm = base[(long long)p * qt * 2], ps = base[(long long)p * qt * 2 + 1];
+        if (pm != -INFINITY) a += (double)(ps * expf(pm - M));
+      }
+      a = warp_sum(a);
+      l = M + logf((float)a);
+    } else {
+      l = lse[q];
+      __syncwarp();                  // every lane has read lse[q] before lane 0 writes it back
     }
-    a = warp_sum(a);
     long long t = targets[q];
     t = t < 0 ? 0 : (t >= Nr ? Nr - 1 : t);
     float d = 0.f;
     for (int k = lane; k < D; k += 32) d = fmaf(__bfloat162float(queries[(long long)q * D + k]), __bfloat162float(regions[t * D + k]), d);
     d = warp_sum(d);
+    if (mem_rows > 0) l = logaddexpf_(l, mem_lse<32>(mem_part, mem_nparts, q, lane));
     if (lane == 0) {
-      const float l = M + logf((float)a);
       lse[q] = l;
       tgt_logit[q] = d;
       acc[0] += (double)l - (double)d * (double)inv_tau;
@@ -671,19 +684,32 @@ extern "C" int cor_sim_lse_parts_ls(int engine, const void* regions, const void*
 
 static int infonce_tail(const float* lse_part, int nparts, int qt, const void* regions, const void* queries, const long long* targets, int Nr,
                         int Nq, int D, float inv_tau, const float* scale, float* lse, float* nce, float* tgt_logit, const float* seg,
-                        const float* fgbg, float w_fg, float w_bg, float w_nce, float* total, cor_stream_t stream) {
-  COR_REQUIRE(lse_part && regions && queries && targets && lse && nce && tgt_logit, "cor_infonce_tail: null pointer");
-  COR_REQUIRE(nparts > 0 && qt > 0 && Nr > 0 && Nq > 0 && D > 0, "cor_infonce_tail: bad sizes");
+                        const float* fgbg, float w_fg, float w_bg, float w_nce, float* total, cor_stream_t stream,
+                        const float* mem_part = nullptr, int mem_nparts = 0, const int* mem_state = nullptr) {
+  COR_REQUIRE(regions && queries && targets && lse && nce && tgt_logit, "cor_infonce_tail: null pointer");
+  COR_REQUIRE((!lse_part || (nparts > 0 && qt > 0)) && Nr > 0 && Nq > 0 && D > 0, "cor_infonce_tail: bad sizes");
   COR_REQUIRE(!total || (seg && fgbg), "cor_infonce_tail: total needs seg and fgbg");
+  COR_REQUIRE(!mem_part || (mem_state && mem_nparts > 0), "cor_infonce_tail_mem: memory partials need mem_state and mem_nparts > 0");
   infonce_tail_kernel<<<1, 1024, 0, as_stream(stream)>>>(lse_part, nparts, qt, (const bf16*)regions, (const bf16*)queries, targets, Nr, Nq, D,
-                                                        inv_tau, scale, lse, nce, tgt_logit, seg, fgbg, w_fg, w_bg, w_nce, total);
+                                                        inv_tau, scale, lse, nce, tgt_logit, seg, fgbg, w_fg, w_bg, w_nce, total, mem_part,
+                                                        mem_nparts, mem_state);
   return check_launch("infonce_tail_kernel");
+}
+
+extern "C" int cor_infonce_tail_mem(const float* lse_part, int nparts, int qt, const void* regions, const void* queries,
+                                    const long long* targets, int Nr, int Nq, int D, float inv_tau, const float* logit_scale,
+                                    const float* mem_part, int mem_nparts, const int* mem_state, float* lse, float* nce,
+                                    float* tgt_logit, const float* seg, const float* fgbg, float w_fg, float w_bg, float w_nce,
+                                    float* total, cor_stream_t stream) {
+  return infonce_tail(lse_part, nparts, qt, regions, queries, targets, Nr, Nq, D, inv_tau, logit_scale, lse, nce, tgt_logit, seg, fgbg,
+                      w_fg, w_bg, w_nce, total, stream, mem_part, mem_nparts, mem_state);
 }
 
 extern "C" int cor_infonce_tail(const float* lse_part, int nparts, int qt, const void* regions, const void* queries,
                                 const long long* targets, int Nr, int Nq, int D, float inv_tau, float* lse, float* nce, float* tgt_logit,
                                 const float* seg, const float* fgbg, float w_fg, float w_bg, float w_nce, float* total,
                                 cor_stream_t stream) {
+  COR_REQUIRE(lse_part, "cor_infonce_tail: null lse_part");
   return infonce_tail(lse_part, nparts, qt, regions, queries, targets, Nr, Nq, D, inv_tau, nullptr, lse, nce, tgt_logit, seg, fgbg, w_fg,
                       w_bg, w_nce, total, stream);
 }
@@ -693,6 +719,7 @@ extern "C" int cor_infonce_tail_ls(const float* lse_part, int nparts, int qt, co
                                    float* tgt_logit, const float* seg, const float* fgbg, float w_fg, float w_bg, float w_nce, float* total,
                                    cor_stream_t stream) {
   COR_REQUIRE(logit_scale, "cor_infonce_tail_ls: null logit_scale");
+  COR_REQUIRE(lse_part, "cor_infonce_tail_ls: null lse_part");
   return infonce_tail(lse_part, nparts, qt, regions, queries, targets, Nr, Nq, D, 0.f, logit_scale, lse, nce, tgt_logit, seg, fgbg, w_fg,
                       w_bg, w_nce, total, stream);
 }

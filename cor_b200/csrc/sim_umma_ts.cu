@@ -37,12 +37,13 @@ struct TsSmemTail {
 
 __global__ void __launch_bounds__(320, 1) sim_umma_ts_kernel(const __grid_constant__ CUtensorMap tmR, const bf16* __restrict__ queries, int Nr,
                                                              int Nq, int nkb, int nstages, float inv_tau, const float* __restrict__ scale,
-                                                             float* __restrict__ part) {
+                                                             float* __restrict__ part, const int* __restrict__ count) {
   extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t* base = reinterpret_cast<uint8_t*>(((uintptr_t)smem + 1023) & ~(uintptr_t)1023);
   uint8_t* r_smem = base;
   TsSmemTail* tail = reinterpret_cast<TsSmemTail*>(r_smem + (size_t)nstages * kTsBBytes);
 
+  if (count) Nr = min(Nr, max(*count, 0));       // a region memory: only its filled rows; no tiles at all when it is empty
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int q0 = blockIdx.y * kTsBM;
   const int nhalf = (Nq - q0 > kTsHalf) ? 2 : 1;
@@ -222,8 +223,10 @@ __global__ void __launch_bounds__(320, 1) sim_umma_ts_kernel(const __grid_consta
 
 // LSE-only launcher (sim_umma.cu stores S with the kernel that keeps both operands in shared memory).  Returns the
 // number of partial records per query tile in *nparts.
+static_assert(kTsBM == kMemQT, "a region memory's scan partials are laid out per kTsBM-query tile");
+
 int sim_umma_ts_launch(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, const float* scale, void* work,
-                       int* nparts, cudaStream_t st) {
+                       int* nparts, cudaStream_t st, const int* count) {
   const int qtiles = ceil_div(Nq, kTsBM), ntiles = ceil_div(Nr, kTsBN);
   CUtensorMap tmR;
   int rc = umma::encode_tmap_bf16_2d(&tmR, regions, (uint64_t)Nr, (uint64_t)D, kTsBN, kTsBK);
@@ -237,7 +240,7 @@ int sim_umma_ts_launch(const void* regions, const void* queries, int Nr, int Nq,
   const size_t smem = (size_t)nstages * kTsBBytes + sizeof(TsSmemTail) + 1024;
   COR_CUDA(cudaFuncSetAttribute(sim_umma_ts_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   sim_umma_ts_kernel<<<dim3(gx, qtiles), 320, smem, st>>>(tmR, reinterpret_cast<const bf16*>(queries), Nr, Nq, nkb, nstages, inv_tau,
-                                                         scale, reinterpret_cast<float*>(work));
+                                                         scale, reinterpret_cast<float*>(work), count);
   *nparts = gx;
   return check_launch("sim_umma_ts_kernel");
 }

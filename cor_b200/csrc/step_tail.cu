@@ -68,17 +68,6 @@ __device__ __forceinline__ void sum_splits(const float* p, int n, long long stri
   }
 }
 
-// "Am I the last CTA?": every thread's global writes are fenced before thread 0 counts; the counter wraps to 0 on the
-// last arrival (atomicInc with limit n - 1), so it is zero again after every launch and every graph replay.
-__device__ __forceinline__ bool arrive_last(unsigned* counter, unsigned n, bool* flag) {
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) *flag = atomicInc(counter, n - 1) == n - 1;
-  __syncthreads();
-  if (*flag) __threadfence();
-  return *flag;
-}
-
 }  // namespace
 
 struct StepTailFwd {
@@ -87,6 +76,7 @@ struct StepTailFwd {
   const float* seg; float w_fg, w_bg, w_nce;
   float* fg; bf16* fg16; float* inv_fg; float* bg; float* inv_bg; float* out4; float* aux;
   float* lse; float* nce; float* tgt; float* total; float* lse_part; unsigned* counter;
+  const float* mem_part; int mem_nparts; const int* mem_state;     // region memory's scan partials (cor_memory_scan) or NULL
 };
 
 // grid = ceil(B*M / 8), block = 256 (warp per region row), dynamic smem = kQT * C floats.
@@ -226,8 +216,10 @@ __global__ void __launch_bounds__(256, 1) step_tail_fwd_kernel(const StepTailFwd
     }
 #pragma unroll
     for (int o = 8; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+    float l = Mx + logf((float)acc);
+    // a region memory: its partials merged in after this batch's, only when it holds rows (an empty one changes no bit)
+    if (a.mem_part && __ldcg(a.mem_state + 1) > 0) l = logaddexpf_(l, mem_lse<16>(a.mem_part, a.mem_nparts, q, j));
     if (j == 0 && q < Nq) {
-      const float l = Mx + logf((float)acc);
       a.lse[q] = l;
       lse_s[q] = l;
     }
@@ -492,9 +484,11 @@ static int step_tail_fwd(const float* part, int nsplit, long long split_stride, 
                          const float* stats, const void* queries_bf16, const float* comb, const long long* targets, float inv_tau,
                          const float* scale, const float* seg, float w_fg, float w_bg, float w_nce, float* fg, void* fg_bf16, float* inv_fg,
                          float* bg, float* inv_bg, float* fgbg_out4, float* aux, float* lse, float* nce, float* tgt_logit, float* total,
-                         void* work, unsigned* counter, cor_stream_t stream) {
+                         void* work, unsigned* counter, cor_stream_t stream, const float* mem_part = nullptr, int mem_nparts = 0,
+                         const int* mem_state = nullptr) {
   int rc = tail_shape_ok(B, M, C, "cor_step_tail_fwd");
   if (rc) return rc;
+  COR_REQUIRE(!mem_part || (mem_state && mem_nparts > 0), "cor_step_tail_fwd_mem: memory partials need mem_state and mem_nparts > 0");
   COR_REQUIRE(part && stats && queries_bf16 && comb && targets && seg && fg && fg_bf16 && inv_fg && bg && inv_bg && fgbg_out4 && aux &&
                   lse && nce && tgt_logit && total && work && counter,
               "cor_step_tail_fwd: null pointer");
@@ -503,7 +497,7 @@ static int step_tail_fwd(const float* part, int nsplit, long long split_stride, 
               "cor_step_tail_fwd: bad partial layout or alignment (nsplit=%d Rp=%d M=%d)", nsplit, Rp, M);
   StepTailFwd a{part, nsplit, split_stride, (long long)Rp * C, B, M, C, p_total, stats, (const bf16*)queries_bf16, comb, targets, inv_tau,
                 scale, seg, w_fg, w_bg, w_nce, fg, (bf16*)fg_bf16, inv_fg, bg, inv_bg, fgbg_out4, aux, lse, nce, tgt_logit, total,
-                (float*)work, counter};
+                (float*)work, counter, mem_part, mem_nparts, mem_state};
   const int grid = ceil_div((long long)B * M, 8);
   step_tail_fwd_kernel<<<grid, 256, (size_t)kQT * C * sizeof(float), as_stream(stream)>>>(a);
   return check_launch("step_tail_fwd_kernel");
@@ -526,6 +520,17 @@ extern "C" int cor_step_tail_fwd_ls(const float* part, int nsplit, long long spl
   COR_REQUIRE(logit_scale, "cor_step_tail_fwd_ls: null logit_scale");
   return step_tail_fwd(part, nsplit, split_stride, Rp, B, M, C, p_total, stats, queries_bf16, comb, targets, 0.f, logit_scale, seg, w_fg,
                        w_bg, w_nce, fg, fg_bf16, inv_fg, bg, inv_bg, fgbg_out4, aux, lse, nce, tgt_logit, total, work, counter, stream);
+}
+
+extern "C" int cor_step_tail_fwd_mem(const float* part, int nsplit, long long split_stride, int Rp, int B, int M, int C, float p_total,
+                                     const float* stats, const void* queries_bf16, const float* comb, const long long* targets, float inv_tau,
+                                     const float* logit_scale, const float* mem_part, int mem_nparts, const int* mem_state, const float* seg,
+                                     float w_fg, float w_bg, float w_nce, float* fg, void* fg_bf16, float* inv_fg, float* bg, float* inv_bg,
+                                     float* fgbg_out4, float* aux, float* lse, float* nce, float* tgt_logit, float* total, void* work,
+                                     unsigned* counter, cor_stream_t stream) {
+  return step_tail_fwd(part, nsplit, split_stride, Rp, B, M, C, p_total, stats, queries_bf16, comb, targets, inv_tau, logit_scale, seg, w_fg,
+                       w_bg, w_nce, fg, fg_bf16, inv_fg, bg, inv_bg, fgbg_out4, aux, lse, nce, tgt_logit, total, work, counter, stream,
+                       mem_part, mem_nparts, mem_state);
 }
 
 static int step_tail_bwd(const void* regions_bf16, const void* queries_bf16, const long long* targets, const float* lse, int B, int M,

@@ -38,6 +38,9 @@ _KERNELS_PER_CALL = {
     "cor_sim_stream_fwd_ls": 2, "cor_sim_umma_fwd_ls": 2, "cor_sim_lse_parts_ls": 1, "cor_infonce_tail_ls": 1, "cor_infonce_fwd_ls": 1,
     "cor_infonce_bwd_ls": 2, "cor_infonce_bwd_umma_ls": 4, "cor_step_tail_fwd_ls": 1, "cor_step_tail_bwd_ls": 1,
     "cor_peer_gather_sim_ls": 1,
+    # cross-batch region memory: cor_memory_dq is 2 launches, 3 with the logit scale's gradient (its caller passes the count)
+    "cor_memory_reset": 1, "cor_memory_enqueue": 1, "cor_memory_scan": 1, "cor_infonce_tail_mem": 1, "cor_step_tail_fwd_mem": 1,
+    "cor_memory_dq": 2,
 }
 
 
@@ -48,10 +51,11 @@ TIMING = {"events": None}
 _raw_stream = getattr(torch._C, "_cuda_getCurrentRawStream", None)
 
 
-def _call(name: str, dev, *args):
+def _call(name: str, dev, *args, launches: Optional[int] = None):
     """One C-ABI call on ``dev``'s current stream.  Host cost matters for the launch-bound small shapes (a few dozen calls
     per module forward): the device guard is taken only when ``dev`` is not already current and the stream handle comes
-    from the raw accessor (no Stream object)."""
+    from the raw accessor (no Stream object).  ``launches`` overrides the table's kernel count for entries whose count
+    depends on their arguments."""
     lib = L.load()
     ev = TIMING["events"]
     idx = dev.index
@@ -68,7 +72,7 @@ def _call(name: str, dev, *args):
                 ev.setdefault(name, []).append((a, b))
             else:
                 rc = getattr(lib, name)(*args, stream_ptr())
-    LAUNCHES["count"] += _KERNELS_PER_CALL.get(name, 1)
+    LAUNCHES["count"] += _KERNELS_PER_CALL.get(name, 1) if launches is None else launches
     check(rc, name)
 
 
@@ -521,6 +525,53 @@ def _sim_lse_parts(r16, q16, inv_tau, engine, scale=None):
     return work, nparts.value, qt.value
 
 
+def check_memory(memory, D: int, dev, who: str) -> None:
+    """A region memory (``region.RegionMemory``) serves queries of its own width on its own device."""
+    if memory is None:
+        return
+    if not all(hasattr(memory, a) for a in ("bank", "state", "K", "C", "enqueues")):
+        raise CorError(f"{who}: memory must be a RegionMemory, got {type(memory).__name__}")
+    if memory.C != D:
+        raise CorError(f"{who}: the memory holds rows of width C={memory.C}, the queries have D={D}")
+    if dev is not None and memory.bank.device != dev:
+        raise CorError(f"{who}: the memory is on {memory.bank.device}, the call on {dev}")
+
+
+def _memory_scan_work(memory, Nq: int, D: int, dev) -> torch.Tensor:
+    return _work(L.load().cor_memory_scan_work_bytes(Nq, memory.K, D), dev)
+
+
+def _memory_scan(memory, q16, inv_tau, scale=None, work=None):
+    """Log-sum-exp partials of the queries against the memory's valid rows (tensor cores): (work, nparts) for the
+    ``_mem`` tail entries.  ``work``: a buffer from _memory_scan_work allocated on the stream that consumes the partials."""
+    dev = q16.device
+    Nq, D = q16.shape
+    if work is None:
+        work = _memory_scan_work(memory, Nq, D, dev)
+    nparts = C.c_int(0)
+    _call("cor_memory_scan", dev, ptr(memory.bank), memory.K, ptr(memory.state), ptr(q16), Nq, D, _f(inv_tau), ptr(scale), ptr(work),
+          C.byref(nparts))
+    return work, nparts.value
+
+
+def _memory_dq(memory, q16, lse, inv_tau, scale, g_loss, g_mul, g_queries, g_scale):
+    """ADD the memory rows' share of the InfoNCE gradient into g_queries [Nq, D] and g_scale (either may be None)."""
+    if g_queries is None and g_scale is None:
+        return
+    dev = q16.device
+    Nq, D = q16.shape
+    work = _work(L.load().cor_memory_dq_work_bytes(Nq, memory.K, D), dev)
+    _call("cor_memory_dq", dev, ptr(memory.bank), memory.K, ptr(memory.state), ptr(q16), Nq, D, _f(inv_tau), ptr(scale), ptr(lse),
+          ptr(g_loss), _f(g_mul), ptr(g_queries), ptr(g_scale), ptr(work), launches=1 + (g_queries is not None) + (g_scale is not None))
+
+
+def check_memory_unchanged(mem_rec, who: str) -> None:
+    """A backward over memory rows needs the rows its forward scored: refuse it after an enqueue in between."""
+    if mem_rec is not None and mem_rec[0].enqueues != mem_rec[1]:
+        raise CorError(f"{who}: the region memory was enqueued between forward and backward, so the rows the forward scored "
+                       "may have been overwritten; enqueue after backward()")
+
+
 def _to_bf16_rows(x: torch.Tensor) -> torch.Tensor:
     """[.., D] -> bf16 [rows, D] on our own cast kernel (fp32 input) -- not an ATen copy."""
     x2 = x.reshape(-1, x.shape[-1])
@@ -549,8 +600,9 @@ def _infonce_bwd_dense(Nq: int, Nr: int, D: int, engine: str) -> bool:
 
 class _InfoNCEFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, regions, queries, targets, tau, engine, regions_bf16, logit_scale):
+    def forward(ctx, regions, queries, targets, tau, engine, regions_bf16, logit_scale, memory):
         dev = require_cuda(regions, queries, targets, logit_scale)
+        check_memory(memory, queries.shape[-1], dev, "infonce_loss")
         r16 = regions_bf16.reshape(-1, regions_bf16.shape[-1]).contiguous() if regions_bf16 is not None else _to_bf16_rows(regions)
         q16 = _to_bf16_rows(queries)
         Nr, D = r16.shape
@@ -560,8 +612,16 @@ class _InfoNCEFn(torch.autograd.Function):
         _, lse = _sim_forward(r16, q16, inv_tau, False, True, engine, logit_scale)
         loss = torch.empty(1, dtype=torch.float32, device=dev)
         tgt = torch.empty((Nq,), dtype=torch.float32, device=dev)
-        name, ta = _tau_arg("cor_infonce_fwd", inv_tau, logit_scale)
-        _call(name, dev, ptr(r16), ptr(q16), ptr(tg), ptr(lse), Nr, Nq, D, ta, ptr(loss), ptr(tgt))
+        if memory is None:
+            name, ta = _tau_arg("cor_infonce_fwd", inv_tau, logit_scale)
+            _call(name, dev, ptr(r16), ptr(q16), ptr(tg), ptr(lse), Nr, Nq, D, ta, ptr(loss), ptr(tgt))
+        else:
+            # the tail entry in its lse-in form: it merges the memory's partials into the current rows' lse (in place) and
+            # forms the loss as cor_infonce_fwd does, so an empty memory changes no bit
+            mwork, mparts = _memory_scan(memory, q16, inv_tau, logit_scale)
+            _call("cor_infonce_tail_mem", dev, None, 0, 0, ptr(r16), ptr(q16), ptr(tg), Nr, Nq, D, _f(inv_tau), ptr(logit_scale),
+                  ptr(mwork), mparts, ptr(memory.state), ptr(lse), ptr(loss), ptr(tgt), None, None, _f(0.0), _f(0.0), _f(0.0), None)
+        ctx.mem = None if memory is None else (memory, memory.enqueues)
         # the scale is saved as an input: an in-place write to it before backward trips autograd's version check
         ctx.save_for_backward(r16, q16, tg, lse, logit_scale)
         ctx.engine = engine
@@ -571,6 +631,7 @@ class _InfoNCEFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, g):
+        check_memory_unchanged(ctx.mem, "infonce_loss backward")
         r16, q16, tg, lse, sc = ctx.saved_tensors
         inv_tau, rdt, qdt, rshape, qshape, r_need, q_need = ctx.cfg
         s_need = sc is not None and ctx.needs_input_grad[6]
@@ -596,19 +657,26 @@ class _InfoNCEFn(torch.autograd.Function):
             work = _work(lib.cor_sim_work_bytes(Nq, Nr, D), dev)
             name, ta = _tau_arg("cor_infonce_bwd", inv_tau, sc)
             _call(name, dev, ptr(r16), ptr(q16), ptr(tg), ptr(lse), Nr, Nq, D, ta, ptr(gl), _f(1.0), ptr(gr), ptr(gq), *gs_arg, ptr(work))
-        return ((gr.view(rshape).to(rdt) if r_need else None), (gq.view(qshape).to(qdt) if q_need else None), None, None, None, None, gs)
+        if ctx.mem is not None:          # the memory rows' share, added into what the current rows' backward wrote
+            _memory_dq(ctx.mem[0], q16, lse, inv_tau, sc, gl, 1.0, gq if q_need else None, gs)
+        return ((gr.view(rshape).to(rdt) if r_need else None), (gq.view(qshape).to(qdt) if q_need else None), None, None, None, None, gs,
+                None)
 
 
 def infonce_loss(regions: torch.Tensor, queries: torch.Tensor, targets: torch.Tensor, tau: Optional[float] = None, engine: str = "auto",
-                 regions_bf16: Optional[torch.Tensor] = None, logit_scale: Optional[torch.Tensor] = None) -> torch.Tensor:
+                 regions_bf16: Optional[torch.Tensor] = None, logit_scale: Optional[torch.Tensor] = None, memory=None) -> torch.Tensor:
     """mean_q CE(s * S[q,:], targets[q]) with S = queries @ regions^T (bf16 operands, fp32 accumulate) and s = 1/tau
     (tau defaults to 0.07).  Gradients flow straight through the bf16 rounding to ``regions`` and ``queries``.
 
     ``logit_scale``: a learnable temperature -- a 0-dim float32 CUDA tensor s > 0 used in place of 1/tau (pass one or
     the other).  The kernels read it from device memory, and when it requires grad d loss / d s reaches it through
-    autograd, e.g. ``logit_scale = log_s.exp()`` with a parameter ``log_s`` as in CLIP."""
+    autograd, e.g. ``logit_scale = log_s.exp()`` with a parameter ``log_s`` as in CLIP.
+
+    ``memory``: a ``region.RegionMemory`` whose valid rows join the negatives of every query (never a target, no gradient
+    of their own); the queries and the scale get the memory terms of their gradient.  Enqueue into it after backward()."""
     check_logit_scale(logit_scale, tau, "infonce_loss")
-    return _InfoNCEFn.apply(regions, queries, targets, 0.07 if tau is None else float(tau), engine, regions_bf16, logit_scale)
+    check_memory(memory, queries.shape[-1], None, "infonce_loss")
+    return _InfoNCEFn.apply(regions, queries, targets, 0.07 if tau is None else float(tau), engine, regions_bf16, logit_scale, memory)
 
 
 def topk_retrieve(regions: torch.Tensor, queries: torch.Tensor, k: int, engine: str = "auto"):

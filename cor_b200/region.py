@@ -20,7 +20,72 @@ from . import peer
 from ._lib import CorError
 
 __all__ = ["pool_regions", "region_query_similarity", "region_infonce_loss", "topk_regions", "region_step", "RegionStepOut",
-           "StepBuffers"]
+           "StepBuffers", "RegionMemory"]
+
+
+class RegionMemory:
+    """Cross-batch memory of region embeddings (as XBM, "Cross-Batch Memory for Embedding Learning"): a ring of at most
+    ``capacity`` bf16 unit rows of width ``C`` whose valid rows serve the InfoNCE of ``region_step``,
+    ``region_infonce_loss`` and ``ops.infonce_loss`` (``memory=``) as extra negatives.  Memory rows are never targets and
+    get no gradient; the queries and the logit scale get the memory terms of theirs.
+
+    The head and fill count live in device memory ({head, count} in ``state``), so a captured CUDA graph that enqueues
+    advances them at every replay.  Enqueue AFTER backward(): a backward whose forward scored the memory raises
+    ``CorError`` if the memory was enqueued in between (``enqueues`` counts the calls on the host).  Each rank of a
+    data-parallel job owns its memory and scores it against its own queries only.  C must be 64, 128, 192 or 256."""
+
+    def __init__(self, capacity: int, C: int, device="cuda"):
+        from . import _lib as L
+        if int(capacity) < 1:
+            raise CorError(f"RegionMemory: capacity must be >= 1, got {capacity}")
+        if int(C) not in (64, 128, 192, 256):
+            raise CorError(f"RegionMemory: C={C} must be 64, 128, 192 or 256 (the widths the tensor-core kernels take)")
+        device = torch.device(device)
+        if device.type != "cuda":
+            raise CorError(f"RegionMemory: the memory lives on a CUDA device, got {device}")
+        self.K, self.C = int(capacity), int(C)
+        # zero rows: the last partly filled tile of a scan reads rows past the fill, which must be finite
+        self.bank = torch.zeros((self.K, self.C), dtype=torch.bfloat16, device=device)
+        self.state = torch.zeros(L.load().cor_memory_state_words(), dtype=torch.int32, device=device)
+        self.enqueues = 0
+
+    @property
+    def device(self):
+        return self.bank.device
+
+    def enqueue(self, rows: torch.Tensor) -> None:
+        """Push ``rows`` (fp32 or bf16 [..., C], e.g. ``RegionStepOut.regions``; 1 <= n <= capacity rows) as bf16 at the
+        head, overwriting the oldest rows once full.  One kernel on the current stream, no host synchronisation."""
+        from . import _lib as L
+        if rows.dtype not in (torch.float32, torch.bfloat16):
+            raise CorError(f"RegionMemory.enqueue: rows must be float32 or bfloat16, got {rows.dtype}")
+        if rows.dim() < 1 or rows.shape[-1] != self.C:
+            raise CorError(f"RegionMemory.enqueue: rows {tuple(rows.shape)} must be [..., C={self.C}]")
+        n = rows.numel() // self.C
+        if not 1 <= n <= self.K:
+            raise CorError(f"RegionMemory.enqueue: {n} rows, the memory takes 1 to {self.K} at once")
+        dev = L.require_cuda(rows)
+        if dev != self.device:
+            raise CorError(f"RegionMemory.enqueue: rows on {dev}, the memory on {self.device}")
+        rc = rows.detach().reshape(n, self.C).contiguous()
+        ops._call("cor_memory_enqueue", dev, ops.ptr(rc), L.dtype_code(rc), n, self.C, ops.ptr(self.bank), self.K, ops.ptr(self.state))
+        self.enqueues += 1
+
+    def reset(self) -> None:
+        """Empty the memory (one memset of the state on the current stream)."""
+        ops._call("cor_memory_reset", self.device, ops.ptr(self.state))
+        self.enqueues += 1
+
+    def count(self) -> int:
+        """Valid rows (synchronises with the device)."""
+        return int(self.state[1].item())
+
+    def rows(self) -> torch.Tensor:
+        """The valid rows, oldest first, as bf16 [count, C] (synchronises with the device)."""
+        head, count = (int(v) for v in self.state[:2].tolist())
+        if count < self.K:
+            return self.bank[:count].clone()
+        return torch.cat([self.bank[head:], self.bank[:head]])
 
 
 def pool_regions(emb: torch.Tensor, masks: torch.Tensor, background: bool = False, engine: str = "auto", want_bf16: bool = True):
@@ -36,12 +101,13 @@ def region_query_similarity(regions: torch.Tensor, queries: torch.Tensor, engine
 
 def region_infonce_loss(regions: torch.Tensor, queries: torch.Tensor, targets: torch.Tensor, tau: Optional[float] = None,
                         gather: bool = True, engine: str = "auto", regions_bf16: Optional[torch.Tensor] = None,
-                        logit_scale: Optional[torch.Tensor] = None) -> torch.Tensor:
+                        logit_scale: Optional[torch.Tensor] = None, memory: Optional[RegionMemory] = None) -> torch.Tensor:
     """InfoNCE of each local query against ALL regions.  With ``gather`` (and an initialised process
     group) the region rows are all-gathered across ranks first and ``targets`` -- indices into the
     LOCAL region rows -- are offset by rank * n_local.  tau (default 0.07) is a build choice (the reference defines
     none); ``logit_scale`` replaces 1/tau with a device tensor that can be learned (see ``ops.infonce_loss``).  Each
-    rank's loss is the mean over its own queries, so the scale's gradient is rank-local, like the queries'."""
+    rank's loss is the mean over its own queries, so the scale's gradient is rank-local, like the queries'.  ``memory``
+    (a :class:`RegionMemory`) adds its valid rows to every query's negatives; each rank scores its own memory."""
     ops.check_logit_scale(logit_scale, tau, "region_infonce_loss")
     regions = regions.reshape(-1, regions.shape[-1])
     rank, ws = cdist.world()
@@ -50,7 +116,7 @@ def region_infonce_loss(regions: torch.Tensor, queries: torch.Tensor, targets: t
         regions = cdist.all_gather_rows(regions)
         targets = targets + rank * n_local
         regions_bf16 = None
-    return ops.infonce_loss(regions, queries.reshape(-1, queries.shape[-1]), targets, tau, engine, regions_bf16, logit_scale)
+    return ops.infonce_loss(regions, queries.reshape(-1, queries.shape[-1]), targets, tau, engine, regions_bf16, logit_scale, memory)
 
 
 def topk_regions(regions: torch.Tensor, queries: torch.Tensor, k: int, sharded: bool = False, engine: str = "auto"):
@@ -148,7 +214,7 @@ class _FusedStepFn(torch.autograd.Function):
     pooling engine applies; the modular ops remain the general path."""
 
     @staticmethod
-    def forward(ctx, pred, emb, comb, masks, tau, nce_weight, gather, sim_engine, bg_mode, w_fg, w_bg, logit_scale):
+    def forward(ctx, pred, emb, comb, masks, tau, nce_weight, gather, sim_engine, bg_mode, w_fg, w_bg, logit_scale, memory):
         from . import _lib as L
         ptr, _f, _ll, call = ops.ptr, ops._f, ops._ll, ops._call
         dev = L.require_cuda(pred, emb, comb, masks, logit_scale)
@@ -199,11 +265,18 @@ class _FusedStepFn(torch.autograd.Function):
                     ev_px.record(side)
         q16 = torch.empty((B, comb_c.shape[1]), dtype=torch.bfloat16, device=dev)
         ev_q = None
+        mem_args = ()
+        # allocated on the consuming stream: its block is reused only after the tail that reads it
+        mwork = ops._memory_scan_work(memory, B, comb_c.shape[1], dev) if memory is not None else None
         with torch.cuda.stream(side if side is not None else cur):
             call("cor_cast_cat_bf16", dev, ptr(comb_c), comb_c.shape[1], None, 0, _ll(B), ptr(q16))   # bf16 queries, off the main chain
             if side is not None:
                 ev_q = torch.cuda.Event()
                 ev_q.record(side)
+            if memory is not None:
+                # the region memory's scan needs only the queries and the bank: a parallel branch beside the mask resample
+                mwork, mparts = ops._memory_scan(memory, q16, 1.0 / float(tau), sc, mwork)
+                mem_args = (ptr(mwork), mparts, ptr(memory.state))
             call("cor_seg_loss_fwd", dev, ptr(pred_c), L.dtype_code(pred_c), ptr(gt), L.dtype_code(gt), _f(ops._mask_scale(gt, None)), N, H, W,
                  Hm, Wm, _ll(gt.stride(0)), None, _f(0.25), _f(-1.0), _f(1.0), ptr(out8), ptr(per), ptr(t_save), ptr(w_save),
                  ptr(seg_work))
@@ -238,9 +311,13 @@ class _FusedStepFn(torch.autograd.Function):
             work = ops._work(lib.cor_step_tail_work_bytes(B, M, Cc), dev)
             if side is not None:
                 cur.wait_stream(side)        # join: the total needs the segmentation loss, the scores the bf16 queries
-            name, ta = tau_arg("cor_step_tail_fwd", inv_tau)
+            if memory is None:
+                name, ta = tau_arg("cor_step_tail_fwd", inv_tau)
+                tas = (ta,)
+            else:                            # the same kernel, the memory's partials merged into the log-sum-exp
+                name, tas = "cor_step_tail_fwd_mem", (_f(inv_tau), ptr(sc), *mem_args)
             call(name, dev, ptr(part), ks, _ll(B * Rp * Cc), Rp, B, M, Cc, _f(float(P)), ptr(stats), ptr(q16), ptr(comb_c),
-                 ptr(targets), ta, ptr(out8), _f(w_fg), _f(w_bg), _f(nce_weight), ptr(fg), ptr(fg16), ptr(inv_fg), ptr(bg),
+                 ptr(targets), *tas, ptr(out8), _f(w_fg), _f(w_bg), _f(nce_weight), ptr(fg), ptr(fg16), ptr(inv_fg), ptr(bg),
                  ptr(inv_bg), ptr(out4), ptr(aux), ptr(lse), ptr(nce), ptr(tgt), ptr(loss), ptr(work), ptr(ctx.tail))
         else:
             fg = torch.empty((B * M, Cc), **f32)
@@ -295,14 +372,19 @@ class _FusedStepFn(torch.autograd.Function):
             lse = torch.empty((B,), **f32)
             if side is not None:
                 cur.wait_stream(side)        # join: the total needs the segmentation and fg/bg losses
-            name, ta = tau_arg("cor_infonce_tail", inv_tau)
-            call(name, dev, ptr(sim_work), nparts, qt, ptr(r16), ptr(q16), ptr(targets), r16.shape[0], B, Cc, ta,
+            if memory is None:
+                name, ta = tau_arg("cor_infonce_tail", inv_tau)
+                tas = (ta,)
+            else:                            # each rank merges ITS memory, scored against its own queries
+                name, tas = "cor_infonce_tail_mem", (_f(inv_tau), ptr(sc), *mem_args)
+            call(name, dev, ptr(sim_work), nparts, qt, ptr(r16), ptr(q16), ptr(targets), r16.shape[0], B, Cc, *tas,
                  ptr(lse), ptr(nce), ptr(tgt), ptr(out8), ptr(out4), _f(w_fg), _f(w_bg), _f(nce_weight), ptr(loss))
         # the scale is saved as an input: an in-place write to it before backward trips autograd's version check
         ctx.save_for_backward(pred_c, t_save, w_save, per, fg, bg, inv_fg, inv_bg, comb_c, stats, out4, aux, r16, q16, targets, lse, w32, sc)
         ctx.cfg = (B, M, Cc, h, w, float(inv_tau), float(nce_weight), int(bg_mode), float(w_fg), float(w_bg), ws, offset, n_local,
                    pred.dtype, emb.dtype, comb.dtype, tuple(comb.shape), need_pred, need_emb, comb.requires_grad)
         ctx.px = px
+        ctx.mem = None if memory is None else (memory, memory.enqueues)
         ctx.w16 = (w16, getattr(w16, "_cor_epoch", -1))      # not a saved tensor: a cached operand buffer, validated by its epoch
         ctx.mark_non_differentiable(fg, out8, out4, nce)
         ctx.set_materialize_grads(False)     # no zero-filled gradients for the auxiliary outputs
@@ -320,7 +402,8 @@ class _FusedStepFn(torch.autograd.Function):
         P = h * w
         f32 = dict(dtype=torch.float32, device=dev)
         if g_loss is None:
-            return (None,) * 12
+            return (None,) * 13
+        ops.check_memory_unchanged(ctx.mem, "region_step backward")
         g = g_loss.reshape(1).float().contiguous()
         g_pred = g_emb = g_comb = None
         need_scale = sc is not None and ctx.needs_input_grad[11]
@@ -370,6 +453,8 @@ class _FusedStepFn(torch.autograd.Function):
             call(name, dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), B, M, Cc, ta, ptr(g), _f(nce_weight),
                  ptr(fg), ptr(inv_fg), ptr(stats), ptr(comb_c), ptr(out4), ptr(aux), _f(w_fg), _f(w_bg), ptr(a16), Kp, ptr(g_q),
                  *gs_arg, ptr(work), ptr(ctx.tail))
+            if ctx.mem is not None:
+                ops._memory_dq(ctx.mem[0], q16, lse, inv_tau, sc, g, nce_weight, g_q, g_scale)
             if need_comb:
                 g_comb = g_q.view(comb_shape).to(comb_dt)
             if need_emb:
@@ -408,6 +493,8 @@ class _FusedStepFn(torch.autograd.Function):
             g_bg = torch.empty((B, Cc), **f32) if bg_mode == 1 else None
             call("cor_fgbg_loss_bwd", dev, ptr(fg), _ll(M * Cc), ptr(bg), _ll(Cc), ptr(comb_c), _ll(Cc), B, Cc, bg_mode, ptr(out4), ptr(aux),
                  ptr(g), _ll(0), _f(w_fg), _f(w_bg), ptr(g_regions), _ll(M * Cc), 1, ptr(g_bg), _ll(Cc), ptr(g_q), _ll(Cc), 1)
+            if ctx.mem is not None:          # this rank's memory, against this rank's queries
+                ops._memory_dq(ctx.mem[0], q16, lse, inv_tau, sc, g, nce_weight, g_q if need_comb else None, g_scale)
             if need_comb:
                 g_comb = g_q.view(comb_shape).to(comb_dt)
             if need_emb:
@@ -443,7 +530,7 @@ class _FusedStepFn(torch.autograd.Function):
             cur.wait_stream(side)
         if g_pred is not None:
             g_pred = g_pred.to(pred_dt)
-        return g_pred, g_emb, g_comb, None, None, None, None, None, None, None, None, g_scale
+        return g_pred, g_emb, g_comb, None, None, None, None, None, None, None, None, g_scale, None
 
 
 def _fused_ok(emb, masks, pool_engine):
@@ -454,7 +541,8 @@ def _fused_ok(emb, masks, pool_engine):
 
 def region_step(pred: torch.Tensor, emb: torch.Tensor, comb: torch.Tensor, masks: torch.Tensor, *, tau: Optional[float] = None,
                 nce_weight: float = 1.0, gather: bool = True, pool_engine: str = "auto", sim_engine: str = "auto",
-                bg_mode: int = 0, fused: bool = True, logit_scale: Optional[torch.Tensor] = None) -> RegionStepOut:
+                bg_mode: int = 0, fused: bool = True, logit_scale: Optional[torch.Tensor] = None,
+                memory: Optional[RegionMemory] = None) -> RegionStepOut:
     """One forward of the whole region path for a batch of triplets with M candidate masks each
     (mask 0 of every image is the ground-truth ``query_mask``):
 
@@ -467,6 +555,11 @@ def region_step(pred: torch.Tensor, emb: torch.Tensor, comb: torch.Tensor, masks
     ``logit_scale`` is a 0-dim float32 tensor s > 0 on the step's device, passed instead of ``tau``.  The kernels read
     it from device memory, and d loss / d s reaches it through autograd when it requires grad.
 
+    ``memory`` (a :class:`RegionMemory` of width C on the step's device) adds its valid rows to every query's InfoNCE
+    negatives: nce = mean_b (logsumexp over the current rows and the memory - target logit).  The step stays on its fused
+    kernels; the memory is scanned on tensor cores beside the mask resample.  Push the batch with
+    ``memory.enqueue(out.regions)`` after backward() (``StepBuffers.capture(memory=...)`` does it inside the graph).
+
     ONE pass over the masks and ONE pass over the feature map serve fg, bg and all M regions.  With bf16
     features and >= 16 masks the step runs as a single fused autograd node (tensor-core pooling, hand
     written backward); other shapes compose the modular ops.
@@ -474,6 +567,7 @@ def region_step(pred: torch.Tensor, emb: torch.Tensor, comb: torch.Tensor, masks
     ops.check_logit_scale(logit_scale, tau, "region_step")
     if logit_scale is not None and logit_scale.device != emb.device:
         raise CorError(f"region_step: logit_scale is on {logit_scale.device}, the step on {emb.device}")
+    ops.check_memory(memory, emb.shape[1], emb.device if emb.is_cuda else None, "region_step")
     B, M = masks.shape[:2]
     if comb.shape[0] != B or emb.shape[0] != B or pred.shape[0] != B:
         raise CorError("region_step: batch sizes differ")
@@ -482,7 +576,7 @@ def region_step(pred: torch.Tensor, emb: torch.Tensor, comb: torch.Tensor, masks
                        "(the kernels read the queries with the feature map's row width)")
     if fused and _fused_ok(emb, masks, pool_engine) and pred.dim() == 4 and pred.shape[1] == 1:
         loss, out8, out4, nce, fg = _FusedStepFn.apply(pred, emb, comb, masks, 0.07 if tau is None else float(tau), float(nce_weight),
-                                                       bool(gather), sim_engine, int(bg_mode), 5.0, 5.0, logit_scale)
+                                                       bool(gather), sim_engine, int(bg_mode), 5.0, 5.0, logit_scale, memory)
         return RegionStepOut(loss=loss, seg=out8[0], fg=out4[0], bg=out4[1], nce=nce[0], regions=fg.view(B, M, -1))
     pool = ops.region_pool(emb, masks, transform=ops.W_CLAMP, normalize=True, pair=True, engine=pool_engine, want_bf16=True)
     Cc = pool.fg.shape[-1]
@@ -491,7 +585,7 @@ def region_step(pred: torch.Tensor, emb: torch.Tensor, comb: torch.Tensor, masks
     losses, _ = ops.fgbg_losses(pool.fg[:, 0, :], pool.bg[:, 0, :], q, pool.stats.view(B, M, 4)[:, 0, :], bg_mode)
     seg = ops.seg_loss(pred, masks[:, 0:1])
     nce = region_infonce_loss(pool.fg.reshape(B * M, Cc), q, gt_rows, tau, gather, sim_engine,
-                              regions_bf16=pool.fg_bf16, logit_scale=logit_scale)
+                              regions_bf16=pool.fg_bf16, logit_scale=logit_scale, memory=memory)
     loss = seg + 5 * losses[0] + 5 * losses[1] + nce_weight * nce
     return RegionStepOut(loss=loss, seg=seg, fg=losses[0], bg=losses[1], nce=nce, regions=pool.fg.detach())
 
@@ -508,7 +602,11 @@ class StepBuffers:
 
     ``capture(logit_scale=s)`` (s a 0-dim float32 tensor on the device) learns the temperature: the graph reads ``s``
     from device memory at every replay, so a value written into it (``s.copy_(log_s.exp())``) takes effect without a
-    recapture, and d loss / d s lands in ``self.grads["logit_scale"]``, overwritten by every replay."""
+    recapture, and d loss / d s lands in ``self.grads["logit_scale"]``, overwritten by every replay.
+
+    ``capture(memory=m)`` / ``run(..., memory=m)`` (m a :class:`RegionMemory`): every step scores against the memory, then
+    after the backward pushes its regions with ``m.enqueue``, inside the graph, so each replay advances the memory.
+    ``capture`` leaves the memory as it found it (its warm-up steps are undone)."""
 
     def __init__(self, B, M, C=256, h=64, w=64, H=1024, W=1024, hp=256, wp=256, D=None, device="cuda",
                  emb_dtype=torch.bfloat16, mask_dtype=torch.float32):
@@ -541,11 +639,14 @@ class StepBuffers:
         emb = self.d["emb"].detach().requires_grad_(backward and emb_grad)
         kw = dict(kw)
         scale = kw.pop("logit_scale", None)
+        memory = kw.pop("memory", None)
         if scale is not None:
             scale = scale.detach().requires_grad_(backward)      # a leaf over the caller's storage: read in place
-        out = region_step(pred, emb, comb, self.d["masks"], logit_scale=scale, **kw)
+        out = region_step(pred, emb, comb, self.d["masks"], logit_scale=scale, memory=memory, **kw)
         if backward:
             out.loss.backward(gradient=self._seed)      # a resident 1.0: no per-step fill kernel from autograd
+        if memory is not None:
+            memory.enqueue(out.regions)                  # after the backward, which needs the rows the forward scored
         grads = {"pred": pred.grad, "comb": comb.grad, "emb": emb.grad}
         if scale is not None:
             grads["logit_scale"] = scale.grad
@@ -553,6 +654,8 @@ class StepBuffers:
 
     def capture(self, backward: bool = True, emb_grad: bool = True, warmup: int = 3, **kw):
         """Warm up on a side stream, then capture fwd+bwd of the step into a CUDA graph."""
+        memory = kw.get("memory")
+        saved = (memory.bank.clone(), memory.state.clone()) if memory is not None else None
         side = torch.cuda.Stream(device=self.device)
         side.wait_stream(torch.cuda.current_stream(self.device))
         with torch.cuda.stream(side):
@@ -560,6 +663,10 @@ class StepBuffers:
                 self._step(backward, emb_grad, kw)
         torch.cuda.current_stream(self.device).wait_stream(side)
         torch.cuda.synchronize(self.device)
+        if saved is not None:                            # undo the warm-up's enqueues
+            memory.bank.copy_(saved[0])
+            memory.state.copy_(saved[1])
+            torch.cuda.synchronize(self.device)
         n0 = ops.LAUNCHES["count"]
         g = torch.cuda.CUDAGraph()
         with torch.cuda.graph(g):

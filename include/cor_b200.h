@@ -296,6 +296,53 @@ int cor_infonce_bwd_umma_ls(const void* regions, const void* queries, int Nr, in
                             const float* lse, const long long* targets, const float* g_loss, float g_mul, float* g_regions,
                             float* g_queries, float* g_logit_scale, void* work, cor_stream_t stream);
 
+/* ------------------------------------------------------------------------------------------
+ * Cross-batch region memory (csrc/memory.cu; Class N, as XBM): a ring of K bf16 unit rows of width D in {64,128,192,256}
+ * (bank [K, D]) that serve the InfoNCE as extra negatives.  state: cor_memory_state_words() int32 on the device,
+ * {head, count, arrival counter, 0}, all zero for an empty memory (one memset) and advanced on the device only, so a
+ * captured CUDA graph moves it at every replay.  The valid rows are bank[0, min(K, count)): the ring is full before it
+ * wraps.  Every entry checks its arguments before any device query (COR_EINVAL).
+ *   cor_memory_enqueue: rows [n, C] f32 or bf16 (16-byte aligned, 1 <= n <= K) -> bank rows (head + i) mod K as bf16
+ *     (round to nearest even); then head = (head + n) mod K, count = min(count + n, K).  One launch, no host sync.
+ *   cor_memory_scan: the log-sum-exp partials of s * queries [Nq, D] bf16 against the valid rows (s = inv_tau, or
+ *     *logit_scale when non-NULL), on the tensor-core kernel that keeps the queries in tensor memory: work
+ *     (cor_memory_scan_work_bytes) holds [ceil(Nq / 256)][*nparts][256][2] (running max, sum); the grid is sized for K
+ *     and CTAs past the fill leave (-inf, 0).  One launch.
+ *   cor_infonce_tail_mem, cor_step_tail_fwd_mem: cor_infonce_tail and cor_step_tail_fwd (inv_tau, or *logit_scale when
+ *     non-NULL) that also merge such partials (mem_part, mem_nparts, the memory's mem_state) into lse:
+ *     lse = logaddexp(lse_current, lse_memory), formed only when count > 0 -- an empty memory leaves lse, nce and total
+ *     bit-equal to mem_part == NULL, which is the entry without the suffix.  cor_infonce_tail_mem also takes
+ *     lse_part == NULL: lse [Nq] then holds the current rows' log-sum-exp on entry (from cor_sim_*_fwd) and nce is formed
+ *     as cor_infonce_fwd forms its loss -- bit-equal to it for an empty memory.
+ *   cor_memory_dq: ADDS the memory rows' share of the InfoNCE gradient, for upstream *g_loss * g_mul:
+ *     g_queries [Nq, D] += g s / Nq sum_j p_qj m_j and *g_logit_scale += g / Nq sum_j p_qj S_qj with p_qj =
+ *     exp(s S_qj - lse[q]) over the valid rows m_j, lse the merged one.  Memory rows are never targets and get no
+ *     gradient.  Either output may be NULL (g_logit_scale needs logit_scale).  The dQ role of the tcgen05 InfoNCE
+ *     backward with the bank as the region operand, then fixed-order folds: 2 launches, 3 with g_logit_scale, 2 without
+ *     g_queries.  work: cor_memory_dq_work_bytes() bytes.  Deterministic.
+ * ---------------------------------------------------------------------------------------- */
+int cor_memory_state_words(void);
+int cor_memory_reset(int* state, cor_stream_t stream);   /* empties the memory: one cudaMemsetAsync of the state */
+int cor_memory_enqueue(const void* rows, int rows_dtype, int n, int C, void* bank, int K, int* state, cor_stream_t stream);
+size_t cor_memory_scan_work_bytes(int Nq, int K, int D);
+int cor_memory_scan(const void* bank, int K, const int* state, const void* queries, int Nq, int D, float inv_tau,
+                    const float* logit_scale, void* work, int* nparts, cor_stream_t stream);
+int cor_infonce_tail_mem(const float* lse_part, int nparts, int qt, const void* regions, const void* queries,
+                         const long long* targets, int Nr, int Nq, int D, float inv_tau, const float* logit_scale,
+                         const float* mem_part, int mem_nparts, const int* mem_state, float* lse, float* nce, float* tgt_logit,
+                         const float* seg, const float* fgbg, float w_fg, float w_bg, float w_nce, float* total,
+                         cor_stream_t stream);
+int cor_step_tail_fwd_mem(const float* part, int nsplit, long long split_stride, int Rp, int B, int M, int C, float p_total,
+                          const float* stats, const void* queries_bf16, const float* comb, const long long* targets, float inv_tau,
+                          const float* logit_scale, const float* mem_part, int mem_nparts, const int* mem_state, const float* seg,
+                          float w_fg, float w_bg, float w_nce, float* fg, void* fg_bf16, float* inv_fg, float* bg, float* inv_bg,
+                          float* fgbg_out4, float* aux, float* lse, float* nce, float* tgt_logit, float* total, void* work,
+                          unsigned* counter, cor_stream_t stream);
+size_t cor_memory_dq_work_bytes(int Nq, int K, int D);
+int cor_memory_dq(const void* bank, int K, const int* state, const void* queries, int Nq, int D, float inv_tau,
+                  const float* logit_scale, const float* lse, const float* g_loss, float g_mul, float* g_queries,
+                  float* g_logit_scale, void* work, cor_stream_t stream);
+
 /* Top-k retrieval: per query the k best regions under (score desc, index asc), where score is the
  * canonical value fl32(sum in fp64 of exact bf16 products).  S is the (tensor-core) prefilter
  * matrix from cor_sim_*; the top (k + slack) prefilter candidates are re-scored exactly.

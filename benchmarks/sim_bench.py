@@ -3,7 +3,6 @@
 events, median of --iters; log-sum-exp checked against an fp32 torch restatement on the same bf16 operands.
 
     python benchmarks/sim_bench.py [--shapes 1024x102400,16x102400,256x4096]
-    COR_B200_LIB=cor_b200/build/ab/libcor_b200_poly1.so python benchmarks/sim_bench.py   # an A/B build (build_variants.sh)
 """
 import argparse
 import json

@@ -7,7 +7,6 @@
 // HBM-bound streaming kernel: every mask byte is read exactly once with 128-bit no-allocate loads;
 // the 4 taps per output pixel hit lines the same CTA streams.  Deterministic: per-CTA partials in
 // double, reduced in fixed order by a second tiny kernel.
-#include <stdlib.h>
 
 #include "common.cuh"
 
@@ -357,8 +356,9 @@ extern "C" int cor_mask_prep(const void* masks, int mask_dtype, float mask_scale
   const long long band_max = ((long long)ceil_div(h, chunks_s) * Hm + h - 1) / h + 2;
   const size_t smem_s = (size_t)2 * max_ro * row_bytes + (size_t)band_max * sizeof(short) + 16;
   // measured on B200 (profiles/): staged beats the two-phase kernel for every mask dtype (f32 0.70 vs 0.73 ms, u8 0.24 vs
-  // 0.49 ms at 1024 masks of 1024^2); COR_PREP_TWO_PHASE=1 forces the two-phase kernel for A/B runs.
-  const bool staged = !getenv("COR_PREP_TWO_PHASE") && (row_bytes % 16 == 0) && (((uintptr_t)masks & 15) == 0) && smem_s <= 96 * 1024 && band_max <= kMaxBand &&
+  // 0.49 ms at 1024 masks of 1024^2); the two-phase kernel takes what staged cannot: up-sampling (Hm < h), unaligned
+  // rows and bands over budget.
+  const bool staged = (row_bytes % 16 == 0) && (((uintptr_t)masks & 15) == 0) && smem_s <= 96 * 1024 && band_max <= kMaxBand &&
                       ceil_div(h, chunks_s) <= max_ro && chunks_s <= h && Hm >= h;
   int chunks = staged ? chunks_s : pick_chunks(n_masks, Hm, Wm, h, es);
   COR_REQUIRE((long long)n_masks * chunks < 2147483647LL, "cor_mask_prep: grid too large");

@@ -6,8 +6,9 @@
 // Neither S nor P ever exists in global memory.  ONE kernel serves both products, with the roles of the operands
 // swapped (mode 0: X = queries, Y = regions, G = dQ;  mode 1: X = regions, Y = queries, G = dR):
 //
-//   a CTA keeps 128 X rows resident in shared memory and walks Y tiles of 64 rows:
-//     GEMM 1   S^(X)[128 x 64] = X Y^T             A = X (K-major, TMA, SW128)      B = Y tile (K-major)
+//   a CTA keeps 128 X rows resident in tensor memory and walks Y tiles of 64 rows through shared memory:
+//     GEMM 1   S^(X)[128 x 64] = X Y^T             A = X (TMEM: row x in lane x, two bf16 per column, stored once by
+//              the epilogue threads)                B = Y tile (K-major, TMA, SW128)
 //     epilogue the thread that owns TMEM lane x turns its S row into bf16 coefficients and stores them into
 //              shared memory in the canonical K-major SW128 layout (manual swizzle) -> A operand of GEMM 2
 //     GEMM 2   G[128 x D] += P[128 x 64] Y          A = P (K-major, K = Y rows)      B = THE SAME Y TILE, read
@@ -15,9 +16,10 @@
 //              8-row x 128-byte groups TMA wrote; LBO = distance between 64-wide d blocks, SBO = 1024 B)
 //   so every Y byte fetched from L2 feeds both GEMMs.  A Y tile stays in shared memory from its load to the end of its
 //   GEMM 2, i.e. through a whole TMA -> GEMM 1 -> epilogue -> GEMM 2 round trip: the tiles are kept SMALL (64 rows, 32 KB
-//   at D = 256) so that FOUR of them fit beside X -- with two 128-row slots the next load could only start when a GEMM 2
+//   at D = 256) and up to four of them are in flight -- with two 128-row slots the next load could only start when a GEMM 2
 //   finished and the tensor pipe idled through every load latency (measured 5 700 cycles per 128 rows against 2 048 of
-//   tensor work).  TMEM: S double-buffered (2 x 64 columns), P double-buffered in shared memory, G in 256 columns.
+//   tensor work).  TMEM: S double-buffered (2 x 64 columns), X in D/2 columns from 128, G in 256 columns; P double-buffered
+//   in shared memory.
 //
 // Warp roles (320 threads): 0..7 = epilogue (warp w owns TMEM lane quarter w % 4 and column half w / 4, i.e. exactly one
 // 128-byte row of one P k-block per thread), 8 = TMA producer, 9 = TMEM owner + MMA issuer (highest warp ids: the
@@ -38,14 +40,11 @@ using namespace umma;
 constexpr int kNbM = 128;                  // X rows per CTA (UMMA M)
 constexpr int kNbN = 64;                   // Y rows per tile (GEMM 1 N, GEMM 2 K)
 constexpr int kNbBK = 64;
-constexpr int kNbBlk = kNbM * kNbBK * 2;   // 16 KB: one 64-wide k-block of the 128 X rows; also one P buffer [128 x 64]
+constexpr int kNbBlk = kNbM * kNbBK * 2;   // 16 KB: one P buffer [128 x 64]
 constexpr int kNbYBlk = kNbN * kNbBK * 2;  // 8 KB: one 64-wide k-block of a Y tile
 constexpr int kNbMaxSlots = 4;
 constexpr int kNbTmaWarp = 8, kNbMmaWarp = 9;
 constexpr int kNbPrefetch = 3;
-#ifndef COR_NCE_TS
-#define COR_NCE_TS 1                       // 1: the X tile lives in TMEM (GEMM 1 in its A-from-TMEM form); 0: in shared memory (A/B)
-#endif
 
 struct NceSmemTail {
   uint64_t xfull, yfull[kNbMaxSlots], yempty[kNbMaxSlots], s_full[2], s_empty[2], p_full[2], p_empty[2], g_full;
@@ -64,7 +63,7 @@ struct NceArgs {
   const int* count;                        // device row count: Y rows past min(Ny, *count) are not scored; or NULL
   const float* g_loss;                     // [1]
   float* out;                              // [gridDim.x][Nx][D] partials (or the result itself when gridDim.x == 1); NULL = not written
-  const bf16* X;                           // [Nx][D] the CTA's rows, read by the epilogue threads when the X tile lives in TMEM
+  const bf16* X;                           // [Nx][D]: the epilogue threads store the CTA's rows into TMEM
 };
 
 // instruction descriptor with an MN-major B operand (bit 16)
@@ -89,12 +88,10 @@ __device__ __forceinline__ uint32_t pack_bf16x2_rn(float lo, float hi) {
   return r;
 }
 
-__global__ void __launch_bounds__(320, 1) nce_bwd_umma_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmY,
-                                                              NceArgs a) {
+__global__ void __launch_bounds__(320, 1) nce_bwd_umma_kernel(const __grid_constant__ CUtensorMap tmY, NceArgs a) {
   extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t* base = reinterpret_cast<uint8_t*>(((uintptr_t)smem + 1023) & ~(uintptr_t)1023);
-  uint8_t* x_smem = base;                                                    // nkb x 16 KB (only when the X tile is not kept in TMEM)
-  uint8_t* y_smem = x_smem + (COR_NCE_TS ? 0 : (size_t)a.nkb * kNbBlk);      // nslots x nkb x 8 KB
+  uint8_t* y_smem = base;                                                    // nslots x nkb x 8 KB
   uint8_t* p_smem = y_smem + (size_t)a.nslots * a.nkb * kNbYBlk;             // 2 buffers x 16 KB
   NceSmemTail* tail = reinterpret_cast<NceSmemTail*>(p_smem + 2 * kNbBlk);
 
@@ -106,9 +103,8 @@ __global__ void __launch_bounds__(320, 1) nce_bwd_umma_kernel(const __grid_const
   const int n_my = (ntiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;      // tiles blockIdx.x, +gridDim.x, ...
 
   if (warp == 0 && lane == 0) {
-    prefetch_tmap(&tmX);
     prefetch_tmap(&tmY);
-    mbar_init(&tail->xfull, COR_NCE_TS ? 4 : 1);
+    mbar_init(&tail->xfull, 4);
     for (int i = 0; i < a.nslots; ++i) { mbar_init(&tail->yfull[i], 1); mbar_init(&tail->yempty[i], 1); }
     for (int i = 0; i < 2; ++i) { mbar_init(&tail->s_full[i], 1); mbar_init(&tail->s_empty[i], 8); }
     for (int i = 0; i < 2; ++i) { mbar_init(&tail->p_full[i], 8); mbar_init(&tail->p_empty[i], 1); }
@@ -121,14 +117,10 @@ __global__ void __launch_bounds__(320, 1) nce_bwd_umma_kernel(const __grid_const
   tc_fence_after();
   const uint32_t tmem = tail->tmem_base;
   const uint32_t tmem_g = tmem + 256u;
-  const uint32_t tmem_x = tmem + 128u;             // TS form: X rows in lanes, D/2 packed-bf16 columns [128, 128 + D/2)
+  const uint32_t tmem_x = tmem + 128u;             // X rows in lanes, D/2 packed-bf16 columns [128, 128 + D/2)
 
   if (warp == kNbTmaWarp) {
     if (lane == 0) {
-#if !COR_NCE_TS
-      mbar_expect_tx(&tail->xfull, (uint32_t)(a.nkb * kNbBlk));
-      for (int kb = 0; kb < a.nkb; ++kb) tma_load_2d(x_smem + kb * kNbBlk, &tmX, &tail->xfull, kb * kNbBK, x0, kEvictNormal);
-#endif
       for (int i = 0; i < n_my && i < kNbPrefetch; ++i)
         for (int kb = 0; kb < a.nkb; ++kb) tma_prefetch_2d(&tmY, kb * kNbBK, ((int)blockIdx.x + i * (int)gridDim.x) * kNbN);
       for (int i = 0; i < n_my; ++i) {
@@ -148,7 +140,7 @@ __global__ void __launch_bounds__(320, 1) nce_bwd_umma_kernel(const __grid_const
       const bool leader = elect_one();
       const uint32_t idesc1 = make_idesc_bf16(kNbM, kNbN);
       const uint32_t idesc2 = make_idesc_bf16_bmn(kNbM, D);
-      const uint32_t x_base = smem_u32(x_smem), y_base = smem_u32(y_smem), p_base = smem_u32(p_smem);
+      const uint32_t y_base = smem_u32(y_smem), p_base = smem_u32(p_smem);
       mbar_wait(&tail->xfull, 0);
       tc_fence_after();
       auto gemm1 = [&](int i) {
@@ -159,19 +151,12 @@ __global__ void __launch_bounds__(320, 1) nce_bwd_umma_kernel(const __grid_const
         if (leader) {
           for (int kb = 0; kb < a.nkb; ++kb) {
             const uint64_t db = make_desc_sw128(y_base + (uint32_t)((slot * a.nkb + kb) * kNbYBlk));
-#if COR_NCE_TS
             // A from TMEM: 16 k-elements = 8 packed columns per MMA; only the Y tile is fetched from shared memory (with both
             // operands there the 64 KB X tile was re-read for every 64-row Y tile: 144 KB of operand fetch per tile against
             // ~1 000 tensor cycles, i.e. shared-memory bandwidth, not the tensor pipe, paced the loop)
 #pragma unroll
             for (int k = 0; k < kNbBK / 16; ++k)
               mma_bf16_ts(tmem + (uint32_t)(buf * kNbN), tmem_x + (uint32_t)(kb * (kNbBK / 2) + k * 8), db + 2 * k, idesc1, (kb | k) != 0);
-#else
-            const uint64_t da = make_desc_sw128(x_base + (uint32_t)(kb * kNbBlk));
-            mma_bf16_ss(tmem + (uint32_t)(buf * kNbN), da, db, idesc1, kb != 0);
-#pragma unroll
-            for (int k = 1; k < kNbBK / 16; ++k) mma_bf16_ss_acc(tmem + (uint32_t)(buf * kNbN), da + 2 * k, db + 2 * k, idesc1);
-#endif
           }
           mma_commit(&tail->s_full[buf]);
         }
@@ -207,7 +192,6 @@ __global__ void __launch_bounds__(320, 1) nce_bwd_umma_kernel(const __grid_const
     const int row = qd * 32 + lane;
     const int xg = x0 + row;
     const bool xok = xg < a.Nx;
-#if COR_NCE_TS
     // ---- this thread's X row -> TMEM (its own lane), two bf16 per 32-bit column; the four warps of column half 0 cover the
     // 128 lanes ----
     if (half == 0) {
@@ -231,7 +215,6 @@ __global__ void __launch_bounds__(320, 1) nce_bwd_umma_kernel(const __grid_const
       __syncwarp();
       if (lane == 0) mbar_arrive(&tail->xfull);
     }
-#endif
     const float log2e = 1.4426950408889634f;
     float c2 = a.c2, gmul = a.gmul;
     if (a.scale) {
@@ -389,13 +372,12 @@ static int nce_launch(const void* X, const void* Y, int Nx, int Ny, int Nq, int 
   const int nkb = D / kNbBK;
   const int xtiles = ceil_div(Nx, kNbM), ytiles = ceil_div(Ny, kNbN);
   const int nsplit = nce_splits(xtiles, ytiles);
-  CUtensorMap tmX, tmY;
-  int rc = encode_tmap_bf16_2d(&tmX, X, (uint64_t)Nx, (uint64_t)D, kNbM, kNbBK);
+  COR_REQUIRE(((uintptr_t)X & 15) == 0, "cor_infonce_bwd_umma: X rows are read as 16-byte vectors: X must be 16-byte aligned");
+  CUtensorMap tmY;
+  int rc = encode_tmap_bf16_2d(&tmY, Y, (uint64_t)Ny, (uint64_t)D, kNbN, kNbBK);
   if (rc) return rc;
-  rc = encode_tmap_bf16_2d(&tmY, Y, (uint64_t)Ny, (uint64_t)D, kNbN, kNbBK);
-  if (rc) return rc;
-  // shared memory: X (nkb blocks) + 2 P buffers + as many whole-Y-tile slots as fit (4 at D = 256)
-  const size_t fixed = (size_t)((COR_NCE_TS ? 0 : nkb) + 2) * kNbBlk + sizeof(NceSmemTail) + 1024;
+  // shared memory: 2 P buffers + as many whole-Y-tile slots as fit, at most kNbMaxSlots
+  const size_t fixed = (size_t)2 * kNbBlk + sizeof(NceSmemTail) + 1024;
   int nslots = (int)((227 * 1024 - fixed) / ((size_t)nkb * kNbYBlk));
   if (nslots > kNbMaxSlots) nslots = kNbMaxSlots;
   COR_REQUIRE(nslots >= 2, "cor_infonce_bwd_umma: shared memory budget (D=%d)", D);
@@ -410,7 +392,7 @@ static int nce_launch(const void* X, const void* Y, int Nx, int Ny, int Nq, int 
   a.X = reinterpret_cast<const bf16*>(X);
   const bool direct = nsplit == 1 && !accumulate;
   a.out = !out ? nullptr : (direct ? out : part);
-  nce_bwd_umma_kernel<<<dim3(nsplit, xtiles), 320, smem, st>>>(tmX, tmY, a);
+  nce_bwd_umma_kernel<<<dim3(nsplit, xtiles), 320, smem, st>>>(tmY, a);
   rc = check_launch("nce_bwd_umma_kernel");
   if (rc || direct || !out) return rc;
   const long long vecs = (long long)Nx * D / 4;

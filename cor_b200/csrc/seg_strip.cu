@@ -234,10 +234,6 @@ int seg_strip_max_strips(int H) { return ceil_div(H, 16); }
 static int strip_rows(int N, int H) {
   // largest strip (least halo re-reads: (R+30)/R of the rows come through L2) that still fills most of the machine's
   // 2-CTAs-per-SM slots in ONE wave (a second, partly filled wave costs more than a few idle slots)
-  if (const char* e = getenv("COR_SEG_STRIP_ROWS")) {      // A/B knob
-    const int r = atoi(e);
-    if (r >= 16 && r <= 256) return r;
-  }
   const long long want = (long long)2 * sm_count() * kStripFill / 100;
   for (int R = 128; R >= 32; R >>= 1)
     if ((long long)N * ceil_div(H, R) >= want) return R;

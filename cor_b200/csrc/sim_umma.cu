@@ -37,16 +37,6 @@ constexpr int kSimMaxKB = 4;                       // D <= 256
 constexpr int kSimTmaWarp = 8, kSimMmaWarp = 9;    // epilogue = warps 0..7
 static_assert(kSimBN == 128, "the epilogue is unrolled for four 32-column chunks");
 
-#ifdef COR_SIM_TRACE
-// Debug build only (benchmarks/build_variants.sh ... "-DCOR_SIM_TRACE"): CTA (0,0) stamps clock64() at the hand-offs of
-// its first 32 tiles: [tile][0] MMA thread starts issuing, [1] all MMAs of the tile issued, [2] epilogue warp 0 sees
-// acc_full, [3] its last TMEM load has landed (buffer released), [4] tile done, [5] producer issued the tile's last stage.
-__device__ long long g_sim_trace[32][8];
-#define SIM_TRACE(tile, ev) do { if (blockIdx.x == 0 && blockIdx.y == 0 && (tile) < 32) g_sim_trace[(tile)][(ev)] = clock64(); } while (0)
-#else
-#define SIM_TRACE(tile, ev) do { } while (0)
-#endif
-
 struct SimSmemTail {
   uint64_t qfull, full[kSimMaxStages], empty[kSimMaxStages], acc_full[2], acc_empty[2];
   uint32_t tmem_base;
@@ -93,13 +83,12 @@ __global__ void __launch_bounds__(320, 1) sim_umma_kernel(const __grid_constant_
           mbar_expect_tx(&tail->full[st], kSimBBytes);
           tma_load_2d(r_smem + st * kSimBBytes, &tmR, &tail->full[st], kb * kSimBK, t * kSimBN, gridDim.y > 1 ? kEvictLast : kEvictFirst);
         }
-        SIM_TRACE((t - (int)blockIdx.x) / (int)gridDim.x, 5);
       }
     }
   } else if (warp == kSimMmaWarp) {
     // The WHOLE warp walks this loop (barrier waits, descriptor arithmetic) and one elected lane issues: with the role
     // wrapped in `if (lane == 0)` the compiler must treat every descriptor as divergent (R2UR + ELECT + BRA.U.ANY around
-    // each UTCHMMA, ~140 cycles per MMA on a lone warp's dependent-issue chain -- measured with the trace build: 4 450
+    // each UTCHMMA, ~140 cycles per MMA on a lone warp's dependent-issue chain -- measured with clock64() stamps: 4 450
     // cycles to issue the 32 MMAs of a tile that the tensor pipe executes in 2 048).
     const bool leader = elect_one();
     const uint32_t idesc = make_idesc_bf16(kSimHalf, kSimBN);
@@ -112,7 +101,6 @@ __global__ void __launch_bounds__(320, 1) sim_umma_kernel(const __grid_constant_
       const int buf = i & 1;
       mbar_wait(&tail->acc_empty[buf], ((i >> 1) & 1) ^ 1);
       tc_fence_after();
-      if (leader) SIM_TRACE(i, 0);
       for (int kb = 0; kb < nkb; ++kb) {
         if (!ready) mbar_wait(&tail->full[st], ph);
         tc_fence_after();
@@ -136,7 +124,6 @@ __global__ void __launch_bounds__(320, 1) sim_umma_kernel(const __grid_constant_
       }
       if (leader) {
         mma_commit(&tail->acc_full[buf]);
-        SIM_TRACE(i, 1);
       }
       __syncwarp();
     }
@@ -169,7 +156,6 @@ __global__ void __launch_bounds__(320, 1) sim_umma_kernel(const __grid_constant_
       const int buf = i & 1;
       mbar_wait(&tail->acc_full[buf], (i >> 1) & 1);
       tc_fence_after();
-      if (warp == 0 && lane == 0) SIM_TRACE(i, 2);
       if (active) {
         const int r0 = t * kSimBN;
         const uint32_t taddr = tmem + ((uint32_t)(qd * 32) << 16) + (uint32_t)((buf * 2 + hf) * kSimBN);
@@ -192,9 +178,7 @@ __global__ void __launch_bounds__(320, 1) sim_umma_kernel(const __grid_constant_
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(&tail->acc_empty[buf]);
-        if (warp == 0 && lane == 0) SIM_TRACE(i, 3);
         if (nch > 3) proc(vb, r0, 96);
-        if (warp == 0 && lane == 0) SIM_TRACE(i, 4);
       } else {
         tc_fence_before();
         __syncwarp();
@@ -262,11 +246,3 @@ extern "C" int cor_sim_umma_fwd_ls(const void* regions, const void* queries, int
   COR_REQUIRE(logit_scale, "cor_sim_umma_fwd_ls: null logit_scale");
   return cor::sim_umma_launch(regions, queries, Nr, Nq, D, 0.f, logit_scale, S, lse, work, nullptr, nullptr, as_stream(stream));
 }
-
-#ifdef COR_SIM_TRACE
-extern "C" int cor_debug_sim_trace(long long* host_out) {
-  COR_CUDA(cudaDeviceSynchronize());
-  COR_CUDA(cudaMemcpyFromSymbol(host_out, cor::g_sim_trace, sizeof(long long) * 32 * 8));
-  return COR_OK;
-}
-#endif

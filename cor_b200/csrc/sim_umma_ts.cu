@@ -26,9 +26,6 @@ constexpr int kTsHalf = 128, kTsBM = 256, kTsBN = 128, kTsBK = 64;
 constexpr int kTsBBytes = kTsBN * kTsBK * 2;     // 16 KB: one stage of regions
 constexpr int kTsMaxStages = 14;
 constexpr int kTsTmaWarp = 8, kTsMmaWarp = 9;
-#ifndef COR_SIM_TS_POLY_OF4
-#define COR_SIM_TS_POLY_OF4 0          // of every 4 element pairs, how many take the FMA-pipe exp2 instead of MUFU (A/B knob)
-#endif
 
 struct TsSmemTail {
   uint64_t afull, full[kTsMaxStages], empty[kTsMaxStages], acc_full[2], acc_empty[2];
@@ -159,14 +156,9 @@ __global__ void __launch_bounds__(320, 1) sim_umma_ts_kernel(const __grid_consta
 #pragma unroll
         for (int j = 0; j < 16; ++j) {
           const uint64_t x2 = fma2(pack2u(v[2 * j], v[2 * j + 1]), C2, NM);
-          uint64_t e2;
-          if ((j % 4) < COR_SIM_TS_POLY_OF4) {
-            e2 = exp2_poly2(x2);
-          } else {
-            float x0, x1;
-            unpack2(x2, x0, x1);
-            e2 = pack2(ex2_approx(x0), ex2_approx(x1));
-          }
+          float x0, x1;
+          unpack2(x2, x0, x1);
+          const uint64_t e2 = pack2(ex2_approx(x0), ex2_approx(x1));
           if (j & 1) a1 = add2(a1, e2);
           else a0 = add2(a0, e2);
         }

@@ -188,36 +188,10 @@ __device__ __forceinline__ uint64_t add2(uint64_t a, uint64_t b) {
   asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
   return d;
 }
-__device__ __forceinline__ uint64_t sub2(uint64_t a, uint64_t b) {
-  uint64_t d;
-  asm("sub.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(a), "l"(b));
-  return d;
-}
 __device__ __forceinline__ float max3(float a, float b, float c) {
   float d;
   asm("max.f32 %0, %1, %2, %3;" : "=f"(d) : "f"(a), "f"(b), "f"(c));
   return d;
-}
-
-// 2^x for a PAIR of arguments x <= 0 on the FMA pipe (no MUFU): Cody-Waite split x = n + f, n = round(x) taken from the
-// low mantissa bits of x + 1.5*2^23, 2^f on [-0.5, 0.5] by a degree-5 minimax polynomial (max relative error 2.4e-7, the
-// same as ex2.approx), then n added into the exponent field.  Arguments below -126 are clamped (result ~1e-38).
-__device__ __forceinline__ uint64_t exp2_poly2(uint64_t x2) {
-  float x0, x1;
-  unpack2(x2, x0, x1);
-  x2 = pack2(fmaxf(x0, -126.f), fmaxf(x1, -126.f));
-  const uint64_t magic = pack2(12582912.f, 12582912.f);
-  const uint64_t t2 = add2(x2, magic);
-  const uint64_t f2 = sub2(x2, sub2(t2, magic));
-  uint64_t p2 = pack2(0x1.5c08e4p-10f, 0x1.5c08e4p-10f);
-  p2 = fma2(p2, f2, pack2(0x1.3d0c52p-7f, 0x1.3d0c52p-7f));
-  p2 = fma2(p2, f2, pack2(0x1.c6b6e4p-5f, 0x1.c6b6e4p-5f));
-  p2 = fma2(p2, f2, pack2(0x1.ebf918p-3f, 0x1.ebf918p-3f));
-  p2 = fma2(p2, f2, pack2(0x1.62e428p-1f, 0x1.62e428p-1f));
-  p2 = fma2(p2, f2, pack2(0x1.000002p+0f, 0x1.000002p+0f));
-  const uint32_t r0 = (uint32_t)p2 + ((uint32_t)t2 << 23);
-  const uint32_t r1 = (uint32_t)(p2 >> 32) + ((uint32_t)(t2 >> 32) << 23);
-  return pack2u(r0, r1);
 }
 
 // D[tmem] (+)= A[tmem] * B[smem]^T : A rows in TMEM lanes, K elements packed two bf16 per 32-bit column

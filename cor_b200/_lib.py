@@ -30,21 +30,41 @@ class CorError(RuntimeError):
     """A libcor_b200 call returned a non-zero status."""
 
 
+# C types of the header -> ctypes.  Every pointer is a c_void_p; a type outside this table is an error, not a guess.
+_SCALARS = {"int": C.c_int, "float": C.c_float, "long long": C.c_longlong, "size_t": C.c_size_t, "cor_stream_t": C.c_void_p}
+_DECL = re.compile(r"^[ \t]*([A-Za-z_][\w \t*]*?)\s*\b(cor_\w+)\s*\(([^;]*?)\)\s*;", re.M)
+
+
+def _ctype(fn: str, t: str, returned: bool = False):
+    t = " ".join(t.replace("*", " * ").split())
+    if returned and t == "const char *":
+        return C.c_char_p                     # cor_last_error(): check() decodes it
+    if "*" in t and re.fullmatch(r"[\w *]+", t):
+        return C.c_void_p
+    if t in _SCALARS:
+        return _SCALARS[t]
+    raise CorError(f"{fn}: no ctypes mapping for the type `{t}` declared in the header")
+
+
+def declarations(header: str = HEADER):
+    """{name: (restype, argtypes)} of every function the header declares, typed from the header itself."""
+    if not os.path.exists(header):
+        raise CorError(f"{header} not found: the C ABI header types every entry of libcor_b200.so")
+    text = re.sub(r"/\*.*?\*/|//[^\n]*", "", open(header).read(), flags=re.S)
+    decls = {}
+    for ret, name, params in _DECL.findall(text):
+        params = [] if params.strip() in ("", "void") else params.split(",")
+        decls[name] = (_ctype(name, ret, returned=True), [_ctype(name, re.sub(r"\b\w+\s*$", "", p)) for p in params])
+    return decls
+
+
 def declared_symbols(header: str = HEADER):
     """Names of every function include/cor_b200.h declares (used by the CPU export test)."""
-    text = re.sub(r"/\*.*?\*/", "", open(header).read(), flags=re.S)
-    return sorted(set(re.findall(r"\b(cor_[a-z0-9_]+)\s*\(", text)))
-
-
-def _sig(lib, name, restype, *argtypes):
-    fn = getattr(lib, name)
-    fn.restype = restype
-    fn.argtypes = list(argtypes)
-    return fn
+    return sorted(declarations(header))
 
 
 def load(path: str = LIB_PATH):
-    """dlopen the library (works without a GPU: cudart is linked statically) and type every entry.
+    """dlopen the library (works without a GPU: cudart is linked statically) and type every entry from the header.
     ``COR_B200_LIB`` points at another build of the same ABI (A/B runs of two kernel versions on one box)."""
     global _lib
     with _lock:
@@ -55,107 +75,11 @@ def load(path: str = LIB_PATH):
             raise CorError(
                 f"{path} not found: build it with `python -m cor_b200.build` (nvcc, sm_100a). "
                 "cor_b200 has no CPU or PyTorch fallback by design.")
+        decls = declarations()
         lib = C.CDLL(path)
-        p, i, f, ll, sz = C.c_void_p, C.c_int, C.c_float, C.c_longlong, C.c_size_t
-        _sig(lib, "cor_abi_version", i)
-        _sig(lib, "cor_last_error", C.c_char_p)
-        _sig(lib, "cor_device_info", i, C.POINTER(i), C.POINTER(i), C.POINTER(i))
-        _sig(lib, "cor_mask_prep_work_bytes", sz, i, i, i, i, i)
-        _sig(lib, "cor_mask_prep", i, p, i, f, i, i, i, i, i, i, p, p, ll, i, ll, p, p, p)
-        _sig(lib, "cor_pool_stream_fwd", i, p, i, p, ll, i, i, i, i, i, p, p, p)
-        _sig(lib, "cor_pool_umma_work_bytes", sz, i, i, i, i)
-        _sig(lib, "cor_pool_umma_ksplit", i, i, i, i)
-        _sig(lib, "cor_pool_umma_fwd", i, p, p, i, i, i, i, p, p)
-        _sig(lib, "cor_rows_finalize", i, p, i, ll, i, ll, p, i, f, i, i, i, i, p, f, p, p, p, p)
-        _sig(lib, "cor_rows_finalize_bwd", i, p, p, p, p, i, f, i, i, i, i, i, f, p, p)
-        _sig(lib, "cor_pool_bwd_feat", i, p, p, p, ll, i, i, i, i, i, p, i, p)
-        _sig(lib, "cor_pool_bwd_umma_ok", i, i, i, i, i, i)
-        _sig(lib, "cor_pool_bwd_umma", i, p, p, p, ll, i, i, i, i, i, p, i, p)
-        _sig(lib, "cor_pool_bwd_maps", i, p, i, p, ll, p, p, p, i, i, i, i, p, p)
-        _sig(lib, "cor_fgbg_aux_floats", sz, i, i)
-        _sig(lib, "cor_fgbg_loss_fwd", i, p, ll, p, ll, p, ll, p, ll, i, i, i, p, p, p)
-        _sig(lib, "cor_fgbg_loss_bwd", i, p, ll, p, ll, p, ll, i, i, i, p, p, p, ll, f, f, p, ll, i, p, ll, p, ll, i, p)
-        _sig(lib, "cor_step_tail_counter_words", i)
-        _sig(lib, "cor_step_tail_work_bytes", sz, i, i, i)
-        _sig(lib, "cor_step_tail_fwd", i, p, i, ll, i, i, i, i, f, p, p, p, p, f, p, f, f, f, p, p, p, p, p, p, p, p, p, p, p, p, p, p)
-        _sig(lib, "cor_step_tail_bwd", i, p, p, p, p, i, i, i, f, p, f, p, p, p, p, p, p, f, f, p, i, p, p, p, p)
-        _sig(lib, "cor_step_tail_fwd_ls", i, p, i, ll, i, i, i, i, f, p, p, p, p, p, p, f, f, f, p, p, p, p, p, p, p, p, p, p, p, p, p, p)
-        _sig(lib, "cor_step_tail_bwd_ls", i, p, p, p, p, i, i, i, p, p, f, p, p, p, p, p, p, f, f, p, i, p, p, p, p, p)
-        _sig(lib, "cor_seg_loss_work_bytes", sz, i, i, i)
-        _sig(lib, "cor_seg_loss_npartials", i)
-        fp = C.POINTER(C.c_float)
-        _sig(lib, "cor_seg_loss_fwd", i, p, i, p, i, f, i, i, i, i, i, ll, fp, f, f, f, p, p, p, p, p, p)
-        _sig(lib, "cor_seg_loss_bwd", i, p, i, p, p, p, i, i, i, fp, f, f, f, p, p, i, p)
-        _sig(lib, "cor_sim_work_bytes", sz, i, i, i)
-        _sig(lib, "cor_sim_stream_fwd", i, p, p, i, i, i, f, p, p, p, p)
-        _sig(lib, "cor_sim_umma_fwd", i, p, p, i, i, i, f, p, p, p, p)
-        _sig(lib, "cor_infonce_fwd", i, p, p, p, p, i, i, i, f, p, p, p)
-        _sig(lib, "cor_sim_lse_parts", i, i, p, p, i, i, i, f, p, C.POINTER(i), C.POINTER(i), p)
-        _sig(lib, "cor_infonce_tail", i, p, i, i, p, p, p, i, i, i, f, p, p, p, p, p, f, f, f, p, p)
-        _sig(lib, "cor_infonce_bwd", i, p, p, p, p, i, i, i, f, p, f, p, p, p, p)
-        _sig(lib, "cor_infonce_bwd_umma_work_bytes", sz, i, i, i)
-        _sig(lib, "cor_infonce_bwd_umma", i, p, p, i, i, i, f, p, p, p, f, p, p, p, p)
-        # the same entries with the logit scale read from device memory (and its gradient written there)
-        _sig(lib, "cor_sim_stream_fwd_ls", i, p, p, i, i, i, p, p, p, p, p)
-        _sig(lib, "cor_sim_umma_fwd_ls", i, p, p, i, i, i, p, p, p, p, p)
-        _sig(lib, "cor_sim_lse_parts_ls", i, i, p, p, i, i, i, p, p, C.POINTER(i), C.POINTER(i), p)
-        _sig(lib, "cor_infonce_tail_ls", i, p, i, i, p, p, p, i, i, i, p, p, p, p, p, p, f, f, f, p, p)
-        _sig(lib, "cor_infonce_fwd_ls", i, p, p, p, p, i, i, i, p, p, p, p)
-        _sig(lib, "cor_infonce_bwd_ls", i, p, p, p, p, i, i, i, p, p, f, p, p, p, p, p)
-        _sig(lib, "cor_infonce_bwd_umma_ls", i, p, p, i, i, i, p, p, p, p, f, p, p, p, p, p)
-        # cross-batch region memory
-        _sig(lib, "cor_memory_state_words", i)
-        _sig(lib, "cor_memory_reset", i, p, p)
-        _sig(lib, "cor_memory_enqueue", i, p, i, i, i, p, i, p, p)
-        _sig(lib, "cor_memory_scan_work_bytes", sz, i, i, i)
-        _sig(lib, "cor_memory_scan", i, p, i, p, p, i, i, f, p, p, C.POINTER(i), p)
-        _sig(lib, "cor_infonce_tail_mem", i, p, i, i, p, p, p, i, i, i, f, p, p, i, p, p, p, p, p, p, f, f, f, p, p)
-        _sig(lib, "cor_step_tail_fwd_mem", i, p, i, ll, i, i, i, i, f, p, p, p, p, f, p, p, i, p, p, f, f, f, p, p, p, p, p, p, p, p, p,
-             p, p, p, p, p)
-        _sig(lib, "cor_memory_dq_work_bytes", sz, i, i, i)
-        _sig(lib, "cor_memory_dq", i, p, i, p, p, i, i, f, p, p, p, f, p, p, p, p)
-        _sig(lib, "cor_topk", i, p, p, p, i, i, i, i, p, p, p)
-        _sig(lib, "cor_l2_normalize", i, p, i, i, i, p, p, p, p)
-        _sig(lib, "cor_gemm_bf16_work_bytes", sz, i, i, i, i, i)
-        _sig(lib, "cor_gemm_bf16", i, p, i, ll, ll, p, i, ll, ll, i, i, i, i, f, p, i, p, p, p, i, ll, p, i, ll, p, i, p, p)
-        _sig(lib, "cor_cast_cat_bf16", i, p, i, p, i, ll, p, p)
-        _sig(lib, "cor_cast_pad_rows_bf16", i, p, i, i, i, i, p, p)
-        _sig(lib, "cor_act_bwd_work_bytes", sz, ll, i)
-        _sig(lib, "cor_act_bwd", i, p, i, p, p, p, p, i, ll, i, p, p, p, p, p)
-        _sig(lib, "cor_dwconv7_work_bytes", sz, i, i, i, i)
-        _sig(lib, "cor_dwconv7_cl", i, p, p, p, p, i, i, i, i, i, p)
-        _sig(lib, "cor_dwconv7_cl_wgrad", i, p, p, p, p, i, i, i, i, p, p)
-        _sig(lib, "cor_ln_rows_work_bytes", sz, ll, i)
-        _sig(lib, "cor_ln_rows_fwd", i, p, p, p, ll, i, f, i, p, i, p, p)
-        _sig(lib, "cor_ln_rows_bwd", i, p, i, p, p, p, p, ll, i, i, p, p, p, p, p)
-        _sig(lib, "cor_ln_cf_work_bytes", sz, ll, i, ll)
-        _sig(lib, "cor_ln_cf_fwd", i, p, p, p, ll, i, ll, f, i, p, p)
-        _sig(lib, "cor_ln_cf_bwd", i, p, p, p, p, ll, i, ll, f, i, p, p, p, p, p)
-        _sig(lib, "cor_adapter_tail_weights", i, p, i, i, i, i, i, p, p, p)
-        _sig(lib, "cor_adapter_tail_bwd", i, p, p, p, i, i, i, i, p, p)
-        _sig(lib, "cor_hyper_logits_work_bytes", sz, i, i, i, ll)
-        _sig(lib, "cor_hyper_logits_fwd", i, p, p, i, p, i, i, i, i, i, i, ll, p)
-        _sig(lib, "cor_hyper_logits_bwd", i, p, p, i, p, i, p, p, i, i, i, i, i, ll, p, p)
-        _sig(lib, "cor_val_post_work_bytes", sz, i, i, i)
-        _sig(lib, "cor_val_post", i, p, i, i, i, i, i, i, i, p, p, p, i, f, p, p, p)
-        _sig(lib, "cor_soft_metrics", i, p, p, i, f, i, ll, f, p, p, p)
-        pp = C.POINTER(C.c_void_p)
-        _sig(lib, "cor_peer_max_world", i)
-        _sig(lib, "cor_peer_flag_bytes", sz)
-        _sig(lib, "cor_peer_state_bytes", sz)
-        _sig(lib, "cor_peer_error_word", i)
-        _sig(lib, "cor_peer_alloc", i, i, sz, pp)
-        _sig(lib, "cor_peer_free", i, p)
-        _sig(lib, "cor_peer_export", i, p, C.c_char_p)
-        _sig(lib, "cor_peer_open", i, i, C.c_char_p, pp)
-        _sig(lib, "cor_peer_close", i, p)
-        _sig(lib, "cor_peer_signal", i, p, p, i, i, i, p)
-        _sig(lib, "cor_peer_wait_exit", i, p, p, i, i, i, p)
-        _sig(lib, "cor_peer_gather_rows", i, p, p, ll, p, p, i, i, i, p)
-        _sig(lib, "cor_peer_reduce_rows", i, p, p, ll, p, p, i, i, i, p)
-        _sig(lib, "cor_peer_gather_sim_work_bytes", sz)
-        _sig(lib, "cor_peer_gather_sim", i, p, p, ll, i, p, i, f, p, p, p, p, i, i, i, p)
-        _sig(lib, "cor_peer_gather_sim_ls", i, p, p, ll, i, p, i, p, p, p, p, p, i, i, i, p)
+        for name, (restype, argtypes) in decls.items():
+            fn = getattr(lib, name)
+            fn.restype, fn.argtypes = restype, argtypes
         if lib.cor_abi_version() != ABI_VERSION:
             raise CorError(f"ABI version mismatch: library {lib.cor_abi_version()}, binding {ABI_VERSION}; rebuild with `python -m cor_b200.build`")
         _lib = lib

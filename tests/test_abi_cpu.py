@@ -3,6 +3,7 @@ symbol include/cor_b200.h declares; the product path refuses CPU tensors instead
 import ctypes
 import inspect
 import os
+import re
 
 import pytest
 import torch
@@ -25,6 +26,34 @@ def test_library_exports_every_declared_symbol(lib):
     missing = [n for n in names if not hasattr(raw, n)]
     assert not missing, f"declared in include/cor_b200.h but not exported: {missing}"
     assert lib.cor_abi_version() == _lib.ABI_VERSION == 3
+    # every entry is typed from its declaration: one argtype per parameter, the declared return type
+    text = re.sub(r"/\*.*?\*/", "", open(_lib.HEADER).read(), flags=re.S)
+    returns = {"int": ctypes.c_int, "size_t": ctypes.c_size_t, "const char*": ctypes.c_char_p}
+    for n in names:
+        ret, params = re.search(rf"^(int|size_t|const char\*) {n}\(([^)]*)\);", text, flags=re.M).groups()
+        fn = getattr(lib, n)
+        assert len(fn.argtypes) == (0 if params == "void" else params.count(",") + 1), n
+        assert fn.restype is returns[ret], n
+
+
+def test_header_types_are_derived_and_unknown_types_refused(tmp_path):
+    """The binding types each entry from its C declaration; a parameter type it has no mapping for fails at load."""
+    h = tmp_path / "cor.h"
+    h.write_text("#define COR_ABI_VERSION 3\n"
+                 "enum { COR_X = 0, COR_Y = 1 };\n"
+                 "typedef void* cor_stream_t;\n"
+                 "/* cor_in_comment(int x); */\n"
+                 "size_t cor_a(void);   // a size query\n"
+                 "int cor_b(const void* const* src, int n /* rows */, float s,\n"
+                 "          long long ld, unsigned* counter, cor_stream_t stream);\n")
+    c = ctypes
+    assert _lib.declarations(str(h)) == {"cor_a": (c.c_size_t, []),
+                                         "cor_b": (c.c_int, [c.c_void_p, c.c_int, c.c_float, c.c_longlong, c.c_void_p, c.c_void_p])}
+    h.write_text(h.read_text() + "int cor_c(const float* x, double eps, cor_stream_t stream);\n")
+    with pytest.raises(_lib.CorError, match=r"cor_c: .*`double`"):
+        _lib.declared_symbols(str(h))
+    with pytest.raises(_lib.CorError, match="not found"):
+        _lib.declarations(str(tmp_path / "missing.h"))
 
 
 def test_no_torch_types_in_the_header():

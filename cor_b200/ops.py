@@ -497,6 +497,15 @@ def _tau_arg(name: str, inv_tau: float, scale: Optional[torch.Tensor]):
     return (name, _f(inv_tau)) if scale is None else (name + "_ls", ptr(scale))
 
 
+def _tail_entry(name: str, inv_tau: float, scale: Optional[torch.Tensor], mem_args: Optional[tuple]):
+    """(entry name, tau-position arguments) of an InfoNCE tail entry: the choice of ``_tau_arg``, or with a region memory's
+    ``mem_args`` = (mem_part, mem_nparts, mem_state) the ``_mem`` twin, which takes inv_tau and the scale (NULL: inv_tau)."""
+    if mem_args is None:
+        name, ta = _tau_arg(name, inv_tau, scale)
+        return name, (ta,)
+    return name + "_mem", (_f(inv_tau), ptr(scale), *mem_args)
+
+
 def _sim_forward(r16, q16, inv_tau, want_S, want_lse, engine, scale=None):
     dev = r16.device
     Nr, D = r16.shape
@@ -619,8 +628,9 @@ class _InfoNCEFn(torch.autograd.Function):
             # the tail entry in its lse-in form: it merges the memory's partials into the current rows' lse (in place) and
             # forms the loss as cor_infonce_fwd does, so an empty memory changes no bit
             mwork, mparts = _memory_scan(memory, q16, inv_tau, logit_scale)
-            _call("cor_infonce_tail_mem", dev, None, 0, 0, ptr(r16), ptr(q16), ptr(tg), Nr, Nq, D, _f(inv_tau), ptr(logit_scale),
-                  ptr(mwork), mparts, ptr(memory.state), ptr(lse), ptr(loss), ptr(tgt), None, None, _f(0.0), _f(0.0), _f(0.0), None)
+            name, tas = _tail_entry("cor_infonce_tail", inv_tau, logit_scale, (ptr(mwork), mparts, ptr(memory.state)))
+            _call(name, dev, None, 0, 0, ptr(r16), ptr(q16), ptr(tg), Nr, Nq, D, *tas, ptr(lse), ptr(loss), ptr(tgt), None, None,
+                  _f(0.0), _f(0.0), _f(0.0), None)
         ctx.mem = None if memory is None else (memory, memory.enqueues)
         # the scale is saved as an input: an in-place write to it before backward trips autograd's version check
         ctx.save_for_backward(r16, q16, tg, lse, logit_scale)

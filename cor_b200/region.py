@@ -8,16 +8,21 @@ column of the similarity matrix equals the cosine inside ``fg_feat_similarity_lo
 """
 from __future__ import annotations
 
+import functools
 import os
+from collections import namedtuple
 from dataclasses import dataclass
 from typing import Optional
 
 import torch
 
+from . import _lib as L
 from . import dist as cdist
 from . import ops
 from . import peer
 from ._lib import CorError
+from .linear import gemm
+from .ops import _f, _ll, ptr
 
 __all__ = ["pool_regions", "region_query_similarity", "region_infonce_loss", "topk_regions", "region_step", "RegionStepOut",
            "StepBuffers", "RegionMemory"]
@@ -35,7 +40,6 @@ class RegionMemory:
     data-parallel job owns its memory and scores it against its own queries only.  C must be 64, 128, 192 or 256."""
 
     def __init__(self, capacity: int, C: int, device="cuda"):
-        from . import _lib as L
         if int(capacity) < 1:
             raise CorError(f"RegionMemory: capacity must be >= 1, got {capacity}")
         if int(C) not in (64, 128, 192, 256):
@@ -56,7 +60,6 @@ class RegionMemory:
     def enqueue(self, rows: torch.Tensor) -> None:
         """Push ``rows`` (fp32 or bf16 [..., C], e.g. ``RegionStepOut.regions``; 1 <= n <= capacity rows) as bf16 at the
         head, overwriting the oldest rows once full.  One kernel on the current stream, no host synchronisation."""
-        from . import _lib as L
         if rows.dtype not in (torch.float32, torch.bfloat16):
             raise CorError(f"RegionMemory.enqueue: rows must be float32 or bfloat16, got {rows.dtype}")
         if rows.dim() < 1 or rows.shape[-1] != self.C:
@@ -140,30 +143,17 @@ class RegionStepOut:
     regions: torch.Tensor          # [B, M, C] unit rows (detached view for retrieval)
 
 
-_target_cache = {}
-
-
+@functools.cache
 def _target_rows(dev, B, M, offset):
-    """Row index of every triplet's ground-truth region (b * M + offset), cached per shape."""
-    key = (dev.index, B, M, offset)
-    t = _target_cache.get(key)
-    if t is None:
-        # never evicted (a few bytes each): captured graphs hold the raw pointer
-        t = torch.arange(B, device=dev, dtype=torch.int64) * M + offset
-        _target_cache[key] = t
-    return t
+    """Row index of every triplet's ground-truth region (b * M + offset), cached per shape and never evicted (a few bytes
+    each): captured graphs hold the raw pointer."""
+    return torch.arange(B, device=dev, dtype=torch.int64) * M + offset
 
 
-_side_streams = {}
-
-
+@functools.cache
 def _side_stream(dev):
     """One extra stream per device for the branch of the step that does not depend on the pooled rows."""
-    st = _side_streams.get(dev.index)
-    if st is None:
-        st = torch.cuda.Stream(device=dev)
-        _side_streams[dev.index] = st
-    return st
+    return torch.cuda.Stream(device=dev)
 
 
 def _overlap_enabled():
@@ -178,19 +168,11 @@ def _step_tail_ok(B: int, M: int, C: int, multi_rank: bool, bg_mode: int, sim_en
             and ops._sim_engine(B, B * M, C, sim_engine) == "stream")
 
 
-_tail_counters = {}
-
-
+@functools.cache
 def _tail_counter(dev, B, M, C):
-    """Zero-initialised arrival counters of the step-tail kernels, cached per shape: every launch leaves them zero again."""
-    key = (dev.index, B, M, C)
-    t = _tail_counters.get(key)
-    if t is None:
-        # never evicted (128 bytes each): captured graphs hold the raw pointer
-        from . import _lib as L
-        t = torch.zeros(L.load().cor_step_tail_counter_words(), dtype=torch.int32, device=dev)
-        _tail_counters[key] = t
-    return t
+    """Zero-initialised arrival counters of the step-tail kernels, cached per shape: every launch leaves them zero again.
+    Never evicted (128 bytes each): captured graphs hold the raw pointer."""
+    return torch.zeros(L.load().cor_step_tail_counter_words(), dtype=torch.int32, device=dev)
 
 
 def _peer_fused_ok(n_queries: int, C: int, n_regions: int = 0, sim_engine: str = "auto") -> bool:
@@ -207,329 +189,336 @@ def _peer_fused_ok(n_queries: int, C: int, n_regions: int = 0, sim_engine: str =
     return ops._sim_engine(n_queries, n_regions, C, sim_engine) != "umma"
 
 
+# the fused step's shape and scalars, fixed before its first launch and read again by its backward.  ws: the ranks whose
+# rows the InfoNCE scores (1 unless the rows are gathered); offset: this rank's first row among them
+_StepCfg = namedtuple("_StepCfg", "B M Cc h w inv_tau nce_weight bg_mode w_fg w_bg ws offset pred_dt emb_dt comb_dt comb_shape "
+                                  "need_pred need_emb need_comb")
+# the tensors the step's backward reads, kept through save_for_backward
+_Saved = namedtuple("_Saved", "pred_c t_save w_save per fg bg inv_fg inv_bg comb_c stats out4 aux r16 q16 targets lse w32 scale")
+_Side = namedtuple("_Side", "q16 ev_q ev_px mem_args out8 t_save w_save per scratch")
+_Rows = namedtuple("_Rows", "fg inv_fg bg inv_bg out4 aux lse nce tgt loss")
+
+
+def _side_branch(cfg, dev, cur, side, px, pred_c, masks, comb_c, memory, sc) -> _Side:
+    """What needs neither the resampled weights nor the pooled rows, issued FIRST on the side stream (a parallel branch once
+    captured in a CUDA graph), else on the current one: the peer-exit wait, the bf16 queries, the memory scan and the
+    segmentation loss, whose instruction-bound tiles run underneath the HBM-bound mask resample.  ``scratch``: the work
+    buffers the side stream writes, to keep alive until the tail joins it."""
+    lib = L.load()
+    f32 = dict(dtype=torch.float32, device=dev)
+    gt = masks[:, 0]                       # [B,Hm,Wm] view; read in place through its sample stride
+    Hm, Wm = gt.shape[1:]
+    if not (gt.stride(2) == 1 and gt.stride(1) == Wm):
+        gt = gt.contiguous()
+    N, D = comb_c.shape
+    H, W = pred_c.shape[2:]
+    out8 = torch.empty(8, **f32)
+    per = torch.empty((N, lib.cor_seg_loss_npartials()), **f32)
+    t_save = torch.empty((N, H, W), **f32) if cfg.need_pred else None
+    w_save = torch.empty((N, H, W), **f32) if cfg.need_pred else None
+    seg_work = ops._work(lib.cor_seg_loss_work_bytes(N, H, W), dev)
+    stream = side if side is not None else cur
+    if side is not None:
+        side.wait_stream(cur)
+    # "Have my peers finished reading the rows I published last step?" is asked HERE, at the very start of the step (one
+    # 32-thread CTA polling local flags): by the time the row epilogue needs the answer the 0.7 ms mask resample has gone
+    # by, so the wait never sits on the critical path.
+    ev_px = mem_args = None
+    if px is not None:
+        with torch.cuda.stream(stream):
+            px.before_produce(0)
+        ev_px = side.record_event() if side is not None else None
+    q16 = torch.empty((N, D), dtype=torch.bfloat16, device=dev)
+    # allocated on the consuming stream: its block is reused only after the tail that reads it
+    mwork = ops._memory_scan_work(memory, N, D, dev) if memory is not None else None
+    with torch.cuda.stream(stream):
+        ops._call("cor_cast_cat_bf16", dev, ptr(comb_c), D, None, 0, _ll(N), ptr(q16))
+        ev_q = side.record_event() if side is not None else None
+        if memory is not None:
+            mwork, mparts = ops._memory_scan(memory, q16, cfg.inv_tau, sc, mwork)
+            mem_args = (ptr(mwork), mparts, ptr(memory.state))
+        ops._call("cor_seg_loss_fwd", dev, ptr(pred_c), L.dtype_code(pred_c), ptr(gt), L.dtype_code(gt), _f(ops._mask_scale(gt, None)),
+                  N, H, W, Hm, Wm, _ll(gt.stride(0)), None, _f(0.25), _f(-1.0), _f(1.0), ptr(out8), ptr(per), ptr(t_save),
+                  ptr(w_save), ptr(seg_work))
+    return _Side(q16, ev_q, ev_px, mem_args, out8, t_save, w_save, per, (seg_work, mwork))
+
+
+def _pool(cfg, dev, emb_c, masks):
+    """masks -> bf16 weights in the cached GEMM operand (+ raw fp32 weights for the backward) + full-resolution stats, then
+    the pooling GEMM: (w16, w32, stats, split-K partials [ksplit, B, Rp, C]), row M = the all-ones weight row's sum."""
+    B, M, Cc, P = cfg.B, cfg.M, cfg.Cc, cfg.h * cfg.w
+    Rp = (M + 1 + 15) // 16 * 16
+    w16 = ops._umma_weight_buffer(dev, B, Rp, M, P)
+    w32, stats = ops.mask_prep(masks.reshape(B * M, *masks.shape[2:]), (cfg.h, cfg.w), ops.W_CLAMP, want_f32=cfg.need_emb,
+                               bf16_out=w16, group=M, group_stride=Rp * P)
+    part = torch.empty((L.load().cor_pool_umma_ksplit(B, Cc, P), B, Rp, Cc), dtype=torch.float32, device=dev)
+    ops._call("cor_pool_umma_fwd", dev, ptr(emb_c), ptr(w16), B, Cc, P, Rp, ptr(part))
+    return w16, w32, stats, part
+
+
+def _row_outputs(dev, B, M, Cc) -> _Rows:
+    """What either tail writes: unit rows + inverse norms, the GT masks' bg rows + inverse norms, the fg / bg losses + their
+    auxiliaries, and the InfoNCE's log-sum-exp, mean and target logits with the step's total loss."""
+    e = lambda *shape: torch.empty(shape, dtype=torch.float32, device=dev)
+    return _Rows(fg=e(B * M, Cc), inv_fg=e(B * M), bg=e(B, Cc), inv_bg=e(B), out4=e(4), aux=e(L.load().cor_fgbg_aux_floats(B, Cc)),
+                 lse=e(B), nce=e(1), tgt=e(B), loss=e(1))
+
+
+def _tail_forward(cfg, dev, cur, side, part, stats, comb_c, sc, sd, counter):
+    """The region tail in ONE launch (csrc/step_tail.cu): unit rows (+ bf16 copy), their scores against the queries, the bg
+    rows and fg / bg cosine statistics of the GT masks, and in its last CTA the log-sum-exp merge (with the memory's
+    partials), the InfoNCE, fg / bg losses and the total.  Returns (_Rows, the scored bf16 rows, their targets)."""
+    B, M, Cc, Rp = cfg.B, cfg.M, cfg.Cc, part.shape[2]
+    o = _row_outputs(dev, B, M, Cc)
+    fg16 = torch.empty((B * M, Cc), dtype=torch.bfloat16, device=dev)
+    targets = _target_rows(dev, B, M, 0)
+    work = ops._work(L.load().cor_step_tail_work_bytes(B, M, Cc), dev)
+    if side is not None:
+        cur.wait_stream(side)            # join: the total needs the segmentation loss, the scores the bf16 queries
+    name, tas = ops._tail_entry("cor_step_tail_fwd", cfg.inv_tau, sc, sd.mem_args)
+    ops._call(name, dev, ptr(part), part.shape[0], _ll(B * Rp * Cc), Rp, B, M, Cc, _f(float(cfg.h * cfg.w)), ptr(stats), ptr(sd.q16),
+              ptr(comb_c), ptr(targets), *tas, ptr(sd.out8), _f(cfg.w_fg), _f(cfg.w_bg), _f(cfg.nce_weight), ptr(o.fg), ptr(fg16),
+              ptr(o.inv_fg), ptr(o.bg), ptr(o.inv_bg), ptr(o.out4), ptr(o.aux), ptr(o.lse), ptr(o.nce), ptr(o.tgt), ptr(o.loss), ptr(work),
+              ptr(counter))
+    return o, fg16, targets
+
+
+def _chain_forward(cfg, dev, cur, side, part, stats, comb_c, sc, sd, px, sim_engine):
+    """The region tail as a kernel chain where the one-launch tail does not serve: the row epilogue, the bg rows and fg / bg
+    losses on the side stream, the gather (or fused gather + similarity) and cor_infonce_tail.  Returns as _tail_forward."""
+    B, M, Cc = cfg.B, cfg.M, cfg.Cc
+    ks, Rp = part.shape[0], part.shape[2]
+    n_local, split = B * M, B * Rp * Cc
+    o = _row_outputs(dev, B, M, Cc)
+    # multi-GPU: the bf16 rows land directly in this rank's peer-mapped buffer (cor_b200/peer.py), else in a local one
+    fg16 = px.pub if px is not None else torch.empty((n_local, Cc), dtype=torch.bfloat16, device=dev)
+    if sd.ev_px is not None:
+        cur.wait_event(sd.ev_px)
+    ops._call("cor_rows_finalize", dev, ptr(part), M, _ll(Rp * Cc), ks, _ll(split), ptr(stats[:, 3:]), 4, _f(1e-8), n_local, Cc, 1, 1,
+              None, _f(0.0), ptr(o.fg), ptr(fg16), ptr(o.inv_fg))
+    if px is not None:
+        px.signal(0)                     # the bg rows, fg/bg loss and segmentation loss below hide the rank skew
+    # background rows + fg / bg cosine losses on the GT rows (row b*M of fg, row b of bg): a second branch off the fg rows,
+    # on the side stream, parallel to the similarity / InfoNCE chain below
+    if side is not None:
+        side.wait_stream(cur)
+    with torch.cuda.stream(side if side is not None else cur):
+        ops._call("cor_rows_finalize", dev, ptr(part), 1, _ll(Rp * Cc), ks, _ll(split), ptr(stats[:, 3:]), 4 * M, _f(1e-8), B, Cc, 1, 1,
+                  ptr(part[0, :, M, :]), _f(float(cfg.h * cfg.w)), ptr(o.bg), None, ptr(o.inv_bg))
+        ops._call("cor_fgbg_loss_fwd", dev, ptr(o.fg), _ll(M * Cc), ptr(o.bg), _ll(Cc), ptr(comb_c), _ll(Cc), ptr(stats), _ll(4 * M), B,
+                  Cc, cfg.bg_mode, ptr(o.out4), ptr(o.aux))
+    # InfoNCE of every composed query against all (gathered) regions
+    if sd.ev_q is not None:
+        cur.wait_event(sd.ev_q)
+    r16, fused_parts = fg16, None
+    if cfg.ws > 1:
+        r16 = torch.empty((cfg.ws * n_local, Cc), dtype=torch.bfloat16, device=dev)
+        if px is not None and _peer_fused_ok(B, Cc, cfg.ws * n_local, sim_engine):
+            # ONE kernel: pull the peers' rows over NVLink, keep a local copy for the backward, and score every row against
+            # this rank's queries while it is in registers (all-gather fused with its consumer)
+            fused_parts = px.gather_sim(r16, sd.q16, cfg.inv_tau, sc)
+        elif px is not None:
+            px.gather(r16)               # our own pull-over-NVLink kernel: no NCCL on the data path
+        else:
+            torch.distributed.all_gather_into_tensor(r16, fg16)
+    targets = _target_rows(dev, B, M, cfg.offset)
+    # similarity with its log-sum-exp partials left in the work buffer, then ONE tail kernel: partial merge (with this rank's
+    # memory, scored against its own queries) -> lse, target logits, InfoNCE mean and the step's total loss
+    sim_work, nparts, qt = fused_parts if fused_parts is not None else ops._sim_lse_parts(r16, sd.q16, cfg.inv_tau, sim_engine, sc)
+    if side is not None:
+        cur.wait_stream(side)            # join: the total needs the segmentation and fg/bg losses
+    name, tas = ops._tail_entry("cor_infonce_tail", cfg.inv_tau, sc, sd.mem_args)
+    ops._call(name, dev, ptr(sim_work), nparts, qt, ptr(r16), ptr(sd.q16), ptr(targets), r16.shape[0], B, Cc, *tas, ptr(o.lse),
+              ptr(o.nce), ptr(o.tgt), ptr(sd.out8), ptr(o.out4), _f(cfg.w_fg), _f(cfg.w_bg), _f(cfg.nce_weight), ptr(o.loss))
+    return o, r16, targets
+
+
+def _seg_backward(cfg, s, g, cur, side):
+    """Gradient of the segmentation loss wrt pred (None when pred needs none), on the side stream when there is one."""
+    if not cfg.need_pred:
+        return None
+    N, H, W = s.t_save.shape
+    gp = torch.empty_like(s.pred_c)
+    if side is not None:
+        side.wait_stream(cur)
+    with torch.cuda.stream(side if side is not None else cur):
+        ops._call("cor_seg_loss_bwd", gp.device, ptr(s.pred_c), L.dtype_code(s.pred_c), ptr(s.t_save), ptr(s.w_save), ptr(s.per), N, H,
+                  W, None, _f(1.0), _f(0.25), _f(-1.0), ptr(g), ptr(gp), L.dtype_code(gp))
+    return gp
+
+
+def _pool_bwd_gemm(a16, w16, B, Cc, P, Kp, out_dtype):
+    """d emb[b] (C x P) = gs[b]^T (C x M) w[b] (M x P) -> [B*C, P]: one batched tcgen05 GEMM on the bf16 weights the forward's
+    pooling GEMM used (the caller checked that no later forward of this shape has rewritten them), both operands MN-major
+    as they lie.  ``a16`` holds the gradient rows in bf16, zero-padded to whole 64-row K blocks (Kp), which makes the
+    weight rows beyond M (the ones row, the next image) irrelevant.  Persistent tiles with coalesced stores: 2-3x faster
+    than the one-shot pool_bwd_umma kernel, which rebuilds both operands from fp32."""
+    Rp = w16.shape[1]
+    return gemm(a16, w16.view(B * Rp, P), Cc, P, Kp, a_mn=True, b_mn=True, batch=B, a_batch_rows=Kp, b_batch_rows=Rp, out_dtype=out_dtype)
+
+
+def _tail_backward(ctx, s, g, g_scale):
+    """(g_emb, g_comb) from ONE launch: InfoNCE + fg-loss gradient of every row, through the row epilogue, cast to bf16 into
+    the K-padded operand of the pooling-backward GEMM; and the query gradient (+ fg / bg terms) in extra CTAs, one set per
+    query.  Then the memory's share of the query gradient, and the GEMM."""
+    cfg = ctx.cfg
+    B, M, Cc = cfg.B, cfg.M, cfg.Cc
+    dev = s.fg.device
+    Kp = (M + 63) // 64 * 64
+    a16 = torch.empty((B * Kp, Cc), dtype=torch.bfloat16, device=dev) if cfg.need_emb else None
+    g_q = torch.empty((B, Cc), dtype=torch.float32, device=dev) if cfg.need_comb else None
+    work = ops._work(L.load().cor_step_tail_work_bytes(B, M, Cc), dev)
+    name, ta = ops._tau_arg("cor_step_tail_bwd", cfg.inv_tau, s.scale)
+    gs_arg = () if s.scale is None else (ptr(g_scale),)          # the _ls backward entries take the gradient pointer
+    ops._call(name, dev, ptr(s.r16), ptr(s.q16), ptr(s.targets), ptr(s.lse), B, M, Cc, ta, ptr(g), _f(cfg.nce_weight), ptr(s.fg),
+              ptr(s.inv_fg), ptr(s.stats), ptr(s.comb_c), ptr(s.out4), ptr(s.aux), _f(cfg.w_fg), _f(cfg.w_bg), ptr(a16), Kp, ptr(g_q),
+              *gs_arg, ptr(work), ptr(ctx.tail))
+    if ctx.mem is not None:
+        ops._memory_dq(ctx.mem[0], s.q16, s.lse, cfg.inv_tau, s.scale, g, cfg.nce_weight, g_q, g_scale)
+    g_comb = g_q.view(cfg.comb_shape).to(cfg.comb_dt) if cfg.need_comb else None
+    if not cfg.need_emb:
+        return None, g_comb
+    out_dt = cfg.emb_dt if cfg.emb_dt in (torch.float32, torch.bfloat16) else torch.float32
+    return _pool_bwd_gemm(a16, ctx.w16[0], B, Cc, cfg.h * cfg.w, Kp, out_dt).view(B, Cc, cfg.h, cfg.w).to(cfg.emb_dt), g_comb
+
+
+def _chain_backward(ctx, s, g, g_scale, g_pred, gemm_ok, cur, side, ev_px):
+    """Backward of the kernel chain, and of a one-launch tail whose bf16 weights were rewritten since: (g_emb, g_comb, g_pred),
+    the last computed here, between the signal and the pull, when there is a peer exchange and no side stream."""
+    cfg, px = ctx.cfg, ctx.px
+    B, M, Cc, P = cfg.B, cfg.M, cfg.Cc, cfg.h * cfg.w
+    dev = s.fg.device
+    lib = L.load()
+    f32 = dict(dtype=torch.float32, device=dev)
+    # InfoNCE backward first: it WRITES g_regions (this rank's rows) and g_queries ...
+    Nr = s.r16.shape[0]
+    g_regions = torch.empty((B * M, Cc), **f32)
+    g_q = torch.empty((B, Cc), **f32)
+    work = ops._work(lib.cor_sim_work_bytes(B, Nr, Cc), dev)
+    if ev_px is not None:
+        cur.wait_event(ev_px)
+    # several ranks: gradient of every gathered row, then a reduce-scatter back to the owning rank: measured faster than a
+    # collective-free backward that all-gathers the queries instead (profiles/README.md)
+    g_rows = g_regions if cfg.ws == 1 else px.gall if px is not None else torch.empty((Nr, Cc), **f32)
+    name, ta = ops._tau_arg("cor_infonce_bwd", cfg.inv_tau, s.scale)
+    gs_arg = () if s.scale is None else (ptr(g_scale),)
+    ops._call(name, dev, ptr(s.r16), ptr(s.q16), ptr(s.targets), ptr(s.lse), Nr, B, Cc, ta, ptr(g), _f(cfg.nce_weight), ptr(g_rows),
+              ptr(g_q), *gs_arg, ptr(work))
+    if px is not None:
+        px.signal(1)
+        if side is None:
+            g_pred = _seg_backward(cfg, s, g, cur, None)   # independent work between the signal and the pull hides the rank skew
+        px.reduce(g_regions)             # fixed rank order: bit-identical from run to run
+    elif cfg.ws > 1:
+        torch.distributed.reduce_scatter_tensor(g_regions, g_rows, op=torch.distributed.ReduceOp.SUM)
+    # ... then the fg/bg backward ADDS its GT-row gradients into g_regions (row b*M) and g_queries
+    g_bg = torch.empty((B, Cc), **f32) if cfg.bg_mode == 1 else None
+    ops._call("cor_fgbg_loss_bwd", dev, ptr(s.fg), _ll(M * Cc), ptr(s.bg), _ll(Cc), ptr(s.comb_c), _ll(Cc), B, Cc, cfg.bg_mode, ptr(s.out4),
+              ptr(s.aux), ptr(g), _ll(0), _f(cfg.w_fg), _f(cfg.w_bg), ptr(g_regions), _ll(M * Cc), 1, ptr(g_bg), _ll(Cc), ptr(g_q), _ll(Cc), 1)
+    if ctx.mem is not None:              # this rank's memory, against this rank's queries
+        ops._memory_dq(ctx.mem[0], s.q16, s.lse, cfg.inv_tau, s.scale, g, cfg.nce_weight, g_q if cfg.need_comb else None, g_scale)
+    g_comb = g_q.view(cfg.comb_shape).to(cfg.comb_dt) if cfg.need_comb else None
+    if not cfg.need_emb:
+        return None, g_comb, g_pred
+    gs_fg = torch.empty((B * M, Cc), **f32)
+    ops._call("cor_rows_finalize_bwd", dev, ptr(g_regions), ptr(s.fg), ptr(s.inv_fg), ptr(s.stats[:, 3:]), 4, _f(1e-8), B * M, Cc, 1, 1,
+              0, _f(0.0), ptr(gs_fg))
+    out_dt = cfg.emb_dt if cfg.emb_dt in (torch.float32, torch.bfloat16) else torch.float32
+    if gemm_ok:                          # implies bg_mode 0: no background gradient
+        Kp = (M + 63) // 64 * 64
+        a16 = torch.empty((B * Kp, Cc), dtype=torch.bfloat16, device=dev)
+        ops._call("cor_cast_pad_rows_bf16", dev, ptr(gs_fg), B, M, Kp, Cc, ptr(a16))
+        return _pool_bwd_gemm(a16, ctx.w16[0], B, Cc, P, Kp, out_dt).view(B, Cc, cfg.h, cfg.w).to(cfg.emb_dt), g_comb, g_pred
+    gs_bg_full = None
+    if g_bg is not None:                 # paired bg mode: background gradient lives on the GT rows only
+        gs_bg = torch.empty((B, Cc), **f32)
+        ops._call("cor_rows_finalize_bwd", dev, ptr(g_bg), ptr(s.bg), ptr(s.inv_bg), ptr(s.stats[:, 3:]), 4 * M, _f(1e-8), B, Cc, 1, 1, 1,
+                  _f(float(P)), ptr(gs_bg))
+        gs_bg_full = torch.zeros((B, M, Cc), **f32)
+        gs_bg_full[:, 0, :] = gs_bg
+    g_emb = torch.empty((B, Cc, cfg.h, cfg.w), dtype=out_dt, device=dev)
+    name = "cor_pool_bwd_umma" if lib.cor_pool_bwd_umma_ok(B, Cc, P, M, int(gs_bg_full is not None)) else "cor_pool_bwd_feat"
+    ops._call(name, dev, ptr(gs_fg), ptr(gs_bg_full), ptr(s.w32), _ll(P), B, Cc, P, M, ops.W_CLAMP, ptr(g_emb), L._DTYPES[g_emb.dtype])
+    return g_emb.to(cfg.emb_dt), g_comb, g_pred
+
+
 class _FusedStepFn(torch.autograd.Function):
-    """The whole region path as ONE autograd node: every kernel of the forward is launched back to
-    back on the current stream, the backward is written out by hand, and no tensor glue (slices,
-    zeros + scatter, tiny adds) sits between them.  Used by :func:`region_step` when the tensor-core
-    pooling engine applies; the modular ops remain the general path."""
+    """The whole region path as ONE autograd node, hand-written backward, no tensor glue (slices, zeros + scatter, tiny adds)
+    between its kernels: the side branch, the pooling, then the one-launch tail where it applies, else the kernel chain.
+    Used by :func:`region_step` when the tensor-core pooling engine applies; the modular ops remain the general path."""
 
     @staticmethod
     def forward(ctx, pred, emb, comb, masks, tau, nce_weight, gather, sim_engine, bg_mode, w_fg, w_bg, logit_scale, memory):
-        from . import _lib as L
-        ptr, _f, _ll, call = ops.ptr, ops._f, ops._ll, ops._call
         dev = L.require_cuda(pred, emb, comb, masks, logit_scale)
         sc = logit_scale                       # device logit scale (replaces 1/tau in every InfoNCE launch) or None
-        tau_arg = lambda name, inv_tau: ops._tau_arg(name, inv_tau, sc)
-        lib = L.load()
         B, M = masks.shape[:2]
         Cc, h, w = emb.shape[1:]
-        P = h * w
         if masks.dtype not in (torch.float32, torch.bfloat16, torch.uint8):
             masks = masks.float()            # bool / fp16 / fp64 masks: one conversion serves mask_prep and the seg loss
         emb_c = emb.contiguous()
         pred_c = ops._as_supported_float(pred)
         comb_c = comb.reshape(B, -1).float().contiguous()
-        f32 = dict(dtype=torch.float32, device=dev)
-        need_emb = emb.requires_grad
-        # 5. segmentation loss against the GT mask, resample fused.  It depends on neither the resampled weights nor the
-        #    pooled rows, so it is issued FIRST, on a side stream (a parallel branch once the step is captured in a CUDA
-        #    graph): its instruction-bound tiles run underneath the HBM-bound mask resample.
-        gt = masks[:, 0]                       # [B,Hm,Wm] view; read in place through its sample stride
-        Hm, Wm = gt.shape[1:]
-        if not (gt.stride(2) == 1 and gt.stride(1) == Wm):
-            gt = gt.contiguous()
-        N = B
-        H, W = pred_c.shape[2:]
-        out8 = torch.empty(8, **f32)
-        per = torch.empty((N, lib.cor_seg_loss_npartials()), **f32)
-        need_pred = pred.requires_grad
-        t_save = torch.empty((N, H, W), **f32) if need_pred else None
-        w_save = torch.empty((N, H, W), **f32) if need_pred else None
-        seg_work = ops._work(lib.cor_seg_loss_work_bytes(N, H, W), dev)
+        rank, ws = cdist.world()
+        multi_rank = gather and ws > 1
+        cfg = _StepCfg(B, M, Cc, h, w, 1.0 / float(tau), float(nce_weight), int(bg_mode), float(w_fg), float(w_bg), ws if multi_rank else 1,
+                       rank * B * M if multi_rank else 0, pred.dtype, emb.dtype, comb.dtype, tuple(comb.shape), pred.requires_grad,
+                       emb.requires_grad, comb.requires_grad)
         cur = torch.cuda.current_stream(dev)
         side = _side_stream(dev) if _overlap_enabled() else None
-        if side is not None:
-            side.wait_stream(cur)
-        # multi-GPU: the bf16 rows land directly in this rank's peer-mapped buffer (cor_b200/peer.py), else in a local one.
-        # "Have my peers finished reading what I published last step?" is asked HERE, on the side stream at the very
-        # start of the step (one 32-thread CTA polling local flags): by the time the row epilogue needs the answer the
-        # 0.7 ms mask resample has gone by, so the wait never sits on the critical path.
-        rank, ws = cdist.world()
-        px = peer.get_exchange(B * M, Cc, dev) if (gather and ws > 1) else None
-        ev_px = None
-        if px is not None:
-            with torch.cuda.stream(side if side is not None else cur):
-                px.before_produce(0)
-                if side is not None:
-                    ev_px = torch.cuda.Event()
-                    ev_px.record(side)
-        q16 = torch.empty((B, comb_c.shape[1]), dtype=torch.bfloat16, device=dev)
-        ev_q = None
-        mem_args = ()
-        # allocated on the consuming stream: its block is reused only after the tail that reads it
-        mwork = ops._memory_scan_work(memory, B, comb_c.shape[1], dev) if memory is not None else None
-        with torch.cuda.stream(side if side is not None else cur):
-            call("cor_cast_cat_bf16", dev, ptr(comb_c), comb_c.shape[1], None, 0, _ll(B), ptr(q16))   # bf16 queries, off the main chain
-            if side is not None:
-                ev_q = torch.cuda.Event()
-                ev_q.record(side)
-            if memory is not None:
-                # the region memory's scan needs only the queries and the bank: a parallel branch beside the mask resample
-                mwork, mparts = ops._memory_scan(memory, q16, 1.0 / float(tau), sc, mwork)
-                mem_args = (ptr(mwork), mparts, ptr(memory.state))
-            call("cor_seg_loss_fwd", dev, ptr(pred_c), L.dtype_code(pred_c), ptr(gt), L.dtype_code(gt), _f(ops._mask_scale(gt, None)), N, H, W,
-                 Hm, Wm, _ll(gt.stride(0)), None, _f(0.25), _f(-1.0), _f(1.0), ptr(out8), ptr(per), ptr(t_save), ptr(w_save),
-                 ptr(seg_work))
-        # 1. masks -> bf16 weights (+ raw fp32 weights for the backward) + full-resolution stats
-        Rp = (M + 1 + 15) // 16 * 16
-        w16 = ops._umma_weight_buffer(dev, B, Rp, M, P)
-        w32, stats = ops.mask_prep(masks.reshape(B * M, *masks.shape[2:]), (h, w), ops.W_CLAMP, want_f32=need_emb, bf16_out=w16,
-                                   group=M, group_stride=Rp * P)
-        # 2. pooling GEMM (split-K partials), 3. row epilogues: all fg rows, bg rows of the GT masks only
-        ks = lib.cor_pool_umma_ksplit(B, Cc, P)
-        part = torch.empty((ks, B, Rp, Cc), **f32)
-        call("cor_pool_umma_fwd", dev, ptr(emb_c), ptr(w16), B, Cc, P, Rp, ptr(part))
-        tail = _step_tail_ok(B, M, Cc, gather and ws > 1, int(bg_mode), sim_engine)
-        ctx.tail = _tail_counter(dev, B, M, Cc) if tail else None
-        if tail:
-            # 3.-6. in ONE launch: unit rows (+ bf16 copy), their scores against the queries, the bg rows and fg / bg cosine
-            # statistics of the GT masks, and in its last CTA the log-sum-exp merge, the InfoNCE, fg / bg losses and the total
-            fg = torch.empty((B * M, Cc), **f32)
-            fg16 = torch.empty((B * M, Cc), dtype=torch.bfloat16, device=dev)
-            inv_fg = torch.empty((B * M,), **f32)
-            bg = torch.empty((B, Cc), **f32)
-            inv_bg = torch.empty((B,), **f32)
-            out4 = torch.empty(4, **f32)
-            aux = torch.empty(lib.cor_fgbg_aux_floats(B, Cc), **f32)
-            r16, offset, ws, n_local = fg16, 0, 1, B * M
-            targets = _target_rows(dev, B, M, 0)
-            lse = torch.empty((B,), **f32)
-            nce = torch.empty(1, **f32)
-            tgt = torch.empty((B,), **f32)
-            loss = torch.empty(1, **f32)
-            inv_tau = 1.0 / float(tau)
-            work = ops._work(lib.cor_step_tail_work_bytes(B, M, Cc), dev)
-            if side is not None:
-                cur.wait_stream(side)        # join: the total needs the segmentation loss, the scores the bf16 queries
-            if memory is None:
-                name, ta = tau_arg("cor_step_tail_fwd", inv_tau)
-                tas = (ta,)
-            else:                            # the same kernel, the memory's partials merged into the log-sum-exp
-                name, tas = "cor_step_tail_fwd_mem", (_f(inv_tau), ptr(sc), *mem_args)
-            call(name, dev, ptr(part), ks, _ll(B * Rp * Cc), Rp, B, M, Cc, _f(float(P)), ptr(stats), ptr(q16), ptr(comb_c),
-                 ptr(targets), *tas, ptr(out8), _f(w_fg), _f(w_bg), _f(nce_weight), ptr(fg), ptr(fg16), ptr(inv_fg), ptr(bg),
-                 ptr(inv_bg), ptr(out4), ptr(aux), ptr(lse), ptr(nce), ptr(tgt), ptr(loss), ptr(work), ptr(ctx.tail))
+        px = peer.get_exchange(B * M, Cc, dev) if multi_rank else None
+        sd = _side_branch(cfg, dev, cur, side, px, pred_c, masks, comb_c, memory, sc)
+        w16, w32, stats, part = _pool(cfg, dev, emb_c, masks)
+        ctx.tail = _tail_counter(dev, B, M, Cc) if _step_tail_ok(B, M, Cc, multi_rank, cfg.bg_mode, sim_engine) else None
+        if ctx.tail is not None:
+            o, r16, targets = _tail_forward(cfg, dev, cur, side, part, stats, comb_c, sc, sd, ctx.tail)
         else:
-            fg = torch.empty((B * M, Cc), **f32)
-            fg16 = px.pub if px is not None else torch.empty((B * M, Cc), dtype=torch.bfloat16, device=dev)
-            if ev_px is not None:
-                cur.wait_event(ev_px)
-            inv_fg = torch.empty((B * M,), **f32)
-            split = B * Rp * Cc
-            call("cor_rows_finalize", dev, ptr(part), M, _ll(Rp * Cc), ks, _ll(split), ptr(stats[:, 3:]), 4, _f(1e-8), B * M, Cc, 1, 1,
-                 None, _f(0.0), ptr(fg), ptr(fg16), ptr(inv_fg))
-            if px is not None:
-                px.signal(0)                     # the bg rows, fg/bg loss and segmentation loss below hide the rank skew
-            # 4. background rows + fg / bg cosine losses on the GT rows (row b*M of fg, row b of bg): a second branch off the
-            #    fg rows, on the side stream, parallel to the similarity / InfoNCE chain below
-            bg = torch.empty((B, Cc), **f32)
-            inv_bg = torch.empty((B,), **f32)
-            out4 = torch.empty(4, **f32)
-            aux = torch.empty(lib.cor_fgbg_aux_floats(B, Cc), **f32)
-            if side is not None:
-                side.wait_stream(cur)
-            with torch.cuda.stream(side if side is not None else cur):
-                call("cor_rows_finalize", dev, ptr(part), 1, _ll(Rp * Cc), ks, _ll(split), ptr(stats[:, 3:]), 4 * M, _f(1e-8), B, Cc, 1, 1,
-                     ptr(part[0, :, M, :]), _f(float(P)), ptr(bg), None, ptr(inv_bg))
-                call("cor_fgbg_loss_fwd", dev, ptr(fg), _ll(M * Cc), ptr(bg), _ll(Cc), ptr(comb_c), _ll(Cc), ptr(stats), _ll(4 * M), B, Cc,
-                     int(bg_mode), ptr(out4), ptr(aux))
-            # 6. InfoNCE of every composed query against all (gathered) regions
-            if ev_q is not None:
-                cur.wait_event(ev_q)
-            n_local = B * M
-            inv_tau = 1.0 / float(tau)
-            fused_parts = None
-            if gather and ws > 1:
-                r16 = torch.empty((ws * n_local, Cc), dtype=torch.bfloat16, device=dev)
-                if px is not None and _peer_fused_ok(B, Cc, ws * n_local, sim_engine):
-                    # ONE kernel: pull the peers' rows over NVLink, keep a local copy for the backward, and score every row
-                    # against this rank's queries while it is in registers (all-gather fused with its consumer)
-                    fused_parts = px.gather_sim(r16, q16, inv_tau, sc)
-                elif px is not None:
-                    px.gather(r16)               # our own pull-over-NVLink kernel: no NCCL on the data path
-                else:
-                    torch.distributed.all_gather_into_tensor(r16, fg16)
-                offset = rank * n_local
-            else:
-                r16, offset, ws = fg16, 0, 1
-            targets = _target_rows(dev, B, M, offset)
-            nce = torch.empty(1, **f32)
-            tgt = torch.empty((B,), **f32)
-            loss = torch.empty(1, **f32)
-            # similarity with its log-sum-exp partials left in the work buffer, then ONE tail kernel: partial merge -> lse,
-            # target logits, InfoNCE mean and the step's total loss
-            sim_work, nparts, qt = fused_parts if fused_parts is not None else ops._sim_lse_parts(r16, q16, inv_tau, sim_engine, sc)
-            lse = torch.empty((B,), **f32)
-            if side is not None:
-                cur.wait_stream(side)        # join: the total needs the segmentation and fg/bg losses
-            if memory is None:
-                name, ta = tau_arg("cor_infonce_tail", inv_tau)
-                tas = (ta,)
-            else:                            # each rank merges ITS memory, scored against its own queries
-                name, tas = "cor_infonce_tail_mem", (_f(inv_tau), ptr(sc), *mem_args)
-            call(name, dev, ptr(sim_work), nparts, qt, ptr(r16), ptr(q16), ptr(targets), r16.shape[0], B, Cc, *tas,
-                 ptr(lse), ptr(nce), ptr(tgt), ptr(out8), ptr(out4), _f(w_fg), _f(w_bg), _f(nce_weight), ptr(loss))
+            o, r16, targets = _chain_forward(cfg, dev, cur, side, part, stats, comb_c, sc, sd, px, sim_engine)
         # the scale is saved as an input: an in-place write to it before backward trips autograd's version check
-        ctx.save_for_backward(pred_c, t_save, w_save, per, fg, bg, inv_fg, inv_bg, comb_c, stats, out4, aux, r16, q16, targets, lse, w32, sc)
-        ctx.cfg = (B, M, Cc, h, w, float(inv_tau), float(nce_weight), int(bg_mode), float(w_fg), float(w_bg), ws, offset, n_local,
-                   pred.dtype, emb.dtype, comb.dtype, tuple(comb.shape), need_pred, need_emb, comb.requires_grad)
-        ctx.px = px
+        ctx.save_for_backward(*_Saved(pred_c=pred_c, t_save=sd.t_save, w_save=sd.w_save, per=sd.per, fg=o.fg, bg=o.bg, inv_fg=o.inv_fg,
+                                      inv_bg=o.inv_bg, comb_c=comb_c, stats=stats, out4=o.out4, aux=o.aux, r16=r16, q16=sd.q16,
+                                      targets=targets, lse=o.lse, w32=w32, scale=sc))
+        ctx.cfg, ctx.px = cfg, px
         ctx.mem = None if memory is None else (memory, memory.enqueues)
         ctx.w16 = (w16, getattr(w16, "_cor_epoch", -1))      # not a saved tensor: a cached operand buffer, validated by its epoch
-        ctx.mark_non_differentiable(fg, out8, out4, nce)
+        ctx.mark_non_differentiable(o.fg, sd.out8, o.out4, o.nce)
         ctx.set_materialize_grads(False)     # no zero-filled gradients for the auxiliary outputs
-        return loss[0], out8, out4, nce, fg
+        return o.loss[0], sd.out8, o.out4, o.nce, o.fg
 
     @staticmethod
     def backward(ctx, g_loss, *_unused):
-        from . import _lib as L
-        ptr, _f, _ll, call = ops.ptr, ops._f, ops._ll, ops._call
-        (pred_c, t_save, w_save, per, fg, bg, inv_fg, inv_bg, comb_c, stats, out4, aux, r16, q16, targets, lse, w32, sc) = ctx.saved_tensors
-        (B, M, Cc, h, w, inv_tau, nce_weight, bg_mode, w_fg, w_bg, ws, offset, n_local, pred_dt, emb_dt, comb_dt, comb_shape,
-         need_pred, need_emb, need_comb) = ctx.cfg
-        dev = fg.device
-        lib = L.load()
-        P = h * w
-        f32 = dict(dtype=torch.float32, device=dev)
         if g_loss is None:
             return (None,) * 13
         ops.check_memory_unchanged(ctx.mem, "region_step backward")
+        cfg, s, px = ctx.cfg, _Saved(*ctx.saved_tensors), ctx.px
+        dev = s.fg.device
         g = g_loss.reshape(1).float().contiguous()
-        g_pred = g_emb = g_comb = None
-        need_scale = sc is not None and ctx.needs_input_grad[11]
         # d loss / d scale: written by the InfoNCE backward over THIS rank's queries (the launch that writes g_queries)
-        g_scale = torch.empty((), **f32) if need_scale else None
-        tau_arg = lambda name: ops._tau_arg(name, inv_tau, sc)
-        gs_arg = () if sc is None else (ptr(g_scale),)          # the _ls backward entries take the gradient pointer
+        g_scale = torch.empty((), dtype=torch.float32, device=dev) if s.scale is not None and ctx.needs_input_grad[11] else None
         cur = torch.cuda.current_stream(dev)
-        side = _side_stream(dev) if (_overlap_enabled() and need_pred) else None
-
-        def seg_bwd():
-            if not need_pred:
-                return None
-            N, H, W = t_save.shape
-            gp = torch.empty_like(pred_c)
+        side = _side_stream(dev) if (_overlap_enabled() and cfg.need_pred) else None
+        ev_px = None
+        if px is not None and cfg.ws > 1:
+            # as in the forward: ask early, on the side stream, whether the peers are done with last step's `gall`
             if side is not None:
                 side.wait_stream(cur)
             with torch.cuda.stream(side if side is not None else cur):
-                call("cor_seg_loss_bwd", dev, ptr(pred_c), L.dtype_code(pred_c), ptr(t_save), ptr(w_save), ptr(per), N, H, W, None, _f(1.0),
-                     _f(0.25), _f(-1.0), ptr(g), ptr(gp), L.dtype_code(gp))
-            return gp
-
-        px = ctx.px
-        ev_px = None
-        if px is not None and ws > 1:
-            # same idea as in the forward: ask early, on the side stream, whether the peers are done with last step's `gall`
-            if side is not None:
-                side.wait_stream(cur)
-                with torch.cuda.stream(side):
-                    px.before_produce(1)
-                    ev_px = torch.cuda.Event()
-                    ev_px.record(side)
-            else:
                 px.before_produce(1)
-        if px is None or side is not None:
-            g_pred = seg_bwd()               # side stream: runs underneath the InfoNCE / pooling backward
+            ev_px = side.record_event() if side is not None else None
+        # on the side stream it runs underneath the InfoNCE / pooling backward
+        g_pred = _seg_backward(cfg, s, g, cur, side) if px is None or side is not None else None
         w16, w16_epoch = ctx.w16
-        gemm_ok = bg_mode != 1 and w16 is not None and getattr(w16, "_cor_epoch", -1) == w16_epoch and Cc % 8 == 0 and P % 8 == 0
-        if ctx.tail is not None and (gemm_ok or not need_emb):
-            # ONE launch: InfoNCE + fg-loss gradient of every row, through the row epilogue, cast to bf16 into the K-padded
-            # operand of the pooling-backward GEMM; and the query gradient (+ fg / bg terms) in extra CTAs, one set per query
-            Kp = (M + 63) // 64 * 64
-            a16 = torch.empty((B * Kp, Cc), dtype=torch.bfloat16, device=dev) if need_emb else None
-            g_q = torch.empty((B, Cc), **f32) if need_comb else None
-            work = ops._work(lib.cor_step_tail_work_bytes(B, M, Cc), dev)
-            name, ta = tau_arg("cor_step_tail_bwd")
-            call(name, dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), B, M, Cc, ta, ptr(g), _f(nce_weight),
-                 ptr(fg), ptr(inv_fg), ptr(stats), ptr(comb_c), ptr(out4), ptr(aux), _f(w_fg), _f(w_bg), ptr(a16), Kp, ptr(g_q),
-                 *gs_arg, ptr(work), ptr(ctx.tail))
-            if ctx.mem is not None:
-                ops._memory_dq(ctx.mem[0], q16, lse, inv_tau, sc, g, nce_weight, g_q, g_scale)
-            if need_comb:
-                g_comb = g_q.view(comb_shape).to(comb_dt)
-            if need_emb:
-                from .linear import gemm
-                Rp = w16.shape[1]
-                out_dt = emb_dt if emb_dt in (torch.float32, torch.bfloat16) else torch.float32
-                g_emb = gemm(a16, w16.view(B * Rp, P), Cc, P, Kp, a_mn=True, b_mn=True, batch=B, a_batch_rows=Kp, b_batch_rows=Rp,
-                             out_dtype=out_dt).view(B, Cc, h, w).to(emb_dt)
+        gemm_ok = (cfg.bg_mode != 1 and w16 is not None and getattr(w16, "_cor_epoch", -1) == w16_epoch and cfg.Cc % 8 == 0
+                   and (cfg.h * cfg.w) % 8 == 0)
+        # a tail forward whose bf16 weights a later forward of this shape rewrote takes the chain's fp32 pooling backward
+        use_tail = ctx.tail is not None and (gemm_ok or not cfg.need_emb)
+        if use_tail:
+            g_emb, g_comb = _tail_backward(ctx, s, g, g_scale)
         else:
-            # InfoNCE backward first: it WRITES g_regions (this rank's rows) and g_queries ...
-            Nr = r16.shape[0]
-            g_regions = torch.empty((n_local, Cc), **f32)
-            g_q = torch.empty((B, Cc), **f32)
-            work = ops._work(lib.cor_sim_work_bytes(B, Nr, Cc), dev)
-            if ws > 1:
-                # gradient of every gathered row, then a reduce-scatter back to the owning rank: measured faster than a
-                # collective-free backward that all-gathers the queries instead (profiles/README.md)
-                if ev_px is not None:
-                    cur.wait_event(ev_px)
-                g_all = px.gall if px is not None else torch.empty((Nr, Cc), **f32)
-                name, ta = tau_arg("cor_infonce_bwd")
-                call(name, dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), Nr, B, Cc, ta, ptr(g), _f(nce_weight),
-                     ptr(g_all), ptr(g_q), *gs_arg, ptr(work))
-                if px is not None:
-                    px.signal(1)
-                    if side is None:
-                        g_pred = seg_bwd()       # independent work between the signal and the pull hides the rank skew
-                    px.reduce(g_regions)         # fixed rank order: bit-identical from run to run
-                else:
-                    torch.distributed.reduce_scatter_tensor(g_regions, g_all, op=torch.distributed.ReduceOp.SUM)
-            else:
-                name, ta = tau_arg("cor_infonce_bwd")
-                call(name, dev, ptr(r16), ptr(q16), ptr(targets), ptr(lse), Nr, B, Cc, ta, ptr(g), _f(nce_weight),
-                     ptr(g_regions), ptr(g_q), *gs_arg, ptr(work))
-            # ... then the fg/bg backward ADDS its GT-row gradients into g_regions (row b*M) and g_queries
-            g_bg = torch.empty((B, Cc), **f32) if bg_mode == 1 else None
-            call("cor_fgbg_loss_bwd", dev, ptr(fg), _ll(M * Cc), ptr(bg), _ll(Cc), ptr(comb_c), _ll(Cc), B, Cc, bg_mode, ptr(out4), ptr(aux),
-                 ptr(g), _ll(0), _f(w_fg), _f(w_bg), ptr(g_regions), _ll(M * Cc), 1, ptr(g_bg), _ll(Cc), ptr(g_q), _ll(Cc), 1)
-            if ctx.mem is not None:          # this rank's memory, against this rank's queries
-                ops._memory_dq(ctx.mem[0], q16, lse, inv_tau, sc, g, nce_weight, g_q if need_comb else None, g_scale)
-            if need_comb:
-                g_comb = g_q.view(comb_shape).to(comb_dt)
-            if need_emb:
-                gs_fg = torch.empty((B * M, Cc), **f32)
-                call("cor_rows_finalize_bwd", dev, ptr(g_regions), ptr(fg), ptr(inv_fg), ptr(stats[:, 3:]), 4, _f(1e-8), B * M, Cc, 1, 1, 0,
-                     _f(0.0), ptr(gs_fg))
-                gs_bg_full = None
-                if g_bg is not None:          # paired bg mode: background gradient lives on the GT rows only
-                    gs_bg = torch.empty((B, Cc), **f32)
-                    call("cor_rows_finalize_bwd", dev, ptr(g_bg), ptr(bg), ptr(inv_bg), ptr(stats[:, 3:]), 4 * M, _f(1e-8), B, Cc, 1, 1, 1,
-                         _f(float(P)), ptr(gs_bg))
-                    gs_bg_full = torch.zeros((B, M, Cc), **f32)
-                    gs_bg_full[:, 0, :] = gs_bg
-                g_emb_c = torch.empty((B, Cc, h, w), dtype=emb_dt if emb_dt in (torch.float32, torch.bfloat16) else torch.float32, device=dev)
-                if gs_bg_full is None and gemm_ok:
-                    # d emb[b] (C x P) = gs[b]^T (C x M) w[b] (M x P): one batched tcgen05 GEMM on the bf16 weights the forward's
-                    # pooling GEMM used (still in their buffer: no later forward of this shape has rewritten them), both operands
-                    # MN-major as they lie; the gradient rows are cast to bf16 and zero-padded to a whole 64-row K block, which makes
-                    # the other operand's rows beyond M (the ones row, the next image) irrelevant.  Persistent tiles with coalesced
-                    # stores: 2-3x faster than the one-shot pool_bwd_umma kernel, which rebuilds both operands from fp32.
-                    from .linear import gemm
-                    Kp = (M + 63) // 64 * 64
-                    a16 = torch.empty((B * Kp, Cc), dtype=torch.bfloat16, device=dev)
-                    call("cor_cast_pad_rows_bf16", dev, ptr(gs_fg), B, M, Kp, Cc, ptr(a16))
-                    Rp = w16.shape[1]
-                    g_emb_c = gemm(a16, w16.view(B * Rp, P), Cc, P, Kp, a_mn=True, b_mn=True, batch=B, a_batch_rows=Kp, b_batch_rows=Rp,
-                                   out_dtype=g_emb_c.dtype).view(B, Cc, h, w)
-                else:
-                    name = "cor_pool_bwd_umma" if lib.cor_pool_bwd_umma_ok(B, Cc, P, M, int(gs_bg_full is not None)) else "cor_pool_bwd_feat"
-                    call(name, dev, ptr(gs_fg), ptr(gs_bg_full), ptr(w32), _ll(P), B, Cc, P, M, ops.W_CLAMP, ptr(g_emb_c), L._DTYPES[g_emb_c.dtype])
-                g_emb = g_emb_c.to(emb_dt)
+            g_emb, g_comb, g_pred = _chain_backward(ctx, s, g, g_scale, g_pred, gemm_ok, cur, side, ev_px)
         if side is not None:
             cur.wait_stream(side)
         if g_pred is not None:
-            g_pred = g_pred.to(pred_dt)
+            g_pred = g_pred.to(cfg.pred_dt)
         return g_pred, g_emb, g_comb, None, None, None, None, None, None, None, None, g_scale, None
 
 

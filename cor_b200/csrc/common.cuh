@@ -30,6 +30,27 @@ int sim_umma_ts_launch(const void* regions, const void* queries, int Nr, int Nq,
 // queries per tile of the log-sum-exp partials sim_umma_ts_launch leaves: the layout of a region memory's scan
 constexpr int kMemQT = 256;
 
+// Top-k candidate segments of the selecting epilogue of sim_umma_ts_kernel: per (query tile, CTA, query) a list of at
+// most `cap` (prefilter key, region index) entries, entry j of query t of a tile at [(qtile * nparts + cta) * cap + j]
+// [kMemQT] + t, in increasing region index; its length in cnt [qtile][nparts][kMemQT].  Each list holds that CTA's top
+// `ncand` regions under (key desc, index asc), plus entries that have not yet been compacted away.
+struct TopkSegments {
+  uint32_t* key;
+  int* idx;
+  int* cnt;
+  int cap, ncand;
+};
+// the selecting instantiation (sim_umma_ts.cu); *nparts = CTAs per query tile (<= max(1, sm_count() / ceil(Nq / 256)))
+int sim_umma_ts_select_launch(const void* regions, const void* queries, int Nr, int Nq, int D, TopkSegments seg, int* nparts,
+                              cudaStream_t st);
+
+// order-preserving float -> uint32 key of the top-k prefilter (larger float, larger key)
+__device__ __forceinline__ uint32_t fkey(float x) {
+  const uint32_t u = __float_as_uint(x);
+  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+__device__ __forceinline__ float fkey_inv(uint32_t k) { return __uint_as_float((k & 0x80000000u) ? (k & 0x7fffffffu) : ~k); }
+
 #define COR_REQUIRE(cond, ...)          \
   do {                                  \
     if (!(cond)) {                      \

@@ -450,45 +450,42 @@ __global__ void __launch_bounds__(256) infonce_bwd_q_kernel(const float* __restr
 }
 
 // ---- top-k: radix select on the prefilter scores, exact fp64 re-score, bitonic sort -----------------------
+// Two candidate sources share the select and the re-score / sort: a row of S (topk_kernel, cor_topk) and the candidate
+// lists of the selecting similarity epilogue (topk_select_kernel, cor_topk_select).
 constexpr int kTopkMaxCand = 512;
 
-__device__ __forceinline__ uint32_t fkey(float x) {
-  const uint32_t u = __float_as_uint(x);
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
+struct TopkShared {
+  unsigned hist[256];
+  unsigned sel_prefix, sel_remaining, n_gt, n_eq, warp_off[9];
+  unsigned long long cand[kTopkMaxCand];
+  int cand_idx[kTopkMaxCand];
+};
 
-__global__ void __launch_bounds__(256) topk_kernel(const float* __restrict__ S, const bf16* __restrict__ regions, const bf16* __restrict__ queries,
-                                                   int Nr, int D, int k, int ncand, long long* __restrict__ idx_out,
-                                                   float* __restrict__ score_out) {
-  __shared__ unsigned hist[256];
-  __shared__ unsigned sel_prefix, sel_remaining, n_gt, n_eq, warp_off[9];
-  __shared__ unsigned long long cand[kTopkMaxCand];
-  __shared__ int cand_idx[kTopkMaxCand];
-  const int q = blockIdx.x;
-  const float* row = S + (long long)q * Nr;
+// Block-wide (256 threads) radix select over the items u in [0, n) for which key_at(u, key) is true: sel_prefix = the key
+// of the need-th largest, sel_remaining = how many items with exactly that key belong to the top need.
+template <class KeyAt>
+__device__ void topk_radix_select(int n, unsigned need, KeyAt key_at, TopkShared& sh) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-
-  // 1. radix select: key of the ncand-th largest prefilter score
-  if (threadIdx.x == 0) { sel_prefix = 0; sel_remaining = (unsigned)ncand; }
+  if (threadIdx.x == 0) { sh.sel_prefix = 0; sh.sel_remaining = need; }
   __syncthreads();
   for (int pass = 0; pass < 4; ++pass) {
     const int shift = 24 - 8 * pass;
-    hist[threadIdx.x] = 0;
+    sh.hist[threadIdx.x] = 0;
     __syncthreads();
-    const unsigned prefix = sel_prefix;
+    const unsigned prefix = sh.sel_prefix;
     const unsigned mask = pass == 0 ? 0u : (0xffffffffu << (shift + 8));
-    for (int r = threadIdx.x; r < Nr; r += blockDim.x) {
-      const unsigned key = fkey(row[r]);
-      if ((key & mask) == prefix) atomicAdd(&hist[(key >> shift) & 255u], 1u);
+    for (int r = threadIdx.x; r < n; r += blockDim.x) {
+      unsigned key;
+      if (key_at(r, key) && (key & mask) == prefix) atomicAdd(&sh.hist[(key >> shift) & 255u], 1u);
     }
     __syncthreads();
     if (warp == 0) {
       // digit = largest d with (count of keys whose digit > d) < remaining: warp-parallel suffix scan over
       // the 256 bins (lane l owns bins 8l..8l+7, higher lanes = higher digits)
-      const unsigned rem = sel_remaining;
+      const unsigned rem = sh.sel_remaining;
       unsigned c[8], own = 0;
 #pragma unroll
-      for (int j = 0; j < 8; ++j) { c[j] = hist[lane * 8 + j]; own += c[j]; }
+      for (int j = 0; j < 8; ++j) { c[j] = sh.hist[lane * 8 + j]; own += c[j]; }
       // inclusive suffix sum of `own` over lanes
       unsigned suf = own;
 #pragma unroll
@@ -506,52 +503,26 @@ __global__ void __launch_bounds__(256) topk_kernel(const float* __restrict__ S, 
           if (acc + c[d] >= rem) break;
           acc += c[d];
         }
-        sel_prefix = prefix | ((unsigned)(lane * 8 + d) << shift);
-        sel_remaining = rem - acc;   // how many of the threshold-digit keys are still needed
+        sh.sel_prefix = prefix | ((unsigned)(lane * 8 + d) << shift);
+        sh.sel_remaining = rem - acc;   // how many of the threshold-digit keys are still needed
       }
     }
     __syncthreads();
   }
-  const unsigned T = sel_prefix;
-  const unsigned need_eq = sel_remaining;   // number of keys == T to take (smallest indices first)
+}
 
-  // 2. collect: all keys > T (any order), then the first `need_eq` keys == T in index order
-  if (threadIdx.x == 0) { n_gt = 0; n_eq = 0; }
-  __syncthreads();
-  for (int r0 = 0; r0 < Nr; r0 += blockDim.x) {
-    const int r = r0 + threadIdx.x;
-    const unsigned key = r < Nr ? fkey(row[r]) : 0u;
-    const bool gt = r < Nr && key > T, eq = r < Nr && key == T;
-    if (gt) {
-      const unsigned slot = atomicAdd(&n_gt, 1u);
-      if (slot < (unsigned)kTopkMaxCand) cand_idx[slot] = r;
-    }
-    const unsigned bal = __ballot_sync(0xffffffffu, eq);
-    if (lane == 0) warp_off[warp] = __popc(bal);
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      unsigned run = n_eq;
-      for (int w = 0; w < 8; ++w) { const unsigned c = warp_off[w]; warp_off[w] = run; run += c; }
-      warp_off[8] = run;
-    }
-    __syncthreads();
-    if (eq) {
-      const unsigned pos = warp_off[warp] + __popc(bal & ((1u << lane) - 1u));
-      if (pos < need_eq) cand_idx[ncand - need_eq + pos] = r;
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) n_eq = warp_off[8];
-    __syncthreads();
-  }
-
-  // 3. exact re-score (fp64 accumulation of exact bf16 products, rounded once to fp32) and sort key
+// Exact re-score of the ncand candidates in sh.cand_idx (fp64 accumulation of exact bf16 products, rounded once to fp32),
+// bitonic sort on (score desc, index asc), and the first k to idx_out / score_out row q.
+__device__ void topk_rescore_sort(TopkShared& sh, const bf16* __restrict__ regions, const bf16* __restrict__ queries, int q, int D, int k,
+                                  int ncand, long long* __restrict__ idx_out, float* __restrict__ score_out) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   int npow = 1;
   while (npow < ncand) npow <<= 1;
-  for (int c = threadIdx.x; c < npow; c += blockDim.x) cand[c] = 0ull;   // padding sorts last
+  for (int c = threadIdx.x; c < npow; c += blockDim.x) sh.cand[c] = 0ull;   // padding sorts last
   __syncthreads();
   // one warp per candidate: lanes take 8-element slices of the row pair, fp64 FMA, fixed-order butterfly
   for (int c = warp; c < ncand; c += 8) {
-    const int r = cand_idx[c];
+    const int r = sh.cand_idx[c];
     double acc = 0.0;
     for (int d0 = lane * 8; d0 < D; d0 += 256) {
       const uint4 qa = *reinterpret_cast<const uint4*>(queries + (long long)q * D + d0);
@@ -566,7 +537,7 @@ __global__ void __launch_bounds__(256) topk_kernel(const float* __restrict__ S, 
     acc = warp_sum(acc);
     if (lane == 0) {
       const float sc = (float)acc;
-      cand[c] = ((unsigned long long)fkey(sc) << 32) | (unsigned long long)(0xffffffffu - (unsigned)r);
+      sh.cand[c] = ((unsigned long long)fkey(sc) << 32) | (unsigned long long)(0xffffffffu - (unsigned)r);
     }
   }
   __syncthreads();
@@ -577,20 +548,133 @@ __global__ void __launch_bounds__(256) topk_kernel(const float* __restrict__ S, 
         const int j = i ^ stride;
         if (j > i) {
           const bool desc = (i & size) == 0;
-          const unsigned long long a = cand[i], b = cand[j];
-          if ((a < b) == desc) { cand[i] = b; cand[j] = a; }
+          const unsigned long long a = sh.cand[i], b = sh.cand[j];
+          if ((a < b) == desc) { sh.cand[i] = b; sh.cand[j] = a; }
         }
       }
       __syncthreads();
     }
   }
   for (int c = threadIdx.x; c < k; c += blockDim.x) {
-    const unsigned long long key = cand[c];
-    const unsigned fk = (unsigned)(key >> 32);
-    const unsigned u = (fk & 0x80000000u) ? (fk & 0x7fffffffu) : ~fk;
+    const unsigned long long key = sh.cand[c];
     idx_out[(long long)q * k + c] = (long long)(0xffffffffu - (unsigned)(key & 0xffffffffu));
-    score_out[(long long)q * k + c] = __uint_as_float(u);
+    score_out[(long long)q * k + c] = fkey_inv((unsigned)(key >> 32));
   }
+}
+
+__global__ void __launch_bounds__(256) topk_kernel(const float* __restrict__ S, const bf16* __restrict__ regions, const bf16* __restrict__ queries,
+                                                   int Nr, int D, int k, int ncand, long long* __restrict__ idx_out,
+                                                   float* __restrict__ score_out) {
+  __shared__ TopkShared sh;
+  const int q = blockIdx.x;
+  const float* row = S + (long long)q * Nr;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+
+  // 1. radix select: key of the ncand-th largest prefilter score
+  topk_radix_select(Nr, (unsigned)ncand, [&](int r, unsigned& key) { key = fkey(row[r]); return true; }, sh);
+  const unsigned T = sh.sel_prefix;
+  const unsigned need_eq = sh.sel_remaining;   // number of keys == T to take (smallest indices first)
+
+  // 2. collect: all keys > T (any order), then the first `need_eq` keys == T in index order
+  if (threadIdx.x == 0) { sh.n_gt = 0; sh.n_eq = 0; }
+  __syncthreads();
+  for (int r0 = 0; r0 < Nr; r0 += blockDim.x) {
+    const int r = r0 + threadIdx.x;
+    const unsigned key = r < Nr ? fkey(row[r]) : 0u;
+    const bool gt = r < Nr && key > T, eq = r < Nr && key == T;
+    if (gt) {
+      const unsigned slot = atomicAdd(&sh.n_gt, 1u);
+      if (slot < (unsigned)kTopkMaxCand) sh.cand_idx[slot] = r;
+    }
+    const unsigned bal = __ballot_sync(0xffffffffu, eq);
+    if (lane == 0) sh.warp_off[warp] = __popc(bal);
+    __syncthreads();
+    if (threadIdx.x == 0) {
+      unsigned run = sh.n_eq;
+      for (int w = 0; w < 8; ++w) { const unsigned c = sh.warp_off[w]; sh.warp_off[w] = run; run += c; }
+      sh.warp_off[8] = run;
+    }
+    __syncthreads();
+    if (eq) {
+      const unsigned pos = sh.warp_off[warp] + __popc(bal & ((1u << lane) - 1u));
+      if (pos < need_eq) sh.cand_idx[ncand - need_eq + pos] = r;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) sh.n_eq = sh.warp_off[8];
+    __syncthreads();
+  }
+
+  // 3. exact re-score and sort
+  topk_rescore_sort(sh, regions, queries, q, D, k, ncand, idx_out, score_out);
+}
+
+// Top-k over the candidate lists of the selecting similarity epilogue (TopkSegments): one CTA per query takes the union of
+// its nparts lists, selects the best ncand by (key desc, index asc) and re-scores and sorts them as topk_kernel does.  The
+// lists are not in global index order, so equal keys at the cut are settled by a second select on the region index.
+constexpr int kTopkMaxParts = 1024;
+
+__global__ void __launch_bounds__(256) topk_select_kernel(TopkSegments seg, int nparts, const bf16* __restrict__ regions,
+                                                          const bf16* __restrict__ queries, int D, int k, long long* __restrict__ idx_out,
+                                                          float* __restrict__ score_out) {
+  __shared__ TopkShared sh;
+  __shared__ int off[kTopkMaxParts + 1];
+  const int q = blockIdx.x, tile = q / kMemQT, t = q % kMemQT;
+  const int ncand = seg.ncand;
+  for (int p = threadIdx.x; p < nparts; p += blockDim.x) off[p + 1] = __ldcg(seg.cnt + ((size_t)tile * nparts + p) * kMemQT + t);
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    off[0] = 0;
+    for (int p = 1; p <= nparts; ++p) off[p] += off[p - 1];
+  }
+  __syncthreads();
+  const int n = off[nparts];
+  // item u of the union -> its entry: list p with off[p] <= u < off[p + 1]
+  auto entry = [&](int u) {
+    int lo = 0, hi = nparts;
+    while (hi - lo > 1) {
+      const int mid = (lo + hi) >> 1;
+      if (off[mid] <= u) lo = mid;
+      else hi = mid;
+    }
+    return (((size_t)tile * nparts + lo) * seg.cap + (u - off[lo])) * kMemQT + t;
+  };
+
+  // 1. key of the ncand-th best candidate and how many of its equals to take
+  topk_radix_select(n, (unsigned)ncand, [&](int u, unsigned& key) { key = __ldcg(seg.key + entry(u)); return true; }, sh);
+  const unsigned T = sh.sel_prefix, need_eq = sh.sel_remaining;
+  __syncthreads();
+  // 2. keys > T go in; count the keys == T
+  if (threadIdx.x == 0) { sh.n_gt = 0; sh.n_eq = 0; }
+  __syncthreads();
+  for (int u = threadIdx.x; u < n; u += blockDim.x) {
+    const size_t e = entry(u);
+    const unsigned key = __ldcg(seg.key + e);
+    if (key > T) sh.cand_idx[atomicAdd(&sh.n_gt, 1u)] = __ldcg(seg.idx + e);
+    else if (key == T) atomicAdd(&sh.n_eq, 1u);
+  }
+  __syncthreads();
+  // 3. the need_eq smallest indices among the keys == T: all of them, or those at or above the need_eq-th largest ~index
+  unsigned ti = 0u;
+  if (sh.n_eq > need_eq) {
+    topk_radix_select(n, need_eq, [&](int u, unsigned& key) {
+      const size_t e = entry(u);
+      key = ~(unsigned)__ldcg(seg.idx + e);
+      return __ldcg(seg.key + e) == T;
+    }, sh);
+    ti = sh.sel_prefix;
+  }
+  __syncthreads();                                 // every thread has read n_eq and sel_prefix
+  if (threadIdx.x == 0) sh.n_eq = 0;
+  __syncthreads();
+  for (int u = threadIdx.x; u < n; u += blockDim.x) {
+    const size_t e = entry(u);
+    if (__ldcg(seg.key + e) != T) continue;
+    const int r = __ldcg(seg.idx + e);
+    if (~(unsigned)r >= ti) sh.cand_idx[ncand - need_eq + atomicAdd(&sh.n_eq, 1u)] = r;
+  }
+  __syncthreads();
+  // 4. exact re-score and sort
+  topk_rescore_sort(sh, regions, queries, q, D, k, ncand, idx_out, score_out);
 }
 
 }  // namespace cor
@@ -794,14 +878,62 @@ extern "C" int cor_infonce_bwd_ls(const void* regions, const void* queries, cons
                      stream);
 }
 
+// ncand = min(k + max(16, k / 2), 512) prefilter candidates per query, before the cap at Nr
+static int topk_ncand(int k) {
+  const int slack = k / 2 < 16 ? 16 : k / 2;
+  return k + slack < kTopkMaxCand ? k + slack : kTopkMaxCand;
+}
+
 extern "C" int cor_topk(const float* S, const void* regions, const void* queries, int Nr, int Nq, int D, int k, long long* idx,
                         float* score, cor_stream_t stream) {
   COR_REQUIRE(S && regions && queries && idx && score, "cor_topk: null pointer");
   COR_REQUIRE(k > 0 && k <= Nr && k <= 256, "cor_topk: need 0 < k <= min(Nr, 256) (k=%d, Nr=%d)", k, Nr);
-  int slack = k / 2 < 16 ? 16 : k / 2;
-  int ncand = k + slack;
+  int ncand = topk_ncand(k);
   if (ncand > Nr) ncand = Nr;
-  if (ncand > kTopkMaxCand) ncand = kTopkMaxCand;
   topk_kernel<<<Nq, 256, 0, as_stream(stream)>>>(S, (const bf16*)regions, (const bf16*)queries, Nr, D, k, ncand, idx, score);
   return check_launch("topk_kernel");
+}
+
+// candidate lists: key and index [qtiles][parts][cap][256] each, then the lengths [qtiles][parts][256]; cap = ncand + 128
+static TopkSegments topk_segments(void* work, int Nq, int Nr, int k, int parts) {
+  const int ncand = topk_ncand(k), cap = ncand + 128;
+  const size_t entries = (size_t)ceil_div(Nq, kMemQT) * parts * cap * kMemQT;
+  TopkSegments seg;
+  seg.key = (uint32_t*)work;
+  seg.idx = (int*)(seg.key + entries);
+  seg.cnt = seg.idx + entries;
+  seg.cap = cap;
+  seg.ncand = ncand < Nr ? ncand : Nr;
+  return seg;
+}
+
+static int topk_select_parts(int Nq) {
+  const int gx = sm_count() / ceil_div(Nq, kMemQT);
+  return gx < 1 ? 1 : gx;
+}
+
+extern "C" size_t cor_topk_select_work_bytes(int Nq, int Nr, int D, int k) {
+  (void)D;
+  if (Nq <= 0 || Nr <= 0 || k <= 0 || k > 256) return 0;
+  const int parts = topk_select_parts(Nq);
+  const size_t lists = (size_t)ceil_div(Nq, kMemQT) * parts * kMemQT;
+  return lists * ((size_t)(topk_ncand(k) + 128) * 8 + 4);
+}
+
+extern "C" int cor_topk_select(const void* regions, const void* queries, int Nr, int Nq, int D, int k, long long* idx, float* score,
+                               void* work, cor_stream_t stream) {
+  COR_REQUIRE(regions && queries && idx && score && work, "cor_topk_select: null pointer");
+  COR_REQUIRE(Nr > 0 && Nq > 0, "cor_topk_select: need Nr >= 1 and Nq >= 1 (Nr=%d Nq=%d)", Nr, Nq);
+  COR_REQUIRE(k > 0 && k <= Nr && k <= 256, "cor_topk_select: need 0 < k <= min(Nr, 256) (k=%d, Nr=%d)", k, Nr);
+  COR_REQUIRE(D == 64 || D == 128 || D == 192 || D == 256, "cor_topk_select: D=%d must be 64, 128, 192 or 256", D);
+  COR_REQUIRE((((uintptr_t)queries) & 15) == 0, "cor_topk_select: queries must be 16-byte aligned");
+  cudaStream_t st = as_stream(stream);
+  const TopkSegments seg = topk_segments(work, Nq, Nr, k, topk_select_parts(Nq));
+  int nparts = 0;
+  int rc = cor::sim_umma_ts_select_launch(regions, queries, Nr, Nq, D, seg, &nparts, st);
+  if (rc) return rc;
+  COR_REQUIRE(nparts <= kTopkMaxParts, "cor_topk_select: %d lists per query (at most %d)", nparts, kTopkMaxParts);
+  // the arrays are sized for the most CTAs per query tile; both kernels index the lists by the nparts CTAs that ran
+  topk_select_kernel<<<Nq, 256, 0, st>>>(seg, nparts, (const bf16*)regions, (const bf16*)queries, D, k, idx, score);
+  return check_launch("topk_select_kernel");
 }

@@ -14,6 +14,15 @@
 // With <= 128 queries there is one half and its accumulator alternates between the two slots tile by tile.
 // Warp roles (320 threads): 0..7 epilogue (lane quarter w % 4, half w / 4), 8 TMA producer, 9 TMEM owner + MMA issuer.
 // LSE partials in the work buffer as [qtile][gridDim.x][256][2], the layout sim_lse_combine_kernel and cor_infonce_tail read.
+//
+// The selecting instantiation (kSelect, cor_topk_select) keeps the same TMA / MMA roles and replaces the log-sum-exp by a
+// top-k candidate list per (query, CTA) in the work buffer (TopkSegments, common.cuh), so S is never written.  A thread
+// appends a score only if it beats its threshold th (a register, -inf at first).  Once its list could not take another
+// tile's 128 scores, it compacts the list in place, stably, to its best ncand under (key desc, index asc) and raises th
+// to the key of the last entry kept; later entries must beat th strictly.  A CTA walks its tiles in increasing region
+// index, so an equal key that arrives later ranks below every equal key already kept: each list keeps its CTA's exact
+// top ncand, ties included, and the union of the lists holds the global top ncand.  At most one compaction per thread
+// per tile, after the thread has released the accumulator, so the MMAs of the next tile run under it.
 #include <stdlib.h>
 
 #include "umma.cuh"
@@ -32,9 +41,59 @@ struct TsSmemTail {
   uint32_t tmem_base;
 };
 
+// Stable in-place compaction of one thread's candidate list (entry j at key[j * kTsBM]) from cnt > ncand entries, all with
+// key >= lo and none above hi, to its best ncand under (key desc, index asc).  The cut key T is found by counting the keys
+// at 15 pivots spread over [lo, hi]: each pass narrows the interval 16-fold (at most 8 passes over 32-bit keys) and stops
+// early once a pivot has exactly ncand keys at or above it.  Returns the key of the worst entry kept.  Rare in a random
+// gallery, once per tile when the scores rise with the index; out of line so that it costs the tile loop no registers.
+__device__ __noinline__ uint32_t ts_compact(uint32_t* __restrict__ key, int* __restrict__ idx, int cnt, int ncand, uint32_t lo, uint32_t hi) {
+  int above = 0;                                   // entries with key > hi
+  uint32_t T;
+  int need_eq;                                     // entries with key == T to keep (the first ones: smallest indices)
+  for (;;) {
+    if (lo == hi) { T = lo; need_eq = ncand - above; break; }
+    const uint64_t span = (uint64_t)(hi - lo) + 1u;
+    uint32_t p[15];
+    int c[15];
+#pragma unroll
+    for (int j = 0; j < 15; ++j) { p[j] = lo + (uint32_t)((span * (uint64_t)(j + 1)) >> 4); c[j] = 0; }
+    for (int e = 0; e < cnt; ++e) {
+      const uint32_t x = key[(size_t)e * kTsBM];
+#pragma unroll
+      for (int j = 0; j < 15; ++j) c[j] += x >= p[j] ? 1 : 0;
+    }
+    int jj = -1;                                   // counts fall with j: the last pivot with >= ncand keys at or above it
+#pragma unroll
+    for (int j = 0; j < 15; ++j) if (c[j] >= ncand) jj = j;
+    if (jj >= 0 && c[jj] == ncand) { T = p[jj] - 1u; need_eq = 0; break; }   // p[jj] > lo: #{key >= lo} > ncand throughout
+    uint32_t nhi = hi;
+    int nabove = above;
+#pragma unroll
+    for (int j = 0; j < 15; ++j) if (j == jj + 1) { nhi = p[j] - 1u; nabove = c[j]; }
+#pragma unroll
+    for (int j = 0; j < 15; ++j) if (j == jj) lo = p[j];
+    hi = nhi;
+    above = nabove;
+  }
+  int w = 0, eq = 0;
+  uint32_t kmin = 0xffffffffu;
+  for (int e = 0; e < cnt; ++e) {
+    const uint32_t x = key[(size_t)e * kTsBM];
+    bool keep = x > T;
+    if (x == T) { keep = eq < need_eq; eq += keep ? 1 : 0; }
+    if (keep) {
+      if (w != e) { key[(size_t)w * kTsBM] = x; idx[(size_t)w * kTsBM] = idx[(size_t)e * kTsBM]; }
+      ++w;
+      kmin = min(kmin, x);
+    }
+  }
+  return kmin;
+}
+
+template <bool kSelect>
 __global__ void __launch_bounds__(320, 1) sim_umma_ts_kernel(const __grid_constant__ CUtensorMap tmR, const bf16* __restrict__ queries, int Nr,
                                                              int Nq, int nkb, int nstages, float inv_tau, const float* __restrict__ scale,
-                                                             float* __restrict__ part, const int* __restrict__ count) {
+                                                             float* __restrict__ part, const int* __restrict__ count, TopkSegments seg) {
   extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t* base = reinterpret_cast<uint8_t*>(((uintptr_t)smem + 1023) & ~(uintptr_t)1023);
   uint8_t* r_smem = base;
@@ -137,47 +196,9 @@ __global__ void __launch_bounds__(320, 1) sim_umma_ts_kernel(const __grid_consta
     __syncwarp();
     if (lane == 0) mbar_arrive(&tail->afull);
 
-    if (scale) inv_tau = __ldg(scale);
-    const float c2 = inv_tau * 1.4426950408889634f;
-    float m = -INFINITY, ssum = 0.f;
-    auto proc = [&](uint32_t (&v)[32], int r0, int col) {
-      const int nval = min(32, Nr - (r0 + col));
-      if (nval == 32) {
-        float t10[10];
-#pragma unroll
-        for (int j = 0; j < 10; ++j) t10[j] = max3(__uint_as_float(v[3 * j]), __uint_as_float(v[3 * j + 1]), __uint_as_float(v[3 * j + 2]));
-        const float u0 = max3(t10[0], t10[1], t10[2]), u1 = max3(t10[3], t10[4], t10[5]), u2 = max3(t10[6], t10[7], t10[8]);
-        const float u3 = max3(t10[9], __uint_as_float(v[30]), __uint_as_float(v[31]));
-        const float cm = fmaxf(max3(u0, u1, u2), u3);
-        if (cm > m) { ssum *= ex2_approx((m - cm) * c2); m = cm; }
-        const float mc = m * c2;
-        const uint64_t C2 = pack2(c2, c2), NM = pack2(-mc, -mc);
-        uint64_t a0 = 0ull, a1 = 0ull;
-#pragma unroll
-        for (int j = 0; j < 16; ++j) {
-          const uint64_t x2 = fma2(pack2u(v[2 * j], v[2 * j + 1]), C2, NM);
-          float x0, x1;
-          unpack2(x2, x0, x1);
-          const uint64_t e2 = pack2(ex2_approx(x0), ex2_approx(x1));
-          if (j & 1) a1 = add2(a1, e2);
-          else a0 = add2(a0, e2);
-        }
-        float s0, s1;
-        unpack2(add2(a0, a1), s0, s1);
-        ssum += s0 + s1;
-      } else {
-        float cm = -INFINITY;
-#pragma unroll
-        for (int j = 0; j < 32; ++j)
-          if (j < nval) cm = fmaxf(cm, __uint_as_float(v[j]));
-        if (cm > m) { ssum *= ex2_approx((m - cm) * c2); m = cm; }
-        const float mc = m * c2;
-#pragma unroll
-        for (int j = 0; j < 32; ++j)
-          if (j < nval) ssum += ex2_approx(fmaf(__uint_as_float(v[j]), c2, -mc));
-      }
-    };
-    if (active) {
+    // this CTA's tiles, in increasing region index: accumulator -> registers -> proc(v, r0, col) per 32 columns, then
+    // after() once the accumulator is released
+    auto walk = [&](auto&& proc, auto&& after) {
       int i = 0;
       for (int t = blockIdx.x; t < ntiles; t += gridDim.x, ++i) {
         const int seq = i * nhalf + hf, slot = seq & 1, use = seq >> 1;
@@ -202,10 +223,100 @@ __global__ void __launch_bounds__(320, 1) sim_umma_ts_kernel(const __grid_consta
         __syncwarp();
         if (lane == 0) mbar_arrive(&tail->acc_empty[slot]);     // accumulator in registers: the MMAs of the next use may start
         if (nch > 3) proc(vb, r0, 96);
+        after();
       }
-      float* o = part + (((long long)blockIdx.y * gridDim.x + blockIdx.x) * kTsBM + hf * kTsHalf + qd * 32 + lane) * 2;
-      o[0] = m * inv_tau;
-      o[1] = ssum;
+    };
+    if constexpr (kSelect) {
+      const bool mine = active && q < Nq;
+      const int tq = hf * kTsHalf + qd * 32 + lane;
+      const size_t s0 = ((size_t)blockIdx.y * gridDim.x + blockIdx.x) * (size_t)seg.cap * kTsBM + tq;
+      uint32_t* skey = seg.key + s0;
+      int* sidx = seg.idx + s0;
+      float th = mine ? -INFINITY : INFINITY;       // padding queries never append
+      uint32_t kmax = 0u;
+      int cnt = 0;
+      auto proc = [&](uint32_t (&v)[32], int r0, int col) {
+        const int nval = min(32, Nr - (r0 + col));
+        float cm = -INFINITY;
+        if (nval == 32) {
+          float t10[10];
+#pragma unroll
+          for (int j = 0; j < 10; ++j) t10[j] = max3(__uint_as_float(v[3 * j]), __uint_as_float(v[3 * j + 1]), __uint_as_float(v[3 * j + 2]));
+          cm = fmaxf(max3(max3(t10[0], t10[1], t10[2]), max3(t10[3], t10[4], t10[5]), max3(t10[6], t10[7], t10[8])),
+                     max3(t10[9], __uint_as_float(v[30]), __uint_as_float(v[31])));
+        } else {
+#pragma unroll
+          for (int j = 0; j < 32; ++j)
+            if (j < nval) cm = fmaxf(cm, __uint_as_float(v[j]));
+        }
+        if (!(cm > th)) return;
+#pragma unroll
+        for (int j = 0; j < 32; ++j) {
+          const float x = __uint_as_float(v[j]);
+          if (j < nval && x > th) {
+            const uint32_t kx = fkey(x == 0.f ? 0.f : x);     // -0 and +0 are one key, as th compares them
+            skey[(size_t)cnt * kTsBM] = kx;
+            sidx[(size_t)cnt * kTsBM] = r0 + col + j;
+            ++cnt;
+            kmax = max(kmax, kx);
+          }
+        }
+      };
+      auto after = [&]() {
+        if (cnt > seg.cap - kTsBN) th = fkey_inv(ts_compact(skey, sidx, cnt, seg.ncand, fkey(th), kmax)), cnt = seg.ncand;
+        __syncwarp();                                  // tcgen05.ld is warp-collective
+      };
+      if (active) {
+        walk(proc, after);
+        seg.cnt[((size_t)blockIdx.y * gridDim.x + blockIdx.x) * kTsBM + tq] = cnt;
+      }
+    } else {
+      if (scale) inv_tau = __ldg(scale);
+      const float c2 = inv_tau * 1.4426950408889634f;
+      float m = -INFINITY, ssum = 0.f;
+      auto proc = [&](uint32_t (&v)[32], int r0, int col) {
+        const int nval = min(32, Nr - (r0 + col));
+        if (nval == 32) {
+          float t10[10];
+#pragma unroll
+          for (int j = 0; j < 10; ++j) t10[j] = max3(__uint_as_float(v[3 * j]), __uint_as_float(v[3 * j + 1]), __uint_as_float(v[3 * j + 2]));
+          const float u0 = max3(t10[0], t10[1], t10[2]), u1 = max3(t10[3], t10[4], t10[5]), u2 = max3(t10[6], t10[7], t10[8]);
+          const float u3 = max3(t10[9], __uint_as_float(v[30]), __uint_as_float(v[31]));
+          const float cm = fmaxf(max3(u0, u1, u2), u3);
+          if (cm > m) { ssum *= ex2_approx((m - cm) * c2); m = cm; }
+          const float mc = m * c2;
+          const uint64_t C2 = pack2(c2, c2), NM = pack2(-mc, -mc);
+          uint64_t a0 = 0ull, a1 = 0ull;
+#pragma unroll
+          for (int j = 0; j < 16; ++j) {
+            const uint64_t x2 = fma2(pack2u(v[2 * j], v[2 * j + 1]), C2, NM);
+            float x0, x1;
+            unpack2(x2, x0, x1);
+            const uint64_t e2 = pack2(ex2_approx(x0), ex2_approx(x1));
+            if (j & 1) a1 = add2(a1, e2);
+            else a0 = add2(a0, e2);
+          }
+          float s0, s1;
+          unpack2(add2(a0, a1), s0, s1);
+          ssum += s0 + s1;
+        } else {
+          float cm = -INFINITY;
+#pragma unroll
+          for (int j = 0; j < 32; ++j)
+            if (j < nval) cm = fmaxf(cm, __uint_as_float(v[j]));
+          if (cm > m) { ssum *= ex2_approx((m - cm) * c2); m = cm; }
+          const float mc = m * c2;
+#pragma unroll
+          for (int j = 0; j < 32; ++j)
+            if (j < nval) ssum += ex2_approx(fmaf(__uint_as_float(v[j]), c2, -mc));
+        }
+      };
+      if (active) {
+        walk(proc, [] {});
+        float* o = part + (((long long)blockIdx.y * gridDim.x + blockIdx.x) * kTsBM + hf * kTsHalf + qd * 32 + lane) * 2;
+        o[0] = m * inv_tau;
+        o[1] = ssum;
+      }
     }
   }
   tc_fence_before();
@@ -213,12 +324,11 @@ __global__ void __launch_bounds__(320, 1) sim_umma_ts_kernel(const __grid_consta
   if (warp == kTsMmaWarp) tmem_dealloc(tmem, 512);
 }
 
-// LSE-only launcher (sim_umma.cu stores S with the kernel that keeps both operands in shared memory).  Returns the
-// number of partial records per query tile in *nparts.
-static_assert(kTsBM == kMemQT, "a region memory's scan partials are laid out per kTsBM-query tile");
+static_assert(kTsBM == kMemQT, "a region memory's scan partials and the top-k lists are laid out per kTsBM-query tile");
 
-int sim_umma_ts_launch(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, const float* scale, void* work,
-                       int* nparts, cudaStream_t st, const int* count) {
+template <bool kSelect>
+static int ts_launch(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, const float* scale, void* work,
+                     int* nparts, cudaStream_t st, const int* count, TopkSegments seg) {
   const int qtiles = ceil_div(Nq, kTsBM), ntiles = ceil_div(Nr, kTsBN);
   CUtensorMap tmR;
   int rc = umma::encode_tmap_bf16_2d(&tmR, regions, (uint64_t)Nr, (uint64_t)D, kTsBN, kTsBK);
@@ -230,11 +340,23 @@ int sim_umma_ts_launch(const void* regions, const void* queries, int Nr, int Nq,
   int nstages = (int)((227 * 1024 - sizeof(TsSmemTail) - 1024) / kTsBBytes);
   if (nstages > kTsMaxStages) nstages = kTsMaxStages;
   const size_t smem = (size_t)nstages * kTsBBytes + sizeof(TsSmemTail) + 1024;
-  COR_CUDA(cudaFuncSetAttribute(sim_umma_ts_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  sim_umma_ts_kernel<<<dim3(gx, qtiles), 320, smem, st>>>(tmR, reinterpret_cast<const bf16*>(queries), Nr, Nq, nkb, nstages, inv_tau,
-                                                         scale, reinterpret_cast<float*>(work), count);
+  COR_CUDA(cudaFuncSetAttribute(sim_umma_ts_kernel<kSelect>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  sim_umma_ts_kernel<kSelect><<<dim3(gx, qtiles), 320, smem, st>>>(tmR, reinterpret_cast<const bf16*>(queries), Nr, Nq, nkb, nstages,
+                                                                   inv_tau, scale, reinterpret_cast<float*>(work), count, seg);
   *nparts = gx;
   return check_launch("sim_umma_ts_kernel");
+}
+
+// LSE-only launcher (sim_umma.cu stores S with the kernel that keeps both operands in shared memory).  Returns the
+// number of partial records per query tile in *nparts.
+int sim_umma_ts_launch(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, const float* scale, void* work,
+                       int* nparts, cudaStream_t st, const int* count) {
+  return ts_launch<false>(regions, queries, Nr, Nq, D, inv_tau, scale, work, nparts, st, count, TopkSegments{});
+}
+
+int sim_umma_ts_select_launch(const void* regions, const void* queries, int Nr, int Nq, int D, TopkSegments seg, int* nparts,
+                              cudaStream_t st) {
+  return ts_launch<true>(regions, queries, Nr, Nq, D, 0.f, nullptr, nullptr, nparts, st, nullptr, seg);
 }
 
 }  // namespace cor

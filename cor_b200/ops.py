@@ -41,6 +41,8 @@ _KERNELS_PER_CALL = {
     # cross-batch region memory: cor_memory_dq is 2 launches, 3 with the logit scale's gradient (its caller passes the count)
     "cor_memory_reset": 1, "cor_memory_enqueue": 1, "cor_memory_scan": 1, "cor_infonce_tail_mem": 1, "cor_step_tail_fwd_mem": 1,
     "cor_memory_dq": 2,
+    # top-k without S: the selecting similarity kernel, then select / re-score / sort
+    "cor_topk_select": 2,
 }
 
 
@@ -689,16 +691,58 @@ def infonce_loss(regions: torch.Tensor, queries: torch.Tensor, targets: torch.Te
     return _InfoNCEFn.apply(regions, queries, targets, 0.07 if tau is None else float(tau), engine, regions_bf16, logit_scale, memory)
 
 
+# Measured on one B200 at 1000 W (profiles/r06_topk_bench.log), D = 256: at k = 10 the fused path takes 2.65 against
+# 12.5 ms at 256 x 1 M and 24.7 against 75.1 ms at 4 096 x 1 M, but 0.195 against 0.040 ms at 256 x 4 096 (S in L2);
+# at k = 256 the S route wins at every size measured, up to S = 16 GB (4 096 x 1 M).  Beyond 16 GB of S the fused path is
+# taken whatever k: its memory does not grow with the gallery.  Sizes between the measured points are not measured.
+_TOPK_FUSED_MAX_K = 10
+_TOPK_FUSED_MIN_ROWS = 1 << 20
+_TOPK_S_MAX_BYTES = 16 << 30
+
+
+def _topk_fused(Nq: int, Nr: int, D: int, k: int, engine: str) -> bool:
+    """Top-k that selects inside the tensor-core similarity kernel (cor_topk_select) instead of writing S."""
+    if engine not in ("auto", "umma") or D not in (64, 128, 192, 256):
+        return False
+    return (k <= _TOPK_FUSED_MAX_K and Nr >= _TOPK_FUSED_MIN_ROWS) or Nq * Nr * 4 > _TOPK_S_MAX_BYTES
+
+
+def _topk_select(r16: torch.Tensor, q16: torch.Tensor, k: int):
+    """cor_topk_select on bf16 rows: (idx, score) without writing S."""
+    dev = r16.device
+    Nr, D = r16.shape
+    Nq = q16.shape[0]
+    idx = torch.empty((Nq, k), dtype=torch.int64, device=dev)
+    score = torch.empty((Nq, k), dtype=torch.float32, device=dev)
+    work = _work(L.load().cor_topk_select_work_bytes(Nq, Nr, D, int(k)), dev)
+    _call("cor_topk_select", dev, ptr(r16), ptr(q16), Nr, Nq, D, int(k), ptr(idx), ptr(score), ptr(work))
+    return idx, score
+
+
 def topk_retrieve(regions: torch.Tensor, queries: torch.Tensor, k: int, engine: str = "auto"):
-    """Per query the k best regions under (score desc, index asc): (idx [Nq,k] int64, score [Nq,k] f32).
-    Prefilter on tensor-core / streaming scores, exact fp64 re-score of the top k+slack candidates."""
+    """Per query the k best regions under (score desc, index asc): (idx [Nq,k] int64, score [Nq,k] f32), 1 <= k <=
+    min(Nr, 256).  Prefilter on tensor-core / streaming scores, exact fp64 re-score of the top k+slack candidates.
+
+    With ``engine`` "auto" or "umma", D in {64, 128, 192, 256} and either k <= 10 on a gallery of at least 2^20 rows or
+    a score matrix S of more than 16 GB, the tensor-core similarity kernel keeps each query's candidates while it
+    scores, so S [Nq, Nr] is never written: the call's memory is the gallery, the queries, the outputs and
+    ``cor_topk_select_work_bytes`` of scratch, which does not grow with Nr.  Other shapes write S (on the tensor cores,
+    or on the CUDA cores with ``engine="stream"`` and other widths) and select from it, which measured faster there.
+    A gallery of bf16 rows is read in place; fp32 rows are first cast to a bf16 copy."""
+    if regions.shape[-1] != queries.shape[-1]:
+        raise CorError(f"topk_retrieve: regions {tuple(regions.shape)} and queries {tuple(queries.shape)} differ in width")
+    Nr = regions.numel() // max(regions.shape[-1], 1)
+    if not 1 <= int(k) <= min(Nr, 256):
+        raise CorError(f"topk_retrieve: need 1 <= k <= min(Nr, 256), got k={k} with Nr={Nr}")
     dev = require_cuda(regions, queries)
     r16, q16 = _to_bf16_rows(regions), _to_bf16_rows(queries)
     Nr, D = r16.shape
     Nq = q16.shape[0]
-    S, _ = _sim_forward(r16, q16, 1.0, True, False, engine)
+    if _topk_fused(Nq, Nr, D, int(k), engine):
+        return _topk_select(r16, q16, int(k))
     idx = torch.empty((Nq, k), dtype=torch.int64, device=dev)
     score = torch.empty((Nq, k), dtype=torch.float32, device=dev)
+    S, _ = _sim_forward(r16, q16, 1.0, True, False, engine)
     _call("cor_topk", dev, ptr(S), ptr(r16), ptr(q16), Nr, Nq, D, int(k), ptr(idx), ptr(score))
     return idx, score
 

@@ -350,6 +350,19 @@ int cor_memory_dq(const void* bank, int K, const int* state, const void* queries
 int cor_topk(const float* S, const void* regions, const void* queries, int Nr, int Nq, int D, int k,
              long long* idx, float* score, cor_stream_t stream);
 
+/* Top-k retrieval without S: the same result as cor_sim_umma_fwd (S) followed by cor_topk, for D in {64, 128, 192, 256}.
+ * The tensor-core similarity kernel that keeps the queries in tensor memory selects while it scores: each (query, CTA)
+ * keeps a list of its best ncand = min(k + max(16, k / 2), Nr, 512) prefilter candidates under (key desc, index asc),
+ * and one CTA per query selects, re-scores exactly and sorts the union of its lists.  Two launches, no host sync,
+ * deterministic, capturable in a CUDA graph.  regions [Nr, D], queries [Nq, D] bf16 (16-byte aligned); 1 <= k <=
+ * min(Nr, 256).  work: cor_topk_select_work_bytes(Nq, Nr, D, k) bytes =
+ *   ceil(Nq / 256) * max(1, SMs / ceil(Nq / 256)) * 256 * (8 * (min(k + max(16, k / 2), 512) + 128) + 4),
+ * which depends on Nq, k and the SM count only, never on Nr (0 for arguments outside the ranges above).  Bad arguments
+ * return COR_EINVAL before any device query. */
+size_t cor_topk_select_work_bytes(int Nq, int Nr, int D, int k);
+int cor_topk_select(const void* regions, const void* queries, int Nr, int Nq, int D, int k, long long* idx, float* score,
+                    void* work, cor_stream_t stream);
+
 /* Row-wise L2 normalise x / max(|x|, 1e-12) (support_branch.py:85, cir_feature_fuse.py:59):
  *   x [n, D] f32/bf16 -> y_f32 and/or y_bf16. */
 int cor_l2_normalize(const void* x, int x_dtype, int n, int D, float* y_f32, void* y_bf16, float* inv_norm,

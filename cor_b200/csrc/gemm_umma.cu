@@ -270,8 +270,10 @@ __global__ void __launch_bounds__(kGmThreads, 1) gemm_umma_kernel(const __grid_c
       const long long roww0 = (long long)b * g.M + mw0;
       auto emit = [&](uint32_t (&v)[32], int nb) {
         if (nb >= g.N) return;
+        // bias and colscale are read as float4 on the fast path: an offset view of either must take the per-element path
         const bool al16 = ((reinterpret_cast<uintptr_t>(g.C) | reinterpret_cast<uintptr_t>(g.pre) | reinterpret_cast<uintptr_t>(g.residual) |
-                            reinterpret_cast<uintptr_t>(g.emul) | reinterpret_cast<uintptr_t>(g.part)) & 15) == 0;
+                            reinterpret_cast<uintptr_t>(g.emul) | reinterpret_cast<uintptr_t>(g.part) | reinterpret_cast<uintptr_t>(g.bias) |
+                            reinterpret_cast<uintptr_t>(g.colscale)) & 15) == 0;
         if (g.ksplit > 1) {
           float* dst = g.part + (((long long)ks * g.batch + b) * g.M + m) * g.N + nb;
           if ((g.N % 4 == 0) && nb + 32 <= g.N && al16) {         // warp-uniform: all lanes take the transposing store

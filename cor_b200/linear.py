@@ -45,9 +45,9 @@ def gemm(a: torch.Tensor, b: torch.Tensor, M: int, N: int, K: int, *, a_mn: bool
     """C[b][m][n] = epilogue(alpha * sum_k A[b](m,k) B[b](n,k)); see include/cor_b200.h (cor_gemm_bf16).  ``a`` / ``b`` are
     2-D bf16 tensors; ``x_mn`` says the operand is stored [K, rows] instead of [rows, K].  Returns C [batch*M, N] (and the
     bf16 pre-activation when ``want_pre``)."""
-    dev = L.require_cuda(a, b, bias, emul, colscale, residual)
     if a.dtype != torch.bfloat16 or b.dtype != torch.bfloat16 or a.dim() != 2 or b.dim() != 2:
         raise CorError("gemm: operands must be 2-D bf16 tensors")
+    dev = L.require_cuda(a, b, bias, emul, colscale, residual)
     a, b = a.contiguous(), b.contiguous()
     lib = L.load()
     C = torch.empty((batch * M, N), dtype=out_dtype, device=dev)
@@ -100,7 +100,7 @@ class _LinearFn(torch.autograd.Function):
         out = gemm(x16, w16, rows, N, K, bias=b32, act=act, emul=m32, colscale=cs, residual=residual, want_pre=want_pre,
                    out_dtype=torch.bfloat16 if out_bf16 else torch.float32)
         y, pre = out if want_pre else (out, None)
-        # relu / sigmoid differentiate through the stored OUTPUT (only used when there is neither scale nor residual)
+        # relu / sigmoid differentiate through the stored OUTPUT (linear() refuses a residual with either, and a mask with sigmoid)
         ctx.save_for_backward(x16, w16, (y.float() if y.dtype != torch.float32 else y) if act in (ACT_RELU, ACT_SIGMOID) else None, pre, m32, cs)
         ctx.cfg = (act, x.shape[1], x.requires_grad, x2 is not None and x2.requires_grad, weight.requires_grad,
                    bias is not None and bias.requires_grad, colscale is not None and colscale.requires_grad,
@@ -140,6 +140,11 @@ def linear(x: torch.Tensor, weight: torch.Tensor, bias: Optional[torch.Tensor] =
     ``F.dropout`` multiplies by); ``colscale`` [out] and ``residual`` [rows, out] are ConvNeXt's layer scale and skip
     connection (mask_adapter.py:215-221), fused into the same GEMM epilogue.  ``out_bf16`` writes the result in bf16 (the next
     GEMM's A operand: no fp32 round trip of a wide hidden activation)."""
+    # relu and sigmoid differentiate through the stored output, which a residual or (for sigmoid) a mask has changed
+    if act in ("relu", "sigmoid") and residual is not None:
+        raise CorError(f"linear: act={act!r} with a residual is not supported (its backward would read relu/sigmoid through the residual)")
+    if act == "sigmoid" and drop_mask is not None:
+        raise CorError("linear: act='sigmoid' with a drop_mask is not supported (its backward would read the sigmoid through the mask)")
     return _LinearFn.apply(x, weight, bias, _ACTS[act], drop_mask, x2, colscale, residual, bool(out_bf16))
 
 

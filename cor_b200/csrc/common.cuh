@@ -23,9 +23,10 @@ int sim_umma_launch(const void* regions, const void* queries, int Nr, int Nq, in
 
 // same, queries held in tensor memory (sim_umma_ts.cu); log-sum-exp partials only: [qtile][*nparts][256][2] in `work`.
 // count non-NULL: the rows actually scored are the first min(Nr, *count), read on the device (a region memory's fill);
-// the grid is sized for Nr and CTAs past the count leave empty partials (-inf, 0).
+// the grid is sized for Nr and CTAs past the count leave empty partials (-inf, 0).  exclude non-NULL: a bit mask
+// [Nq][ceil(Nr / 32)] (bit j of word w set: row 32 w + j is left out of that query's sum; memory.cu builds it).
 int sim_umma_ts_launch(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, const float* scale, void* work,
-                       int* nparts, cudaStream_t st, const int* count = nullptr);
+                       int* nparts, cudaStream_t st, const int* count = nullptr, const unsigned* exclude = nullptr);
 
 // queries per tile of the log-sum-exp partials sim_umma_ts_launch leaves: the layout of a region memory's scan
 constexpr int kMemQT = 256;

@@ -29,6 +29,9 @@
 // register across its Y tiles and leaves one partial per (split, column half, query); nce_scale_fold_kernel sums them.
 // Region memory (mode 0, cor_memory_dq): Y = the memory's bank, its row count read on the device (count), no targets (a
 // memory row is never a positive); both folds ADD into the gradients the current rows' backward already wrote.
+// The excluding instantiation (kExclude, cor_memory_dq_x) reads the scan's bit mask [Nx][ceil(Ny / 32)] (memory.cu): a
+// thread's 32 S columns of a tile are one 32-aligned chunk, so one word per tile; a masked column gets the exponent -inf,
+// as a column past the fill does, hence coefficient 0 and nothing in dQ or the logit-scale partial.
 #include <stdlib.h>
 
 #include "umma.cuh"
@@ -88,7 +91,9 @@ __device__ __forceinline__ uint32_t pack_bf16x2_rn(float lo, float hi) {
   return r;
 }
 
-__global__ void __launch_bounds__(320, 1) nce_bwd_umma_kernel(const __grid_constant__ CUtensorMap tmY, NceArgs a) {
+template <bool kExclude = false>
+__global__ void __launch_bounds__(320, 1) nce_bwd_umma_kernel(const __grid_constant__ CUtensorMap tmY, NceArgs a,
+                                                              const unsigned* __restrict__ exclude = nullptr) {
   extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t* base = reinterpret_cast<uint8_t*>(((uintptr_t)smem + 1023) & ~(uintptr_t)1023);
   uint8_t* y_smem = base;                                                    // nslots x nkb x 8 KB
@@ -242,6 +247,10 @@ __global__ void __launch_bounds__(320, 1) nce_bwd_umma_kernel(const __grid_const
         nl_a = qa < a.Nq ? -__ldg(a.lse + qa) * log2e : -INFINITY;      // exp2(-inf) = 0: columns past Nq contribute nothing
         tg_a = qa < a.Nq ? (int)__ldg(a.targets + qa) : -1;
       }
+      unsigned xw = 0u;                               // kExclude: mask bits of this thread's 32 columns, loaded under the wait
+      if constexpr (kExclude) {
+        if (a.mode == 0 && xok && y0 < a.Ny) xw = __ldg(exclude + (long long)xg * ((a.Ny + 31) / 32) + (y0 >> 5));   // else: past the rows
+      }
       mbar_wait(&tail->s_full[buf], (i >> 1) & 1);
       tc_fence_after();
       const uint32_t taddr = tmem + ((uint32_t)(qd * 32) << 16) + (uint32_t)(buf * kNbN + half * 32);
@@ -260,6 +269,10 @@ __global__ void __launch_bounds__(320, 1) nce_bwd_umma_kernel(const __grid_const
           // columns past Ny get no coefficient (exp2(-inf) = 0): a memory's stale rows in its last tile add nothing
           n0 = y0 + 2 * j < Ny ? my_nl : -INFINITY;
           n1 = y0 + 2 * j + 1 < Ny ? my_nl : -INFINITY;
+          if constexpr (kExclude) {
+            if ((xw >> (2 * j)) & 1u) n0 = -INFINITY;
+            if ((xw >> (2 * j + 1)) & 1u) n1 = -INFINITY;
+          }
           hit0 = (y0 + 2 * j == my_tg);
           hit1 = (y0 + 2 * j + 1 == my_tg);
         } else {
@@ -368,7 +381,8 @@ static int nce_splits(int xtiles, int ytiles) {
 // count: device row count of Y (see NceArgs); accumulate: the fold adds into `out` (then the partials always go to `part`)
 static int nce_launch(const void* X, const void* Y, int Nx, int Ny, int Nq, int D, int mode, float inv_tau, const float* scale,
                       const float* lse, const long long* targets, const float* g_loss, float g_mul, float* out, float* part,
-                      float* lspart, cudaStream_t st, const int* count = nullptr, int accumulate = 0) {
+                      float* lspart, cudaStream_t st, const int* count = nullptr, int accumulate = 0,
+                      const unsigned* exclude = nullptr) {
   const int nkb = D / kNbBK;
   const int xtiles = ceil_div(Nx, kNbM), ytiles = ceil_div(Ny, kNbN);
   const int nsplit = nce_splits(xtiles, ytiles);
@@ -382,7 +396,10 @@ static int nce_launch(const void* X, const void* Y, int Nx, int Ny, int Nq, int 
   if (nslots > kNbMaxSlots) nslots = kNbMaxSlots;
   COR_REQUIRE(nslots >= 2, "cor_infonce_bwd_umma: shared memory budget (D=%d)", D);
   const size_t smem = fixed + (size_t)nslots * nkb * kNbYBlk;
-  COR_CUDA(cudaFuncSetAttribute(nce_bwd_umma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  if (exclude)
+    COR_CUDA(cudaFuncSetAttribute(nce_bwd_umma_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  else
+    COR_CUDA(cudaFuncSetAttribute(nce_bwd_umma_kernel<>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   NceArgs a;
   a.Nx = Nx; a.Ny = Ny; a.Nq = Nq; a.nkb = nkb; a.nslots = nslots; a.mode = mode;
   a.c2 = inv_tau * 1.4426950408889634f;
@@ -392,7 +409,10 @@ static int nce_launch(const void* X, const void* Y, int Nx, int Ny, int Nq, int 
   a.X = reinterpret_cast<const bf16*>(X);
   const bool direct = nsplit == 1 && !accumulate;
   a.out = !out ? nullptr : (direct ? out : part);
-  nce_bwd_umma_kernel<<<dim3(nsplit, xtiles), 320, smem, st>>>(tmY, a);
+  if (exclude)
+    nce_bwd_umma_kernel<true><<<dim3(nsplit, xtiles), 320, smem, st>>>(tmY, a, exclude);
+  else
+    nce_bwd_umma_kernel<><<<dim3(nsplit, xtiles), 320, smem, st>>>(tmY, a);
   rc = check_launch("nce_bwd_umma_kernel");
   if (rc || direct || !out) return rc;
   const long long vecs = (long long)Nx * D / 4;
@@ -469,20 +489,35 @@ extern "C" size_t cor_memory_dq_work_bytes(int Nq, int K, int D) {
   return mem_dq_part_bytes(Nq, K, D) + (size_t)mem_dq_splits(Nq, K) * 2 * Nq * sizeof(float) + 256;
 }
 
-extern "C" int cor_memory_dq(const void* bank, int K, const int* state, const void* queries, int Nq, int D, float inv_tau,
-                             const float* logit_scale, const float* lse, const float* g_loss, float g_mul, float* g_queries,
-                             float* g_logit_scale, void* work, cor_stream_t stream) {
-  COR_REQUIRE(bank && state && queries && lse && g_loss && work, "cor_memory_dq: null pointer");
-  COR_REQUIRE(K >= 1 && Nq >= 1, "cor_memory_dq: need K >= 1 and Nq >= 1 (K=%d Nq=%d)", K, Nq);
-  COR_REQUIRE(D % kNbBK == 0 && D >= kNbBK && D <= 256, "cor_memory_dq: need D in {64,128,192,256} (D=%d)", D);
-  COR_REQUIRE(g_queries || g_logit_scale, "cor_memory_dq: nothing to compute");
-  COR_REQUIRE(!g_logit_scale || logit_scale, "cor_memory_dq: g_logit_scale needs logit_scale");
+static int memory_dq(const char* who, const void* bank, int K, const int* state, const void* queries, int Nq, int D, float inv_tau,
+                     const float* logit_scale, const unsigned* exclude, const float* lse, const float* g_loss, float g_mul, float* g_queries,
+                     float* g_logit_scale, void* work, cor_stream_t stream) {
+  COR_REQUIRE(bank && state && queries && lse && g_loss && work, "%s: null pointer", who);
+  COR_REQUIRE(K >= 1 && Nq >= 1, "%s: need K >= 1 and Nq >= 1 (K=%d Nq=%d)", who, K, Nq);
+  COR_REQUIRE(D % kNbBK == 0 && D >= kNbBK && D <= 256, "%s: need D in {64,128,192,256} (D=%d)", who, D);
+  COR_REQUIRE(g_queries || g_logit_scale, "%s: nothing to compute", who);
+  COR_REQUIRE(!g_logit_scale || logit_scale, "%s: g_logit_scale needs logit_scale", who);
   cudaStream_t st = as_stream(stream);
   float* part = reinterpret_cast<float*>(work);
   float* lspart = g_logit_scale ? reinterpret_cast<float*>(reinterpret_cast<char*>(work) + mem_dq_part_bytes(Nq, K, D)) : nullptr;
   int rc = nce_launch(queries, bank, Nq, K, Nq, D, 0, inv_tau, logit_scale, lse, nullptr, g_loss, g_mul, g_queries, part, lspart, st,
-                      state + 1, 1);
+                      state + 1, 1, exclude);
   if (rc || !g_logit_scale) return rc;
   nce_scale_fold_kernel<<<1, 256, 0, st>>>(lspart, 2 * mem_dq_splits(Nq, K), Nq, g_loss, g_mul, g_logit_scale, 1);
   return check_launch("nce_scale_fold_kernel");
+}
+
+extern "C" int cor_memory_dq(const void* bank, int K, const int* state, const void* queries, int Nq, int D, float inv_tau,
+                             const float* logit_scale, const float* lse, const float* g_loss, float g_mul, float* g_queries,
+                             float* g_logit_scale, void* work, cor_stream_t stream) {
+  return memory_dq("cor_memory_dq", bank, K, state, queries, Nq, D, inv_tau, logit_scale, nullptr, lse, g_loss, g_mul, g_queries,
+                   g_logit_scale, work, stream);
+}
+
+extern "C" int cor_memory_dq_x(const void* bank, int K, const int* state, const void* queries, int Nq, int D, float inv_tau,
+                               const float* logit_scale, const unsigned* exclude, const float* lse, const float* g_loss, float g_mul,
+                               float* g_queries, float* g_logit_scale, void* work, cor_stream_t stream) {
+  COR_REQUIRE(exclude, "cor_memory_dq_x: null exclude");
+  return memory_dq("cor_memory_dq_x", bank, K, state, queries, Nq, D, inv_tau, logit_scale, exclude, lse, g_loss, g_mul, g_queries,
+                   g_logit_scale, work, stream);
 }

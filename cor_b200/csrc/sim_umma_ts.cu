@@ -23,6 +23,12 @@
 // index, so an equal key that arrives later ranks below every equal key already kept: each list keeps its CTA's exact
 // top ncand, ties included, and the union of the lists holds the global top ncand.  At most one compaction per thread
 // per tile, after the thread has released the accumulator, so the MMAs of the next tile run under it.
+//
+// The excluding instantiation (kExclude, cor_memory_scan_x) is the log-sum-exp with a bit mask over the region rows
+// [Nq][ceil(Nr / 32)] (memory.cu): a thread has one mask word per 32 columns and, when it is non-zero, folds only the
+// columns whose bit is clear, so an excluded column adds exactly nothing to (m, ssum).  While every column seen so far is
+// excluded, m stays -inf and ssum 0: a query that excludes them all leaves (-inf, 0), as an empty memory does.  A zero
+// word takes the unmasked code, so with nothing excluded the partials are bit-equal to the unmasked kernel's.
 #include <stdlib.h>
 
 #include "umma.cuh"
@@ -90,15 +96,18 @@ __device__ __noinline__ uint32_t ts_compact(uint32_t* __restrict__ key, int* __r
   return kmin;
 }
 
-template <bool kSelect>
+template <bool kSelect, bool kExclude = false>
 __global__ void __launch_bounds__(320, 1) sim_umma_ts_kernel(const __grid_constant__ CUtensorMap tmR, const bf16* __restrict__ queries, int Nr,
                                                              int Nq, int nkb, int nstages, float inv_tau, const float* __restrict__ scale,
-                                                             float* __restrict__ part, const int* __restrict__ count, TopkSegments seg) {
+                                                             float* __restrict__ part, const int* __restrict__ count, TopkSegments seg,
+                                                             const unsigned* __restrict__ exclude = nullptr) {
+  static_assert(!(kSelect && kExclude), "the exclusion mask belongs to the log-sum-exp epilogue");
   extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t* base = reinterpret_cast<uint8_t*>(((uintptr_t)smem + 1023) & ~(uintptr_t)1023);
   uint8_t* r_smem = base;
   TsSmemTail* tail = reinterpret_cast<TsSmemTail*>(r_smem + (size_t)nstages * kTsBBytes);
 
+  const int xwords = (Nr + 31) / 32;               // kExclude: mask words per query
   if (count) Nr = min(Nr, max(*count, 0));       // a region memory: only its filled rows; no tiles at all when it is empty
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int q0 = blockIdx.y * kTsBM;
@@ -312,7 +321,41 @@ __global__ void __launch_bounds__(320, 1) sim_umma_ts_kernel(const __grid_consta
         }
       };
       if (active) {
-        walk(proc, [] {});
+        if constexpr (kExclude) {
+          // the four mask words of a tile are loaded one tile ahead, under the wait for its accumulator
+          const unsigned* xrow = exclude + (size_t)min(q, Nq - 1) * xwords;
+          unsigned xcur[4], xnext[4];
+          auto load4 = [&](int t) {
+#pragma unroll
+            for (int c = 0; c < 4; ++c) xnext[c] = (q < Nq && t * 4 + c < xwords) ? __ldg(xrow + t * 4 + c) : 0u;
+          };
+          load4(blockIdx.x);
+          auto proc_x = [&](uint32_t (&v)[32], int r0, int col) {
+            if (col == 0) {
+#pragma unroll
+              for (int c = 0; c < 4; ++c) xcur[c] = xnext[c];
+              load4(r0 / kTsBN + (int)gridDim.x);
+            }
+            const unsigned xw = xcur[col >> 5];
+            if (!xw) {
+              proc(v, r0, col);
+              return;
+            }
+            const int nval = min(32, Nr - (r0 + col));
+            float cm = -INFINITY;
+#pragma unroll
+            for (int j = 0; j < 32; ++j)
+              if (j < nval && !((xw >> j) & 1u)) cm = fmaxf(cm, __uint_as_float(v[j]));
+            if (cm > m) { ssum *= ex2_approx((m - cm) * c2); m = cm; }
+            const float mc = m * c2;
+#pragma unroll
+            for (int j = 0; j < 32; ++j)
+              if (j < nval && !((xw >> j) & 1u)) ssum += ex2_approx(fmaf(__uint_as_float(v[j]), c2, -mc));
+          };
+          walk(proc_x, [] {});
+        } else {
+          walk(proc, [] {});
+        }
         float* o = part + (((long long)blockIdx.y * gridDim.x + blockIdx.x) * kTsBM + hf * kTsHalf + qd * 32 + lane) * 2;
         o[0] = m * inv_tau;
         o[1] = ssum;
@@ -326,9 +369,9 @@ __global__ void __launch_bounds__(320, 1) sim_umma_ts_kernel(const __grid_consta
 
 static_assert(kTsBM == kMemQT, "a region memory's scan partials and the top-k lists are laid out per kTsBM-query tile");
 
-template <bool kSelect>
+template <bool kSelect, bool kExclude = false>
 static int ts_launch(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, const float* scale, void* work,
-                     int* nparts, cudaStream_t st, const int* count, TopkSegments seg) {
+                     int* nparts, cudaStream_t st, const int* count, TopkSegments seg, const unsigned* exclude = nullptr) {
   const int qtiles = ceil_div(Nq, kTsBM), ntiles = ceil_div(Nr, kTsBN);
   CUtensorMap tmR;
   int rc = umma::encode_tmap_bf16_2d(&tmR, regions, (uint64_t)Nr, (uint64_t)D, kTsBN, kTsBK);
@@ -340,17 +383,23 @@ static int ts_launch(const void* regions, const void* queries, int Nr, int Nq, i
   int nstages = (int)((227 * 1024 - sizeof(TsSmemTail) - 1024) / kTsBBytes);
   if (nstages > kTsMaxStages) nstages = kTsMaxStages;
   const size_t smem = (size_t)nstages * kTsBBytes + sizeof(TsSmemTail) + 1024;
-  COR_CUDA(cudaFuncSetAttribute(sim_umma_ts_kernel<kSelect>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  sim_umma_ts_kernel<kSelect><<<dim3(gx, qtiles), 320, smem, st>>>(tmR, reinterpret_cast<const bf16*>(queries), Nr, Nq, nkb, nstages,
-                                                                   inv_tau, scale, reinterpret_cast<float*>(work), count, seg);
+  COR_CUDA(cudaFuncSetAttribute(sim_umma_ts_kernel<kSelect, kExclude>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  if constexpr (kExclude)
+    sim_umma_ts_kernel<kSelect, true><<<dim3(gx, qtiles), 320, smem, st>>>(tmR, reinterpret_cast<const bf16*>(queries), Nr, Nq, nkb,
+                                                                           nstages, inv_tau, scale, reinterpret_cast<float*>(work), count,
+                                                                           seg, exclude);
+  else
+    sim_umma_ts_kernel<kSelect><<<dim3(gx, qtiles), 320, smem, st>>>(tmR, reinterpret_cast<const bf16*>(queries), Nr, Nq, nkb, nstages,
+                                                                     inv_tau, scale, reinterpret_cast<float*>(work), count, seg);
   *nparts = gx;
   return check_launch("sim_umma_ts_kernel");
 }
 
 // LSE-only launcher (sim_umma.cu stores S with the kernel that keeps both operands in shared memory).  Returns the
-// number of partial records per query tile in *nparts.
+// number of partial records per query tile in *nparts.  exclude non-NULL: the excluding instantiation.
 int sim_umma_ts_launch(const void* regions, const void* queries, int Nr, int Nq, int D, float inv_tau, const float* scale, void* work,
-                       int* nparts, cudaStream_t st, const int* count) {
+                       int* nparts, cudaStream_t st, const int* count, const unsigned* exclude) {
+  if (exclude) return ts_launch<false, true>(regions, queries, Nr, Nq, D, inv_tau, scale, work, nparts, st, count, TopkSegments{}, exclude);
   return ts_launch<false>(regions, queries, Nr, Nq, D, inv_tau, scale, work, nparts, st, count, TopkSegments{});
 }
 

@@ -41,6 +41,8 @@ _KERNELS_PER_CALL = {
     # cross-batch region memory: cor_memory_dq is 2 launches, 3 with the logit scale's gradient (its caller passes the count)
     "cor_memory_reset": 1, "cor_memory_enqueue": 1, "cor_memory_scan": 1, "cor_infonce_tail_mem": 1, "cor_step_tail_fwd_mem": 1,
     "cor_memory_dq": 2,
+    # region memory with row ids: the exclusion mask, and the scan / dQ twins that read it
+    "cor_memory_enqueue_ids": 1, "cor_memory_exclude": 1, "cor_memory_scan_x": 1, "cor_memory_dq_x": 2,
     # top-k without S: the selecting similarity kernel, then select / re-score / sort
     "cor_topk_select": 2,
 }
@@ -548,32 +550,70 @@ def check_memory(memory, D: int, dev, who: str) -> None:
         raise CorError(f"{who}: the memory is on {memory.bank.device}, the call on {dev}")
 
 
+def check_query_ids(query_ids, memory, Nq: int, dev, who: str) -> None:
+    """Query ids (int64 [Nq] on the call's device) name each query's own object, whose memory rows are left out of its
+    negatives: they need a memory whose rows carry ids."""
+    if query_ids is None:
+        return
+    if memory is None:
+        raise CorError(f"{who}: query_ids select memory rows to leave out; pass them together with memory=")
+    if not hasattr(memory, "ids"):
+        raise CorError(f"{who}: query_ids need a RegionMemory that keeps row ids")
+    if not isinstance(query_ids, torch.Tensor) or query_ids.dtype != torch.int64:
+        raise CorError(f"{who}: query_ids must be an int64 tensor, got "
+                       + (str(query_ids.dtype) if isinstance(query_ids, torch.Tensor) else type(query_ids).__name__))
+    if tuple(query_ids.shape) != (Nq,):
+        raise CorError(f"{who}: query_ids {tuple(query_ids.shape)} must be [{Nq}], one per query")
+    if not query_ids.is_cuda or (dev is not None and query_ids.device != dev):
+        raise CorError(f"{who}: query_ids are on {query_ids.device}, the call on {dev if dev is not None else 'a CUDA device'}")
+
+
+def _memory_exclude_work(memory, Nq: int, dev) -> torch.Tensor:
+    return _work(L.load().cor_memory_exclude_bytes(Nq, memory.K), dev)
+
+
+def _memory_exclude(memory, query_ids, work=None):
+    """The bit mask [Nq][ceil(K / 32)] of the memory slots whose id is the query's: read by the scan and the dQ (``_x``
+    entries).  ``work``: a buffer from _memory_exclude_work allocated on the stream that reads the mask last."""
+    dev = query_ids.device
+    Nq = query_ids.shape[0]
+    if work is None:
+        work = _memory_exclude_work(memory, Nq, dev)
+    _call("cor_memory_exclude", dev, ptr(memory.ids), memory.K, ptr(memory.state), ptr(query_ids.contiguous()), Nq, ptr(work))
+    return work
+
+
 def _memory_scan_work(memory, Nq: int, D: int, dev) -> torch.Tensor:
     return _work(L.load().cor_memory_scan_work_bytes(Nq, memory.K, D), dev)
 
 
-def _memory_scan(memory, q16, inv_tau, scale=None, work=None):
+def _memory_scan(memory, q16, inv_tau, scale=None, work=None, exclude=None):
     """Log-sum-exp partials of the queries against the memory's valid rows (tensor cores): (work, nparts) for the
-    ``_mem`` tail entries.  ``work``: a buffer from _memory_scan_work allocated on the stream that consumes the partials."""
+    ``_mem`` tail entries.  ``work``: a buffer from _memory_scan_work allocated on the stream that consumes the partials.
+    ``exclude``: a mask from _memory_exclude, whose rows the scan leaves out."""
     dev = q16.device
     Nq, D = q16.shape
     if work is None:
         work = _memory_scan_work(memory, Nq, D, dev)
     nparts = C.c_int(0)
-    _call("cor_memory_scan", dev, ptr(memory.bank), memory.K, ptr(memory.state), ptr(q16), Nq, D, _f(inv_tau), ptr(scale), ptr(work),
-          C.byref(nparts))
+    x = () if exclude is None else (ptr(exclude),)
+    _call("cor_memory_scan" if exclude is None else "cor_memory_scan_x", dev, ptr(memory.bank), memory.K, ptr(memory.state), ptr(q16), Nq,
+          D, _f(inv_tau), ptr(scale), *x, ptr(work), C.byref(nparts))
     return work, nparts.value
 
 
-def _memory_dq(memory, q16, lse, inv_tau, scale, g_loss, g_mul, g_queries, g_scale):
-    """ADD the memory rows' share of the InfoNCE gradient into g_queries [Nq, D] and g_scale (either may be None)."""
+def _memory_dq(memory, q16, lse, inv_tau, scale, g_loss, g_mul, g_queries, g_scale, exclude=None):
+    """ADD the memory rows' share of the InfoNCE gradient into g_queries [Nq, D] and g_scale (either may be None), leaving
+    out the rows ``exclude`` masks."""
     if g_queries is None and g_scale is None:
         return
     dev = q16.device
     Nq, D = q16.shape
     work = _work(L.load().cor_memory_dq_work_bytes(Nq, memory.K, D), dev)
-    _call("cor_memory_dq", dev, ptr(memory.bank), memory.K, ptr(memory.state), ptr(q16), Nq, D, _f(inv_tau), ptr(scale), ptr(lse),
-          ptr(g_loss), _f(g_mul), ptr(g_queries), ptr(g_scale), ptr(work), launches=1 + (g_queries is not None) + (g_scale is not None))
+    x = () if exclude is None else (ptr(exclude),)
+    _call("cor_memory_dq" if exclude is None else "cor_memory_dq_x", dev, ptr(memory.bank), memory.K, ptr(memory.state), ptr(q16), Nq, D,
+          _f(inv_tau), ptr(scale), *x, ptr(lse), ptr(g_loss), _f(g_mul), ptr(g_queries), ptr(g_scale), ptr(work),
+          launches=1 + (g_queries is not None) + (g_scale is not None))
 
 
 def check_memory_unchanged(mem_rec, who: str) -> None:
@@ -611,7 +651,7 @@ def _infonce_bwd_dense(Nq: int, Nr: int, D: int, engine: str) -> bool:
 
 class _InfoNCEFn(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, regions, queries, targets, tau, engine, regions_bf16, logit_scale, memory):
+    def forward(ctx, regions, queries, targets, tau, engine, regions_bf16, logit_scale, memory, query_ids):
         dev = require_cuda(regions, queries, targets, logit_scale)
         check_memory(memory, queries.shape[-1], dev, "infonce_loss")
         r16 = regions_bf16.reshape(-1, regions_bf16.shape[-1]).contiguous() if regions_bf16 is not None else _to_bf16_rows(regions)
@@ -623,17 +663,19 @@ class _InfoNCEFn(torch.autograd.Function):
         _, lse = _sim_forward(r16, q16, inv_tau, False, True, engine, logit_scale)
         loss = torch.empty(1, dtype=torch.float32, device=dev)
         tgt = torch.empty((Nq,), dtype=torch.float32, device=dev)
+        check_query_ids(query_ids, memory, Nq, dev, "infonce_loss")
+        excl = _memory_exclude(memory, query_ids) if query_ids is not None else None
         if memory is None:
             name, ta = _tau_arg("cor_infonce_fwd", inv_tau, logit_scale)
             _call(name, dev, ptr(r16), ptr(q16), ptr(tg), ptr(lse), Nr, Nq, D, ta, ptr(loss), ptr(tgt))
         else:
             # the tail entry in its lse-in form: it merges the memory's partials into the current rows' lse (in place) and
             # forms the loss as cor_infonce_fwd does, so an empty memory changes no bit
-            mwork, mparts = _memory_scan(memory, q16, inv_tau, logit_scale)
+            mwork, mparts = _memory_scan(memory, q16, inv_tau, logit_scale, exclude=excl)
             name, tas = _tail_entry("cor_infonce_tail", inv_tau, logit_scale, (ptr(mwork), mparts, ptr(memory.state)))
             _call(name, dev, None, 0, 0, ptr(r16), ptr(q16), ptr(tg), Nr, Nq, D, *tas, ptr(lse), ptr(loss), ptr(tgt), None, None,
                   _f(0.0), _f(0.0), _f(0.0), None)
-        ctx.mem = None if memory is None else (memory, memory.enqueues)
+        ctx.mem = None if memory is None else (memory, memory.enqueues, excl)
         # the scale is saved as an input: an in-place write to it before backward trips autograd's version check
         ctx.save_for_backward(r16, q16, tg, lse, logit_scale)
         ctx.engine = engine
@@ -670,13 +712,14 @@ class _InfoNCEFn(torch.autograd.Function):
             name, ta = _tau_arg("cor_infonce_bwd", inv_tau, sc)
             _call(name, dev, ptr(r16), ptr(q16), ptr(tg), ptr(lse), Nr, Nq, D, ta, ptr(gl), _f(1.0), ptr(gr), ptr(gq), *gs_arg, ptr(work))
         if ctx.mem is not None:          # the memory rows' share, added into what the current rows' backward wrote
-            _memory_dq(ctx.mem[0], q16, lse, inv_tau, sc, gl, 1.0, gq if q_need else None, gs)
+            _memory_dq(ctx.mem[0], q16, lse, inv_tau, sc, gl, 1.0, gq if q_need else None, gs, ctx.mem[2])
         return ((gr.view(rshape).to(rdt) if r_need else None), (gq.view(qshape).to(qdt) if q_need else None), None, None, None, None, gs,
-                None)
+                None, None)
 
 
 def infonce_loss(regions: torch.Tensor, queries: torch.Tensor, targets: torch.Tensor, tau: Optional[float] = None, engine: str = "auto",
-                 regions_bf16: Optional[torch.Tensor] = None, logit_scale: Optional[torch.Tensor] = None, memory=None) -> torch.Tensor:
+                 regions_bf16: Optional[torch.Tensor] = None, logit_scale: Optional[torch.Tensor] = None, memory=None,
+                 query_ids: Optional[torch.Tensor] = None) -> torch.Tensor:
     """mean_q CE(s * S[q,:], targets[q]) with S = queries @ regions^T (bf16 operands, fp32 accumulate) and s = 1/tau
     (tau defaults to 0.07).  Gradients flow straight through the bf16 rounding to ``regions`` and ``queries``.
 
@@ -685,10 +728,16 @@ def infonce_loss(regions: torch.Tensor, queries: torch.Tensor, targets: torch.Te
     autograd, e.g. ``logit_scale = log_s.exp()`` with a parameter ``log_s`` as in CLIP.
 
     ``memory``: a ``region.RegionMemory`` whose valid rows join the negatives of every query (never a target, no gradient
-    of their own); the queries and the scale get the memory terms of their gradient.  Enqueue into it after backward()."""
+    of their own); the queries and the scale get the memory terms of their gradient.  Enqueue into it after backward().
+
+    ``query_ids``: int64 [Nq] on the queries' device, with ``memory`` only.  A memory row whose id (``RegionMemory.enqueue``
+    ``ids=``) is >= 0 and equals the query's id is left out of that query's negatives and of its gradients, e.g. earlier
+    pooled rows of the object the query is looking for.  A negative id matches nothing."""
     check_logit_scale(logit_scale, tau, "infonce_loss")
     check_memory(memory, queries.shape[-1], None, "infonce_loss")
-    return _InfoNCEFn.apply(regions, queries, targets, 0.07 if tau is None else float(tau), engine, regions_bf16, logit_scale, memory)
+    check_query_ids(query_ids, memory, queries.numel() // queries.shape[-1] if queries.dim() else 0, None, "infonce_loss")
+    return _InfoNCEFn.apply(regions, queries, targets, 0.07 if tau is None else float(tau), engine, regions_bf16, logit_scale, memory,
+                            query_ids)
 
 
 # Measured on one B200 at 1000 W (profiles/r06_topk_bench.log), D = 256: at k = 10 the fused path takes 2.65 against

@@ -37,7 +37,12 @@ class RegionMemory:
     The head and fill count live in device memory ({head, count} in ``state``), so a captured CUDA graph that enqueues
     advances them at every replay.  Enqueue AFTER backward(): a backward whose forward scored the memory raises
     ``CorError`` if the memory was enqueued in between (``enqueues`` counts the calls on the host).  Each rank of a
-    data-parallel job owns its memory and scores it against its own queries only.  C must be 64, 128, 192 or 256."""
+    data-parallel job owns its memory and scores it against its own queries only.  C must be 64, 128, 192 or 256.
+
+    Every slot also carries an int64 row id (``ids``, -1 = none), set by ``enqueue(rows, ids=...)``.  A call given
+    ``query_ids`` leaves each query's same-id rows out of its negatives and its gradients: with the target object's id on
+    the rows pushed from a step, a later step that looks for the same object does not score it as a negative (XBM keeps
+    a label with every memory row for this reason)."""
 
     def __init__(self, capacity: int, C: int, device="cuda"):
         if int(capacity) < 1:
@@ -51,15 +56,20 @@ class RegionMemory:
         # zero rows: the last partly filled tile of a scan reads rows past the fill, which must be finite
         self.bank = torch.zeros((self.K, self.C), dtype=torch.bfloat16, device=device)
         self.state = torch.zeros(L.load().cor_memory_state_words(), dtype=torch.int32, device=device)
+        self.ids = torch.full((self.K,), -1, dtype=torch.int64, device=device)
         self.enqueues = 0
 
     @property
     def device(self):
         return self.bank.device
 
-    def enqueue(self, rows: torch.Tensor) -> None:
+    def enqueue(self, rows: torch.Tensor, ids: Optional[torch.Tensor] = None) -> None:
         """Push ``rows`` (fp32 or bf16 [..., C], e.g. ``RegionStepOut.regions``; 1 <= n <= capacity rows) as bf16 at the
-        head, overwriting the oldest rows once full.  One kernel on the current stream, no host synchronisation."""
+        head, overwriting the oldest rows once full.  One kernel on the current stream, no host synchronisation.
+
+        ``ids``: int64 row ids on the memory's device, shaped ``rows.shape[:-1]`` (one per row) or, for rows [B, M, C],
+        [B]: the id of each image's row 0 (the ground-truth region of ``region_step``), its other rows getting -1.  Without
+        ``ids`` every pushed row gets -1."""
         if rows.dtype not in (torch.float32, torch.bfloat16):
             raise CorError(f"RegionMemory.enqueue: rows must be float32 or bfloat16, got {rows.dtype}")
         if rows.dim() < 1 or rows.shape[-1] != self.C:
@@ -70,8 +80,23 @@ class RegionMemory:
         dev = L.require_cuda(rows)
         if dev != self.device:
             raise CorError(f"RegionMemory.enqueue: rows on {dev}, the memory on {self.device}")
+        group = 1
+        if ids is not None:
+            lead = tuple(rows.shape[:-1])
+            if not isinstance(ids, torch.Tensor) or ids.dtype != torch.int64:
+                raise CorError("RegionMemory.enqueue: ids must be an int64 tensor, got "
+                               + (str(ids.dtype) if isinstance(ids, torch.Tensor) else type(ids).__name__))
+            if rows.dim() == 3 and tuple(ids.shape) == lead[:1]:
+                group = rows.shape[1]
+            elif tuple(ids.shape) != lead:
+                raise CorError(f"RegionMemory.enqueue: ids {tuple(ids.shape)} must be {lead} (one per row)"
+                               + (f" or {lead[:1]} (one per image, on its row 0)" if rows.dim() == 3 else ""))
+            if ids.device != self.device:
+                raise CorError(f"RegionMemory.enqueue: ids on {ids.device}, the memory on {self.device}")
+            ids = ids.contiguous()
         rc = rows.detach().reshape(n, self.C).contiguous()
-        ops._call("cor_memory_enqueue", dev, ops.ptr(rc), L.dtype_code(rc), n, self.C, ops.ptr(self.bank), self.K, ops.ptr(self.state))
+        ops._call("cor_memory_enqueue_ids", dev, ops.ptr(rc), L.dtype_code(rc), n, self.C, ops.ptr(self.bank), self.K, ops.ptr(self.state),
+                  ops.ptr(self.ids), ops.ptr(ids), group)
         self.enqueues += 1
 
     def reset(self) -> None:
@@ -90,6 +115,13 @@ class RegionMemory:
             return self.bank[:count].clone()
         return torch.cat([self.bank[head:], self.bank[:head]])
 
+    def row_ids(self) -> torch.Tensor:
+        """The ids of the valid rows, oldest first, as int64 [count], in the order of ``rows()`` (synchronises)."""
+        head, count = (int(v) for v in self.state[:2].tolist())
+        if count < self.K:
+            return self.ids[:count].clone()
+        return torch.cat([self.ids[head:], self.ids[:head]])
+
 
 def pool_regions(emb: torch.Tensor, masks: torch.Tensor, background: bool = False, engine: str = "auto", want_bf16: bool = True):
     """emb [B,C,h,w] x candidate masks [B,M,H,W] -> ops.RegionPool with unit rows fg [B,M,C]
@@ -104,13 +136,16 @@ def region_query_similarity(regions: torch.Tensor, queries: torch.Tensor, engine
 
 def region_infonce_loss(regions: torch.Tensor, queries: torch.Tensor, targets: torch.Tensor, tau: Optional[float] = None,
                         gather: bool = True, engine: str = "auto", regions_bf16: Optional[torch.Tensor] = None,
-                        logit_scale: Optional[torch.Tensor] = None, memory: Optional[RegionMemory] = None) -> torch.Tensor:
+                        logit_scale: Optional[torch.Tensor] = None, memory: Optional[RegionMemory] = None,
+                        query_ids: Optional[torch.Tensor] = None) -> torch.Tensor:
     """InfoNCE of each local query against ALL regions.  With ``gather`` (and an initialised process
     group) the region rows are all-gathered across ranks first and ``targets`` -- indices into the
     LOCAL region rows -- are offset by rank * n_local.  tau (default 0.07) is a build choice (the reference defines
     none); ``logit_scale`` replaces 1/tau with a device tensor that can be learned (see ``ops.infonce_loss``).  Each
     rank's loss is the mean over its own queries, so the scale's gradient is rank-local, like the queries'.  ``memory``
-    (a :class:`RegionMemory`) adds its valid rows to every query's negatives; each rank scores its own memory."""
+    (a :class:`RegionMemory`) adds its valid rows to every query's negatives; each rank scores its own memory.
+    ``query_ids`` (int64, one per local query, with ``memory``): leave each query's same-id memory rows out (see
+    ``ops.infonce_loss``); each rank's ids are those of its own queries and memory."""
     ops.check_logit_scale(logit_scale, tau, "region_infonce_loss")
     regions = regions.reshape(-1, regions.shape[-1])
     rank, ws = cdist.world()
@@ -119,7 +154,8 @@ def region_infonce_loss(regions: torch.Tensor, queries: torch.Tensor, targets: t
         regions = cdist.all_gather_rows(regions)
         targets = targets + rank * n_local
         regions_bf16 = None
-    return ops.infonce_loss(regions, queries.reshape(-1, queries.shape[-1]), targets, tau, engine, regions_bf16, logit_scale, memory)
+    return ops.infonce_loss(regions, queries.reshape(-1, queries.shape[-1]), targets, tau, engine, regions_bf16, logit_scale, memory,
+                            query_ids)
 
 
 def topk_regions(regions: torch.Tensor, queries: torch.Tensor, k: int, sharded: bool = False, engine: str = "auto"):
@@ -195,15 +231,16 @@ _StepCfg = namedtuple("_StepCfg", "B M Cc h w inv_tau nce_weight bg_mode w_fg w_
                                   "need_pred need_emb need_comb")
 # the tensors the step's backward reads, kept through save_for_backward
 _Saved = namedtuple("_Saved", "pred_c t_save w_save per fg bg inv_fg inv_bg comb_c stats out4 aux r16 q16 targets lse w32 scale")
-_Side = namedtuple("_Side", "q16 ev_q ev_px mem_args out8 t_save w_save per scratch")
+_Side = namedtuple("_Side", "q16 ev_q ev_px mem_args excl out8 t_save w_save per scratch")
 _Rows = namedtuple("_Rows", "fg inv_fg bg inv_bg out4 aux lse nce tgt loss")
 
 
-def _side_branch(cfg, dev, cur, side, px, pred_c, masks, comb_c, memory, sc) -> _Side:
+def _side_branch(cfg, dev, cur, side, px, pred_c, masks, comb_c, memory, sc, query_ids) -> _Side:
     """What needs neither the resampled weights nor the pooled rows, issued FIRST on the side stream (a parallel branch once
     captured in a CUDA graph), else on the current one: the peer-exit wait, the bf16 queries, the memory scan and the
     segmentation loss, whose instruction-bound tiles run underneath the HBM-bound mask resample.  ``scratch``: the work
-    buffers the side stream writes, to keep alive until the tail joins it."""
+    buffers the side stream writes, to keep alive until the tail joins it.  ``excl``: with ``query_ids``, the memory's
+    exclusion mask, built just before the scan and kept for the backward's memory dQ."""
     lib = L.load()
     f32 = dict(dtype=torch.float32, device=dev)
     gt = masks[:, 0]                       # [B,Hm,Wm] view; read in place through its sample stride
@@ -231,16 +268,20 @@ def _side_branch(cfg, dev, cur, side, px, pred_c, masks, comb_c, memory, sc) -> 
     q16 = torch.empty((N, D), dtype=torch.bfloat16, device=dev)
     # allocated on the consuming stream: its block is reused only after the tail that reads it
     mwork = ops._memory_scan_work(memory, N, D, dev) if memory is not None else None
+    # its last reader is the memory dQ of the backward, on the current stream
+    excl = ops._memory_exclude_work(memory, N, dev) if query_ids is not None else None
     with torch.cuda.stream(stream):
         ops._call("cor_cast_cat_bf16", dev, ptr(comb_c), D, None, 0, _ll(N), ptr(q16))
         ev_q = side.record_event() if side is not None else None
         if memory is not None:
-            mwork, mparts = ops._memory_scan(memory, q16, cfg.inv_tau, sc, mwork)
+            if excl is not None:
+                ops._memory_exclude(memory, query_ids, excl)
+            mwork, mparts = ops._memory_scan(memory, q16, cfg.inv_tau, sc, mwork, excl)
             mem_args = (ptr(mwork), mparts, ptr(memory.state))
         ops._call("cor_seg_loss_fwd", dev, ptr(pred_c), L.dtype_code(pred_c), ptr(gt), L.dtype_code(gt), _f(ops._mask_scale(gt, None)),
                   N, H, W, Hm, Wm, _ll(gt.stride(0)), None, _f(0.25), _f(-1.0), _f(1.0), ptr(out8), ptr(per), ptr(t_save),
                   ptr(w_save), ptr(seg_work))
-    return _Side(q16, ev_q, ev_px, mem_args, out8, t_save, w_save, per, (seg_work, mwork))
+    return _Side(q16, ev_q, ev_px, mem_args, excl, out8, t_save, w_save, per, (seg_work, mwork))
 
 
 def _pool(cfg, dev, emb_c, masks):
@@ -374,7 +415,7 @@ def _tail_backward(ctx, s, g, g_scale):
               ptr(s.inv_fg), ptr(s.stats), ptr(s.comb_c), ptr(s.out4), ptr(s.aux), _f(cfg.w_fg), _f(cfg.w_bg), ptr(a16), Kp, ptr(g_q),
               *gs_arg, ptr(work), ptr(ctx.tail))
     if ctx.mem is not None:
-        ops._memory_dq(ctx.mem[0], s.q16, s.lse, cfg.inv_tau, s.scale, g, cfg.nce_weight, g_q, g_scale)
+        ops._memory_dq(ctx.mem[0], s.q16, s.lse, cfg.inv_tau, s.scale, g, cfg.nce_weight, g_q, g_scale, ctx.mem[2])
     g_comb = g_q.view(cfg.comb_shape).to(cfg.comb_dt) if cfg.need_comb else None
     if not cfg.need_emb:
         return None, g_comb
@@ -416,7 +457,8 @@ def _chain_backward(ctx, s, g, g_scale, g_pred, gemm_ok, cur, side, ev_px):
     ops._call("cor_fgbg_loss_bwd", dev, ptr(s.fg), _ll(M * Cc), ptr(s.bg), _ll(Cc), ptr(s.comb_c), _ll(Cc), B, Cc, cfg.bg_mode, ptr(s.out4),
               ptr(s.aux), ptr(g), _ll(0), _f(cfg.w_fg), _f(cfg.w_bg), ptr(g_regions), _ll(M * Cc), 1, ptr(g_bg), _ll(Cc), ptr(g_q), _ll(Cc), 1)
     if ctx.mem is not None:              # this rank's memory, against this rank's queries
-        ops._memory_dq(ctx.mem[0], s.q16, s.lse, cfg.inv_tau, s.scale, g, cfg.nce_weight, g_q if cfg.need_comb else None, g_scale)
+        ops._memory_dq(ctx.mem[0], s.q16, s.lse, cfg.inv_tau, s.scale, g, cfg.nce_weight, g_q if cfg.need_comb else None, g_scale,
+                       ctx.mem[2])
     g_comb = g_q.view(cfg.comb_shape).to(cfg.comb_dt) if cfg.need_comb else None
     if not cfg.need_emb:
         return None, g_comb, g_pred
@@ -448,7 +490,7 @@ class _FusedStepFn(torch.autograd.Function):
     Used by :func:`region_step` when the tensor-core pooling engine applies; the modular ops remain the general path."""
 
     @staticmethod
-    def forward(ctx, pred, emb, comb, masks, tau, nce_weight, gather, sim_engine, bg_mode, w_fg, w_bg, logit_scale, memory):
+    def forward(ctx, pred, emb, comb, masks, tau, nce_weight, gather, sim_engine, bg_mode, w_fg, w_bg, logit_scale, memory, query_ids):
         dev = L.require_cuda(pred, emb, comb, masks, logit_scale)
         sc = logit_scale                       # device logit scale (replaces 1/tau in every InfoNCE launch) or None
         B, M = masks.shape[:2]
@@ -466,7 +508,7 @@ class _FusedStepFn(torch.autograd.Function):
         cur = torch.cuda.current_stream(dev)
         side = _side_stream(dev) if _overlap_enabled() else None
         px = peer.get_exchange(B * M, Cc, dev) if multi_rank else None
-        sd = _side_branch(cfg, dev, cur, side, px, pred_c, masks, comb_c, memory, sc)
+        sd = _side_branch(cfg, dev, cur, side, px, pred_c, masks, comb_c, memory, sc, query_ids)
         w16, w32, stats, part = _pool(cfg, dev, emb_c, masks)
         ctx.tail = _tail_counter(dev, B, M, Cc) if _step_tail_ok(B, M, Cc, multi_rank, cfg.bg_mode, sim_engine) else None
         if ctx.tail is not None:
@@ -478,7 +520,7 @@ class _FusedStepFn(torch.autograd.Function):
                                       inv_bg=o.inv_bg, comb_c=comb_c, stats=stats, out4=o.out4, aux=o.aux, r16=r16, q16=sd.q16,
                                       targets=targets, lse=o.lse, w32=w32, scale=sc))
         ctx.cfg, ctx.px = cfg, px
-        ctx.mem = None if memory is None else (memory, memory.enqueues)
+        ctx.mem = None if memory is None else (memory, memory.enqueues, sd.excl)
         ctx.w16 = (w16, getattr(w16, "_cor_epoch", -1))      # not a saved tensor: a cached operand buffer, validated by its epoch
         ctx.mark_non_differentiable(o.fg, sd.out8, o.out4, o.nce)
         ctx.set_materialize_grads(False)     # no zero-filled gradients for the auxiliary outputs
@@ -487,7 +529,7 @@ class _FusedStepFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g_loss, *_unused):
         if g_loss is None:
-            return (None,) * 13
+            return (None,) * 14
         ops.check_memory_unchanged(ctx.mem, "region_step backward")
         cfg, s, px = ctx.cfg, _Saved(*ctx.saved_tensors), ctx.px
         dev = s.fg.device
@@ -519,7 +561,7 @@ class _FusedStepFn(torch.autograd.Function):
             cur.wait_stream(side)
         if g_pred is not None:
             g_pred = g_pred.to(cfg.pred_dt)
-        return g_pred, g_emb, g_comb, None, None, None, None, None, None, None, None, g_scale, None
+        return g_pred, g_emb, g_comb, None, None, None, None, None, None, None, None, g_scale, None, None
 
 
 def _fused_ok(emb, masks, pool_engine):
@@ -531,7 +573,7 @@ def _fused_ok(emb, masks, pool_engine):
 def region_step(pred: torch.Tensor, emb: torch.Tensor, comb: torch.Tensor, masks: torch.Tensor, *, tau: Optional[float] = None,
                 nce_weight: float = 1.0, gather: bool = True, pool_engine: str = "auto", sim_engine: str = "auto",
                 bg_mode: int = 0, fused: bool = True, logit_scale: Optional[torch.Tensor] = None,
-                memory: Optional[RegionMemory] = None) -> RegionStepOut:
+                memory: Optional[RegionMemory] = None, query_ids: Optional[torch.Tensor] = None) -> RegionStepOut:
     """One forward of the whole region path for a batch of triplets with M candidate masks each
     (mask 0 of every image is the ground-truth ``query_mask``):
 
@@ -549,6 +591,10 @@ def region_step(pred: torch.Tensor, emb: torch.Tensor, comb: torch.Tensor, masks
     kernels; the memory is scanned on tensor cores beside the mask resample.  Push the batch with
     ``memory.enqueue(out.regions)`` after backward() (``StepBuffers.capture(memory=...)`` does it inside the graph).
 
+    ``query_ids`` (int64 [B] on the step's device, with ``memory``): an id per triplet, e.g. its target object's.  Memory
+    rows with the same id (pushed by ``memory.enqueue(out.regions, ids=query_ids)``) are left out of that triplet's
+    negatives and gradients, so an earlier pooled row of the object it looks for is not scored against it.
+
     ONE pass over the masks and ONE pass over the feature map serve fg, bg and all M regions.  With bf16
     features and >= 16 masks the step runs as a single fused autograd node (tensor-core pooling, hand
     written backward); other shapes compose the modular ops.
@@ -558,6 +604,7 @@ def region_step(pred: torch.Tensor, emb: torch.Tensor, comb: torch.Tensor, masks
         raise CorError(f"region_step: logit_scale is on {logit_scale.device}, the step on {emb.device}")
     ops.check_memory(memory, emb.shape[1], emb.device if emb.is_cuda else None, "region_step")
     B, M = masks.shape[:2]
+    ops.check_query_ids(query_ids, memory, B, emb.device if emb.is_cuda else None, "region_step")
     if comb.shape[0] != B or emb.shape[0] != B or pred.shape[0] != B:
         raise CorError("region_step: batch sizes differ")
     if comb.numel() != B * emb.shape[1]:
@@ -565,7 +612,7 @@ def region_step(pred: torch.Tensor, emb: torch.Tensor, comb: torch.Tensor, masks
                        "(the kernels read the queries with the feature map's row width)")
     if fused and _fused_ok(emb, masks, pool_engine) and pred.dim() == 4 and pred.shape[1] == 1:
         loss, out8, out4, nce, fg = _FusedStepFn.apply(pred, emb, comb, masks, 0.07 if tau is None else float(tau), float(nce_weight),
-                                                       bool(gather), sim_engine, int(bg_mode), 5.0, 5.0, logit_scale, memory)
+                                                       bool(gather), sim_engine, int(bg_mode), 5.0, 5.0, logit_scale, memory, query_ids)
         return RegionStepOut(loss=loss, seg=out8[0], fg=out4[0], bg=out4[1], nce=nce[0], regions=fg.view(B, M, -1))
     pool = ops.region_pool(emb, masks, transform=ops.W_CLAMP, normalize=True, pair=True, engine=pool_engine, want_bf16=True)
     Cc = pool.fg.shape[-1]
@@ -574,7 +621,7 @@ def region_step(pred: torch.Tensor, emb: torch.Tensor, comb: torch.Tensor, masks
     losses, _ = ops.fgbg_losses(pool.fg[:, 0, :], pool.bg[:, 0, :], q, pool.stats.view(B, M, 4)[:, 0, :], bg_mode)
     seg = ops.seg_loss(pred, masks[:, 0:1])
     nce = region_infonce_loss(pool.fg.reshape(B * M, Cc), q, gt_rows, tau, gather, sim_engine,
-                              regions_bf16=pool.fg_bf16, logit_scale=logit_scale, memory=memory)
+                              regions_bf16=pool.fg_bf16, logit_scale=logit_scale, memory=memory, query_ids=query_ids)
     loss = seg + 5 * losses[0] + 5 * losses[1] + nce_weight * nce
     return RegionStepOut(loss=loss, seg=seg, fg=losses[0], bg=losses[1], nce=nce, regions=pool.fg.detach())
 
@@ -595,10 +642,15 @@ class StepBuffers:
 
     ``capture(memory=m)`` / ``run(..., memory=m)`` (m a :class:`RegionMemory`): every step scores against the memory, then
     after the backward pushes its regions with ``m.enqueue``, inside the graph, so each replay advances the memory.
-    ``capture`` leaves the memory as it found it (its warm-up steps are undone)."""
+    ``capture`` leaves the memory as it found it (its warm-up steps are undone).
+
+    ``ids=True`` adds a static int64 buffer ``d["ids"]`` [B], one id per triplet (e.g. its target object's), that
+    ``load`` fills like the others.  With a memory every step then scores with ``query_ids=d["ids"]`` and pushes its
+    regions with ``ids=d["ids"]`` (on each image's ground-truth row), so a replay never scores a triplet against earlier
+    pooled rows of its own target."""
 
     def __init__(self, B, M, C=256, h=64, w=64, H=1024, W=1024, hp=256, wp=256, D=None, device="cuda",
-                 emb_dtype=torch.bfloat16, mask_dtype=torch.float32):
+                 emb_dtype=torch.bfloat16, mask_dtype=torch.float32, ids: bool = False):
         if D is not None and D != C:
             raise CorError(f"StepBuffers: the composed query width D={D} must equal the feature channels C={C}")
         D = C
@@ -606,6 +658,8 @@ class StepBuffers:
         mk = lambda shape, dt: torch.empty(shape, dtype=dt, device=self.device)
         self.d = {"pred": mk((B, 1, hp, wp), emb_dtype), "emb": mk((B, C, h, w), emb_dtype), "comb": mk((B, 1, D), torch.float32),
                   "masks": mk((B, M, H, W), mask_dtype)}
+        if ids:
+            self.d["ids"] = mk((B,), torch.int64)
         self.loss_host = torch.empty((), dtype=torch.float32).pin_memory()
         self._seed = torch.ones((), dtype=torch.float32, device=self.device)
         self.graph = None
@@ -631,11 +685,12 @@ class StepBuffers:
         memory = kw.pop("memory", None)
         if scale is not None:
             scale = scale.detach().requires_grad_(backward)      # a leaf over the caller's storage: read in place
-        out = region_step(pred, emb, comb, self.d["masks"], logit_scale=scale, memory=memory, **kw)
+        ids = self.d.get("ids") if memory is not None else None
+        out = region_step(pred, emb, comb, self.d["masks"], logit_scale=scale, memory=memory, query_ids=ids, **kw)
         if backward:
             out.loss.backward(gradient=self._seed)      # a resident 1.0: no per-step fill kernel from autograd
         if memory is not None:
-            memory.enqueue(out.regions)                  # after the backward, which needs the rows the forward scored
+            memory.enqueue(out.regions, ids=ids)         # after the backward, which needs the rows the forward scored
         grads = {"pred": pred.grad, "comb": comb.grad, "emb": emb.grad}
         if scale is not None:
             grads["logit_scale"] = scale.grad
@@ -644,7 +699,7 @@ class StepBuffers:
     def capture(self, backward: bool = True, emb_grad: bool = True, warmup: int = 3, **kw):
         """Warm up on a side stream, then capture fwd+bwd of the step into a CUDA graph."""
         memory = kw.get("memory")
-        saved = (memory.bank.clone(), memory.state.clone()) if memory is not None else None
+        saved = (memory.bank.clone(), memory.state.clone(), memory.ids.clone()) if memory is not None else None
         side = torch.cuda.Stream(device=self.device)
         side.wait_stream(torch.cuda.current_stream(self.device))
         with torch.cuda.stream(side):
@@ -655,6 +710,7 @@ class StepBuffers:
         if saved is not None:                            # undo the warm-up's enqueues
             memory.bank.copy_(saved[0])
             memory.state.copy_(saved[1])
+            memory.ids.copy_(saved[2])
             torch.cuda.synchronize(self.device)
         n0 = ops.LAUNCHES["count"]
         g = torch.cuda.CUDAGraph()

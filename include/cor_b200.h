@@ -320,6 +320,19 @@ int cor_infonce_bwd_umma_ls(const void* regions, const void* queries, int Nr, in
  *     gradient.  Either output may be NULL (g_logit_scale needs logit_scale).  The dQ role of the tcgen05 InfoNCE
  *     backward with the bank as the region operand, then fixed-order folds: 2 launches, 3 with g_logit_scale, 2 without
  *     g_queries.  work: cor_memory_dq_work_bytes() bytes.  Deterministic.
+ * Row ids (as XBM's labels), so that a query's own object is not among its memory negatives: ids_ring is int64 [K] on the
+ * device, one id per slot, -1 = no id (a negative id matches nothing).
+ *   cor_memory_enqueue_ids: cor_memory_enqueue that also writes ids_ring at the same slots: row i gets ids[i / group] when
+ *     i % group == 0, else -1; every row gets -1 when ids is NULL (no stale id survives a wrap).  group >= 1 divides n:
+ *     1 = one id per row, M = one id per image of n = B M rows, on its row 0.  One launch.
+ *   cor_memory_exclude: the exclusion mask exclude [Nq][ceil(K / 32)] uint32 (cor_memory_exclude_bytes(Nq, K) bytes) from
+ *     ids_ring, the fill count in state and query_ids [Nq] int64: bit j of word w is set iff slot r = 32 w + j is valid
+ *     (r < count), ids_ring[r] >= 0 and ids_ring[r] == query_ids[q].  One launch; build it once per forward, after the
+ *     enqueues the forward sees, and keep it for the backward.
+ *   cor_memory_scan_x, cor_memory_dq_x: cor_memory_scan and cor_memory_dq that leave every masked (query, slot) pair out:
+ *     it adds exactly nothing to the query's log-sum-exp partials, its gradient or the logit scale's (a query whose every
+ *     valid row is masked gets the partials (-inf, 0) of an empty memory).  With no bit set the results are bit-equal
+ *     to the entries without the suffix.  exclude must not be NULL.
  * ---------------------------------------------------------------------------------------- */
 int cor_memory_state_words(void);
 int cor_memory_reset(int* state, cor_stream_t stream);   /* empties the memory: one cudaMemsetAsync of the state */
@@ -342,6 +355,16 @@ size_t cor_memory_dq_work_bytes(int Nq, int K, int D);
 int cor_memory_dq(const void* bank, int K, const int* state, const void* queries, int Nq, int D, float inv_tau,
                   const float* logit_scale, const float* lse, const float* g_loss, float g_mul, float* g_queries,
                   float* g_logit_scale, void* work, cor_stream_t stream);
+int cor_memory_enqueue_ids(const void* rows, int rows_dtype, int n, int C, void* bank, int K, int* state, long long* ids_ring,
+                           const long long* ids, int group, cor_stream_t stream);
+size_t cor_memory_exclude_bytes(int Nq, int K);
+int cor_memory_exclude(const long long* ids_ring, int K, const int* state, const long long* query_ids, int Nq, unsigned* exclude,
+                       cor_stream_t stream);
+int cor_memory_scan_x(const void* bank, int K, const int* state, const void* queries, int Nq, int D, float inv_tau,
+                      const float* logit_scale, const unsigned* exclude, void* work, int* nparts, cor_stream_t stream);
+int cor_memory_dq_x(const void* bank, int K, const int* state, const void* queries, int Nq, int D, float inv_tau,
+                    const float* logit_scale, const unsigned* exclude, const float* lse, const float* g_loss, float g_mul,
+                    float* g_queries, float* g_logit_scale, void* work, cor_stream_t stream);
 
 /* Top-k retrieval: per query the k best regions under (score desc, index asc), where score is the
  * canonical value fl32(sum in fp64 of exact bf16 products).  S is the (tensor-core) prefilter
